@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path (BASELINE.json): decode tok/s and % of the HBM roofline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one decode step of the workload's batch through the whole model (all layers + lm_head + arg-max).
 Default workload: Mistral-7B-v0.1 bf16, batch 1, 2k context (the configuration the headline metric is quoted on).
@@ -96,19 +96,38 @@ def ncu_traffic_per_step():
         return None, None
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each array the last timed step handed its caller, as out_dir/<name>.npy -- token ids as float64 (exact),
+    real values as float32 (float64 stays float64).  The inputs are seeded, so two builds run with the same arguments can be
+    compared output for output."""
+    conv = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        conv[name] = a.astype(np.float32 if a.dtype.kind == "f" and a.dtype.itemsize <= 4 else np.float64)
+    total = sum(a.nbytes for a in conv.values())
+    if total > DUMP_MAX_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_MAX_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in conv.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def minilm_measure(local_rank, b, t, repeats, e2e_iters, warm=3):
-    """-> dict(device ms/batch, e2e s/batch) for b x t synthetic sentences on this rank's GPU."""
+    """-> dict(device ms/batch, e2e s/batch, embeddings of the timed batch) for b x t synthetic sentences on this rank's GPU."""
     from fastllm_b200 import models
     m = models.MiniLMModel(models.BertConfig(), None, local_rank, random_seed=0)
     ids = (np.arange(b * t, dtype=np.uint64).reshape(b, t) * 7919 % 30000 + 3).astype(np.uint32)
     for _ in range(warm):
         m.embed_ids(ids)
-    _, ms = m.embed_ids_timed(ids, repeats)
+    emb, ms = m.embed_ids_timed(ids, repeats)
     t0 = time.perf_counter()
     for _ in range(e2e_iters):
         m.embed_ids(ids)                                   # host ids in (H2D), f32 [b, 384] out (D2H)
     e2e_s = (time.perf_counter() - t0) / e2e_iters
-    return {"ms": ms / repeats, "e2e_s": e2e_s}
+    return {"ms": ms / repeats, "e2e_s": e2e_s, "embeddings": emb}
 
 
 def cpu_minilm_sample(b=16, t=128, iters=2):
@@ -148,6 +167,8 @@ def run_minilm(args, rank, world, local_rank):
         t1w = time.time()
         time.sleep(0.12)
     launches = models.launch_count() - l0
+    if args.dump_outputs and rank == 0:           # every rank embeds the same sentences
+        dump_outputs(args.dump_outputs, {"embeddings": r["embeddings"]})
     tt = torch.tensor([r["ms"], r["e2e_s"]], dtype=torch.float64, device="cuda")
     if dist is not None:
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
@@ -533,11 +554,19 @@ def run_ours(args, rank, world, local_rank):
         barrier()
         l0 = models.launch_count()
         t_wall0 = time.time()
-        _, ms = cache.decode_greedy_loop(first, ctx, K)
+        timed_ids, ms = cache.decode_greedy_loop(first, ctx, K)
         barrier()
         t_wall1 = time.time()
         time.sleep(0.12)                                      # let the sampler flush its last lines
     gpu_launches = models.launch_count() - l0
+    if args.dump_outputs:
+        last_ids = timed_ids[-1]                              # [local_batch]: the token ids the last timed step returned
+        if use_ep:                                            # sequences are dealt out to the ranks: collect them in order
+            parts = [None] * world
+            dist.all_gather_object(parts, last_ids)
+            last_ids = np.concatenate(parts)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"next_token_ids": last_ids})
     ms = max_over_ranks(ms)
     value = jobs * batch * K / (ms / 1e3)
 
@@ -787,7 +816,7 @@ def run_prefill(args, rank, world, local_rank):
         torch.cuda.synchronize()
 
     model, _ = cls.initialize_model(cf, None, "bf16", local_rank, random_seed=0, std=0.02)
-    K, W = min(args.steps, 16), min(args.warmup, 3)
+    K, W = args.steps, min(args.warmup, 3)
     ids = (np.arange(T, dtype=np.uint64) * 7919 % 150000 + 3).astype(np.uint32)[None]
     cache = models.DeviceCache(model.dev, 1, T + 264)
     with ClockSampler(local_rank) as clk:
@@ -805,6 +834,8 @@ def run_prefill(args, rank, world, local_rank):
         barrier()
         t_wall1 = time.time()
         launches = models.launch_count() - l0
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {"next_token_ids": nxt})
         _, dec_ms = cache.decode_greedy_loop(nxt, T, 256)
         time.sleep(0.12)
     tt = torch.tensor([dt, dec_ms], dtype=torch.float64, device="cuda")
@@ -851,6 +882,7 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-extras", action="store_true", help="default workload: skip the batch sweep / Mixtral / MiniLM / parity legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned to its caller as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
@@ -869,9 +901,8 @@ def main():
             return
         run_reference(args, rank)
         return
-    import __graft_entry__ as g
-    if rank == 0 or not os.path.exists(os.path.join(ROOT, "fastllm_b200", "libfastllm_b200.so")):
-        g.build()
+    from fastllm_b200 import _lib
+    _lib.load()         # built by __graft_entry__.build(): the benchmark compiles nothing, so it also runs from a read-only tree
     if args.workload == "minilm_256x128":
         run_minilm(args, rank, world, local_rank)
     elif args.workload == "qwen25_7b_prefill4k":
@@ -881,4 +912,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True      # the project's modules load lazily below: leave no __pycache__ in the tree
     main()

@@ -63,6 +63,23 @@ def test_reference_arm_times_whole_steps_with_every_core_under_a_launcher_that_p
     assert r1.returncode == 0 and r1.stdout.strip() == ""
 
 
+def test_dump_outputs_writes_exact_ids_and_refuses_more_than_64_mb(tmp_path):
+    """--dump-outputs: one DIR/<name>.npy per output, token ids as float64 (every uint32 exactly), real values as float32; an
+    output set above 64 MB is refused before anything is written."""
+    import numpy as np
+    import pytest
+    import bench
+    ids = np.array([5, 151935, 2**32 - 1], dtype=np.uint32)
+    emb = np.linspace(-1, 1, 12, dtype=np.float32).reshape(3, 4)
+    bench.dump_outputs(str(tmp_path / "out"), {"next_token_ids": ids, "embeddings": emb})
+    got_ids, got_emb = np.load(tmp_path / "out" / "next_token_ids.npy"), np.load(tmp_path / "out" / "embeddings.npy")
+    assert got_ids.dtype == np.float64 and np.array_equal(got_ids, ids)
+    assert got_emb.dtype == np.float32 and np.array_equal(got_emb, emb)
+    with pytest.raises(ValueError):
+        bench.dump_outputs(str(tmp_path / "big"), {"x": np.zeros((8 << 20) + 1, dtype=np.float64)})
+    assert not (tmp_path / "big").exists()
+
+
 def test_compare_sharded_counts_rows_only_while_routing_agrees():
     """bench.compare_sharded with router records: a sequence rerouted on a near-tie leaves the comparison from that step on; a
     disagreement off a tie, or a large error in a row that was routed identically, fails the check."""
