@@ -68,7 +68,7 @@ __device__ __forceinline__ void store_out2(const AttnArgs& a, size_t idx, float 
 // ---------------------------------------------------------------------------------------------------------------------
 // batched decode, stream-K: a fixed grid of resident CTAs splits the batch's whole K|V page stream evenly
 // ---------------------------------------------------------------------------------------------------------------------
-// attn_gqa_decode_kernel above hands each (split, kv head, sequence) to a CTA: the number of CTAs is a multiple of the pairs, not of
+// A kernel that hands each (split, kv head, sequence) to a CTA (round 1): the number of CTAs is a multiple of the pairs, not of
 // the machine (batch 64 x 8 kv heads x 3 splits = 1536 CTAs on 444 slots = 3.46 waves; Mixtral's batch 32 = 256 CTAs on 444
 // slots), every CTA re-pays set-up, q conversion and merge, and its cp.async ring drains at every CTA boundary.  Here the pages
 // of all (sequence, kv head) pairs form ONE list (pair-major) cut into gridDim.x equal ranges:
@@ -83,7 +83,10 @@ __device__ __forceinline__ void store_out2(const AttnArgs& a, size_t idx, float 
 constexpr int kSkConsumerWarps = 4;
 constexpr int kSkConsumers = kSkConsumerWarps * 32;
 constexpr int kSkThreads = kSkConsumers + 32;
-constexpr int kSkMaxStages = 4;
+// K|V stages of the ring; with up to 3 resident CTAs per SM (attn_sk_plan in fl_lib.cu).  Measured on Mistral-7B at 2k context:
+// batch 64 is the same with 3 stages x 2 CTAs (6.83 vs 6.84 ms/step), batch 8 is better with more, smaller ranges (4.07 vs
+// 4.17 ms/step); 4 stages x 1 CTA loses 14 %.
+constexpr int kSkStages = 2;
 
 // element offset of (row, col) inside a staged 64 x D K or V page.  D >= 64: [D / 64 halves][64 rows][128 bytes] with the TMA
 // engine's 128-byte swizzle (16-byte chunk index XOR row & 7); D < 64 (test-size heads): the plain [64][D] box, no swizzle.
@@ -98,7 +101,6 @@ struct SkArgs {
     float* sk_acc;        // [gridDim.x][2][n_rep][D] partial numerators of the pairs a CTA shares with its neighbours
     float* sk_ml;         // [gridDim.x][2][n_rep][2] their running max / denominator
     int b;                // sequences in the step
-    int nstages;          // K|V stages of the ring
     int layer_row0;       // row of this layer's page 0 / kv head 0 in the pool-wide tensor maps
 };
 
@@ -117,17 +119,16 @@ __global__ void __launch_bounds__(kSkThreads) attn_sk_decode_kernel(const __grid
     uint16_t* qlo = qhi + 16 * D;
     float* red_o = reinterpret_cast<float*>(sksm);
     uint16_t* ring = reinterpret_cast<uint16_t*>(sksm + ((front + 1023) & ~1023));
-    __shared__ __align__(8) uint64_t full[kSkMaxStages];
-    __shared__ __align__(8) uint64_t empty[kSkMaxStages];
+    __shared__ __align__(8) uint64_t full[kSkStages];
+    __shared__ __align__(8) uint64_t empty[kSkStages];
     __shared__ float red_m[NW][16], red_l[NW][16], mrg_w[NW][16], mrg_den[16], mrg_star[16];
     __shared__ int prefix[kMaxBatch + 1];        // pages of the sequences before s
     __shared__ int s_len[kMaxBatch], s_slot[kMaxBatch];
     __shared__ int s_last, s_i0, s_i1;
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, tq = lane & 3;
-    const int NST = k.nstages;
     if (tid == 0) {
-        for (int s = 0; s < NST; ++s) {
+        for (int s = 0; s < kSkStages; ++s) {
             mbar_init(&full[s], 1);
             mbar_init(&empty[s], NW);
         }
@@ -205,8 +206,8 @@ __global__ void __launch_bounds__(kSkThreads) attn_sk_decode_kernel(const __grid
                 }
                 r &= 0x7FFFFFFF;
                 if (lane == 0) {
-                    const int st = c % NST;
-                    mbar_wait(&empty[st], ((c / NST) & 1) ^ 1);
+                    const int st = c % kSkStages;
+                    mbar_wait(&empty[st], ((c / kSkStages) & 1) ^ 1);
                     mbar_expect_tx(&full[st], 2u * TILE * 2u);
                     uint16_t* kd = ring + (size_t)st * 2 * TILE;
                     if constexpr (D >= 64) {
@@ -253,8 +254,8 @@ __global__ void __launch_bounds__(kSkThreads) attn_sk_decode_kernel(const __grid
             open = true;
             from_start = (p == 0);
         }
-        const int st = c % NST;
-        mbar_wait(&full[st], (c / NST) & 1);
+        const int st = c % kSkStages;
+        mbar_wait(&full[st], (c / kSkStages) & 1);
         const uint16_t* kt = ring + (size_t)st * 2 * TILE;
         const uint16_t* vt = kt + TILE;
         const int key0 = p * kKvPage + warp * 16;

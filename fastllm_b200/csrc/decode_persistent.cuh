@@ -91,7 +91,6 @@ struct PkArgs {
     int xs_floats;        // shared-memory activation / scratch region capacity (floats)
     int kcap;             // largest K of any phase rounded up to whole chunks (x_hi at xs, x_lo at xs + (kcap + 8) bf16)
     const CUtensorMap* tmaps;   // [4 L + 1] weight-stream descriptors, indexed by the phase id g
-    int static_num;             // static share of a phase's blocks in 32nds (the rest is the pool)
     unsigned int* pool;         // [4 L + 1] ticket counters of the phases' dynamic block pools (zero between uses)
     int partial_rows;     // rows of the per-warp partial buffer
     // ---- tensor parallelism inside the kernel: all-reduce over NVLink peer memory (no NCCL call, no extra launch) ----
@@ -102,8 +101,6 @@ struct PkArgs {
     float* peer_logits[8];           // rank r's full-vocabulary logits [Vfull]
     unsigned int ar_epoch0;          // exchanges completed on this communicator before this launch
     int* comm_err;                   // set to 1 when a peer did not show up within the spin budget
-    int flags;            // dev knob (FL_PK_FLAGS) bit 0: prefetch this CTA's KV pages into L2 at the top of P1; bits 1-3: timing
-                          // experiments with garbage results (2: no arithmetic, 4: no attention, 8: no weight traffic)
     long long* dbg;       // optional: CTA 0 writes %globaltimer at the phase boundaries of layer L/2 (FL_PK_DEBUG=1)
 };
 
@@ -119,15 +116,15 @@ struct PkSplit {
     int pool0, npool;  // pool = blocks [pool0, pool0 + npool)
     int ncc;           // column chunks per block
 };
-constexpr int kPkStaticNum = 30;      // default static share of a phase's blocks, in 32nds (PkArgs.static_num)
+constexpr int kPkStaticNum = 30;      // static share of a phase's blocks, in 32nds (the rest is the pool)
 constexpr int kPkPoolCap = 8;      // pool blocks one CTA may take per phase (bounds the per-CTA partial-sum buffer)
 
-__device__ __forceinline__ PkSplit pk_split(int N, int K, int cta, int ncta, bool dynamic, int static_num) {
+__device__ __forceinline__ PkSplit pk_split(int N, int K, int cta, int ncta, bool dynamic) {
     PkSplit p;
     const int nblk = N / kPkBlockRows;
     p.ncc = (K + kPkChunkCols - 1) / kPkChunkCols;
     if (dynamic) {
-        const int S = (int)((long long)nblk * static_num / 32) / ncta;
+        const int S = (int)((long long)nblk * kPkStaticNum / 32) / ncta;
         p.s0 = cta * S; p.s1 = p.s0 + S;
         p.pool0 = ncta * S; p.npool = nblk - p.pool0;
     } else {
@@ -258,7 +255,7 @@ __global__ void __launch_bounds__(kPkThreads, 1) decode_persistent_kernel(const 
                 const uint16_t* W;
                 int N, K;
                 pk_phase(a, g, W, N, K);
-                const PkSplit sp = pk_split(N, K, cta, ncta, dynamic, a.static_num);
+                const PkSplit sp = pk_split(N, K, cta, ncta, dynamic);
                 const bool pdbg = a.dbg != nullptr && cta == 0 && g < 4 * a.L && (g >> 2) == a.L / 2;
                 int pn = 0;
                 auto fetch_block = [&](int blk) {
@@ -273,10 +270,6 @@ __global__ void __launch_bounds__(kPkThreads, 1) decode_persistent_kernel(const 
                             if (pn < 8) a.dbg[660 + (g & 3) * 10 + pn] = t;
                             a.dbg[660 + (g & 3) * 10 + 8] = t;
                             a.dbg[660 + (g & 3) * 10 + 9] = ++pn;
-                        }
-                        if (a.flags & 8) {      // timing experiment: no weight traffic at all (results are garbage)
-                            mbar_arrive(&full[st]);
-                            continue;
                         }
                         mbar_expect_tx(&full[st], kPkStageBytes);      // the whole box always arrives (out-of-range columns as zeros)
                         // weights are dead once staged: evict_first keeps the L2 for the KV cache and the activations
@@ -360,7 +353,6 @@ __global__ void __launch_bounds__(kPkThreads, 1) decode_persistent_kernel(const 
             // c % NS: faster with the weight traffic switched off, 0.8-3.6 % SLOWER in the real run on all three models: dropped.)
             constexpr int KPW = kPkChunkCols / 16 / kPkConsumerWarps;      // k-steps per warp per full chunk (8)
             const uint16_t* xcol = xrow + (col0 + bk + warp * 16);
-            if (!(a.flags & 2))      // (timing experiment: bit 1 skips the arithmetic)
 #pragma unroll
             for (int h = 0; h < KPW; h += 4) {
                 uint32_t af[4][4], bf[4][2];
@@ -537,6 +529,11 @@ __global__ void __launch_bounds__(kPkThreads, 1) decode_persistent_kernel(const 
     const int n_rep = a.nh / a.nkv;
     constexpr int LPT = D / 8, TPW = 32 / LPT;
     const int grp = lane / LPT, gl = lane % LPT;
+    // this CTA's first attention item, opaque to the optimiser: starting the item loop at `cta` itself lets the compiler keep values
+    // derived from it live across every weight phase, and the q|k|v phase then spills its MMA accumulators (ptxas at 168 registers;
+    // Mistral-7B and TinyLlama batch 1 measured 0.9 % and 1.7 % slower per step)
+    int item0 = cta;
+    asm volatile("" : "+r"(item0));
 
     for (int step = 0; step < a.nsteps; ++step) {
         const uint32_t tok_id = __ldcg(a.ids);
@@ -556,21 +553,6 @@ __global__ void __launch_bounds__(kPkThreads, 1) decode_persistent_kernel(const 
             dbg_i = 0;
             dbg_layer = l;
             stamp(l);
-            if (a.flags & 1) {   // pull the K/V pages of this CTA's attention item(s) of this layer towards L2 while P1 runs
-                const int npages = (len + kKvPage - 1) / kKvPage;
-                const int per = (npages + a.nsplit - 1) / a.nsplit;
-                for (int item = cta; item < a.nkv * a.nsplit; item += ncta) {
-                    const int kvh = item / a.nsplit, split = item % a.nsplit;
-                    const int p0 = split * per, p1 = min(p0 + per, npages);
-                    constexpr int kLines = kKvPage * D * 2 / 128;          // 128-byte lines per K (or V) page chunk
-                    for (int i = tid; i < (p1 - p0) * 2 * kLines; i += kPkConsumers) {
-                        const int pg = p0 + i / (2 * kLines), rem = i % (2 * kLines);
-                        const size_t base = ((size_t)__ldg(a.page_table + pg) * a.nkv + kvh) * (size_t)(kKvPage * D);
-                        const uint16_t* src = (rem < kLines ? kpool : vpool) + base + (size_t)(rem % kLines) * 64;
-                        asm volatile("prefetch.global.L2 [%0];" ::"l"(src));
-                    }
-                }
-            }
             if (l == 0) {      // page-table entries of this CTA's attention items (constant during the launch): towards L1, off the
                                // load -> load dependency chain of every layer's attention phase
                 const int npages = (len + kKvPage - 1) / kKvPage;
@@ -624,7 +606,7 @@ __global__ void __launch_bounds__(kPkThreads, 1) decode_persistent_kernel(const 
                 const int per = (npages + a.nsplit - 1) / a.nsplit;
                 float* gacc = xs;                            // [NG][HG][D]
                 float* gml = xs + NG * HG * D;               // [NG][HG][2]
-                for (int item = (a.flags & 4) ? a.nkv * a.nsplit : cta; item < a.nkv * a.nsplit; item += ncta) {      // (bit 2: timing experiment without attention)
+                for (int item = item0; item < a.nkv * a.nsplit; item += ncta) {
                     const int kvh = item / a.nsplit, split = item % a.nsplit;
                     const int tok0 = split * per * kKvPage, tok1 = min(min((split + 1) * per, npages) * kKvPage, len);
                     const int gidx = warp * TPW + grp;

@@ -78,12 +78,6 @@ static __global__ void advance_state_kernel(StepState* st, int b, int t, int rop
 }
 
 // ---- tensor-parallel glue -------------------------------------------------------------------------------------------------
-// resid += delta (the all-reduced o_proj / down_proj output)
-static __global__ void add_rows_kernel(float* __restrict__ resid, const float* __restrict__ delta, int n) {
-    pdl_launch_dependents();
-    pdl_wait();
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) resid[i] += delta[i];
-}
 // out = sum over split-K slices (fixed order)
 static __global__ void sum_slices_kernel(const float* __restrict__ y, int nsl, long long stride, int n, float* __restrict__ out) {
     pdl_launch_dependents();

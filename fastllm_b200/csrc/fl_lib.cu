@@ -117,41 +117,32 @@ static void launch_attn(LaunchCtx& lc, int d, int nsplit, int nkv, int rows, siz
     }
 }
 
-// tensor-core attention of the dense path (attn_mma.cuh): batched decode (one CTA per split x kv head x sequence) or prefill
-// (one CTA per 64-query tile x q head x sequence)
+// mma.sync prefill attention of the dense path (attn_prefill_kernel, attn_mma.cuh): one CTA per 64-query tile x q head x sequence,
+// for the multi-token calls that the tcgen05 kernel (attn_prefill_tc_kernel) does not take
 static size_t attn_prefill_smem_bytes(int d) {
     return (size_t)(2 * kPrefillBM + 4 * kKvPage) * d * 2;
 }
 
 // stream-K batched decode (attn_sk_decode_kernel): q tiles / merge scratch in front, then the K|V ring
-static size_t attn_sk_smem_bytes(int d, int n_rep, int stages) {
+static size_t attn_sk_smem_bytes(int d, int n_rep) {
     const size_t front = std::max<size_t>((size_t)2 * 16 * d * 2, (size_t)kSkConsumerWarps * n_rep * d * 4);
-    return ((front + 1023) & ~(size_t)1023) + (size_t)stages * 2 * kKvPage * d * 2;
+    return ((front + 1023) & ~(size_t)1023) + (size_t)kSkStages * 2 * kKvPage * d * 2;
 }
-struct SkPlan { int stages = 0, ctas = 0; size_t smem = 0; };
-// ring depth and resident CTAs per SM: 2 stages x 3 CTAs (the runtime's occupancy answer caps the CTAs).  Measured on Mistral-7B
-// at 2k context: batch 64 is the same with 3 stages x 2 CTAs (6.83 vs 6.84 ms/step), batch 8 is better with more, smaller ranges
-// (4.07 vs 4.17 ms/step); 4 stages x 1 CTA loses 14 %.  FL_ATTN_SK_STAGES / FL_ATTN_SK_CTAS override (dev knobs).
+struct SkPlan { int ctas = 0; size_t smem = 0; };
+// resident CTAs per SM: 3, capped by the runtime's occupancy answer (the ring depth and why: kSkStages in attn_mma.cuh)
 template <int D>
 static SkPlan attn_sk_plan_d(int n_rep) {
-    static const int env_st = std::getenv("FL_ATTN_SK_STAGES") ? std::atoi(std::getenv("FL_ATTN_SK_STAGES")) : 0;
-    static const int env_ct = std::getenv("FL_ATTN_SK_CTAS") ? std::atoi(std::getenv("FL_ATTN_SK_CTAS")) : 0;
     static std::map<int, SkPlan> memo;
     static std::mutex mu;
     std::lock_guard<std::mutex> lk(mu);
     auto it = memo.find(n_rep);
     if (it != memo.end()) return it->second;
-    auto fit = [&](int st) {
-        int n = 0;
-        FL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, attn_sk_decode_kernel<D>, kSkThreads, attn_sk_smem_bytes(D, n_rep, st)));
-        return n;
-    };
     SkPlan p;
-    p.stages = env_st >= 1 && env_st <= kSkMaxStages ? env_st : 2;
-    p.ctas = std::min(3, fit(p.stages));
-    if (env_ct >= 1) p.ctas = std::min(p.ctas, env_ct);
+    p.smem = attn_sk_smem_bytes(D, n_rep);
+    int fit = 0;
+    FL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fit, attn_sk_decode_kernel<D>, kSkThreads, p.smem));
+    p.ctas = std::min(3, fit);
     FL_CHECK(p.ctas >= 1, FL_ERR_UNSUPPORTED, "stream-K attention does not fit an SM");
-    p.smem = attn_sk_smem_bytes(D, n_rep, p.stages);
     memo[n_rep] = p;
     return p;
 }
@@ -662,8 +653,7 @@ static void plan_persistent(fl_cache& c) {
     const size_t fixed = (size_t)p.xs_floats * 4 + (size_t)p.partial_rows * kPkConsumerWarps * 4 + (size_t)kAttnMaxRep * kKvPage * 4 + 64 * 4;
     const size_t avail = 232448 - 2048;   // 227 KB opt-in limit minus static shared memory and slack
     if (fixed + 2 * (size_t)kPkStageBytes > avail) return;
-    static const int max_stages = std::getenv("FL_PK_MAXSTAGES") ? std::max(2, std::atoi(std::getenv("FL_PK_MAXSTAGES"))) : kPkMaxStages;      // dev knob
-    p.nstages = (int)std::min<size_t>(std::min(max_stages, kPkMaxStages), (avail - fixed) / kPkStageBytes);
+    p.nstages = (int)std::min<size_t>(kPkMaxStages, (avail - fixed) / kPkStageBytes);
     p.smem = (size_t)p.nstages * kPkStageBytes + fixed;
     p.nsplit = std::max(1, std::min(c.pages_per_seq, kNumSMs / w.nkv));
     if (p.nsplit > c.nsplit) p.nsplit = c.nsplit;            // partial buffers are sized for c.nsplit
@@ -699,17 +689,6 @@ static void launch_persistent(fl_cache& c, int nsteps, bool feedback) {
     a.tmaps = w.pk_tmaps.p;
     if (c.pk_pool.p == nullptr) c.pk_pool.alloc(4 * (size_t)w.L + 1, true);
     a.pool = c.pk_pool.p;
-    {
-        const char* sn = std::getenv("FL_PK_STATIC");      // dev knob: static share of the blocks in 32nds
-        a.static_num = sn ? std::max(0, std::min(32, std::atoi(sn))) : kPkStaticNum;
-        // every pool block needs a taker: a CTA takes at most kPkPoolCap tickets per phase, so a share that leaves more than
-        // kNumSMs * kPkPoolCap blocks in some phase's pool (only reachable through the knob) falls back to the all-static split
-        for (int N : {w.nqkv, w.H, 2 * w.I, w.V}) {
-            const int nblk = N / kPkBlockRows;
-            const int S = (int)((long long)nblk * a.static_num / 32) / kNumSMs;
-            if (nblk - kNumSMs * S > kNumSMs * kPkPoolCap) a.static_num = 32;
-        }
-    }
     a.tp = w.tp; a.rank = w.rank;
     if (w.tp > 1) {
         for (int r = 0; r < w.tp; ++r) {
@@ -722,10 +701,6 @@ static void launch_persistent(fl_cache& c, int nsteps, bool feedback) {
         a.comm_err = (int*)((uint8_t*)g_peer.local + PeerComm::kErrOff);
         a.ar_epoch0 = g_peer.ar_epoch;
         g_peer.ar_epoch += (unsigned int)nsteps * (2u * (unsigned int)w.L + 1u);
-    }
-    {
-        const char* fl = std::getenv("FL_PK_FLAGS");
-        a.flags = fl ? std::atoi(fl) : 0;
     }
     static long long* dbg_buf = nullptr;
     const bool dbg = env_flag("FL_PK_DEBUG");
@@ -1113,7 +1088,7 @@ static int pick_ksplit(int tiles, int nk, int R) {
 // which the consumer kernel sums in a fixed order (deterministic, no atomics, no memset).
 //   R <= 128 (decode batches, short prefills): swap-AB -- the weights are the 128-row MMA operand, the activations a tiny
 //             N = R tile, the result is stored transposed; the only large shared-memory traffic is the weight stream.
-//   R  > 128 (prefill): tokens are the M dimension, 128 x 128 output tiles.
+//   R  > 128 (prefill): tokens are the M dimension, 128 x 256 output tiles.
 static int dense_gemm(fl_cache& c, LaunchCtx& lc, const char* tag, int R, int N, int K, const CUtensorMap& tmW, float* out,
                       const uint16_t* xhi = nullptr, const uint16_t* xlo = nullptr, uint16_t* silu_hi = nullptr, uint16_t* silu_lo = nullptr) {
     if (!xhi) { xhi = c.dw.xhi.p; xlo = c.dw.xlo.p; }
@@ -1122,8 +1097,7 @@ static int dense_gemm(fl_cache& c, LaunchCtx& lc, const char* tag, int R, int N,
     // prefill: 128 tokens x 256 weight rows per tile.  The hi/lo activation pair makes a k-block 2 x 16 KB of A next to the weight
     // tile, and the GEMM is bound by the shared-memory fill rate (L2 -> SM), not by the tensor pipe: a 256-row weight tile is
     // 64 KB per 2 x 128 x 256 x 64 MACs where the 128-row one is 48 KB per half of that -- 1.5x the arithmetic per staged byte.
-    static const int prefill_bn = env_flag("FL_PREFILL_BN128") ? 128 : 256;      // dev knob: the 128-row tile of round 1
-    const int tiles = swap ? (N + 127) / 128 : ((R + kGemmBM - 1) / kGemmBM) * ((N + prefill_bn - 1) / prefill_bn);
+    const int tiles = swap ? (N + 127) / 128 : ((R + kGemmBM - 1) / kGemmBM) * ((N + 255) / 256);
     const int ks = swap ? pick_ksplit(tiles, nk, R) : 1;
     ProfEntry pe;
     const bool prof = g_prof.on && !lc.capturing;
@@ -1139,10 +1113,6 @@ static int dense_gemm(fl_cache& c, LaunchCtx& lc, const char* tag, int R, int N,
         const int bn = R <= 16 ? 16 : (R <= 32 ? 32 : (R <= 64 ? 64 : 128));
         const CUtensorMap hi = make_tmap_bf16(xhi, R, K, K, bn), lo = make_tmap_bf16(xlo, R, K, K, bn);
         GemmArgs g{N, R, K, nullptr, nullptr, 0, out, N, ks, (long long)R * N};     // M = weight rows, N = activation rows
-        static const bool w_prefetch = env_flag("FL_GEMM_WPREFETCH");     // experimental (DESIGN.md section 9): not yet measured on a GPU
-        g.w_prefetch = (w_prefetch && pdl) ? 1 : 0;
-        static const int gemm_dbg = std::getenv("FL_GEMM_DBG") ? std::atoi(std::getenv("FL_GEMM_DBG")) : 0;
-        g.dbg = gemm_dbg;
         switch (bn) {
             case 16: launch_gemm_tc<16, GEPI_F32_T, DUAL_B>(lc.stream, pdl, tiles * ks, tmW, hi, lo, g); break;
             case 32: launch_gemm_tc<32, GEPI_F32_T, DUAL_B>(lc.stream, pdl, tiles * ks, tmW, hi, lo, g); break;
@@ -1153,12 +1123,10 @@ static int dense_gemm(fl_cache& c, LaunchCtx& lc, const char* tag, int R, int N,
         const CUtensorMap hi = make_tmap_bf16(xhi, R, K, K, kGemmBM), lo = make_tmap_bf16(xlo, R, K, K, kGemmBM);
         if (silu_hi != nullptr) {       // prefill gate|up: SiLU(gate) * up + hi/lo split fused into the epilogue
             GemmArgs g{R, N, K, nullptr, nullptr, 0, silu_hi, N / 2, 1, 0, silu_lo};
-            if (prefill_bn == 256) launch_gemm_tc<256, GEPI_SILU_HL, DUAL_A>(lc.stream, pdl, tiles, hi, lo, tmW, g);
-            else launch_gemm_tc<128, GEPI_SILU_HL, DUAL_A>(lc.stream, pdl, tiles, hi, lo, tmW, g);
+            launch_gemm_tc<256, GEPI_SILU_HL, DUAL_A>(lc.stream, pdl, tiles, hi, lo, tmW, g);
         } else {
             GemmArgs g{R, N, K, nullptr, nullptr, 0, out, N, 1, (long long)R * N};
-            if (prefill_bn == 256) launch_gemm_tc<256, GEPI_F32, DUAL_A>(lc.stream, pdl, tiles, hi, lo, tmW, g);
-            else launch_gemm_tc<128, GEPI_F32, DUAL_A>(lc.stream, pdl, tiles, hi, lo, tmW, g);
+            launch_gemm_tc<256, GEPI_F32, DUAL_A>(lc.stream, pdl, tiles, hi, lo, tmW, g);
         }
     }
     if (prof) {
@@ -1222,9 +1190,8 @@ static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool
 
     auto prep = [&](const char* tag, PrepArgs pa, int rows_out) {
         pa.xhi = d.xhi.p; pa.xlo = d.xlo.p; pa.eps = w.cfg.norm_eps; pa.t = t;
-        // many rows (prefill): the register-resident 256-thread kernel (dense_prep_rows_kernel); FL_PREP_ROWS=0 keeps the one-CTA-per-row kernel
-        static const bool rows_kernel = !std::getenv("FL_PREP_ROWS") || std::atoi(std::getenv("FL_PREP_ROWS")) != 0;
-        if (rows_kernel && rows_out >= 512 && pa.norm_w != nullptr && pa.embed == nullptr && pa.K <= 8192 && pa.K % 4 == 0) {
+        // many rows (prefill): the register-resident 256-thread kernel (dense_prep_rows_kernel)
+        if (rows_out >= 512 && pa.norm_w != nullptr && pa.embed == nullptr && pa.K <= 8192 && pa.K % 4 == 0) {
             if (pa.K <= 4096)
                 launch(lc, tag, 0, dense_prep_rows_kernel<4>, dim3(rows_out), dim3(kPrepRowsThreads), 0, pa);
             else
@@ -1246,8 +1213,7 @@ static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool
         int ks = dense_gemm(c, lc, "gemm_tc_qkv", R, w.nqkv, w.H, lw.tm_wqkv, d.y.p);
         QkvEpiArgs qa{ks, (long long)R * w.nqkv, d.y.p, lw.bqkv, d.q.p, kpool, vpool, c.page_table.p, c.pages_per_seq, c.state.p, w.rope_cos,
                       w.rope_sin, w.nh, w.nkv, w.d, w.max_pos, t, w.nqkv, tc_prefill ? d.vt.p : nullptr, vt_pages};
-        static const bool qkv_rows = !std::getenv("FL_QKV_ROWS") || std::atoi(std::getenv("FL_QKV_ROWS")) != 0;      // A/B knob
-        if (qkv_rows && t >= 64 && t % kQkvRowsPerThread == 0)      // prefill: eight rows per thread (dense_qkv_epi_rows_kernel)
+        if (t >= 64 && t % kQkvRowsPerThread == 0)      // prefill: eight rows per thread (dense_qkv_epi_rows_kernel)
             launch(lc, "dense_qkv_rope_append", 0, dense_qkv_epi_rows_kernel, dim3((w.nqkv / 2 + 255) / 256, R / kQkvRowsPerThread), dim3(256), 0, qa);
         else
             launch(lc, "dense_qkv_rope_append", 0, dense_qkv_epi_kernel, dim3((w.nqkv / 2 + 255) / 256, R), dim3(256), 0, qa);
@@ -1265,7 +1231,7 @@ static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool
                 FL_CHECK(c.kv_tmaps && w.nh / w.nkv <= 16, FL_ERR_UNSUPPORTED, "batched decode attention: GQA group > 16 heads or KV pool beyond 2^31 rows");
                 const SkPlan pl = attn_sk_plan(w.d, w.nh / w.nkv);
                 SkArgs sk{};
-                sk.a = at; sk.sk_acc = d.sk_acc.p; sk.sk_ml = d.sk_ml.p; sk.b = b; sk.nstages = pl.stages;
+                sk.a = at; sk.sk_acc = d.sk_acc.p; sk.sk_ml = d.sk_ml.p; sk.b = b;
                 sk.layer_row0 = (int)((size_t)l * (c.layer_pool_elems / w.d));
                 launch_attn_sk(lc, w.d, pl, kv_bytes, c.tm_kpool, c.tm_vpool, sk);
             } else {

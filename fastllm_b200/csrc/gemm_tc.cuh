@@ -18,7 +18,7 @@
 
 namespace fl {
 
-enum : int { GEPI_BIAS_BF16 = 0, GEPI_BIAS_GELU_BF16 = 1, GEPI_BIAS_RESID_F32 = 2, GEPI_F32 = 3, GEPI_ATOMIC_F32 = 4, GEPI_F32_T = 5, GEPI_SILU_HL = 6 };
+enum : int { GEPI_BIAS_BF16 = 0, GEPI_BIAS_GELU_BF16 = 1, GEPI_BIAS_RESID_F32 = 2, GEPI_F32 = 3, GEPI_F32_T = 5, GEPI_SILU_HL = 6 };
 enum : int { DUAL_NONE = 0, DUAL_A = 1, DUAL_B = 2 };
 
 constexpr int kGemmBM = 128;
@@ -33,10 +33,9 @@ struct GemmArgs {
     int ldr;
     void* out;                  // bf16 or f32 [M, ldo]
     int ldo;
-    int ksplit;                 // >1: K is cut into ksplit ranges handled by different work items (GEPI_F32 / GEPI_ATOMIC_F32)
+    int ksplit;                 // >1: K is cut into ksplit ranges handled by different work items (GEPI_F32)
     long long split_stride;     // GEPI_F32 with ksplit > 1: split s writes its partial sums to out + s * split_stride (deterministic)
     void* out2 = nullptr;       // GEPI_SILU_HL: the lo half ([M, ldo] bf16, like `out` = the hi half)
-    int w_prefetch = 0;         // DUAL_B: request the first ring-full of WEIGHT tiles before griddepcontrol.wait (see the producer)
     // GROUPED swap-AB GEMM (DUAL_B + GEPI_F32_T; the Mixtral experts): A stacks `M / grp_m` weight matrices of grp_m rows each,
     // B stacks one block of grp_cap (<= BN) activation rows per group -- the rows routed to that expert, gathered -- and group j
     // multiplies ITS rows with ITS matrix: out[slice][j * grp_cap + n][row within the group].  grp_cnt[j] (device memory, written
@@ -45,8 +44,6 @@ struct GemmArgs {
     int grp_m = 0;
     int grp_cap = 0;
     const int* grp_cnt = nullptr;
-    int dbg = 0;                // dev knob FL_GEMM_DBG (timing experiments only, results are garbage): bit 0 = DUAL_B without the
-                                // activation loads, bit 1 = no MMAs (the issuer releases a stage as soon as it has landed)
 };
 
 // ---- PTX wrappers ------------------------------------------------------------------------------------------------------
@@ -183,7 +180,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     constexpr uint32_t kBOff = (DUAL == DUAL_A ? 2 : 1) * kABytes;
     // DUAL_B: the hi and lo activation tiles sit back to back in a stage ([BN rows x 128 B] each, same swizzle), so ONE MMA of
     // N = 2 BN multiplies the weight tile with both -- half the tcgen05.mma instructions per staged byte (at N = 16 the issue rate
-    // of these tiny MMAs, not the weight stream, was the limit: FL_GEMM_DBG=2 measured it) -- into two accumulator column blocks
+    // of these tiny MMAs, not the weight stream, was the limit, measured in round 2) -- into two accumulator column blocks
     // [W.hi | W.lo] that the epilogue adds.
     constexpr int kMmaN = (DUAL == DUAL_B) ? 2 * BN : BN;
     static_assert(kMmaN <= 256, "UMMA N <= 256");
@@ -244,25 +241,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     if (warp == 0) {
         // ===== TMA producer =====
         if (lane == 0) {
-            // Swap-AB decode GEMMs are short (one work item per CTA, 5-40 us) and sit in a chain GEMM -> element-wise -> GEMM, so the
-            // ~2 us between the dependency wait and the first landed weight tile is a fixed tax on every one of them.  The WEIGHT
-            // operand does not depend on the previous kernel (it is constant after upload), so with w_prefetch the first ring-full of
-            // weight tiles is requested BEFORE griddepcontrol.wait: the CTA becomes resident as soon as the previous GEMM's CTA on
-            // this SM exits (every kernel of the chain calls launch_dependents at entry) and fills its ring while the element-wise
-            // kernel in between runs.  The stage barrier still expects the whole stage; the activation tiles that complete it are
-            // requested after the wait.  (The first pass over the ring needs no empty-slot wait: the slots have never been used.)
-            uint32_t pre = 0;
-            if (DUAL == DUAL_B && g.w_prefetch) {
-                for (int item = blockIdx.x; item < ntiles && pre < (uint32_t)kStages; item += gridDim.x) {
-                    const int tile = item / ksplit, ks = item % ksplit;
-                    const int m0 = (tile / nt) * kGemmBM;
-                    const int kb1 = min((ks + 1) * nkps, nk);
-                    for (int kb = ks * nkps; kb < kb1 && pre < (uint32_t)kStages; ++kb, ++pre) {
-                        mbar_expect_tx(&full[pre], kStageBytes);
-                        tma_load_2d(gsm + (size_t)pre * kStageBytes, &tmA, kb * kGemmBK, m0, &full[pre]);
-                    }
-                }
-            }
             pdl_wait();
             asm volatile("fence.proxy.async;" ::: "memory");      // the previous kernel's generic-proxy stores -> TMA reads
             uint32_t c = 0;
@@ -275,17 +253,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                 for (int kb = ks * nkps; kb < kb1; ++kb, ++c) {
                     const int st = c % kStages;
                     uint8_t* sa = gsm + (size_t)st * kStageBytes;
-                    if (DUAL == DUAL_B && c < pre) {       // weight tile already on its way; complete the stage with the activations
-                        tma_load_2d(sa + kBOff, &tmA2, kb * kGemmBK, n0, &full[st]);
-                        tma_load_2d(sa + kBOff + kBBytes, &tmB, kb * kGemmBK, n0, &full[st]);
-                        continue;
-                    }
                     mbar_wait(&empty[st], ((c / kStages) & 1) ^ 1);
-                    if (DUAL == DUAL_B && (g.dbg & 1)) {        // timing experiment: the weight stream alone
-                        mbar_expect_tx(&full[st], kABytes);
-                        tma_load_2d(sa, &tmA, kb * kGemmBK, m0, &full[st]);
-                        continue;
-                    }
                     mbar_expect_tx(&full[st], kStageBytes);
                     if (DUAL == DUAL_B) {       // tmA = weights, tmA2 / tmB = activation hi / lo
                         tma_load_2d(sa, &tmA, kb * kGemmBK, m0, &full[st]);
@@ -321,10 +289,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                     const int st = c % kStages;
                     mbar_wait(&full[st], (c / kStages) & 1);
                     tc_fence_after();
-                    if (g.dbg & 2) {            // timing experiment: no tensor-core work, the stage goes straight back
-                        mbar_arrive(&empty[st]);
-                        continue;
-                    }
                     const uint8_t* sa = gsm + (size_t)st * kStageBytes;
                     const uint64_t adesc = umma_smem_desc_sw128(sa), bdesc = umma_smem_desc_sw128(sa + kBOff);
 #pragma unroll
@@ -462,26 +426,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                 }
                 if (row < row_lim) {
                     const int col = n0 + c0;
-                    if (EPI == GEPI_BIAS_BF16 || EPI == GEPI_BIAS_GELU_BF16) {
-                        uint16_t* o = reinterpret_cast<uint16_t*>(g.out) + (size_t)row * g.ldo + col;
-#pragma unroll
-                        for (int j = 0; j < 32; j += 8) {
-                            if (col + j < g.N) {
-                                uint32_t pk[4];
-                                const float4 b0 = g.bias ? *reinterpret_cast<const float4*>(g.bias + col + j) : make_float4(0.f, 0.f, 0.f, 0.f);
-                                const float4 b1 = g.bias ? *reinterpret_cast<const float4*>(g.bias + col + j + 4) : make_float4(0.f, 0.f, 0.f, 0.f);
-                                const float bb[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
-#pragma unroll
-                                for (int e = 0; e < 8; e += 2) {
-                                    float v0 = __uint_as_float(r[j + e]) + bb[e];
-                                    float v1 = __uint_as_float(r[j + e + 1]) + bb[e + 1];
-                                    if (EPI == GEPI_BIAS_GELU_BF16) { v0 = gelu_tanh_f(v0); v1 = gelu_tanh_f(v1); }
-                                    pk[e >> 1] = pack_bf16x2(v0, v1);
-                                }
-                                *reinterpret_cast<uint4*>(o + j) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
-                            }
-                        }
-                    } else if (EPI == GEPI_SILU_HL) {
+                    if (EPI == GEPI_SILU_HL) {
                         // gate|up GEMM of the prefill: columns interleave gate_j (even) and up_j (odd); act_j = silu(gate_j) * up_j
                         // is written straight as the hi/lo bf16 operand of the down_proj GEMM ([M, N/2] each)
                         uint16_t* oh = reinterpret_cast<uint16_t*>(g.out) + (size_t)row * g.ldo + (col >> 1);
@@ -509,32 +454,13 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 #pragma unroll
                         for (int j = 0; j < 32; ++j)
                             if (col + j < col_lim) o[(size_t)(col + j) * g.ldo] = __uint_as_float(r[j]);
-                    } else if (EPI == GEPI_ATOMIC_F32) {
-                        // split-K partial sums meet in a pre-zeroed f32 buffer (vector red.global.add, sm_90+)
-                        float* o = reinterpret_cast<float*>(g.out) + (size_t)row * g.ldo + col;
-#pragma unroll
-                        for (int j = 0; j < 32; j += 4)
-                            if (col + j < g.N)
-                                atomicAdd(reinterpret_cast<float4*>(o + j), make_float4(__uint_as_float(r[j]), __uint_as_float(r[j + 1]),
-                                                                                        __uint_as_float(r[j + 2]), __uint_as_float(r[j + 3])));
-                    } else {
-                        float* o = reinterpret_cast<float*>(g.out) + (EPI == GEPI_F32 ? (size_t)ksi * (size_t)g.split_stride : 0) + (size_t)row * g.ldo + col;
-                        const uint16_t* rs = (EPI == GEPI_BIAS_RESID_F32 && g.resid) ? g.resid + (size_t)row * g.ldr + col : nullptr;
+                    } else {      // GEPI_F32
+                        float* o = reinterpret_cast<float*>(g.out) + (size_t)ksi * (size_t)g.split_stride + (size_t)row * g.ldo + col;
 #pragma unroll
                         for (int j = 0; j < 32; j += 4) {
                             if (col + j < g.N) {
                                 float4 v;
                                 v.x = __uint_as_float(r[j]); v.y = __uint_as_float(r[j + 1]); v.z = __uint_as_float(r[j + 2]); v.w = __uint_as_float(r[j + 3]);
-                                if (EPI == GEPI_BIAS_RESID_F32) {
-                                    if (g.bias) {
-                                        const float4 bv = *reinterpret_cast<const float4*>(g.bias + col + j);
-                                        v.x += bv.x; v.y += bv.y; v.z += bv.z; v.w += bv.w;
-                                    }
-                                    if (rs) {
-                                        const uint2 rr = *reinterpret_cast<const uint2*>(rs + j);
-                                        v.x += bf16lo(rr.x); v.y += bf16hi(rr.x); v.z += bf16lo(rr.y); v.w += bf16hi(rr.y);
-                                    }
-                                }
                                 *reinterpret_cast<float4*>(o + j) = v;
                             }
                         }

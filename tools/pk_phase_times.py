@@ -1,5 +1,5 @@
 import numpy as np, os, sys
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 os.environ.setdefault("FL_PK_DEBUG", "0")
 from fastllm_b200 import models, presets
 cls, cf = presets.PRESETS["mistral7b"]
