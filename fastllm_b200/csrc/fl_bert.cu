@@ -10,8 +10,6 @@
 
 namespace fl {
 
-static inline size_t align_up_b(size_t x, size_t a) { return (x + a - 1) / a * a; }
-
 // ---- TMA descriptors (driver entry point fetched through the runtime: no link-time libcuda dependency) -----------------
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
@@ -84,36 +82,13 @@ CUtensorMap make_tmap_kv(const void* ptr, uint64_t rows, uint32_t head_dim) {
 // Every kernel of the encoder is launched with programmatic stream serialization: each calls griddepcontrol.launch_dependents at
 // entry and griddepcontrol.wait before it touches anything the previous kernel wrote, so a kernel's prologue (barrier / TMEM
 // set-up, descriptor fetch, block scheduling) overlaps its predecessor's tail instead of following it.
-static bool g_bert_pdl = !env_flag("FL_NO_PDL");
-template <typename... KArgs, typename... Args>
-static void blaunch(cudaStream_t st, void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, Args&&... args) {
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    if (g_bert_pdl) {
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 1;
-    }
-    FL_CUDA(cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...));
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-}
-
 template <int EPI>
-static void launch_gemm(cudaStream_t st, const CUtensorMap& tmA, const CUtensorMap& tmB, const GemmArgs& g) {
+static void launch_gemm(LaunchCtx& lc, const char* tag, const CUtensorMap& tmA, const CUtensorMap& tmB, const GemmArgs& g) {
     constexpr int BN = kBertBN;
     const size_t smem = gemm_smem_bytes(BN, DUAL_NONE) + (gemm_epi_staged(EPI) ? kEpiStageBytes : 0);
-    static bool attr_set = false;
-    if (!attr_set) {
-        FL_CUDA(cudaFuncSetAttribute(gemm_tc_kernel<BN, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        attr_set = true;
-    }
     const int tiles = ((g.M + kGemmBM - 1) / kGemmBM) * ((g.N + BN - 1) / BN);
-    blaunch(st, gemm_tc_kernel<BN, EPI>, dim3(std::min(tiles, kNumSMs)), dim3(kGemmThreads), smem, tmA, tmA, tmB, g);
+    launch(lc, tag, (uint64_t)g.N * g.K * 2, gemm_tc_kernel<BN, EPI>, dim3(std::min(tiles, kNumSMs)), dim3(kGemmThreads), smem, tmA, tmA, tmB,
+           g);
 }
 
 // ---- weights -------------------------------------------------------------------------------------------------------------
@@ -126,7 +101,7 @@ void bert_build(BertModel& m) {
     FL_CHECK(m.H % 64 == 0 && m.I % 64 == 0 && m.H <= 512, FL_ERR_UNSUPPORTED, "BERT path needs hidden/intermediate % 64 == 0 and hidden <= 512");
     const size_t H = m.H, I = m.I;
     size_t off = 0;
-    auto take = [&](size_t bytes) { size_t o = off; off = align_up_b(off + bytes, 256); return o; };
+    auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
     const size_t o_w = take((size_t)m.V * H * 2), o_p = take((size_t)m.maxpos * H * 2), o_lw = take(H * 4), o_lb = take(H * 4);
     struct LO { size_t wqkv, wo, wi, wo2, bqkv, bo, bi, bo2, l1w, l1b, l2w, l2b; };
     std::vector<LO> lo(m.L);
@@ -205,13 +180,6 @@ static std::vector<std::string> bert_expected(const BertModel& m) {
     return v;
 }
 
-static uint16_t h_bf16(float f) {
-    uint32_t b;
-    std::memcpy(&b, &f, 4);
-    if ((b & 0x7FFFFFFFu) > 0x7F800000u) return (uint16_t)((b >> 16) | 0x40u);   // NaN stays NaN (quiet), as half::bf16::from_f32 does
-    return (uint16_t)((b + 0x7FFFu + ((b >> 16) & 1u)) >> 16);
-}
-
 void bert_put_tensor(BertModel& m, const char* name, int dtype, const int64_t* shape, int rank, const void* host) {
     FL_CHECK(!m.finalized, FL_ERR_STATE, "model already finalized");
     const std::string n(name);
@@ -226,7 +194,7 @@ void bert_put_tensor(BertModel& m, const char* name, int dtype, const int64_t* s
     const float* f = (const float*)host;
     if (r.mat) {
         std::vector<uint16_t> bits((size_t)r.rows * r.cols);
-        for (size_t i = 0; i < bits.size(); ++i) bits[i] = h_bf16(f[i]);
+        for (size_t i = 0; i < bits.size(); ++i) bits[i] = host_f32_to_bf16(f[i]);
         FL_CUDA(cudaMemcpy((uint16_t*)r.base + r.row0 * r.cols, bits.data(), bits.size() * 2, cudaMemcpyHostToDevice));
     } else {
         FL_CUDA(cudaMemcpy((float*)r.base + r.row0, f, (size_t)r.rows * 4, cudaMemcpyHostToDevice));
@@ -282,11 +250,11 @@ static void bert_reserve(BertModel& m, int b, int t) {
 // Enqueue the encoder on m.stream: B1 -> 6 x (B2..B7) -> B8 (SURVEY.md section 2.4)
 static void bert_enqueue(BertModel& m, int b, int t, bool has_mask) {
     const int T = b * t, H = m.H, I = m.I;
-    cudaStream_t st = m.stream;
+    LaunchCtx lc{m.stream};
     const int rows_per_cta = 8;
     const dim3 row_grid((T + rows_per_cta - 1) / rows_per_cta), row_block(rows_per_cta * 32);
-    blaunch(st, embed_ln_kernel, row_grid, row_block, 0, (const uint16_t*)m.wemb, (const uint16_t*)m.pemb, (const float*)m.lnw, (const float*)m.lnb,
-            (const uint32_t*)m.ids.p, T, t, H, m.V, m.maxpos, 1e-12f, m.x.p);
+    launch(lc, "bert_embed_ln", 0, embed_ln_kernel, row_grid, row_block, 0, (const uint16_t*)m.wemb, (const uint16_t*)m.pemb, (const float*)m.lnw,
+           (const float*)m.lnb, (const uint32_t*)m.ids.p, T, t, H, m.V, m.maxpos, 1e-12f, m.x.p);
     const CUtensorMap tm_x = make_tmap_bf16(m.x.p, T, H, H, kGemmBM), tm_x1 = make_tmap_bf16(m.x1.p, T, H, H, kGemmBM),
                       tm_ctx = make_tmap_bf16(m.ctx.p, T, H, H, kGemmBM), tm_h = make_tmap_bf16(m.hbuf.p, T, I, I, kGemmBM);
     const float eps = m.cfg.norm_eps;
@@ -294,24 +262,27 @@ static void bert_enqueue(BertModel& m, int b, int t, bool has_mask) {
     for (int l = 0; l < m.L; ++l) {
         const BertLayerW& w = m.layers[l];
         // B2: fused q|k|v projection + bias -> bf16 [T, 3H]
-        launch_gemm<GEPI_BIAS_BF16>(st, tm_x, w.tm_wqkv, GemmArgs{T, 3 * H, H, w.bqkv, nullptr, 0, m.qkv.p, 3 * H, 1, 0});
+        launch_gemm<GEPI_BIAS_BF16>(lc, "bert_gemm_qkv", tm_x, w.tm_wqkv, GemmArgs{T, 3 * H, H, w.bqkv, nullptr, 0, m.qkv.p, 3 * H, 1, 0});
         // B3+B4: per (sentence, head) softmax(QK^T / sqrt(d)) V, no mask
         if (t <= kBertS)
-            blaunch(st, bert_attn_kernel, dim3(m.nh, b), dim3(128), 0, (const uint16_t*)m.qkv.p, t, H, scale, m.ctx.p);
+            launch(lc, "bert_attn", 0, bert_attn_kernel, dim3(m.nh, b), dim3(128), 0, (const uint16_t*)m.qkv.p, t, H, scale, m.ctx.p);
         else
-            blaunch(st, bert_attn_long_kernel, dim3(m.nh, b, (t + kBertS - 1) / kBertS), dim3(128), 0, (const uint16_t*)m.qkv.p, t, H, scale, m.ctx.p);
+            launch(lc, "bert_attn", 0, bert_attn_long_kernel, dim3(m.nh, b, (t + kBertS - 1) / kBertS), dim3(128), 0, (const uint16_t*)m.qkv.p, t, H,
+                   scale, m.ctx.p);
         // B5: attention output dense + bias + residual -> f32, then LayerNorm -> bf16
-        launch_gemm<GEPI_BIAS_RESID_F32>(st, tm_ctx, w.tm_wo, GemmArgs{T, H, H, w.bo, m.x.p, H, m.pre.p, H, 1, 0});
-        blaunch(st, layernorm_kernel, row_grid, row_block, 0, (const float*)m.pre.p, (const float*)w.ln1w, (const float*)w.ln1b, T, H, eps, m.x1.p);
+        launch_gemm<GEPI_BIAS_RESID_F32>(lc, "bert_gemm_o", tm_ctx, w.tm_wo, GemmArgs{T, H, H, w.bo, m.x.p, H, m.pre.p, H, 1, 0});
+        launch(lc, "bert_layernorm", 0, layernorm_kernel, row_grid, row_block, 0, (const float*)m.pre.p, (const float*)w.ln1w, (const float*)w.ln1b,
+               T, H, eps, m.x1.p);
         // B6: intermediate dense + bias + GELU(tanh) -> bf16 [T, I]
-        launch_gemm<GEPI_BIAS_GELU_BF16>(st, tm_x1, w.tm_wi, GemmArgs{T, I, H, w.bi, nullptr, 0, m.hbuf.p, I, 1, 0});
+        launch_gemm<GEPI_BIAS_GELU_BF16>(lc, "bert_gemm_up_gelu", tm_x1, w.tm_wi, GemmArgs{T, I, H, w.bi, nullptr, 0, m.hbuf.p, I, 1, 0});
         // B7: output dense + bias + residual -> f32, LayerNorm -> bf16
-        launch_gemm<GEPI_BIAS_RESID_F32>(st, tm_h, w.tm_wo2, GemmArgs{T, H, I, w.bo2, m.x1.p, H, m.pre.p, H, 1, 0});
-        blaunch(st, layernorm_kernel, row_grid, row_block, 0, (const float*)m.pre.p, (const float*)w.ln2w, (const float*)w.ln2b, T, H, eps, m.x.p);
+        launch_gemm<GEPI_BIAS_RESID_F32>(lc, "bert_gemm_down", tm_h, w.tm_wo2, GemmArgs{T, H, I, w.bo2, m.x1.p, H, m.pre.p, H, 1, 0});
+        launch(lc, "bert_layernorm", 0, layernorm_kernel, row_grid, row_block, 0, (const float*)m.pre.p, (const float*)w.ln2w, (const float*)w.ln2b,
+               T, H, eps, m.x.p);
     }
     // B8: masked mean pooling + L2 normalise -> f32 [b, H]
-    blaunch(st, pool_l2_kernel, dim3(b), dim3((H + 31) / 32 * 32), 0, (const uint16_t*)m.x.p, has_mask ? (const uint32_t*)m.mask.p : (const uint32_t*)nullptr,
-            t, H, m.out.p);
+    launch(lc, "bert_pool_l2", 0, pool_l2_kernel, dim3(b), dim3((H + 31) / 32 * 32), 0, (const uint16_t*)m.x.p,
+           has_mask ? (const uint32_t*)m.mask.p : (const uint32_t*)nullptr, t, H, m.out.p);
 }
 
 void bert_embed(BertModel& m, const uint32_t* ids, const uint32_t* mask, int b, int t, float* out, float* device_ms) {

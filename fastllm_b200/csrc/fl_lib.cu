@@ -25,14 +25,6 @@ NcclApi g_nccl;
 PeerComm g_peer;
 static std::atomic<int> g_device{-1};
 
-static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
-
-static uint16_t host_f32_to_bf16(float f) {
-    uint32_t b;
-    std::memcpy(&b, &f, 4);
-    if ((b & 0x7FFFFFFFu) > 0x7F800000u) return (uint16_t)((b >> 16) | 0x40u);   // NaN stays NaN (quiet), as half::bf16::from_f32 does
-    return (uint16_t)((b + 0x7FFFu + ((b >> 16) & 1u)) >> 16);
-}
 static float host_f16_to_f32(uint16_t h) {
     const uint32_t sign = (uint32_t)(h >> 15) << 31;
     int exp = (h >> 10) & 0x1F;
@@ -55,6 +47,31 @@ static float host_f16_to_f32(uint16_t h) {
     float f;
     std::memcpy(&f, &bits, 4);
     return f;
+}
+
+// Calls f(std::integral_constant<int, D>{}) for head size d: the one place a runtime head_dim becomes the kernels' template
+// parameter D.  (Kernels built for 64 / 128 only are guarded with `if constexpr` at the call.)
+template <typename F>
+static decltype(auto) with_head_dim(int d, F&& f) {
+    switch (d) {
+        case 16: return f(std::integral_constant<int, 16>{});
+        case 32: return f(std::integral_constant<int, 32>{});
+        case 64: return f(std::integral_constant<int, 64>{});
+        case 128: return f(std::integral_constant<int, 128>{});
+    }
+    throw Error(FL_ERR_UNSUPPORTED, "head_dim must be 16, 32, 64 or 128");
+}
+
+// The same for the N tile (activation rows) of the swap-AB GEMMs.
+template <typename F>
+static decltype(auto) with_tile_n(int bn, F&& f) {
+    switch (bn) {
+        case 16: return f(std::integral_constant<int, 16>{});
+        case 32: return f(std::integral_constant<int, 32>{});
+        case 64: return f(std::integral_constant<int, 64>{});
+        case 128: return f(std::integral_constant<int, 128>{});
+    }
+    throw Error(FL_ERR_INVALID, "internal: GEMM N tile must be 16, 32, 64 or 128");
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -107,14 +124,9 @@ static size_t attn_smem_bytes(int d, int n_rep) {
 }
 
 static void launch_attn(LaunchCtx& lc, int d, int nsplit, int nkv, int rows, size_t smem, uint64_t bytes, const AttnArgs& a) {
-    dim3 g(nsplit, nkv, rows), b(kAttnThreads);
-    switch (d) {
-        case 16: launch(lc, "attn_decode", bytes, attn_decode_kernel<16>, g, b, smem, a); break;
-        case 32: launch(lc, "attn_decode", bytes, attn_decode_kernel<32>, g, b, smem, a); break;
-        case 64: launch(lc, "attn_decode", bytes, attn_decode_kernel<64>, g, b, smem, a); break;
-        case 128: launch(lc, "attn_decode", bytes, attn_decode_kernel<128>, g, b, smem, a); break;
-        default: throw Error(FL_ERR_UNSUPPORTED, "head_dim must be 16, 32, 64 or 128");
-    }
+    with_head_dim(d, [&](auto D) {
+        launch(lc, "attn_decode", bytes, attn_decode_kernel<D>, dim3(nsplit, nkv, rows), dim3(kAttnThreads), smem, a);
+    });
 }
 
 // mma.sync prefill attention of the dense path (attn_prefill_kernel, attn_mma.cuh): one CTA per 64-query tile x q head x sequence,
@@ -131,7 +143,7 @@ static size_t attn_sk_smem_bytes(int d, int n_rep) {
 struct SkPlan { int ctas = 0; size_t smem = 0; };
 // resident CTAs per SM: 3, capped by the runtime's occupancy answer (the ring depth and why: kSkStages in attn_mma.cuh)
 template <int D>
-static SkPlan attn_sk_plan_d(int n_rep) {
+static SkPlan attn_sk_plan(int n_rep) {
     static std::map<int, SkPlan> memo;
     static std::mutex mu;
     std::lock_guard<std::mutex> lk(mu);
@@ -139,6 +151,7 @@ static SkPlan attn_sk_plan_d(int n_rep) {
     if (it != memo.end()) return it->second;
     SkPlan p;
     p.smem = attn_sk_smem_bytes(D, n_rep);
+    ensure_smem_optin((const void*)attn_sk_decode_kernel<D>, p.smem);    // the occupancy answer is 0 above the opt-in limit
     int fit = 0;
     FL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fit, attn_sk_decode_kernel<D>, kSkThreads, p.smem));
     p.ctas = std::min(3, fit);
@@ -146,45 +159,6 @@ static SkPlan attn_sk_plan_d(int n_rep) {
     memo[n_rep] = p;
     return p;
 }
-static SkPlan attn_sk_plan(int d, int n_rep) {
-    switch (d) {
-        case 16: return attn_sk_plan_d<16>(n_rep);
-        case 32: return attn_sk_plan_d<32>(n_rep);
-        case 64: return attn_sk_plan_d<64>(n_rep);
-        case 128: return attn_sk_plan_d<128>(n_rep);
-        default: throw Error(FL_ERR_UNSUPPORTED, "head_dim must be 16, 32, 64 or 128");
-    }
-}
-static void launch_attn_sk(LaunchCtx& lc, int d, const SkPlan& pl, uint64_t bytes, const CUtensorMap& tmk, const CUtensorMap& tmv, const SkArgs& k) {
-    const dim3 g(pl.ctas * kNumSMs), b(kSkThreads);
-    switch (d) {
-        case 16: launch(lc, "attn_sk_decode", bytes, attn_sk_decode_kernel<16>, g, b, pl.smem, tmk, tmv, k); break;
-        case 32: launch(lc, "attn_sk_decode", bytes, attn_sk_decode_kernel<32>, g, b, pl.smem, tmk, tmv, k); break;
-        case 64: launch(lc, "attn_sk_decode", bytes, attn_sk_decode_kernel<64>, g, b, pl.smem, tmk, tmv, k); break;
-        default: launch(lc, "attn_sk_decode", bytes, attn_sk_decode_kernel<128>, g, b, pl.smem, tmk, tmv, k); break;
-    }
-}
-
-template <int D>
-static void attn_mma_set_attrs() {
-    FL_CUDA(cudaFuncSetAttribute(attn_sk_decode_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    if constexpr (D == 64 || D == 128)
-        FL_CUDA(cudaFuncSetAttribute(attn_prefill_tc_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)attn_prefill_tc_smem_bytes(D)));
-    FL_CUDA(cudaFuncSetAttribute(attn_prefill_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)attn_prefill_smem_bytes(D)));
-}
-
-static void launch_attn_prefill(LaunchCtx& lc, int d, dim3 g, uint64_t bytes, const AttnArgs& a) {
-    const size_t smem = attn_prefill_smem_bytes(d);
-    const dim3 b(kMmaAttnThreads);
-    switch (d) {
-        case 16: launch(lc, "attn_prefill", bytes, attn_prefill_kernel<16>, g, b, smem, a); break;
-        case 32: launch(lc, "attn_prefill", bytes, attn_prefill_kernel<32>, g, b, smem, a); break;
-        case 64: launch(lc, "attn_prefill", bytes, attn_prefill_kernel<64>, g, b, smem, a); break;
-        case 128: launch(lc, "attn_prefill", bytes, attn_prefill_kernel<128>, g, b, smem, a); break;
-        default: throw Error(FL_ERR_UNSUPPORTED, "head_dim must be 16, 32, 64 or 128");
-    }
-}
-
 // ------------------------------------------------------------------------------------------------------------------
 // Weights
 // ------------------------------------------------------------------------------------------------------------------
@@ -248,7 +222,7 @@ static void build_weights(Weights& w) {
     w.d = w.H / nh_f;
     w.max_pos = c.max_position_embeddings;
     w.nqkv = (w.nh + 2 * w.nkv) * w.d;
-    FL_CHECK(w.d == 16 || w.d == 32 || w.d == 64 || w.d == 128, FL_ERR_UNSUPPORTED, "head_dim must be 16, 32, 64 or 128");
+    with_head_dim(w.d, [](auto) {});
     FL_CHECK(c.arch != FL_ARCH_BERT, FL_ERR_INVALID, "internal: BERT goes through bert_build");
 
     const size_t A = 256;
@@ -429,7 +403,7 @@ static void put_tensor(Weights& w, const char* name, int dtype, const int64_t* s
     // Names the model does not read are skipped, as candle's VarBuilder ignores the extra entries of the HashMap the loader hands
     // over (huggingface.rs:81-130 loads EVERY tensor of the checkpoint: `self_attn.rotary_emb.inv_freq` in older Llama exports,
     // `visual.*` in Qwen2_5_VLForConditionalGeneration, ...).  finalize() stays the strict gate: a MISSING tensor is an error.
-    if (!route_tensor(w, name, r)) { w.ignored++; return; }
+    if (!route_tensor(w, name, r)) return;
     if (r.base == nullptr) return;       // an expert that lives on another expert-parallel rank
     int64_t numel = 1;
     for (int i = 0; i < rank; ++i) numel *= shape[i];
@@ -584,12 +558,12 @@ static void finalize(Weights& w) {
 static void tp_allreduce_sum(LaunchCtx& lc, float* buf, size_t count) {
     FL_CHECK(g_nccl.comm != nullptr, FL_ERR_STATE, "tensor parallelism: fl_comm_init has not been called");
     g_nccl.check(g_nccl.AllReduce(buf, buf, count, ncclFloat32, ncclSum, g_nccl.comm, lc.stream), "ncclAllReduce");
-    if (lc.capturing) lc.captured++; else g_launches.fetch_add(1, std::memory_order_relaxed);
+    count_launch(lc);
 }
 static void tp_allgather(LaunchCtx& lc, const float* send, float* recv, size_t count) {
     FL_CHECK(g_nccl.comm != nullptr, FL_ERR_STATE, "tensor parallelism: fl_comm_init has not been called");
     g_nccl.check(g_nccl.AllGather(send, recv, count, ncclFloat32, g_nccl.comm, lc.stream), "ncclAllGather");
-    if (lc.capturing) lc.captured++; else g_launches.fetch_add(1, std::memory_order_relaxed);
+    count_launch(lc);
 }
 // All-to-all over the communicator (grouped ncclSend / ncclRecv, ONE fused NCCL launch for all segments): for every segment,
 // rank r receives block `r` of every peer's send buffer into recv[src * bytes ...].  `replicate`: every peer gets the SAME
@@ -613,7 +587,7 @@ static void ep_alltoall(LaunchCtx& lc, const A2aSeg* segs, int nseg) {
         }
     }
     g_nccl.check(g_nccl.GroupEnd(), "ncclGroupEnd");
-    if (lc.capturing) lc.captured++; else g_launches.fetch_add(1, std::memory_order_relaxed);
+    count_launch(lc);
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -660,10 +634,6 @@ static void plan_persistent(fl_cache& c) {
     int coop = 0;
     FL_CUDA(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, w.device));
     if (!coop) return;
-    if (w.d == 64)
-        FL_CUDA(cudaFuncSetAttribute(decode_persistent_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
-    else
-        FL_CUDA(cudaFuncSetAttribute(decode_persistent_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
     c.gbar.alloc(1, true);
     p.ok = true;
 }
@@ -711,22 +681,13 @@ static void launch_persistent(fl_cache& c, int nsteps, bool feedback) {
     a.dbg = dbg ? dbg_buf : nullptr;
     FL_CUDA(cudaMemsetAsync(c.gbar.p, 0, sizeof(unsigned int), c.stream));
     FL_CUDA(cudaMemsetAsync(c.pk_pool.p, 0, (4 * (size_t)w.L + 1) * sizeof(unsigned int), c.stream));   // the kernel re-arms them itself; this covers an aborted launch
-    void* params[] = {&a};
-    const void* fn = (w.d == 64) ? (const void*)decode_persistent_kernel<64> : (const void*)decode_persistent_kernel<128>;
-    ProfEntry pe;
-    if (g_prof.on) {
-        pe.tag = "decode_persistent";
-        pe.bytes = (uint64_t)nsteps * (w.streamed_bytes + (uint64_t)c.kv_len * w.L * w.nkv * w.d * 2 * 2);
-        FL_CUDA(cudaEventCreate(&pe.e0));
-        FL_CUDA(cudaEventCreate(&pe.e1));
-        FL_CUDA(cudaEventRecord(pe.e0, c.stream));
-    }
-    FL_CUDA(cudaLaunchCooperativeKernel(fn, dim3(kNumSMs), dim3(kPkThreads), params, c.pk.smem, c.stream));
-    if (g_prof.on) {
-        FL_CUDA(cudaEventRecord(pe.e1, c.stream));
-        g_prof.entries.push_back(pe);
-    }
-    g_launches.fetch_add(1);
+    LaunchCtx lc{c.stream, /*pdl=*/false};
+    lc.cooperative = true;
+    const uint64_t bytes = (uint64_t)nsteps * (w.streamed_bytes + (uint64_t)c.kv_len * w.L * w.nkv * w.d * 2 * 2);
+    with_head_dim(w.d, [&](auto D) {     // plan_persistent admits head_dim 64 / 128 only
+        if constexpr (D == 64 || D == 128)
+            launch(lc, "decode_persistent", bytes, decode_persistent_kernel<D>, dim3(kNumSMs), dim3(kPkThreads), c.pk.smem, a);
+    });
     if (w.tp > 1)   // every rank received every logits slice in its exchange area: hand them to the usual logits buffer
         FL_CUDA(cudaMemcpyAsync(c.logits.p, (uint8_t*)g_peer.local + PeerComm::kLogitsOff, (size_t)w.Vfull * 4, cudaMemcpyDeviceToDevice, c.stream));
     if (dbg) {
@@ -821,19 +782,6 @@ static void cache_create(fl_cache& c, int max_batch, int max_seq) {
     c.h_slot_tab.alloc(2 * (size_t)max_batch);
     c.sample_out.alloc(1, true);
     plan_persistent(c);
-    const size_t smem = attn_smem_bytes(w.d, w.nh / w.nkv);
-    switch (w.d) {
-        case 16: FL_CUDA(cudaFuncSetAttribute(attn_decode_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); break;
-        case 32: FL_CUDA(cudaFuncSetAttribute(attn_decode_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); break;
-        case 64: FL_CUDA(cudaFuncSetAttribute(attn_decode_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); break;
-        default: FL_CUDA(cudaFuncSetAttribute(attn_decode_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); break;
-    }
-    switch (w.d) {
-        case 16: attn_mma_set_attrs<16>(); break;
-        case 32: attn_mma_set_attrs<32>(); break;
-        case 64: attn_mma_set_attrs<64>(); break;
-        default: attn_mma_set_attrs<128>(); break;
-    }
     FL_CUDA(cudaDeviceSynchronize());
 }
 
@@ -848,12 +796,16 @@ static void cache_destroy_graphs(fl_cache& c) {
 // passes already appended, so the order is causal-correct.
 static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool loop_mode);
 
+// A uniform call of `rows` activation rows runs on the dense (tcgen05) path: 3+ rows, or any Mixtral call.
+static bool uses_dense(const fl_cache& c, int rows) {
+    return (rows >= 3 || c.w->cfg.arch == FL_ARCH_MIXTRAL) && c.w->dense_ok;
+}
+
 static void enqueue_forward(fl_cache& c, LaunchCtx& lc, int b, int t, bool loop_mode) {
     const Weights& w = *c.w;
     const int rows = b * t;
-    const bool moe = w.cfg.arch == FL_ARCH_MIXTRAL;
-    FL_CHECK(!moe || c.dw.rows >= (size_t)rows, FL_ERR_STATE, "internal: Mixtral needs the dense workspace");
-    if ((rows >= 3 || moe) && w.dense_ok && c.dw.rows >= (size_t)rows) {   // workspace is reserved by the caller (never during capture)
+    FL_CHECK(w.cfg.arch != FL_ARCH_MIXTRAL || c.dw.rows >= (size_t)rows, FL_ERR_STATE, "internal: Mixtral needs the dense workspace");
+    if (uses_dense(c, rows) && c.dw.rows >= (size_t)rows) {   // workspace is reserved by the caller (never during capture)
         enqueue_forward_dense(c, lc, b, t, loop_mode);
         return;
     }
@@ -976,23 +928,21 @@ static void enqueue_forward(fl_cache& c, LaunchCtx& lc, int b, int t, bool loop_
 constexpr int kDenseMaxSplit = 16;    // upper bound on the split-K slices of a decode GEMM (see pick_ksplit)
 
 static int pick_ksplit(int tiles, int nk, int R);
-// rows per expert block of the grouped expert GEMMs = their N tile: the smallest of 16 / 32 / 64 / 128 that holds every row
-static int moe_group_cap(int Rm) { return Rm <= 16 ? 16 : (Rm <= 32 ? 32 : (Rm <= 64 ? 64 : 128)); }
+// N tile of a swap-AB GEMM over `rows` (<= 128) activation rows: the smallest of 16 / 32 / 64 / 128 that holds every row; for the
+// grouped expert GEMMs also the rows per expert block
+static int swap_tile_n(int rows) { return rows <= 16 ? 16 : (rows <= 32 ? 32 : (rows <= 64 ? 64 : 128)); }
 
 static void ensure_dense_ws(fl_cache& c, int rows) {
     DenseWs& d = c.dw;
     if ((size_t)rows <= d.rows) return;
     const Weights& w = *c.w;
     FL_CUDA(cudaStreamSynchronize(c.stream));
-    for (auto& kv : c.graphs)            // captured graphs hold the old workspace pointers
-        if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
-    c.graphs.clear();
+    cache_destroy_graphs(c);             // captured graphs hold the old workspace pointers
     const size_t R = rows, nq = (size_t)w.nh * w.d;
     const size_t kmax = std::max<size_t>(std::max<size_t>(w.H, nq), w.I);
     const size_t nmax = std::max<size_t>(std::max<size_t>(w.nqkv, 2 * (size_t)w.I), std::max<size_t>(w.H, w.V));
     d.xhi.alloc(R * kmax); d.xlo.alloc(R * kmax);
     const size_t Rm = w.ep_dp ? R * (size_t)w.ep : R;        // rows the expert GEMMs see
-    d.moe_rows = Rm;
     {   // GEMM output: [ks][rows, N] for the largest N * ks over the model's GEMM shapes at this row count
         size_t need = Rm * nmax;
         auto consider = [&](size_t rows, size_t N, size_t K) {
@@ -1002,7 +952,7 @@ static void ensure_dense_ws(fl_cache& c, int rows) {
         consider(R, w.nqkv, w.H); consider(R, w.H, nq); consider(R, w.V, w.H);
         consider(Rm, 2 * (size_t)w.I, w.H); consider(Rm, w.H, w.I);
         if (w.cfg.arch == FL_ARCH_MIXTRAL) {      // grouped expert GEMMs: E_local stacked matrices x one block of `cap` rows each
-            for (size_t cap = 16; cap <= (size_t)moe_group_cap((int)std::min<size_t>(Rm, 128)); cap *= 2) {
+            for (size_t cap = 16; cap <= (size_t)swap_tile_n((int)std::min<size_t>(Rm, 128)); cap *= 2) {
                 const size_t Rg = (size_t)w.E_local * cap;
                 for (size_t NK : {(size_t)0, (size_t)1}) {
                     const size_t N = NK == 0 ? 2 * (size_t)w.I : w.H, K = NK == 0 ? w.H : w.I;
@@ -1019,8 +969,8 @@ static void ensure_dense_ws(fl_cache& c, int rows) {
     if (w.cfg.arch != FL_ARCH_MIXTRAL && R > 128) { d.xhi2.alloc(R * (size_t)w.I); d.xlo2.alloc(R * (size_t)w.I); }
     if (w.cfg.arch == FL_ARCH_MIXTRAL) {
         // grouped path (calls with <= 128 expert rows): E_local blocks of up to grp_cap rows; masked path (prefill): Rm rows
-        d.grp_cap = moe_group_cap((int)std::min<size_t>(Rm, 128));
-        const size_t Rg = (size_t)w.E_local * d.grp_cap;
+        const size_t grp_cap = swap_tile_n((int)std::min<size_t>(Rm, 128));
+        const size_t Rg = (size_t)w.E_local * grp_cap;
         d.xhi2.alloc(std::max(Rm, Rg) * kmax); d.xlo2.alloc(std::max(Rm, Rg) * kmax);
         d.gx_hi.alloc(Rg * w.H, true); d.gx_lo.alloc(Rg * w.H, true);
         d.grp_cnt.alloc(w.E_local, true); d.grp_pos.alloc(Rm * w.E_local);
@@ -1031,8 +981,8 @@ static void ensure_dense_ws(fl_cache& c, int rows) {
             d.comb.alloc(Rm * w.H);
         }
     }
-    d.chunk = std::min(rows, kMaxBatch);            // split partials of the batched-decode attention: one row per sequence
-    d.counters.alloc((size_t)d.chunk * w.nkv, true);
+    const int chunk = std::min(rows, kMaxBatch);    // split partials of the batched-decode attention: one row per sequence
+    d.counters.alloc((size_t)chunk * w.nkv, true);
     d.sk_acc.alloc((size_t)4 * kNumSMs * 2 * (w.nh / w.nkv) * w.d);
     d.sk_ml.alloc((size_t)4 * kNumSMs * 2 * (w.nh / w.nkv) * 2);
     d.vt_pages_cap = 0;
@@ -1042,29 +992,6 @@ static void ensure_dense_ws(fl_cache& c, int rows) {
         d.tm_vt = make_tmap_bf16(d.vt.p, d.vt_pages_cap * w.nkv * w.d, kKvPage, kKvPage, (uint32_t)w.d);
     }
     d.rows = R;
-}
-
-template <int BN, int EPI, int DUAL>
-static void launch_gemm_tc(cudaStream_t st, bool pdl, int items, const CUtensorMap& a, const CUtensorMap& a2, const CUtensorMap& b, const GemmArgs& g) {
-    const size_t smem = gemm_smem_bytes(BN, DUAL);
-    static bool attr_set = false;
-    if (!attr_set) {
-        FL_CUDA(cudaFuncSetAttribute(gemm_tc_kernel<BN, EPI, DUAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        attr_set = true;
-    }
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3(std::min(items, kNumSMs));
-    cfg.blockDim = dim3(kGemmThreads);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    if (pdl) {
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 1;
-    }
-    FL_CUDA(cudaLaunchKernelEx(&cfg, gemm_tc_kernel<BN, EPI, DUAL>, a, a2, b, g));
 }
 
 // Split-K factor of a swap-AB (decode) GEMM: the one whose work items (output tiles x k slices) fill whole waves of the 148
@@ -1099,41 +1026,27 @@ static int dense_gemm(fl_cache& c, LaunchCtx& lc, const char* tag, int R, int N,
     // 64 KB per 2 x 128 x 256 x 64 MACs where the 128-row one is 48 KB per half of that -- 1.5x the arithmetic per staged byte.
     const int tiles = swap ? (N + 127) / 128 : ((R + kGemmBM - 1) / kGemmBM) * ((N + 255) / 256);
     const int ks = swap ? pick_ksplit(tiles, nk, R) : 1;
-    ProfEntry pe;
-    const bool prof = g_prof.on && !lc.capturing;
-    const bool pdl = lc.pdl && !prof;
-    if (prof) {
-        pe.tag = tag;
-        pe.bytes = (uint64_t)N * K * 2;
-        FL_CUDA(cudaEventCreate(&pe.e0));
-        FL_CUDA(cudaEventCreate(&pe.e1));
-        FL_CUDA(cudaEventRecord(pe.e0, lc.stream));
-    }
+    const uint64_t bytes = (uint64_t)N * K * 2;
+    const dim3 block(kGemmThreads);
     if (swap) {
-        const int bn = R <= 16 ? 16 : (R <= 32 ? 32 : (R <= 64 ? 64 : 128));
+        const int bn = swap_tile_n(R);
         const CUtensorMap hi = make_tmap_bf16(xhi, R, K, K, bn), lo = make_tmap_bf16(xlo, R, K, K, bn);
         GemmArgs g{N, R, K, nullptr, nullptr, 0, out, N, ks, (long long)R * N};     // M = weight rows, N = activation rows
-        switch (bn) {
-            case 16: launch_gemm_tc<16, GEPI_F32_T, DUAL_B>(lc.stream, pdl, tiles * ks, tmW, hi, lo, g); break;
-            case 32: launch_gemm_tc<32, GEPI_F32_T, DUAL_B>(lc.stream, pdl, tiles * ks, tmW, hi, lo, g); break;
-            case 64: launch_gemm_tc<64, GEPI_F32_T, DUAL_B>(lc.stream, pdl, tiles * ks, tmW, hi, lo, g); break;
-            default: launch_gemm_tc<128, GEPI_F32_T, DUAL_B>(lc.stream, pdl, tiles * ks, tmW, hi, lo, g); break;
-        }
+        with_tile_n(bn, [&](auto BN) {
+            launch(lc, tag, bytes, gemm_tc_kernel<BN, GEPI_F32_T, DUAL_B>, dim3(std::min(tiles * ks, kNumSMs)), block, gemm_smem_bytes(BN, DUAL_B),
+                   tmW, hi, lo, g);
+        });
     } else {
         const CUtensorMap hi = make_tmap_bf16(xhi, R, K, K, kGemmBM), lo = make_tmap_bf16(xlo, R, K, K, kGemmBM);
+        const dim3 grid(std::min(tiles, kNumSMs));
         if (silu_hi != nullptr) {       // prefill gate|up: SiLU(gate) * up + hi/lo split fused into the epilogue
             GemmArgs g{R, N, K, nullptr, nullptr, 0, silu_hi, N / 2, 1, 0, silu_lo};
-            launch_gemm_tc<256, GEPI_SILU_HL, DUAL_A>(lc.stream, pdl, tiles, hi, lo, tmW, g);
+            launch(lc, tag, bytes, gemm_tc_kernel<256, GEPI_SILU_HL, DUAL_A>, grid, block, gemm_smem_bytes(256, DUAL_A), hi, lo, tmW, g);
         } else {
             GemmArgs g{R, N, K, nullptr, nullptr, 0, out, N, 1, (long long)R * N};
-            launch_gemm_tc<256, GEPI_F32, DUAL_A>(lc.stream, pdl, tiles, hi, lo, tmW, g);
+            launch(lc, tag, bytes, gemm_tc_kernel<256, GEPI_F32, DUAL_A>, grid, block, gemm_smem_bytes(256, DUAL_A), hi, lo, tmW, g);
         }
     }
-    if (prof) {
-        FL_CUDA(cudaEventRecord(pe.e1, lc.stream));
-        g_prof.entries.push_back(pe);
-    }
-    if (lc.capturing) lc.captured++; else g_launches.fetch_add(1, std::memory_order_relaxed);
     return ks;
 }
 
@@ -1145,30 +1058,13 @@ static int dense_gemm_grouped(fl_cache& c, LaunchCtx& lc, const char* tag, int g
     const int nk = (K + kGemmBK - 1) / kGemmBK;
     const int tiles = groups * ((Ne + kGemmBM - 1) / kGemmBM);
     const int ks = pick_ksplit(tiles, nk, cap);
-    const bool prof = g_prof.on && !lc.capturing;
-    const bool pdl = lc.pdl && !prof;
-    ProfEntry pe;
-    if (prof) {
-        pe.tag = tag;
-        pe.bytes = (uint64_t)groups * Ne * K * 2;
-        FL_CUDA(cudaEventCreate(&pe.e0));
-        FL_CUDA(cudaEventCreate(&pe.e1));
-        FL_CUDA(cudaEventRecord(pe.e0, lc.stream));
-    }
     const CUtensorMap hi = make_tmap_bf16(xhi, (uint64_t)groups * cap, K, K, cap), lo = make_tmap_bf16(xlo, (uint64_t)groups * cap, K, K, cap);
     GemmArgs g{groups * Ne, cap, K, nullptr, nullptr, 0, out, Ne, ks, (long long)groups * cap * Ne};
     g.grp_m = Ne; g.grp_cap = cap; g.grp_cnt = cnt;
-    switch (cap) {
-        case 16: launch_gemm_tc<16, GEPI_F32_T, DUAL_B>(lc.stream, pdl, tiles * ks, tmWall, hi, lo, g); break;
-        case 32: launch_gemm_tc<32, GEPI_F32_T, DUAL_B>(lc.stream, pdl, tiles * ks, tmWall, hi, lo, g); break;
-        case 64: launch_gemm_tc<64, GEPI_F32_T, DUAL_B>(lc.stream, pdl, tiles * ks, tmWall, hi, lo, g); break;
-        default: launch_gemm_tc<128, GEPI_F32_T, DUAL_B>(lc.stream, pdl, tiles * ks, tmWall, hi, lo, g); break;
-    }
-    if (prof) {
-        FL_CUDA(cudaEventRecord(pe.e1, lc.stream));
-        g_prof.entries.push_back(pe);
-    }
-    if (lc.capturing) lc.captured++; else g_launches.fetch_add(1, std::memory_order_relaxed);
+    with_tile_n(cap, [&](auto BN) {
+        launch(lc, tag, (uint64_t)groups * Ne * K * 2, gemm_tc_kernel<BN, GEPI_F32_T, DUAL_B>, dim3(std::min(tiles * ks, kNumSMs)), dim3(kGemmThreads),
+               gemm_smem_bytes(BN, DUAL_B), tmWall, hi, lo, g);
+    });
     return ks;
 }
 
@@ -1177,10 +1073,8 @@ static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool
     DenseWs& d = c.dw;
     const int R = b * t;
     const int nq = w.nh * w.d;
-    const bool saved_pdl = lc.pdl;
     const float qscale = (float)(1.0 / std::sqrt((double)w.d));
     const bool windowed = (w.cfg.arch != FL_ARCH_LLAMA) && w.cfg.sliding_window > 0 && t > 1;
-    const size_t attn_smem = attn_smem_bytes(w.d, w.nh / w.nkv);
     // multi-token calls on empty sequences with head_dim 64 / 128 and more than one page of keys: attention on tcgen05
     // (attn_prefill_tc_kernel; FL_ATTN_PREFILL_MMA=1 keeps the mma.sync kernel, the A/B knob)
     const int vt_pages = (t + kKvPage - 1) / kKvPage;
@@ -1224,28 +1118,31 @@ static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool
             at.out_hi = d.xhi.p; at.out_lo = d.xlo.p; at.nh = w.nh; at.nkv = w.nkv; at.t = t; at.row_base = 0;
             at.sliding_window = windowed ? w.cfg.sliding_window : 0; at.qscale = qscale;
             const uint64_t kv_bytes = (uint64_t)b * (c.kv_len + t) * w.nkv * w.d * 4;
-            if (t == 1) {
-                // stream-K: a fixed grid of resident CTAs, each an equal share of the step's page stream.  The grid does NOT depend
-                // on the KV length: this launch is captured into the step's CUDA graph, which is keyed by (batch, mode) only and
-                // replayed as the context grows.
-                FL_CHECK(c.kv_tmaps && w.nh / w.nkv <= 16, FL_ERR_UNSUPPORTED, "batched decode attention: GQA group > 16 heads or KV pool beyond 2^31 rows");
-                const SkPlan pl = attn_sk_plan(w.d, w.nh / w.nkv);
-                SkArgs sk{};
-                sk.a = at; sk.sk_acc = d.sk_acc.p; sk.sk_ml = d.sk_ml.p; sk.b = b;
-                sk.layer_row0 = (int)((size_t)l * (c.layer_pool_elems / w.d));
-                launch_attn_sk(lc, w.d, pl, kv_bytes, c.tm_kpool, c.tm_vpool, sk);
-            } else {
-                if (tc_prefill) {
-                    TcPrefillArgs tp{};
-                    tp.a = at; tp.layer_row0 = (int)((size_t)l * (c.layer_pool_elems / w.d)); tp.vt_pages = vt_pages;
-                    tp.tau = std::getenv("FL_ATTN_TC_TAU") ? (float)std::atof(std::getenv("FL_ATTN_TC_TAU")) : 8.f;      // 0: O is rescaled on every new row max (tests)
-                    const dim3 g((t + kTcQ - 1) / kTcQ, w.nh, b), blk(kTcThreads);
-                    if (w.d == 64) launch(lc, "attn_prefill_tc", kv_bytes, attn_prefill_tc_kernel<64>, g, blk, attn_prefill_tc_smem_bytes(64), c.tm_kpool, d.tm_vt, tp);
-                    else launch(lc, "attn_prefill_tc", kv_bytes, attn_prefill_tc_kernel<128>, g, blk, attn_prefill_tc_smem_bytes(128), c.tm_kpool, d.tm_vt, tp);
+            const int layer_row0 = (int)((size_t)l * (c.layer_pool_elems / w.d));
+            with_head_dim(w.d, [&](auto D) {
+                if (t == 1) {
+                    // stream-K: a fixed grid of resident CTAs, each an equal share of the step's page stream.  The grid does NOT
+                    // depend on the KV length: this launch is captured into the step's CUDA graph, which is keyed by (batch, mode)
+                    // only and replayed as the context grows.
+                    FL_CHECK(c.kv_tmaps && w.nh / w.nkv <= 16, FL_ERR_UNSUPPORTED, "batched decode attention: GQA group > 16 heads or KV pool beyond 2^31 rows");
+                    const SkPlan pl = attn_sk_plan<D>(w.nh / w.nkv);
+                    SkArgs sk{};
+                    sk.a = at; sk.sk_acc = d.sk_acc.p; sk.sk_ml = d.sk_ml.p; sk.b = b; sk.layer_row0 = layer_row0;
+                    launch(lc, "attn_sk_decode", kv_bytes, attn_sk_decode_kernel<D>, dim3(pl.ctas * kNumSMs), dim3(kSkThreads), pl.smem, c.tm_kpool,
+                           c.tm_vpool, sk);
+                } else if (tc_prefill) {
+                    if constexpr (D == 64 || D == 128) {
+                        TcPrefillArgs tp{};
+                        tp.a = at; tp.layer_row0 = layer_row0; tp.vt_pages = vt_pages;
+                        tp.tau = std::getenv("FL_ATTN_TC_TAU") ? (float)std::atof(std::getenv("FL_ATTN_TC_TAU")) : 8.f;      // 0: O is rescaled on every new row max (tests)
+                        launch(lc, "attn_prefill_tc", kv_bytes, attn_prefill_tc_kernel<D>, dim3((t + kTcQ - 1) / kTcQ, w.nh, b), dim3(kTcThreads),
+                               attn_prefill_tc_smem_bytes(D), c.tm_kpool, d.tm_vt, tp);
+                    }
                 } else {
-                    launch_attn_prefill(lc, w.d, dim3((t + kPrefillBM - 1) / kPrefillBM, w.nh, b), kv_bytes, at);
+                    launch(lc, "attn_prefill", kv_bytes, attn_prefill_kernel<D>, dim3((t + kPrefillBM - 1) / kPrefillBM, w.nh, b), dim3(kMmaAttnThreads),
+                           attn_prefill_smem_bytes(D), at);
                 }
-            }
+            });
         }
         ks = dense_gemm(c, lc, "gemm_tc_o", R, w.H, nq, lw.tm_wo, d.y.p);
         const float* delta = d.y.p;
@@ -1287,7 +1184,7 @@ static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool
             }
             if (Rm <= 128 && !env_flag("FL_MOE_MASKED")) {
                 // decode batches: per-expert row lists + ONE grouped GEMM pair over (expert, weight tile, k slice) work items
-                const int cap = moe_group_cap(Rm), Rg = w.E_local * cap, e0 = w.rank * w.E_local;
+                const int cap = swap_tile_n(Rm), Rg = w.E_local * cap, e0 = w.rank * w.E_local;
                 MoeGatherArgs ga{ex_hi, ex_lo, ex_route, Rm, w.H, w.E, e0, w.E_local, cap, d.gx_hi.p, d.gx_lo.p, d.grp_cnt.p, d.grp_pos.p};
                 launch(lc, "moe_gather", 0, moe_gather_kernel, dim3(w.E_local, std::max(1, std::min(Rm, 2 * kNumSMs / w.E_local))), dim3(256), 0, ga);
                 int ke = dense_gemm_grouped(c, lc, "gemm_tc_moe_w13", w.E_local, cap, 2 * w.I, w.H, lw.tm_ewgu_all, d.y.p, d.gx_hi.p, d.gx_lo.p,
@@ -1357,25 +1254,25 @@ static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool
     launch(lc, "advance_state", 0, advance_state_kernel, dim3(1), dim3(kMaxBatch), 0, c.state.p, b, t, loop_mode ? 1 : 0, c.ids.p,
            (const uint32_t*)c.next_ids.p, loop_mode ? 1 : 0, loop_mode ? c.trace.p : (uint32_t*)nullptr,
            loop_mode ? c.trace_pos.p : (int*)nullptr);
-    lc.pdl = saved_pdl;
 }
 
 // mode 0: one decode step of a uniform batch; 1: the same inside the device-resident greedy loop; 2: one decode step of a ragged
 // batch (fl_forward_slots: always the dense path, whatever the row count)
+static void enqueue_step(fl_cache& c, LaunchCtx& lc, int b, int t, int mode) {
+    if (mode == 2) enqueue_forward_dense(c, lc, b, t, false);
+    else enqueue_forward(c, lc, b, t, mode == 1);
+}
+
 static GraphEntry& get_graph(fl_cache& c, int b, int mode) {
-    const bool loop_mode = mode == 1;
     const GraphKey key{b, mode};
     auto it = c.graphs.find(key);
     if (it != c.graphs.end()) return it->second;
-    LaunchCtx lc;
-    lc.stream = c.stream;
-    lc.pdl = !env_flag("FL_NO_PDL");
+    LaunchCtx lc{c.stream};
     lc.capturing = true;
     cudaGraph_t graph = nullptr;
     FL_CUDA(cudaStreamBeginCapture(c.stream, cudaStreamCaptureModeThreadLocal));
     try {
-        if (mode == 2) enqueue_forward_dense(c, lc, b, 1, false);
-        else enqueue_forward(c, lc, b, 1, loop_mode);
+        enqueue_step(c, lc, b, 1, mode);
     } catch (...) {
         cudaStreamEndCapture(c.stream, &graph);
         if (graph) cudaGraphDestroy(graph);
@@ -1387,6 +1284,34 @@ static GraphEntry& get_graph(fl_cache& c, int b, int mode) {
     FL_CUDA(cudaGraphDestroy(graph));
     e.kernels = lc.captured;
     return c.graphs[key] = e;
+}
+
+// Enqueues `steps` forward steps of b x t rows on the cache's stream (mode as in enqueue_step; several steps only in the greedy
+// loop) and advances kv_len by t per step (not in mode 2: ragged calls keep per-slot lengths).  Batch-1 decode runs in the
+// persistent kernel, all steps in one launch.  Other single-token steps replay the step's CUDA graph, except inside a profile
+// window, whose per-kernel events a graph cannot record.  Everything else is enqueued kernel by kernel.  `ev`, if given, brackets
+// the enqueued work; a graph is captured before it.
+static void run_steps(fl_cache& c, int b, int t, int mode, int steps, const EventPair* ev = nullptr) {
+    const bool persistent = mode != 2 && b == 1 && t == 1 && c.pk.ok;
+    const bool use_graph = !persistent && t == 1 && !g_prof.on && !env_flag("FL_NO_GRAPH");
+    const GraphEntry* g = use_graph ? &get_graph(c, b, mode) : nullptr;
+    if (ev) FL_CUDA(cudaEventRecord(ev->e0, c.stream));
+    if (persistent) {
+        launch_persistent(c, steps, mode == 1);
+        c.kv_len += steps;
+    } else {
+        for (int s = 0; s < steps; ++s) {
+            if (g) {
+                FL_CUDA(cudaGraphLaunch(g->exec, c.stream));
+                g_launches.fetch_add(g->kernels);
+            } else {
+                LaunchCtx lc{c.stream};
+                enqueue_step(c, lc, b, t, mode);
+            }
+            if (mode != 2) c.kv_len += t;
+        }
+    }
+    if (ev) FL_CUDA(cudaEventRecord(ev->e1, c.stream));
 }
 
 static void check_call(fl_cache& c, const uint32_t* ids, int b, int t, size_t rope_offset, int extra_steps) {
@@ -1405,27 +1330,14 @@ static void check_call(fl_cache& c, const uint32_t* ids, int b, int t, size_t ro
 
 static void run_forward(fl_cache& c, const uint32_t* ids, int b, int t, size_t rope_offset) {
     check_call(c, ids, b, t, rope_offset, 0);
-    if ((b * t >= 3 || c.w->cfg.arch == FL_ARCH_MIXTRAL) && c.w->dense_ok) ensure_dense_ws(c, b * t);
+    if (uses_dense(c, b * t)) ensure_dense_ws(c, b * t);
     std::memcpy(c.h_ids.p, ids, (size_t)b * t * 4);
     FL_CUDA(cudaMemcpyAsync(c.ids.p, c.h_ids.p, (size_t)b * t * 4, cudaMemcpyHostToDevice, c.stream));
     set_state_kernel<<<1, 1, 0, c.stream>>>(c.state.p, (int)rope_offset);
     g_launches.fetch_add(1);
-    const bool use_graph = (t == 1) && !g_prof.on && !env_flag("FL_NO_GRAPH");
     c.dw.route_rows = b * t;
     c.fresh_call = c.kv_len == 0 && !c.slots_used;
-    if (b == 1 && t == 1 && c.pk.ok) {
-        launch_persistent(c, 1, false);
-    } else if (use_graph) {
-        GraphEntry& g = get_graph(c, b, 0);
-        FL_CUDA(cudaGraphLaunch(g.exec, c.stream));
-        g_launches.fetch_add(g.kernels);
-    } else {
-        LaunchCtx lc;
-        lc.stream = c.stream;
-        lc.pdl = !env_flag("FL_NO_PDL");
-        enqueue_forward(c, lc, b, t, false);
-    }
-    c.kv_len += t;
+    run_steps(c, b, t, 0, 1);
 }
 
 // Ragged forward (continuous batching): batch row i is the sequence in cache slot slots[i], which holds slot_len[slots[i]]
@@ -1464,16 +1376,7 @@ static void run_forward_slots(fl_cache& c, const int* slots, const uint32_t* ids
     FL_CUDA(cudaMemcpyAsync(c.slot_tab.p, c.h_slot_tab.p, (size_t)2 * n * 4, cudaMemcpyHostToDevice, c.stream));
     set_slots_kernel<<<1, 256, 0, c.stream>>>(c.state.p, c.slot_tab.p, n);
     g_launches.fetch_add(1);
-    if (t == 1 && !g_prof.on && !env_flag("FL_NO_GRAPH")) {
-        GraphEntry& g = get_graph(c, n, 2);
-        FL_CUDA(cudaGraphLaunch(g.exec, c.stream));
-        g_launches.fetch_add(g.kernels);
-    } else {
-        LaunchCtx lc;
-        lc.stream = c.stream;
-        lc.pdl = !env_flag("FL_NO_PDL");
-        enqueue_forward_dense(c, lc, n, t, false);
-    }
+    run_steps(c, n, t, 2, 1);
     for (int i = 0; i < n; ++i) c.slot_len[slots[i]] += t;
 }
 
@@ -1508,6 +1411,21 @@ static void use_device() {
     const int dev = g_device.load();
     FL_CHECK(dev >= 0, FL_ERR_STATE, "fl_init has not been called");
     FL_CUDA(cudaSetDevice(dev));   // no thread-affine state: callers may hop OS threads between calls (SURVEY.md section 8b)
+}
+
+// Body of a forward entry point on model m and its cache c (`args_ok`: the entry point's other pointer arguments are set).
+// A CUDA or NCCL error poisons the cache: a missed peer leaves kv_len / exchange epochs out of step.
+template <typename F>
+static void forward_guard(fl_model* m, fl_cache* c, bool args_ok, F&& body) {
+    FL_CHECK(m && c && args_ok, FL_ERR_INVALID, "NULL argument");
+    FL_CHECK(m->w != nullptr && m->w.get() == c->w.get(), FL_ERR_INVALID, "cache belongs to a different model");
+    use_device();
+    try {
+        body(*c);
+    } catch (const fl::Error& e) {
+        if (e.code == FL_ERR_CUDA || e.code == FL_ERR_NCCL) c->poisoned = true;
+        throw;
+    }
 }
 
 extern "C" {
@@ -1723,93 +1641,55 @@ FL_EXPORT int fl_cache_destroy(fl_cache* c) {
 
 FL_EXPORT int fl_forward(fl_model* m, fl_cache* c, const uint32_t* ids, int b, int t, size_t rope_offset, float* logits_host) {
     FL_API_BEGIN
-    FL_CHECK(m && c && logits_host, FL_ERR_INVALID, "NULL argument");
-    FL_CHECK(m->w != nullptr && m->w.get() == c->w.get(), FL_ERR_INVALID, "cache belongs to a different model");
-    use_device();
-    try {
-        run_forward(*c, ids, b, t, rope_offset);
-        const size_t n = (size_t)b * c->w->Vfull;
-        FL_CUDA(cudaMemcpyAsync(c->h_logits.p, c->logits.p, n * 4, cudaMemcpyDeviceToHost, c->stream));
-        FL_CUDA(cudaStreamSynchronize(c->stream));
+    forward_guard(m, c, logits_host, [&](fl_cache& c) {
+        run_forward(c, ids, b, t, rope_offset);
+        const size_t n = (size_t)b * c.w->Vfull;
+        FL_CUDA(cudaMemcpyAsync(c.h_logits.p, c.logits.p, n * 4, cudaMemcpyDeviceToHost, c.stream));
+        FL_CUDA(cudaStreamSynchronize(c.stream));
         check_peer_error();
-        std::memcpy(logits_host, c->h_logits.p, n * 4);
-    } catch (const fl::Error& e) {
-        if (e.code == FL_ERR_CUDA || e.code == FL_ERR_NCCL) c->poisoned = true;   // a missed peer leaves kv_len / exchange epochs out of step
-        throw;
-    }
+        std::memcpy(logits_host, c.h_logits.p, n * 4);
+    });
     FL_API_END
 }
 
 FL_EXPORT int fl_forward_greedy(fl_model* m, fl_cache* c, const uint32_t* ids, int b, int t, size_t rope_offset, uint32_t* next_ids) {
     FL_API_BEGIN
-    FL_CHECK(m && c && next_ids, FL_ERR_INVALID, "NULL argument");
-    FL_CHECK(m->w != nullptr && m->w.get() == c->w.get(), FL_ERR_INVALID, "cache belongs to a different model");
-    use_device();
-    try {
-        run_forward(*c, ids, b, t, rope_offset);
-        FL_CUDA(cudaMemcpyAsync(c->h_ids.p, c->next_ids.p, (size_t)b * 4, cudaMemcpyDeviceToHost, c->stream));
-        FL_CUDA(cudaStreamSynchronize(c->stream));
+    forward_guard(m, c, next_ids, [&](fl_cache& c) {
+        run_forward(c, ids, b, t, rope_offset);
+        FL_CUDA(cudaMemcpyAsync(c.h_ids.p, c.next_ids.p, (size_t)b * 4, cudaMemcpyDeviceToHost, c.stream));
+        FL_CUDA(cudaStreamSynchronize(c.stream));
         check_peer_error();
-        std::memcpy(next_ids, c->h_ids.p, (size_t)b * 4);
-    } catch (const fl::Error& e) {
-        if (e.code == FL_ERR_CUDA || e.code == FL_ERR_NCCL) c->poisoned = true;   // a missed peer leaves kv_len / exchange epochs out of step
-        throw;
-    }
+        std::memcpy(next_ids, c.h_ids.p, (size_t)b * 4);
+    });
     FL_API_END
 }
 
 FL_EXPORT int fl_decode_greedy_loop(fl_model* m, fl_cache* c, const uint32_t* first_ids, int b, size_t rope_offset, int steps,
                           uint32_t* out_ids, float* elapsed_ms) {
     FL_API_BEGIN
-    FL_CHECK(m && c, FL_ERR_INVALID, "NULL argument");
-    FL_CHECK(m->w != nullptr && m->w.get() == c->w.get(), FL_ERR_INVALID, "cache belongs to a different model");
-    FL_CHECK(steps >= 1, FL_ERR_INVALID, "steps must be >= 1");
-    use_device();
-    try {
-        check_call(*c, first_ids, b, 1, rope_offset, steps - 1);
-        if ((b >= 3 || c->w->cfg.arch == FL_ARCH_MIXTRAL) && c->w->dense_ok) ensure_dense_ws(*c, b);
-        if (c->trace_cap < (size_t)steps * b) {
-            c->trace.alloc((size_t)steps * b);
-            c->trace_cap = (size_t)steps * b;
-            cache_destroy_graphs(*c);   // captured graphs hold the old trace pointer
+    forward_guard(m, c, true, [&](fl_cache& c) {
+        FL_CHECK(steps >= 1, FL_ERR_INVALID, "steps must be >= 1");
+        check_call(c, first_ids, b, 1, rope_offset, steps - 1);
+        if (uses_dense(c, b)) ensure_dense_ws(c, b);
+        if (c.trace_cap < (size_t)steps * b) {
+            c.trace.alloc((size_t)steps * b);
+            c.trace_cap = (size_t)steps * b;
+            cache_destroy_graphs(c);   // captured graphs hold the old trace pointer
         }
-        std::memcpy(c->h_ids.p, first_ids, (size_t)b * 4);
-        FL_CUDA(cudaMemcpyAsync(c->ids.p, c->h_ids.p, (size_t)b * 4, cudaMemcpyHostToDevice, c->stream));
-        FL_CUDA(cudaMemsetAsync(c->trace_pos.p, 0, 4, c->stream));
-        set_state_kernel<<<1, 1, 0, c->stream>>>(c->state.p, (int)rope_offset);
+        std::memcpy(c.h_ids.p, first_ids, (size_t)b * 4);
+        FL_CUDA(cudaMemcpyAsync(c.ids.p, c.h_ids.p, (size_t)b * 4, cudaMemcpyHostToDevice, c.stream));
+        FL_CUDA(cudaMemsetAsync(c.trace_pos.p, 0, 4, c.stream));
+        set_state_kernel<<<1, 1, 0, c.stream>>>(c.state.p, (int)rope_offset);
         g_launches.fetch_add(1);
-        const bool persistent = (b == 1) && c->pk.ok;
-        const bool use_graph = !persistent && !g_prof.on && !env_flag("FL_NO_GRAPH");
-        GraphEntry* g = use_graph ? &get_graph(*c, b, 1) : nullptr;
         EventPair ev;
-        FL_CUDA(cudaEventRecord(ev.e0, c->stream));
-        if (persistent) {
-            launch_persistent(*c, steps, true);   // all steps inside one cooperative launch
-            c->kv_len += steps;
-        }
-        for (int s = 0; s < (persistent ? 0 : steps); ++s) {
-            if (g) {
-                FL_CUDA(cudaGraphLaunch(g->exec, c->stream));
-                g_launches.fetch_add(g->kernels);
-            } else {
-                LaunchCtx lc;
-                lc.stream = c->stream;
-                lc.pdl = !env_flag("FL_NO_PDL");
-                enqueue_forward(*c, lc, b, 1, true);
-            }
-            c->kv_len += 1;
-        }
-        FL_CUDA(cudaEventRecord(ev.e1, c->stream));
-        FL_CUDA(cudaStreamSynchronize(c->stream));
+        run_steps(c, b, 1, 1, steps, &ev);     // batch 1: all steps inside one persistent launch
+        FL_CUDA(cudaStreamSynchronize(c.stream));
         check_peer_error();
         float ms = 0.f;
         FL_CUDA(cudaEventElapsedTime(&ms, ev.e0, ev.e1));
         if (elapsed_ms) *elapsed_ms = ms;
-        if (out_ids) FL_CUDA(cudaMemcpy(out_ids, c->trace.p, (size_t)steps * b * 4, cudaMemcpyDeviceToHost));
-    } catch (const fl::Error& e) {
-        if (e.code == FL_ERR_CUDA || e.code == FL_ERR_NCCL) c->poisoned = true;   // a missed peer leaves kv_len / exchange epochs out of step
-        throw;
-    }
+        if (out_ids) FL_CUDA(cudaMemcpy(out_ids, c.trace.p, (size_t)steps * b * 4, cudaMemcpyDeviceToHost));
+    });
     FL_API_END
 }
 
@@ -1818,6 +1698,15 @@ struct fl_sampler {
     fl::LogitsProcessor lp;
     fl_sampler(uint64_t seed, double temperature) : lp(seed, temperature) {}
 };
+
+// One host-side sample; a sampler error (e.g. logits that are all NaN) is an invalid argument at the C ABI.
+static uint32_t sample_host(fl_sampler* s, const float* logits_host, size_t n) {
+    try {
+        return s->lp.sample(logits_host, n);
+    } catch (const fl::SamplerError& e) {
+        throw fl::Error(FL_ERR_INVALID, e.what());
+    }
+}
 
 FL_EXPORT int fl_sampler_create(uint64_t seed, double temperature, fl_sampler** out) {
     FL_API_BEGIN
@@ -1830,11 +1719,7 @@ FL_EXPORT int fl_sampler_create(uint64_t seed, double temperature, fl_sampler** 
 FL_EXPORT int fl_sampler_sample(fl_sampler* s, const float* logits_host, size_t n, uint32_t* token) {
     FL_API_BEGIN
     FL_CHECK(s && logits_host && token, FL_ERR_INVALID, "NULL argument");
-    try {
-        *token = s->lp.sample(logits_host, n);
-    } catch (const fl::SamplerError& e) {
-        throw fl::Error(FL_ERR_INVALID, e.what());
-    }
+    *token = sample_host(s, logits_host, n);
     FL_API_END
 }
 
@@ -1873,72 +1758,50 @@ FL_EXPORT int fl_sampler_destroy(fl_sampler* s) {
 FL_EXPORT int fl_forward_sample(fl_model* m, fl_cache* c, const uint32_t* ids, int b, int t, size_t rope_offset, fl_sampler* s,
                                 uint32_t* next_id) {
     FL_API_BEGIN
-    FL_CHECK(m && c && s && next_id, FL_ERR_INVALID, "NULL argument");
-    FL_CHECK(m->w != nullptr && m->w.get() == c->w.get(), FL_ERR_INVALID, "cache belongs to a different model");
-    use_device();
-    try {
-        run_forward(*c, ids, b, t, rope_offset);
+    forward_guard(m, c, s && next_id, [&](fl_cache& c) {
+        run_forward(c, ids, b, t, rope_offset);
         // only row 0 is sampled (logits.get(0)?.flatten_all()?, models/mod.rs:421): one V*4-byte read-back into the pinned staging row
-        const size_t n = c->w->Vfull;
-        FL_CUDA(cudaMemcpyAsync(c->h_logits.p, c->logits.p, n * 4, cudaMemcpyDeviceToHost, c->stream));
-        FL_CUDA(cudaStreamSynchronize(c->stream));
+        const size_t n = c.w->Vfull;
+        FL_CUDA(cudaMemcpyAsync(c.h_logits.p, c.logits.p, n * 4, cudaMemcpyDeviceToHost, c.stream));
+        FL_CUDA(cudaStreamSynchronize(c.stream));
         check_peer_error();
-        try {
-            *next_id = s->lp.sample(c->h_logits.p, n);
-        } catch (const fl::SamplerError& e) {
-            throw fl::Error(FL_ERR_INVALID, e.what());
-        }
-    } catch (const fl::Error& e) {
-        if (e.code == FL_ERR_CUDA || e.code == FL_ERR_NCCL) c->poisoned = true;   // a missed peer leaves kv_len / exchange epochs out of step
-        throw;
-    }
+        *next_id = sample_host(s, c.h_logits.p, n);
+    });
     FL_API_END
 }
 
 FL_EXPORT int fl_forward_slots(fl_model* m, fl_cache* c, const int* slots, const uint32_t* ids, int n, int t, const size_t* rope_offsets,
                                float* logits_host) {
     FL_API_BEGIN
-    FL_CHECK(m && c && logits_host, FL_ERR_INVALID, "NULL argument");
-    FL_CHECK(m->w != nullptr && m->w.get() == c->w.get(), FL_ERR_INVALID, "cache belongs to a different model");
-    use_device();
-    try {
-        run_forward_slots(*c, slots, ids, n, t, rope_offsets);
-        const size_t cnt = (size_t)n * c->w->Vfull;
-        FL_CUDA(cudaMemcpyAsync(c->h_logits.p, c->logits.p, cnt * 4, cudaMemcpyDeviceToHost, c->stream));
-        FL_CUDA(cudaStreamSynchronize(c->stream));
+    forward_guard(m, c, logits_host, [&](fl_cache& c) {
+        run_forward_slots(c, slots, ids, n, t, rope_offsets);
+        const size_t cnt = (size_t)n * c.w->Vfull;
+        FL_CUDA(cudaMemcpyAsync(c.h_logits.p, c.logits.p, cnt * 4, cudaMemcpyDeviceToHost, c.stream));
+        FL_CUDA(cudaStreamSynchronize(c.stream));
         check_peer_error();
-        std::memcpy(logits_host, c->h_logits.p, cnt * 4);
-    } catch (const fl::Error& e) {
-        if (e.code == FL_ERR_CUDA || e.code == FL_ERR_NCCL) c->poisoned = true;
-        throw;
-    }
+        std::memcpy(logits_host, c.h_logits.p, cnt * 4);
+    });
     FL_API_END
 }
 
 FL_EXPORT int fl_forward_sample_device(fl_model* m, fl_cache* c, const uint32_t* ids, int b, int t, size_t rope_offset, fl_sampler* s,
                                        uint32_t* next_id) {
     FL_API_BEGIN
-    FL_CHECK(m && c && s && next_id, FL_ERR_INVALID, "NULL argument");
-    FL_CHECK(m->w != nullptr && m->w.get() == c->w.get(), FL_ERR_INVALID, "cache belongs to a different model");
-    use_device();
-    try {
-        run_forward(*c, ids, b, t, rope_offset);
-        const uint32_t* src = c->next_ids.p;                       // temperature below 1e-7: the arg-max the forward already computed
+    forward_guard(m, c, s && next_id, [&](fl_cache& c) {
+        run_forward(c, ids, b, t, rope_offset);
+        const uint32_t* src = c.next_ids.p;                       // temperature below 1e-7: the arg-max the forward already computed
         if (!s->lp.is_argmax()) {
             // row 0 only (logits.get(0)?, models/mod.rs:421); ONE generator draw per sample, exactly as on the host path
             const float u = s->lp.draw_unit();
-            sample_softmax_kernel<<<1, 1024, 0, c->stream>>>(c->logits.p, c->w->Vfull, s->lp.inv_temperature(), u, c->sample_out.p);
+            sample_softmax_kernel<<<1, 1024, 0, c.stream>>>(c.logits.p, c.w->Vfull, s->lp.inv_temperature(), u, c.sample_out.p);
             g_launches.fetch_add(1);
-            src = c->sample_out.p;
+            src = c.sample_out.p;
         }
-        FL_CUDA(cudaMemcpyAsync(c->h_ids.p, src, 4, cudaMemcpyDeviceToHost, c->stream));
-        FL_CUDA(cudaStreamSynchronize(c->stream));
+        FL_CUDA(cudaMemcpyAsync(c.h_ids.p, src, 4, cudaMemcpyDeviceToHost, c.stream));
+        FL_CUDA(cudaStreamSynchronize(c.stream));
         check_peer_error();
-        *next_id = c->h_ids.p[0];
-    } catch (const fl::Error& e) {
-        if (e.code == FL_ERR_CUDA || e.code == FL_ERR_NCCL) c->poisoned = true;
-        throw;
-    }
+        *next_id = c.h_ids.p[0];
+    });
     FL_API_END
 }
 

@@ -57,7 +57,6 @@ struct Weights {
     float* rope_cos = nullptr;  // [max_pos, d/2]
     float* rope_sin = nullptr;
     std::set<std::string> have; // tensor names that arrived
-    int ignored = 0;            // tensors handed over that the architecture does not read (skipped like VarBuilder does)
     bool lm_head_loaded = false;
     bool finalized = false;
     uint64_t streamed_bytes = 0;
@@ -76,7 +75,6 @@ struct PkPlan {
 // Workspace of the dense (tensor-core) path, sized for the largest row count seen so far.
 struct DenseWs {
     size_t rows = 0;
-    int chunk = 0;              // attention rows per launch
     DevBuf<uint16_t> xhi, xlo;  // [rows, Kmax] hi/lo bf16 split of the activations fed to the next GEMM
     DevBuf<float> y;            // [rows, Nmax] GEMM output
     DevBuf<float> resid, q;
@@ -91,11 +89,9 @@ struct DenseWs {
     DevBuf<float> route_margin;     // [L][rows of the call]
     int route_rows = 0;             // rows of the last Mixtral forward
     // grouped expert GEMMs (decode batches): per-expert blocks of gathered rows, their counts, and the row -> slot map
-    int grp_cap = 0;                 // rows per expert block (the GEMM's N tile: 16 / 32 / 64 / 128)
-    DevBuf<uint16_t> gx_hi, gx_lo;   // [E_local * grp_cap, H]
-    DevBuf<int> grp_cnt, grp_pos;    // [E_local], [moe_rows, E_local]
+    DevBuf<uint16_t> gx_hi, gx_lo;   // [E_local * rows per expert block (16 / 32 / 64 / 128), H]
+    DevBuf<int> grp_cnt, grp_pos;    // [E_local], [expert rows (rows, or rows * ep), E_local]
     // expert parallelism with data-parallel attention: dispatch / combine staging (all rows of all ranks, rank-major)
-    size_t moe_rows = 0;         // rows the expert GEMMs see (rows, or rows * ep)
     DevBuf<uint16_t> g_xhi, g_xlo;   // [ep * rows, H] gathered block inputs
     DevBuf<float> g_route;           // [ep * rows, E]
     DevBuf<float> comb;              // [ep sources][rows, H] expert outputs returned to this rank

@@ -1,5 +1,5 @@
-// Host-side runtime pieces shared by the translation units: launch wrapper (PDL + per-kernel event profile +
-// launch counter), device buffer RAII, thread-local error slot.
+// Host-side runtime pieces shared by the translation units: launch wrapper (PDL + opt-in shared memory + per-kernel event
+// profile + launch counter), device buffer RAII, thread-local error slot, host bf16 rounding.
 #pragma once
 #include <atomic>
 #include <cstdlib>
@@ -32,29 +32,65 @@ inline bool env_flag(const char* name) {
     return v != nullptr && v[0] != '\0' && v[0] != '0';
 }
 
+inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
+
+// f32 -> bf16 bits, round to nearest even
+inline uint16_t host_f32_to_bf16(float f) {
+    uint32_t b;
+    std::memcpy(&b, &f, 4);
+    if ((b & 0x7FFFFFFFu) > 0x7F800000u) return (uint16_t)((b >> 16) | 0x40u);   // NaN stays NaN (quiet), as half::bf16::from_f32 does
+    return (uint16_t)((b + 0x7FFFu + ((b >> 16) & 1u)) >> 16);
+}
+
 struct LaunchCtx {
     cudaStream_t stream = nullptr;
-    bool pdl = true;          // programmatic dependent launch on every kernel of the step
+    bool pdl = !env_flag("FL_NO_PDL");   // programmatic dependent launch on every kernel of the step
     bool capturing = false;   // inside cudaStreamBeginCapture: no events, no profile
     uint64_t captured = 0;    // kernels recorded into the graph being captured
+    bool cooperative = false; // cooperative launch: every CTA of the grid co-resident (the persistent decode kernel)
 };
 
-// Launches `kern` with optional PDL.  `tag`/`bytes` feed the per-kernel profile (algorithmic bytes of that launch).
+// One launch (kernel or NCCL call) enqueued on lc: counted into the graph being captured, or into fl_launch_count.
+inline void count_launch(LaunchCtx& lc) {
+    if (lc.capturing)
+        lc.captured++;
+    else
+        g_launches.fetch_add(1, std::memory_order_relaxed);
+}
+
+// Raises `kern`'s opt-in dynamic shared-memory limit to at least `bytes`.  Idempotent and safe from several threads: the largest
+// size set so far is remembered per kernel (attributes are per device; a process drives one, see fl_init).
+inline void ensure_smem_optin(const void* kern, size_t bytes) {
+    static std::mutex mu;
+    static std::map<const void*, size_t> raised;
+    std::lock_guard<std::mutex> lk(mu);
+    size_t& cur = raised[kern];
+    if (bytes <= cur) return;
+    FL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+    cur = bytes;
+}
+
+// Launches `kern` with optional PDL.  `tag`/`bytes` feed the per-kernel profile (algorithmic bytes of that launch).  Inside a
+// profile window kernels run without PDL, so that each one's events bracket it alone.
 template <typename... KArgs, typename... Args>
 inline void launch(LaunchCtx& lc, const char* tag, uint64_t bytes, void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem,
                    Args&&... args) {
+    if (smem > 48 * 1024) ensure_smem_optin((const void*)kern, smem);
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = grid;
     cfg.blockDim = block;
     cfg.dynamicSmemBytes = smem;
     cfg.stream = lc.stream;
-    cudaLaunchAttribute attr[1];
+    cudaLaunchAttribute attr[2];
+    cfg.attrs = attr;
     const bool prof = g_prof.on && !lc.capturing;
     if (lc.pdl && !prof) {
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 1;
+        attr[cfg.numAttrs].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+        attr[cfg.numAttrs++].val.programmaticStreamSerializationAllowed = 1;
+    }
+    if (lc.cooperative) {
+        attr[cfg.numAttrs].id = cudaLaunchAttributeCooperative;
+        attr[cfg.numAttrs++].val.cooperative = 1;
     }
     ProfEntry pe;
     if (prof) {
@@ -69,10 +105,7 @@ inline void launch(LaunchCtx& lc, const char* tag, uint64_t bytes, void (*kern)(
         FL_CUDA(cudaEventRecord(pe.e1, lc.stream));
         g_prof.entries.push_back(pe);
     }
-    if (lc.capturing)
-        lc.captured++;
-    else
-        g_launches.fetch_add(1, std::memory_order_relaxed);
+    count_launch(lc);
 }
 
 // a start / stop event pair that cannot leak when something between create and destroy throws

@@ -195,7 +195,7 @@ FL_EXPORT int fl_comm_ipc_import(const void* handles, int world, int rank);
 FL_EXPORT int fl_comm_destroy(void);
 
 /* ---- measurement hooks (bench.py / tests) ------------------------------------------------------- */
-/* Per-kernel CUDA-event profile of subsequent forwards (eager launches, events on the launching stream). */
+/* Per-kernel CUDA-event profile of subsequent forwards and embeddings (eager launches without PDL, events on the launching stream). */
 FL_EXPORT int fl_prof_begin(void);
 /* Writes a JSON array [{"kernel": name, "launches": n, "ms": total_ms, "bytes": algorithmic_bytes}, ...]. */
 FL_EXPORT int fl_prof_end(char* json_out, size_t cap);
