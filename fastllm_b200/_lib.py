@@ -64,6 +64,7 @@ SYMBOLS = {
     "fl_cache_moe_routing": (_I, [_VP, _I, _VP, _VP]),
     "fl_forward_sample_device": (_I, [_VP, _VP, _VP, _I, _I, _SZ, _VP, C.POINTER(C.c_uint32)]),
     "fl_embed": (_I, [_VP, _VP, _VP, _I, _I, _VP]),
+    "fl_embed_packed": (_I, [_VP, _VP, _VP, _I, _VP]),
     "fl_embed_timed": (_I, [_VP, _VP, _VP, _I, _I, _VP, _I, C.POINTER(C.c_float)]),
     "fl_comm_unique_id": (_I, [_VP]),
     "fl_comm_init": (_I, [_I, _I, _VP]),

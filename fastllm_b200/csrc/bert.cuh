@@ -5,23 +5,33 @@
 //                       more than 128 tokens go through bert_attn_long_kernel (key tiles + online softmax)
 //   layernorm_kernel  : post-LN over (x + f(x)), eps = config.layer_norm_eps (:185-190, :236-241); one-pass var = E[x^2]-mean^2
 //   pool_l2_kernel    : masked mean pooling (divisor = mask_count * hidden [sic], :346-368) + L2 normalise (:341-344)
+// Token rows are packed: sentence s is rows [starts[s], starts[s + 1]) of every [T, .] activation, with no padding between
+// sentences.  A uniform [b, t] batch is the case starts[s] = s * t.  The attention kernels take a work list of BertItem.
+// The sentence tables (positions, starts, items) are written by the host upload that precedes the encoder's first kernel and by
+// no kernel, so every kernel reads them BEFORE pdl_wait: their load latency overlaps the previous kernel's tail.
 #pragma once
 #include "common.cuh"
 #include "mma.cuh"
 
 namespace fl {
 
+// One attention work item: the sentence's first token row and length, and the first query row q0 of the item within the sentence
+// (a multiple of 128; always 0 for bert_attn_kernel, whose sentences are one tile).
+struct __align__(16) BertItem {
+    int row0, len, q0, pad;
+};
+
 // One warp per token row; H multiple of 32*... generic loop.  out bf16 [T, H].
 static __global__ void embed_ln_kernel(const uint16_t* __restrict__ wemb, const uint16_t* __restrict__ pemb, const float* __restrict__ lnw,
-                                const float* __restrict__ lnb, const uint32_t* __restrict__ ids, int T, int t, int H, int vocab, int maxpos,
-                                float eps, uint16_t* __restrict__ out) {
+                                const float* __restrict__ lnb, const uint32_t* __restrict__ ids, const int* __restrict__ positions, int T,
+                                int H, int vocab, int maxpos, float eps, uint16_t* __restrict__ out) {
     pdl_launch_dependents();      // programmatic dependent launch: the next kernel may start its prologue now ...
-    pdl_wait();                   // ... and nothing below runs before the previous kernel has completed
     const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    int pos = row < T ? positions[row] : 0;  // position ids 0..n-1 of each sentence (embeddings.rs:416); a sentence table
+    pdl_wait();                   // ... and nothing below runs before the previous kernel has completed
     if (row >= T) return;
     uint32_t id = ids[row];
     if (id >= (uint32_t)vocab) id = vocab - 1;
-    int pos = row % t;                       // position ids 0..n-1 (embeddings.rs:416)
     if (pos >= maxpos) pos = maxpos - 1;
     const uint16_t* w = wemb + (size_t)id * H;
     const uint16_t* p = pemb + (size_t)pos * H;
@@ -91,13 +101,16 @@ constexpr int kBertS = 128;      // query / key rows per tile (a sentence of <= 
 constexpr int kBertD = 32;       // head dim
 constexpr int kBertLd = 40;      // padded smem row (80 bytes): conflict-free ldmatrix
 
-// grid (heads, sentences), 128 threads: warp w owns query rows [32w, 32w+32).  qkv bf16 [T, 3H] (q | k | v), ctx bf16 [T, H].
-static __global__ void __launch_bounds__(128) bert_attn_kernel(const uint16_t* __restrict__ qkv, int t, int H, float scale, uint16_t* __restrict__ ctx) {
+// grid (heads x items), head fastest; 128 threads: warp w owns query rows [32w, 32w+32).  qkv bf16 [T, 3H] (q | k | v), ctx bf16 [T, H].
+static __global__ void __launch_bounds__(128) bert_attn_kernel(const uint16_t* __restrict__ qkv, const BertItem* __restrict__ items, int nh,
+                                                               int H, float scale, uint16_t* __restrict__ ctx) {
     pdl_launch_dependents();      // programmatic dependent launch: the next kernel may start its prologue now ...
+    const BertItem it = items[blockIdx.x / nh];      // a sentence table
     pdl_wait();                   // ... and nothing below runs before the previous kernel has completed
     __shared__ __align__(16) uint16_t sq[kBertS * kBertLd], sk[kBertS * kBertLd], sv[kBertS * kBertLd];
-    const int head = blockIdx.x, sent = blockIdx.y, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const size_t row0 = (size_t)sent * t;
+    const int head = blockIdx.x % nh, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const size_t row0 = (size_t)it.row0;
+    const int t = it.len;
     const int ld = 3 * H;
     // stage Q, K, V of this (sentence, head): 128 rows x 32 bf16 (64 B) each; rows >= t are zero
     for (int i = tid; i < kBertS * 4; i += 128) {
@@ -191,16 +204,18 @@ static __global__ void __launch_bounds__(128) bert_attn_kernel(const uint16_t* _
 }
 
 // Sentences longer than one 128-row tile (up to max_position_embeddings, 512 for MiniLM: the reference enforces no limit,
-// embeddings.rs:285-286): the same attention, FlashAttention-style.  grid (heads, sentences, ceil(t / 128) query tiles), 128 threads;
+// embeddings.rs:285-286): the same attention, FlashAttention-style.  grid (heads x (sentence, query tile) items), 128 threads;
 // a CTA stages its 128 query rows once and walks the sentence's keys in 128-row tiles with an online softmax (running max / sum per
 // row, accumulator rescaled when the max moves) -- algebraically the reference's max-subtract / exp / sum / div over all keys.
-static __global__ void __launch_bounds__(128) bert_attn_long_kernel(const uint16_t* __restrict__ qkv, int t, int H, float scale,
-                                                                    uint16_t* __restrict__ ctx) {
+static __global__ void __launch_bounds__(128) bert_attn_long_kernel(const uint16_t* __restrict__ qkv, const BertItem* __restrict__ items,
+                                                                    int nh, int H, float scale, uint16_t* __restrict__ ctx) {
     pdl_launch_dependents();      // programmatic dependent launch: the next kernel may start its prologue now ...
+    const BertItem it = items[blockIdx.x / nh];      // a sentence table
     pdl_wait();                   // ... and nothing below runs before the previous kernel has completed
     __shared__ __align__(16) uint16_t sq[kBertS * kBertLd], sk[kBertS * kBertLd], sv[kBertS * kBertLd];
-    const int head = blockIdx.x, sent = blockIdx.y, q0 = blockIdx.z * kBertS, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const size_t row0 = (size_t)sent * t;
+    const int head = blockIdx.x % nh, q0 = it.q0, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const size_t row0 = (size_t)it.row0;
+    const int t = it.len;
     const int ld = 3 * H;
     for (int i = tid; i < kBertS * 4; i += 128) {
         const int r = i >> 2, c = (i & 3) * 8;
@@ -314,17 +329,19 @@ static __global__ void __launch_bounds__(128) bert_attn_long_kernel(const uint16
     }
 }
 
-// mean_pooling + normalize_l2: one CTA per sentence, thread per hidden column (H <= 1024).
-static __global__ void pool_l2_kernel(const uint16_t* __restrict__ x, const uint32_t* __restrict__ mask, int t, int H, float* __restrict__ out) {
+// mean_pooling + normalize_l2: one CTA per sentence, thread per hidden column (H <= 1024); mask (per token row) may be NULL = all ones.
+static __global__ void pool_l2_kernel(const uint16_t* __restrict__ x, const uint32_t* __restrict__ mask, const int* __restrict__ starts, int H,
+                                      float* __restrict__ out) {
     pdl_launch_dependents();      // programmatic dependent launch: the next kernel may start its prologue now ...
+    const int sent = blockIdx.x, c = threadIdx.x;
+    const int r0 = starts[sent], r1 = starts[sent + 1];      // a sentence table
     pdl_wait();                   // ... and nothing below runs before the previous kernel has completed
     __shared__ float red[32];
-    const int sent = blockIdx.x, c = threadIdx.x;
     float acc = 0.f, cnt = 0.f;
-    for (int r = 0; r < t; ++r) {
-        const float m = mask ? (float)mask[(size_t)sent * t + r] : 1.f;
+    for (int r = r0; r < r1; ++r) {
+        const float m = mask ? (float)mask[r] : 1.f;
         cnt += m;
-        if (c < H) acc = fmaf(__uint_as_float((uint32_t)x[((size_t)sent * t + r) * H + c] << 16), m, acc);
+        if (c < H) acc = fmaf(__uint_as_float((uint32_t)x[(size_t)r * H + c] << 16), m, acc);
     }
     const float pooled = acc / (cnt * (float)H);      // divisor = mask_count * hidden (embeddings.rs:359-365); cancelled below
     float sq = (c < H) ? pooled * pooled : 0.f;

@@ -1,7 +1,8 @@
 // BERT / MiniLM sentence-encoder path behind fl_embed (host orchestration), sm_100a.
 // Reference: MiniLMModel::{new, embed_tokens, forward, mean_pooling, normalize_l2, embed} src/models/embeddings.rs:245-447.
+#include <algorithm>
 #include <cmath>
-#include <memory>
+#include <cstring>
 
 #include "bert.cuh"
 #include "bert_model.cuh"
@@ -235,26 +236,35 @@ void bert_finalize(BertModel& m) {
     m.finalized = true;
 }
 
-static void bert_reserve(BertModel& m, int b, int t) {
-    const size_t T = (size_t)b * t;
-    if (T <= m.cap_tokens && (size_t)b <= m.cap_batch) return;
+static void bert_reserve(BertModel& m, size_t T, size_t n, size_t words) {
     const size_t H = m.H, I = m.I;
-    m.cap_tokens = std::max(T, m.cap_tokens);
-    m.cap_batch = std::max((size_t)b, m.cap_batch);
-    const size_t Tc = m.cap_tokens;
-    m.x.alloc(Tc * H); m.x1.alloc(Tc * H); m.ctx.alloc(Tc * H); m.qkv.alloc(Tc * 3 * H); m.hbuf.alloc(Tc * I); m.pre.alloc(Tc * H);
-    m.ids.alloc(Tc); m.mask.alloc(Tc); m.out.alloc(m.cap_batch * H);
-    m.h_ids.alloc(2 * Tc); m.h_out.alloc(m.cap_batch * H);
+    if (T > m.cap_tokens) {
+        m.cap_tokens = T;
+        m.x.alloc(T * H); m.x1.alloc(T * H); m.ctx.alloc(T * H); m.qkv.alloc(T * 3 * H); m.hbuf.alloc(T * I); m.pre.alloc(T * H);
+    }
+    if (n > m.cap_batch) {
+        m.cap_batch = n;
+        m.out.alloc(n * H); m.h_out.alloc(n * H);
+    }
+    if (words > m.cap_words) {
+        m.cap_words = words;
+        m.ids.alloc(words); m.h_ids.alloc(words);
+    }
 }
 
-// Enqueue the encoder on m.stream: B1 -> 6 x (B2..B7) -> B8 (SURVEY.md section 2.4)
-static void bert_enqueue(BertModel& m, int b, int t, bool has_mask) {
-    const int T = b * t, H = m.H, I = m.I;
+// Enqueue the encoder on m.stream over the batch m.batch describes: B1 -> L x (B2..B7) -> B8 (SURVEY.md section 2.4)
+static void bert_enqueue(BertModel& m, bool use_mask) {
+    const BertModel::Batch& bb = m.batch;
+    const int T = bb.T, H = m.H, I = m.I;
+    const int* positions = (const int*)(m.ids.p + bb.o_pos);
+    const int* starts = (const int*)(m.ids.p + bb.o_starts);
+    const BertItem* shorts = (const BertItem*)(m.ids.p + bb.o_short);
+    const BertItem* longs = (const BertItem*)(m.ids.p + bb.o_long);
     LaunchCtx lc{m.stream};
     const int rows_per_cta = 8;
     const dim3 row_grid((T + rows_per_cta - 1) / rows_per_cta), row_block(rows_per_cta * 32);
     launch(lc, "bert_embed_ln", 0, embed_ln_kernel, row_grid, row_block, 0, (const uint16_t*)m.wemb, (const uint16_t*)m.pemb, (const float*)m.lnw,
-           (const float*)m.lnb, (const uint32_t*)m.ids.p, T, t, H, m.V, m.maxpos, 1e-12f, m.x.p);
+           (const float*)m.lnb, (const uint32_t*)m.ids.p, positions, T, H, m.V, m.maxpos, 1e-12f, m.x.p);
     const CUtensorMap tm_x = make_tmap_bf16(m.x.p, T, H, H, kGemmBM), tm_x1 = make_tmap_bf16(m.x1.p, T, H, H, kGemmBM),
                       tm_ctx = make_tmap_bf16(m.ctx.p, T, H, H, kGemmBM), tm_h = make_tmap_bf16(m.hbuf.p, T, I, I, kGemmBM);
     const float eps = m.cfg.norm_eps;
@@ -263,11 +273,12 @@ static void bert_enqueue(BertModel& m, int b, int t, bool has_mask) {
         const BertLayerW& w = m.layers[l];
         // B2: fused q|k|v projection + bias -> bf16 [T, 3H]
         launch_gemm<GEPI_BIAS_BF16>(lc, "bert_gemm_qkv", tm_x, w.tm_wqkv, GemmArgs{T, 3 * H, H, w.bqkv, nullptr, 0, m.qkv.p, 3 * H, 1, 0});
-        // B3+B4: per (sentence, head) softmax(QK^T / sqrt(d)) V, no mask
-        if (t <= kBertS)
-            launch(lc, "bert_attn", 0, bert_attn_kernel, dim3(m.nh, b), dim3(128), 0, (const uint16_t*)m.qkv.p, t, H, scale, m.ctx.p);
-        else
-            launch(lc, "bert_attn", 0, bert_attn_long_kernel, dim3(m.nh, b, (t + kBertS - 1) / kBertS), dim3(128), 0, (const uint16_t*)m.qkv.p, t, H,
+        // B3+B4: per (sentence, head) softmax(QK^T / sqrt(d)) V, no mask; sentences of <= 128 tokens in one tile, longer ones key-tiled
+        if (bb.nshort)
+            launch(lc, "bert_attn", 0, bert_attn_kernel, dim3(m.nh * bb.nshort), dim3(128), 0, (const uint16_t*)m.qkv.p, shorts, m.nh, H, scale,
+                   m.ctx.p);
+        if (bb.nlong)
+            launch(lc, "bert_attn", 0, bert_attn_long_kernel, dim3(m.nh * bb.nlong), dim3(128), 0, (const uint16_t*)m.qkv.p, longs, m.nh, H,
                    scale, m.ctx.p);
         // B5: attention output dense + bias + residual -> f32, then LayerNorm -> bf16
         launch_gemm<GEPI_BIAS_RESID_F32>(lc, "bert_gemm_o", tm_ctx, w.tm_wo, GemmArgs{T, H, H, w.bo, m.x.p, H, m.pre.p, H, 1, 0});
@@ -280,48 +291,99 @@ static void bert_enqueue(BertModel& m, int b, int t, bool has_mask) {
         launch(lc, "bert_layernorm", 0, layernorm_kernel, row_grid, row_block, 0, (const float*)m.pre.p, (const float*)w.ln2w, (const float*)w.ln2b,
                T, H, eps, m.x.p);
     }
-    // B8: masked mean pooling + L2 normalise -> f32 [b, H]
-    launch(lc, "bert_pool_l2", 0, pool_l2_kernel, dim3(b), dim3((H + 31) / 32 * 32), 0, (const uint16_t*)m.x.p,
-           has_mask ? (const uint32_t*)m.mask.p : (const uint32_t*)nullptr, t, H, m.out.p);
+    // B8: masked mean pooling + L2 normalise -> f32 [n, H]
+    launch(lc, "bert_pool_l2", 0, pool_l2_kernel, dim3(bb.n), dim3((H + 31) / 32 * 32), 0, (const uint16_t*)m.x.p,
+           use_mask && bb.mask ? (const uint32_t*)m.ids.p + T : (const uint32_t*)nullptr, starts, H, m.out.p);
 }
 
-void bert_embed(BertModel& m, const uint32_t* ids, const uint32_t* mask, int b, int t, float* out, float* device_ms) {
+// The total token count T of a batch, checked: GemmArgs and the kernels' index arithmetic are int, so T x max(3H, I) must fit in int32.
+static int bert_total_tokens(const BertModel& m, int64_t T) {
+    FL_CHECK(T * std::max(3 * m.H, m.I) <= (int64_t)INT32_MAX, FL_ERR_INVALID,
+             "batch too large: total tokens x max(3 x hidden, intermediate) must fit in int32");
+    return (int)T;
+}
+
+// One encoder pass over n packed sentences (lengths already checked, T = their sum): stage ids | mask | token positions | sentence
+// starts | attention work lists in the pinned buffer, upload them in one copy, run, read back f32 [n, H].  The work lists: a sentence of <= 128 tokens
+// is one bert_attn_kernel item, a longer one is one bert_attn_long_kernel item per 128-row query tile -- the kernel its lone fl_embed
+// uses, so its rows get the same arithmetic.  Both lists hold the sentences in order of decreasing length (most key tiles first), so
+// the longest sentences start first instead of running alone at the end of the launch.
+static void bert_run(BertModel& m, const uint32_t* ids, const uint32_t* mask, const int32_t* lengths, int n, int T, float* out) {
+    std::vector<int> order(n);
+    for (int i = 0; i < n; ++i) order[i] = i;
+    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return lengths[a] > lengths[b]; });
+    int nshort = 0, nlong = 0;
+    for (int i = 0; i < n; ++i) {
+        if (lengths[i] <= kBertS) ++nshort;
+        else nlong += (lengths[i] + kBertS - 1) / kBertS;
+    }
+    BertModel::Batch bb;
+    bb.T = T; bb.n = n; bb.nshort = nshort; bb.nlong = nlong; bb.mask = mask != nullptr;
+    bb.o_pos = (size_t)T * (mask ? 2 : 1);
+    bb.o_starts = bb.o_pos + T;
+    bb.o_short = align_up(bb.o_starts + n + 1, 4);      // BertItem: 16-byte aligned
+    bb.o_long = bb.o_short + 4 * (size_t)nshort;
+    const size_t words = bb.o_long + 4 * (size_t)nlong;
+    std::lock_guard<std::mutex> lock(m.mu);      // embed(&self) may be called from several threads: one workspace
+    bert_reserve(m, T, n, words);
+    m.batch = bb;
+    uint32_t* h = m.h_ids.p;
+    std::memcpy(h, ids, (size_t)T * 4);
+    if (mask) std::memcpy(h + T, mask, (size_t)T * 4);
+    int32_t* positions = (int32_t*)(h + bb.o_pos);
+    int32_t* starts = (int32_t*)(h + bb.o_starts);
+    starts[0] = 0;
+    for (int i = 0; i < n; ++i) {
+        starts[i + 1] = starts[i] + lengths[i];
+        for (int p = 0; p < lengths[i]; ++p) positions[starts[i] + p] = p;
+    }
+    BertItem* shorts = (BertItem*)(h + bb.o_short);
+    BertItem* longs = (BertItem*)(h + bb.o_long);
+    for (int s : order) {
+        if (lengths[s] <= kBertS) *shorts++ = BertItem{starts[s], lengths[s], 0, 0};
+        else for (int q0 = 0; q0 < lengths[s]; q0 += kBertS) *longs++ = BertItem{starts[s], lengths[s], q0, 0};
+    }
+    FL_CUDA(cudaMemcpyAsync(m.ids.p, h, words * 4, cudaMemcpyHostToDevice, m.stream));
+    bert_enqueue(m, true);
+    FL_CUDA(cudaGetLastError());
+    FL_CUDA(cudaMemcpyAsync(m.h_out.p, m.out.p, (size_t)n * m.H * 4, cudaMemcpyDeviceToHost, m.stream));
+    FL_CUDA(cudaStreamSynchronize(m.stream));
+    std::memcpy(out, m.h_out.p, (size_t)n * m.H * 4);
+}
+
+void bert_embed(BertModel& m, const uint32_t* ids, const uint32_t* mask, int b, int t, float* out) {
     FL_CHECK(m.finalized, FL_ERR_STATE, "model not finalized");
     FL_CHECK(ids && out && b >= 1 && t >= 1, FL_ERR_INVALID, "bad arguments");
     // the reference enforces no max_seq_length (embeddings.rs:285-286); what bounds a sentence is its position table: position ids
     // 0..n index a [max_position_embeddings, H] embedding (embeddings.rs:416, 370-378), and candle's index_select fails past it
     FL_CHECK(t <= m.maxpos, FL_ERR_INVALID, "sentence longer than max_position_embeddings (the position-embedding lookup fails in the reference too)");
-    for (int i = 0; i < b * t; ++i) FL_CHECK(ids[i] < (uint32_t)m.V, FL_ERR_INVALID, "token id out of range");
-    std::lock_guard<std::mutex> lock(m.mu);      // embed(&self) may be called from several threads: one workspace
-    bert_reserve(m, b, t);
-    const size_t T = (size_t)b * t;
-    std::memcpy(m.h_ids.p, ids, T * 4);
-    FL_CUDA(cudaMemcpyAsync(m.ids.p, m.h_ids.p, T * 4, cudaMemcpyHostToDevice, m.stream));
-    if (mask) {
-        std::memcpy(m.h_ids.p + T, mask, T * 4);
-        FL_CUDA(cudaMemcpyAsync(m.mask.p, m.h_ids.p + T, T * 4, cudaMemcpyHostToDevice, m.stream));
-    }
-    std::unique_ptr<EventPair> ev;
-    if (device_ms) {
-        ev.reset(new EventPair);
-        FL_CUDA(cudaEventRecord(ev->e0, m.stream));
-    }
-    bert_enqueue(m, b, t, mask != nullptr);
-    if (device_ms) FL_CUDA(cudaEventRecord(ev->e1, m.stream));
-    FL_CUDA(cudaGetLastError());
-    FL_CUDA(cudaMemcpyAsync(m.h_out.p, m.out.p, (size_t)b * m.H * 4, cudaMemcpyDeviceToHost, m.stream));
-    FL_CUDA(cudaStreamSynchronize(m.stream));
-    std::memcpy(out, m.h_out.p, (size_t)b * m.H * 4);
-    if (device_ms) FL_CUDA(cudaEventElapsedTime(device_ms, ev->e0, ev->e1));
+    const int T = bert_total_tokens(m, (int64_t)b * t);
+    for (int i = 0; i < T; ++i) FL_CHECK(ids[i] < (uint32_t)m.V, FL_ERR_INVALID, "token id out of range");
+    const std::vector<int32_t> lengths(b, t);
+    bert_run(m, ids, mask, lengths.data(), b, T, out);
 }
 
-// Device-resident repeat of the encoder on the ids already uploaded by the last bert_embed (benchmark `value`).
+void bert_embed_packed(BertModel& m, const uint32_t* ids, const int32_t* lengths, int n, float* out) {
+    FL_CHECK(m.finalized, FL_ERR_STATE, "model not finalized");
+    FL_CHECK(ids && lengths && out && n >= 1, FL_ERR_INVALID, "bad arguments");
+    int64_t total = 0;
+    for (int i = 0; i < n; ++i) {
+        FL_CHECK(lengths[i] >= 1, FL_ERR_INVALID, "bad arguments");
+        FL_CHECK(lengths[i] <= m.maxpos, FL_ERR_INVALID, "sentence longer than max_position_embeddings (the position-embedding lookup fails in the reference too)");
+        total += lengths[i];
+    }
+    const int T = bert_total_tokens(m, total);
+    for (int i = 0; i < T; ++i) FL_CHECK(ids[i] < (uint32_t)m.V, FL_ERR_INVALID, "token id out of range");
+    bert_run(m, ids, nullptr, lengths, n, T, out);
+}
+
+// Device-resident repeat of the encoder on the batch the last bert_embed uploaded (benchmark `value`).
 void bert_repeat(BertModel& m, int b, int t, int iters, float* elapsed_ms) {
     std::lock_guard<std::mutex> lock(m.mu);
-    FL_CHECK((size_t)b * t <= m.cap_tokens, FL_ERR_STATE, "call fl_embed with this shape first");
+    FL_CHECK(m.batch.n == b && m.batch.T == (int64_t)b * t, FL_ERR_STATE, "call fl_embed with this shape first");
     EventPair ev;
     FL_CUDA(cudaEventRecord(ev.e0, m.stream));
-    for (int i = 0; i < iters; ++i) bert_enqueue(m, b, t, false);
+    for (int i = 0; i < iters; ++i) bert_enqueue(m, false);
     FL_CUDA(cudaEventRecord(ev.e1, m.stream));
     FL_CUDA(cudaStreamSynchronize(m.stream));
     FL_CUDA(cudaGetLastError());

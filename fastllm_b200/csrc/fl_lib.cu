@@ -1810,7 +1810,16 @@ FL_EXPORT int fl_embed(fl_model* m, const uint32_t* ids, const uint32_t* mask, i
     FL_CHECK(m && ids && out, FL_ERR_INVALID, "NULL argument");
     FL_CHECK(m->bert != nullptr, FL_ERR_INVALID, "fl_embed needs a BERT-family model (the reference panics on embedding_size() of chat models, models/mod.rs:97-106)");
     use_device();
-    bert_embed(*m->bert, ids, mask, b, t, out, nullptr);
+    bert_embed(*m->bert, ids, mask, b, t, out);
+    FL_API_END
+}
+
+FL_EXPORT int fl_embed_packed(fl_model* m, const uint32_t* ids, const int32_t* lengths, int n, float* out) {
+    FL_API_BEGIN
+    FL_CHECK(m && ids && lengths && out, FL_ERR_INVALID, "NULL argument");
+    FL_CHECK(m->bert != nullptr, FL_ERR_INVALID, "fl_embed_packed needs a BERT-family model (the reference panics on embedding_size() of chat models, models/mod.rs:97-106)");
+    use_device();
+    bert_embed_packed(*m->bert, ids, lengths, n, out);
     FL_API_END
 }
 
@@ -1819,7 +1828,7 @@ FL_EXPORT int fl_embed_timed(fl_model* m, const uint32_t* ids, const uint32_t* m
     FL_CHECK(m && ids && out && device_ms, FL_ERR_INVALID, "NULL argument");
     FL_CHECK(m->bert != nullptr, FL_ERR_INVALID, "fl_embed_timed needs a BERT-family model");
     use_device();
-    bert_embed(*m->bert, ids, mask, b, t, out, nullptr);
+    bert_embed(*m->bert, ids, mask, b, t, out);
     bert_repeat(*m->bert, b, t, repeats < 1 ? 1 : repeats, device_ms);
     FL_API_END
 }

@@ -699,6 +699,20 @@ class MiniLMModel:
                 out[chunk] = self.embed_ids(np.asarray([sentences[i] for i in chunk], dtype=np.uint32))
         return out
 
+    def embed_packed(self, sentences) -> np.ndarray:
+        """`input: [String]` in ONE encoder pass (fl_embed_packed): the sentences (1-D id sequences of any lengths) are concatenated
+        without padding, and row i equals embed_ids of sentence i alone bit for bit.  Returns f32 [len(sentences), hidden] in request
+        order."""
+        out = np.empty((len(sentences), self.config.hidden_size), dtype=np.float32)
+        if not len(sentences):
+            return out
+        parts = [np.asarray(s, dtype=np.uint32).reshape(-1) for s in sentences]
+        ids = np.ascontiguousarray(np.concatenate(parts), dtype=np.uint32)
+        lengths = np.array([len(p) for p in parts], dtype=np.int32)
+        _lib.check(self.dev.lib.fl_embed_packed(self.dev.h, ids.ctypes.data_as(C.c_void_p), lengths.ctypes.data_as(C.c_void_p),
+                                                len(parts), out.ctypes.data_as(C.c_void_p)))
+        return out
+
     def embed_ids_timed(self, ids: np.ndarray, repeats: int):
         """-> (embeddings, device ms for `repeats` device-resident encoder passes over the uploaded batch)."""
         ids = np.ascontiguousarray(ids, dtype=np.uint32)

@@ -336,6 +336,23 @@ struct MiniLMModel {
             }
         return out;
     }
+    // `input: [String]` in ONE encoder pass (fl_embed_packed): the sentences are concatenated without padding; row i equals
+    // embed_ids of sentence i alone bit for bit; rows come back in request order
+    std::vector<std::vector<float>> embed_packed(const std::vector<std::vector<uint32_t>>& sentences) const {
+        if (sentences.empty()) return {};
+        std::vector<uint32_t> ids;
+        std::vector<int32_t> lengths;
+        for (const auto& s : sentences) {
+            ids.insert(ids.end(), s.begin(), s.end());
+            lengths.push_back((int32_t)s.size());
+        }
+        const size_t H = embedding_size();
+        std::vector<float> e(sentences.size() * H);
+        check(fl_embed_packed(dev->h, ids.data(), lengths.data(), (int)sentences.size(), e.data()));
+        std::vector<std::vector<float>> out(sentences.size());
+        for (size_t i = 0; i < out.size(); ++i) out[i].assign(e.begin() + i * H, e.begin() + (i + 1) * H);
+        return out;
+    }
 };
 
 }  // namespace fastllm

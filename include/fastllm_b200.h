@@ -32,6 +32,9 @@
  *                                are serialised at batch 1, api/chat.rs:206-208; streams run side by side, models/mod.rs:151-175)
  *   fl_embed                  <- EmbeddingModel::embed models/embeddings.rs:397-447 after tokenisation:
  *                                encoder forward + mean_pooling (:346-368) + normalize_l2 (:341-344)
+ *   fl_embed_packed           <- the same embed for a batch of sentences of different lengths in ONE encoder pass (no reference
+ *                                counterpart: api/embeddings.rs takes one string per request); row i is what embed returns for
+ *                                sentence i alone
  */
 #ifndef FASTLLM_B200_H
 #define FASTLLM_B200_H
@@ -181,6 +184,12 @@ FL_EXPORT int fl_forward_sample_device(fl_model* m, fl_cache* c, const uint32_t*
 /* ---- embeddings (BERT family) ------------------------------------------------------------------ */
 /* ids/mask: host u32 [b, t]; mask may be NULL (all ones).  out: host f32 [b, hidden], mean-pooled and L2-normalised. */
 FL_EXPORT int fl_embed(fl_model* m, const uint32_t* ids, const uint32_t* mask, int b, int t, float* out);
+/* Sentences of different lengths in ONE encoder pass, no padding: sentence i is ids[o_i, o_i + lengths[i]) with
+ * o_i = lengths[0] + ... + lengths[i-1]; every token of a sentence is pooled (the all-ones mask a lone sentence has).
+ * out: host f32 [n, hidden].  Row i equals fl_embed(m, ids + o_i, NULL, 1, lengths[i], ...) bit for bit.
+ * FL_ERR_INVALID for a NULL pointer, n < 1, a non-BERT model, a length < 1 or > max_position_embeddings, an id >= vocab, or a
+ * total token count T with T x max(3 x hidden, intermediate) > INT32_MAX; all are rejected before any device work. */
+FL_EXPORT int fl_embed_packed(fl_model* m, const uint32_t* ids, const int32_t* lengths, int n, float* out);
 /* Benchmark hook: one fl_embed, then `repeats` device-resident encoder passes over the same (already uploaded) batch;
  * device_ms = CUDA-event time of those repeats on the model's stream. */
 FL_EXPORT int fl_embed_timed(fl_model* m, const uint32_t* ids, const uint32_t* mask, int b, int t, float* out, int repeats, float* device_ms);
