@@ -9,6 +9,7 @@
 // sentences.  A uniform [b, t] batch is the case starts[s] = s * t.  The attention kernels take a work list of BertItem.
 // The sentence tables (positions, starts, items) are written by the host upload that precedes the encoder's first kernel and by
 // no kernel, so every kernel reads them BEFORE pdl_wait: their load latency overlaps the previous kernel's tail.
+// Shapes: head_dim 32 or 64 (the attention kernels' template parameter), hidden a multiple of 64 and <= 1024.
 #pragma once
 #include "common.cuh"
 #include "mma.cuh"
@@ -21,7 +22,8 @@ struct __align__(16) BertItem {
     int row0, len, q0, pad;
 };
 
-// One warp per token row; H multiple of 32*... generic loop.  out bf16 [T, H].
+// One warp per token row, PER values per lane: H <= 32 * PER (PER = 16 up to hidden 512, 32 up to 1024).  out bf16 [T, H].
+template <int PER>
 static __global__ void embed_ln_kernel(const uint16_t* __restrict__ wemb, const uint16_t* __restrict__ pemb, const float* __restrict__ lnw,
                                 const float* __restrict__ lnb, const uint32_t* __restrict__ ids, const int* __restrict__ positions, int T,
                                 int H, int vocab, int maxpos, float eps, uint16_t* __restrict__ out) {
@@ -35,11 +37,11 @@ static __global__ void embed_ln_kernel(const uint16_t* __restrict__ wemb, const 
     if (pos >= maxpos) pos = maxpos - 1;
     const uint16_t* w = wemb + (size_t)id * H;
     const uint16_t* p = pemb + (size_t)pos * H;
-    float v[16];                             // H <= 512 per warp (32 lanes x 16)
+    float v[PER];
     float s = 0.f, s2 = 0.f;
     const int per = (H + 31) / 32;
 #pragma unroll
-    for (int j = 0; j < 16; ++j) {
+    for (int j = 0; j < PER; ++j) {
         const int c = lane + 32 * j;
         v[j] = 0.f;
         if (j < per && c < H) {
@@ -53,13 +55,15 @@ static __global__ void embed_ln_kernel(const uint16_t* __restrict__ wemb, const 
     const float mean = s / (float)H;
     const float inv = 1.f / sqrtf(s2 / (float)H - mean * mean + eps);
 #pragma unroll
-    for (int j = 0; j < 16; ++j) {
+    for (int j = 0; j < PER; ++j) {
         const int c = lane + 32 * j;
         if (j < per && c < H) out[(size_t)row * H + c] = f32_to_bf16_rne((v[j] - mean) * inv * lnw[c] + lnb[c]);
     }
 }
 
-// LayerNorm over f32 rows [T, H] -> bf16 [T, H]; one warp per row, 128-bit loads / 64-bit stores (H % 4 == 0, H <= 512).
+// LayerNorm over f32 rows [T, H] -> bf16 [T, H]; one warp per row, V4 float4 per lane, 128-bit loads / 64-bit stores
+// (H % 4 == 0, H <= 128 * V4: V4 = 4 up to hidden 512, 8 up to 1024).
+template <int V4>
 static __global__ void layernorm_kernel(const float* __restrict__ x, const float* __restrict__ lnw, const float* __restrict__ lnb, int T, int H,
                                  float eps, uint16_t* __restrict__ out) {
     pdl_launch_dependents();      // programmatic dependent launch: the next kernel may start its prologue now ...
@@ -68,10 +72,10 @@ static __global__ void layernorm_kernel(const float* __restrict__ x, const float
     if (row >= T) return;
     const float4* xr = reinterpret_cast<const float4*>(x + (size_t)row * H);
     const int H4 = H >> 2;
-    float4 v[4];
+    float4 v[V4];
     float s = 0.f, s2 = 0.f;
 #pragma unroll
-    for (int j = 0; j < 4; ++j) {
+    for (int j = 0; j < V4; ++j) {
         const int c = lane + 32 * j;
         v[j] = make_float4(0.f, 0.f, 0.f, 0.f);
         if (c < H4) {
@@ -86,7 +90,7 @@ static __global__ void layernorm_kernel(const float* __restrict__ x, const float
     const float inv = 1.f / sqrtf(s2 / (float)H - mean * mean + eps);
     uint2* orow = reinterpret_cast<uint2*>(out + (size_t)row * H);
 #pragma unroll
-    for (int j = 0; j < 4; ++j) {
+    for (int j = 0; j < V4; ++j) {
         const int c = lane + 32 * j;
         if (c < H4) {
             const float4 w4 = reinterpret_cast<const float4*>(lnw)[c], b4 = reinterpret_cast<const float4*>(lnb)[c];
@@ -96,35 +100,58 @@ static __global__ void layernorm_kernel(const float* __restrict__ x, const float
     }
 }
 
-// ---- fused small-head attention (t <= 128, d = 32) on mma.sync m16n8k16 bf16 ------------------------------------------
+// ---- fused attention (head_dim D = 32 or 64) on mma.sync m16n8k16 bf16 ----------------------------------------------------
 constexpr int kBertS = 128;      // query / key rows per tile (a sentence of <= 128 tokens is ONE tile: bert_attn_kernel)
-constexpr int kBertD = 32;       // head dim
-constexpr int kBertLd = 40;      // padded smem row (80 bytes): conflict-free ldmatrix
+
+// Q | K | V staging of one attention CTA: 3 x 128 rows of D + 8 bf16.  The 8-element pad makes the row 80 bytes (D = 32) or 144
+// bytes (D = 64), so the 8 rows one ldmatrix phase reads fall in distinct bank groups.  30 720 bytes at D = 32 are three static
+// arrays; 55 296 bytes at D = 64 exceed the 48 KB static limit and are dynamic (launched with bert_attn_dyn_smem(64) bytes).
+template <int D>
+constexpr int bert_attn_ld() { return D + 8; }
+constexpr size_t bert_attn_dyn_smem(int d) { return d == 32 ? 0 : (size_t)3 * kBertS * (d + 8) * 2; }
+
+struct BertAttnStage {
+    uint16_t *q, *k, *v;
+};
+template <int D>
+static __device__ __forceinline__ BertAttnStage bert_attn_stage() {
+    static_assert(D == 32 || D == 64, "BERT attention is built for head_dim 32 and 64");
+    constexpr int n = kBertS * bert_attn_ld<D>();
+    if constexpr (D == 32) {
+        __shared__ __align__(16) uint16_t sq[n], sk[n], sv[n];
+        return {sq, sk, sv};
+    } else {
+        extern __shared__ __align__(16) uint16_t bert_attn_dyn[];
+        return {bert_attn_dyn, bert_attn_dyn + n, bert_attn_dyn + 2 * n};
+    }
+}
 
 // grid (heads x items), head fastest; 128 threads: warp w owns query rows [32w, 32w+32).  qkv bf16 [T, 3H] (q | k | v), ctx bf16 [T, H].
+template <int D>
 static __global__ void __launch_bounds__(128) bert_attn_kernel(const uint16_t* __restrict__ qkv, const BertItem* __restrict__ items, int nh,
                                                                int H, float scale, uint16_t* __restrict__ ctx) {
+    constexpr int LD = bert_attn_ld<D>(), KS = D / 16, DT = D / 8;      // row pitch; k16 steps of Q K^T; 8-column output tiles of P V
     pdl_launch_dependents();      // programmatic dependent launch: the next kernel may start its prologue now ...
     const BertItem it = items[blockIdx.x / nh];      // a sentence table
     pdl_wait();                   // ... and nothing below runs before the previous kernel has completed
-    __shared__ __align__(16) uint16_t sq[kBertS * kBertLd], sk[kBertS * kBertLd], sv[kBertS * kBertLd];
+    const auto [sq, sk, sv] = bert_attn_stage<D>();
     const int head = blockIdx.x % nh, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const size_t row0 = (size_t)it.row0;
     const int t = it.len;
     const int ld = 3 * H;
-    // stage Q, K, V of this (sentence, head): 128 rows x 32 bf16 (64 B) each; rows >= t are zero
-    for (int i = tid; i < kBertS * 4; i += 128) {
-        const int r = i >> 2, c = (i & 3) * 8;
+    // stage Q, K, V of this (sentence, head): 128 rows x D bf16 each, in 16-byte chunks; rows >= t are zero
+    for (int i = tid; i < kBertS * DT; i += 128) {
+        const int r = i / DT, c = (i % DT) * 8;
         uint4 q = make_uint4(0, 0, 0, 0), k = q, v = q;
         if (r < t) {
-            const uint16_t* src = qkv + (row0 + r) * ld + head * kBertD + c;
+            const uint16_t* src = qkv + (row0 + r) * ld + head * D + c;
             q = *reinterpret_cast<const uint4*>(src);
             k = *reinterpret_cast<const uint4*>(src + H);
             v = *reinterpret_cast<const uint4*>(src + 2 * H);
         }
-        *reinterpret_cast<uint4*>(sq + r * kBertLd + c) = q;
-        *reinterpret_cast<uint4*>(sk + r * kBertLd + c) = k;
-        *reinterpret_cast<uint4*>(sv + r * kBertLd + c) = v;
+        *reinterpret_cast<uint4*>(sq + r * LD + c) = q;
+        *reinterpret_cast<uint4*>(sk + r * LD + c) = k;
+        *reinterpret_cast<uint4*>(sv + r * LD + c) = v;
     }
     __syncthreads();
     const int g = lane >> 2, tq = lane & 3;
@@ -132,24 +159,24 @@ static __global__ void __launch_bounds__(128) bert_attn_kernel(const uint16_t* _
     for (int mt = 0; mt < 2; ++mt) {
         const int m0 = warp * 32 + mt * 16;
         if (m0 >= t) break;
-        // A fragments of Q: 16 rows x 32 (two k16 steps)
-        uint32_t qa[2][4];
+        // A fragments of Q: 16 rows x D (KS k16 steps)
+        uint32_t qa[KS][4];
 #pragma unroll
-        for (int ks = 0; ks < 2; ++ks) ldmatrix_x4(qa[ks], sq + (m0 + (lane & 15)) * kBertLd + ks * 16 + (lane >> 4) * 8);
+        for (int ks = 0; ks < KS; ++ks) ldmatrix_x4(qa[ks], sq + (m0 + (lane & 15)) * LD + ks * 16 + (lane >> 4) * 8);
         // S = Q K^T : 16 key tiles of 8
         float s[16][4];
 #pragma unroll
         for (int nt = 0; nt < 16; ++nt) {
             s[nt][0] = s[nt][1] = s[nt][2] = s[nt][3] = 0.f;
 #pragma unroll
-            for (int ks = 0; ks < 2; ++ks) {
+            for (int ks = 0; ks < KS; ++ks) {
                 uint32_t kb[2];
-                ldmatrix_x2(kb, sk + (nt * 8 + (lane & 7)) * kBertLd + ks * 16 + ((lane >> 3) & 1) * 8);
+                ldmatrix_x2(kb, sk + (nt * 8 + (lane & 7)) * LD + ks * 16 + ((lane >> 3) & 1) * 8);
                 mma_bf16_16816(s[nt], qa[ks], kb);
             }
         }
         // scores / sqrt(d) (after the matmul, embeddings.rs:155-159), softmax over keys < t; rows g and g+8
-        // (the reference divides by sqrt(d); sqrt(32) is not a power of two, so x * (1/sqrt(d)) differs by <= 1 ulp)
+        // (the reference divides by sqrt(d); sqrt(32) is not a power of two, so x * (1/sqrt(d)) differs by <= 1 ulp; at d = 64 it is exact)
         const float inv_scale = 1.f / scale;
         float mx0 = -INFINITY, mx1 = -INFINITY;
 #pragma unroll
@@ -175,9 +202,9 @@ static __global__ void __launch_bounds__(128) bert_attn_kernel(const uint16_t* _
         sum0 += __shfl_xor_sync(0xFFFFFFFFu, sum0, 1); sum0 += __shfl_xor_sync(0xFFFFFFFFu, sum0, 2);
         sum1 += __shfl_xor_sync(0xFFFFFFFFu, sum1, 1); sum1 += __shfl_xor_sync(0xFFFFFFFFu, sum1, 2);
         // O = P V : the S accumulator layout of key tiles (2j, 2j+1) is exactly the A fragment of k16 step j
-        float o[4][4];
+        float o[DT][4];
 #pragma unroll
-        for (int dt = 0; dt < 4; ++dt) o[dt][0] = o[dt][1] = o[dt][2] = o[dt][3] = 0.f;
+        for (int dt = 0; dt < DT; ++dt) o[dt][0] = o[dt][1] = o[dt][2] = o[dt][3] = 0.f;
 #pragma unroll
         for (int ks = 0; ks < 8; ++ks) {
             uint32_t pa[4];
@@ -186,17 +213,17 @@ static __global__ void __launch_bounds__(128) bert_attn_kernel(const uint16_t* _
             pa[2] = pack_bf16(s[2 * ks + 1][0], s[2 * ks + 1][1]);
             pa[3] = pack_bf16(s[2 * ks + 1][2], s[2 * ks + 1][3]);
 #pragma unroll
-            for (int dt = 0; dt < 4; ++dt) {
+            for (int dt = 0; dt < DT; ++dt) {
                 uint32_t vb[2];
-                ldmatrix_x2_trans(vb, sv + (ks * 16 + (lane & 15)) * kBertLd + dt * 8);
+                ldmatrix_x2_trans(vb, sv + (ks * 16 + (lane & 15)) * LD + dt * 8);
                 mma_bf16_16816(o[dt], pa, vb);
             }
         }
         const float i0 = 1.f / sum0, i1 = 1.f / sum1;
         const int r0 = m0 + g, r1 = m0 + g + 8;
 #pragma unroll
-        for (int dt = 0; dt < 4; ++dt) {
-            const int c = head * kBertD + dt * 8 + tq * 2;
+        for (int dt = 0; dt < DT; ++dt) {
+            const int c = head * D + dt * 8 + tq * 2;
             if (r0 < t) *reinterpret_cast<uint32_t*>(ctx + (row0 + r0) * H + c) = pack_bf16(o[dt][0] * i0, o[dt][1] * i0);
             if (r1 < t) *reinterpret_cast<uint32_t*>(ctx + (row0 + r1) * H + c) = pack_bf16(o[dt][2] * i1, o[dt][3] * i1);
         }
@@ -207,48 +234,50 @@ static __global__ void __launch_bounds__(128) bert_attn_kernel(const uint16_t* _
 // embeddings.rs:285-286): the same attention, FlashAttention-style.  grid (heads x (sentence, query tile) items), 128 threads;
 // a CTA stages its 128 query rows once and walks the sentence's keys in 128-row tiles with an online softmax (running max / sum per
 // row, accumulator rescaled when the max moves) -- algebraically the reference's max-subtract / exp / sum / div over all keys.
+template <int D>
 static __global__ void __launch_bounds__(128) bert_attn_long_kernel(const uint16_t* __restrict__ qkv, const BertItem* __restrict__ items,
                                                                     int nh, int H, float scale, uint16_t* __restrict__ ctx) {
+    constexpr int LD = bert_attn_ld<D>(), KS = D / 16, DT = D / 8;
     pdl_launch_dependents();      // programmatic dependent launch: the next kernel may start its prologue now ...
     const BertItem it = items[blockIdx.x / nh];      // a sentence table
     pdl_wait();                   // ... and nothing below runs before the previous kernel has completed
-    __shared__ __align__(16) uint16_t sq[kBertS * kBertLd], sk[kBertS * kBertLd], sv[kBertS * kBertLd];
+    const auto [sq, sk, sv] = bert_attn_stage<D>();
     const int head = blockIdx.x % nh, q0 = it.q0, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const size_t row0 = (size_t)it.row0;
     const int t = it.len;
     const int ld = 3 * H;
-    for (int i = tid; i < kBertS * 4; i += 128) {
-        const int r = i >> 2, c = (i & 3) * 8;
+    for (int i = tid; i < kBertS * DT; i += 128) {
+        const int r = i / DT, c = (i % DT) * 8;
         uint4 q = make_uint4(0, 0, 0, 0);
-        if (q0 + r < t) q = *reinterpret_cast<const uint4*>(qkv + (row0 + q0 + r) * ld + head * kBertD + c);
-        *reinterpret_cast<uint4*>(sq + r * kBertLd + c) = q;
+        if (q0 + r < t) q = *reinterpret_cast<const uint4*>(qkv + (row0 + q0 + r) * ld + head * D + c);
+        *reinterpret_cast<uint4*>(sq + r * LD + c) = q;
     }
     __syncthreads();
     const int g = lane >> 2, tq = lane & 3;
     const float inv_scale = 1.f / scale;
-    uint32_t qa[2][2][4];
-    float o[2][4][4], mrun[2][2], lrun[2][2];
+    uint32_t qa[2][KS][4];
+    float o[2][DT][4], mrun[2][2], lrun[2][2];
 #pragma unroll
     for (int mt = 0; mt < 2; ++mt) {
 #pragma unroll
-        for (int ks = 0; ks < 2; ++ks) ldmatrix_x4(qa[mt][ks], sq + (warp * 32 + mt * 16 + (lane & 15)) * kBertLd + ks * 16 + (lane >> 4) * 8);
+        for (int ks = 0; ks < KS; ++ks) ldmatrix_x4(qa[mt][ks], sq + (warp * 32 + mt * 16 + (lane & 15)) * LD + ks * 16 + (lane >> 4) * 8);
 #pragma unroll
-        for (int dt = 0; dt < 4; ++dt) o[mt][dt][0] = o[mt][dt][1] = o[mt][dt][2] = o[mt][dt][3] = 0.f;
+        for (int dt = 0; dt < DT; ++dt) o[mt][dt][0] = o[mt][dt][1] = o[mt][dt][2] = o[mt][dt][3] = 0.f;
         mrun[mt][0] = mrun[mt][1] = -INFINITY;
         lrun[mt][0] = lrun[mt][1] = 0.f;
     }
     for (int k0 = 0; k0 < t; k0 += kBertS) {
         __syncthreads();      // the previous key tile is no longer being read
-        for (int i = tid; i < kBertS * 4; i += 128) {
-            const int r = i >> 2, c = (i & 3) * 8;
+        for (int i = tid; i < kBertS * DT; i += 128) {
+            const int r = i / DT, c = (i % DT) * 8;
             uint4 k = make_uint4(0, 0, 0, 0), v = k;
             if (k0 + r < t) {
-                const uint16_t* src = qkv + (row0 + k0 + r) * ld + head * kBertD + c;
+                const uint16_t* src = qkv + (row0 + k0 + r) * ld + head * D + c;
                 k = *reinterpret_cast<const uint4*>(src + H);
                 v = *reinterpret_cast<const uint4*>(src + 2 * H);
             }
-            *reinterpret_cast<uint4*>(sk + r * kBertLd + c) = k;
-            *reinterpret_cast<uint4*>(sv + r * kBertLd + c) = v;
+            *reinterpret_cast<uint4*>(sk + r * LD + c) = k;
+            *reinterpret_cast<uint4*>(sv + r * LD + c) = v;
         }
         __syncthreads();
 #pragma unroll
@@ -259,9 +288,9 @@ static __global__ void __launch_bounds__(128) bert_attn_long_kernel(const uint16
             for (int nt = 0; nt < 16; ++nt) {
                 s[nt][0] = s[nt][1] = s[nt][2] = s[nt][3] = 0.f;
 #pragma unroll
-                for (int ks = 0; ks < 2; ++ks) {
+                for (int ks = 0; ks < KS; ++ks) {
                     uint32_t kb[2];
-                    ldmatrix_x2(kb, sk + (nt * 8 + (lane & 7)) * kBertLd + ks * 16 + ((lane >> 3) & 1) * 8);
+                    ldmatrix_x2(kb, sk + (nt * 8 + (lane & 7)) * LD + ks * 16 + ((lane >> 3) & 1) * 8);
                     mma_bf16_16816(s[nt], qa[mt][ks], kb);
                 }
             }
@@ -292,7 +321,7 @@ static __global__ void __launch_bounds__(128) bert_attn_long_kernel(const uint16
             lrun[mt][0] = lrun[mt][0] * al0 + ps0;      // per-thread partial row sums; the quad is reduced once at the end
             lrun[mt][1] = lrun[mt][1] * al1 + ps1;
 #pragma unroll
-            for (int dt = 0; dt < 4; ++dt) {
+            for (int dt = 0; dt < DT; ++dt) {
                 o[mt][dt][0] *= al0; o[mt][dt][1] *= al0; o[mt][dt][2] *= al1; o[mt][dt][3] *= al1;
             }
 #pragma unroll
@@ -303,9 +332,9 @@ static __global__ void __launch_bounds__(128) bert_attn_long_kernel(const uint16
                 pa[2] = pack_bf16(s[2 * ks + 1][0], s[2 * ks + 1][1]);
                 pa[3] = pack_bf16(s[2 * ks + 1][2], s[2 * ks + 1][3]);
 #pragma unroll
-                for (int dt = 0; dt < 4; ++dt) {
+                for (int dt = 0; dt < DT; ++dt) {
                     uint32_t vb[2];
-                    ldmatrix_x2_trans(vb, sv + (ks * 16 + (lane & 15)) * kBertLd + dt * 8);
+                    ldmatrix_x2_trans(vb, sv + (ks * 16 + (lane & 15)) * LD + dt * 8);
                     mma_bf16_16816(o[mt][dt], pa, vb);
                 }
             }
@@ -321,8 +350,8 @@ static __global__ void __launch_bounds__(128) bert_attn_long_kernel(const uint16
         const float i0 = 1.f / l0, i1 = 1.f / l1;
         const int r0 = m0 + g, r1 = m0 + g + 8;
 #pragma unroll
-        for (int dt = 0; dt < 4; ++dt) {
-            const int c = head * kBertD + dt * 8 + tq * 2;
+        for (int dt = 0; dt < DT; ++dt) {
+            const int c = head * D + dt * 8 + tq * 2;
             if (r0 < t) *reinterpret_cast<uint32_t*>(ctx + (row0 + r0) * H + c) = pack_bf16(o[mt][dt][0] * i0, o[mt][dt][1] * i0);
             if (r1 < t) *reinterpret_cast<uint32_t*>(ctx + (row0 + r1) * H + c) = pack_bf16(o[mt][dt][2] * i1, o[mt][dt][3] * i1);
         }

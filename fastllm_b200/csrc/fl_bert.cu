@@ -31,7 +31,9 @@ static EncodeTiledFn encode_tiled_fn() {
 // Output-tile width of the encoder GEMMs.  With hidden = 384 every GEMM of the model has K-major operands of equal depth, so a
 // 128 x BN tile moves (128 + BN) * K * 2 bytes from L2 for 2 * 128 * BN * K FLOP: 64 FLOP/B at BN = 128 -- L2->SM bound
 // (~7 TB/s chip-wide => ~450 TFLOP/s) long before the tensor pipe.  BN = 192 divides all three widths (1152, 384, 1536), lifts
-// the intensity to 77 FLOP/B and still fits two TMEM accumulator stages (2 x 256 columns).
+// the intensity to 77 FLOP/B and still fits two TMEM accumulator stages (2 x 256 columns).  It also divides every width at hidden
+// 768 (2304, 768, 3072); at hidden 1024, N = 1024 and 4096 end in a partial tile (TMA zero-fills the dead weight rows, the epilogue
+// stores col < N only).  One width for every model, no split-K: a row's sums never depend on the other rows in the batch.
 constexpr int kBertBN = 192;
 
 CUtensorMap make_tmap_bf16(const void* ptr, uint64_t rows, uint64_t cols, uint64_t ld, uint32_t box_rows) {
@@ -98,8 +100,12 @@ void bert_build(BertModel& m) {
     m.H = c.hidden_size; m.I = c.intermediate_size; m.V = c.vocab_size; m.L = c.num_hidden_layers; m.nh = c.num_attention_heads;
     m.d = m.H / m.nh; m.maxpos = c.max_position_embeddings;
     FL_CHECK(m.d * m.nh == m.H, FL_ERR_INVALID, "hidden_size must be divisible by num_attention_heads");
-    FL_CHECK(m.d == kBertD, FL_ERR_UNSUPPORTED, "BERT path is built for head_dim 32 (all-MiniLM-L6-v2); other head sizes not built yet");
-    FL_CHECK(m.H % 64 == 0 && m.I % 64 == 0 && m.H <= 512, FL_ERR_UNSUPPORTED, "BERT path needs hidden/intermediate % 64 == 0 and hidden <= 512");
+    // head_dim: the attention kernels are built for 32 (all-MiniLM-L6-v2) and 64 (BERT-base / -large, e5, gte); the GEMMs take
+    // K and N in 64-column blocks; the LayerNorm kernels hold a row in one warp and pool_l2_kernel a row in one CTA: hidden <= 1024
+    FL_CHECK(m.d == 32 || m.d == 64, FL_ERR_UNSUPPORTED,
+             "BERT path is built for head_dim 32 and 64 (hidden_size / num_attention_heads = " + std::to_string(m.d) + ")");
+    FL_CHECK(m.H % 64 == 0 && m.I % 64 == 0, FL_ERR_UNSUPPORTED, "BERT path needs hidden_size and intermediate_size to be multiples of 64");
+    FL_CHECK(m.H <= 1024, FL_ERR_UNSUPPORTED, "BERT path is built for hidden_size <= 1024");
     const size_t H = m.H, I = m.I;
     size_t off = 0;
     auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
@@ -261,9 +267,17 @@ static void bert_enqueue(BertModel& m, bool use_mask) {
     const BertItem* shorts = (const BertItem*)(m.ids.p + bb.o_short);
     const BertItem* longs = (const BertItem*)(m.ids.p + bb.o_long);
     LaunchCtx lc{m.stream};
+    // the model's kernel instantiations (bert_build admits head_dim 32 / 64 and hidden <= 1024); rows of up to 512 columns take the
+    // narrow LayerNorm kernels, which hold 16 values per lane instead of 32
+    const bool wide = H > 512;
+    const auto embed_ln = wide ? embed_ln_kernel<32> : embed_ln_kernel<16>;
+    const auto layernorm = wide ? layernorm_kernel<8> : layernorm_kernel<4>;
+    const auto attn = m.d == 64 ? bert_attn_kernel<64> : bert_attn_kernel<32>;
+    const auto attn_long = m.d == 64 ? bert_attn_long_kernel<64> : bert_attn_long_kernel<32>;
+    const size_t attn_smem = bert_attn_dyn_smem(m.d);
     const int rows_per_cta = 8;
     const dim3 row_grid((T + rows_per_cta - 1) / rows_per_cta), row_block(rows_per_cta * 32);
-    launch(lc, "bert_embed_ln", 0, embed_ln_kernel, row_grid, row_block, 0, (const uint16_t*)m.wemb, (const uint16_t*)m.pemb, (const float*)m.lnw,
+    launch(lc, "bert_embed_ln", 0, embed_ln, row_grid, row_block, 0, (const uint16_t*)m.wemb, (const uint16_t*)m.pemb, (const float*)m.lnw,
            (const float*)m.lnb, (const uint32_t*)m.ids.p, positions, T, H, m.V, m.maxpos, 1e-12f, m.x.p);
     const CUtensorMap tm_x = make_tmap_bf16(m.x.p, T, H, H, kGemmBM), tm_x1 = make_tmap_bf16(m.x1.p, T, H, H, kGemmBM),
                       tm_ctx = make_tmap_bf16(m.ctx.p, T, H, H, kGemmBM), tm_h = make_tmap_bf16(m.hbuf.p, T, I, I, kGemmBM);
@@ -275,20 +289,20 @@ static void bert_enqueue(BertModel& m, bool use_mask) {
         launch_gemm<GEPI_BIAS_BF16>(lc, "bert_gemm_qkv", tm_x, w.tm_wqkv, GemmArgs{T, 3 * H, H, w.bqkv, nullptr, 0, m.qkv.p, 3 * H, 1, 0});
         // B3+B4: per (sentence, head) softmax(QK^T / sqrt(d)) V, no mask; sentences of <= 128 tokens in one tile, longer ones key-tiled
         if (bb.nshort)
-            launch(lc, "bert_attn", 0, bert_attn_kernel, dim3(m.nh * bb.nshort), dim3(128), 0, (const uint16_t*)m.qkv.p, shorts, m.nh, H, scale,
+            launch(lc, "bert_attn", 0, attn, dim3(m.nh * bb.nshort), dim3(128), attn_smem, (const uint16_t*)m.qkv.p, shorts, m.nh, H, scale,
                    m.ctx.p);
         if (bb.nlong)
-            launch(lc, "bert_attn", 0, bert_attn_long_kernel, dim3(m.nh * bb.nlong), dim3(128), 0, (const uint16_t*)m.qkv.p, longs, m.nh, H,
+            launch(lc, "bert_attn", 0, attn_long, dim3(m.nh * bb.nlong), dim3(128), attn_smem, (const uint16_t*)m.qkv.p, longs, m.nh, H,
                    scale, m.ctx.p);
         // B5: attention output dense + bias + residual -> f32, then LayerNorm -> bf16
         launch_gemm<GEPI_BIAS_RESID_F32>(lc, "bert_gemm_o", tm_ctx, w.tm_wo, GemmArgs{T, H, H, w.bo, m.x.p, H, m.pre.p, H, 1, 0});
-        launch(lc, "bert_layernorm", 0, layernorm_kernel, row_grid, row_block, 0, (const float*)m.pre.p, (const float*)w.ln1w, (const float*)w.ln1b,
+        launch(lc, "bert_layernorm", 0, layernorm, row_grid, row_block, 0, (const float*)m.pre.p, (const float*)w.ln1w, (const float*)w.ln1b,
                T, H, eps, m.x1.p);
         // B6: intermediate dense + bias + GELU(tanh) -> bf16 [T, I]
         launch_gemm<GEPI_BIAS_GELU_BF16>(lc, "bert_gemm_up_gelu", tm_x1, w.tm_wi, GemmArgs{T, I, H, w.bi, nullptr, 0, m.hbuf.p, I, 1, 0});
         // B7: output dense + bias + residual -> f32, LayerNorm -> bf16
         launch_gemm<GEPI_BIAS_RESID_F32>(lc, "bert_gemm_down", tm_h, w.tm_wo2, GemmArgs{T, H, I, w.bo2, m.x1.p, H, m.pre.p, H, 1, 0});
-        launch(lc, "bert_layernorm", 0, layernorm_kernel, row_grid, row_block, 0, (const float*)m.pre.p, (const float*)w.ln2w, (const float*)w.ln2b,
+        launch(lc, "bert_layernorm", 0, layernorm, row_grid, row_block, 0, (const float*)m.pre.p, (const float*)w.ln2w, (const float*)w.ln2b,
                T, H, eps, m.x.p);
     }
     // B8: masked mean pooling + L2 normalise -> f32 [n, H]

@@ -632,6 +632,21 @@ class BertConfig:
     layer_norm_eps: float = 1e-12
     vocab_size: int = 30522
 
+    @classmethod
+    def from_json(cls, path_or_dict) -> "BertConfig":
+        """The seven dimensions from a HuggingFace BERT `config.json` (a path, or the parsed dict).  Every other key
+        (`type_vocab_size`, `architectures`, `hidden_act`, ...) is ignored; a missing dimension raises ValueError naming it."""
+        if isinstance(path_or_dict, dict):
+            d = path_or_dict
+        else:
+            with open(path_or_dict) as f:
+                d = json.load(f)
+        missing = [k for k in cls.__dataclass_fields__ if k not in d]
+        if missing:
+            raise ValueError(f"BERT config.json lacks {', '.join(missing)}")
+        return cls(int(d["hidden_size"]), int(d["num_attention_heads"]), int(d["num_hidden_layers"]), int(d["intermediate_size"]),
+                   int(d["max_position_embeddings"]), float(d["layer_norm_eps"]), int(d["vocab_size"]))
+
 
 class MiniLMModel:
     """MiniLMModel (models/embeddings.rs:245-447) after tokenisation: `embed_ids` takes the token ids (and the tokenizer's

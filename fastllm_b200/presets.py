@@ -1,5 +1,5 @@
 """config.json presets of the BASELINE.json models (sizes only), as the adapters' ConfigFile (llama.rs:17-29 etc.)."""
-from .models import ConfigFile, LlamaWithConfig, MistralWithConfig, MixtralWithConfig, QwenWithConfig
+from .models import BertConfig, ConfigFile, LlamaWithConfig, MistralWithConfig, MixtralWithConfig, QwenWithConfig
 
 # TinyLlama-1.1B-Chat: the shape llama.rs:125-145 hard-codes for its cache
 TINYLLAMA = (LlamaWithConfig, ConfigFile(2048, 5632, 32000, 22, 32, 4, 1e-5, 10000.0, 2048))
@@ -13,3 +13,10 @@ MIXTRAL_8X7B = (MixtralWithConfig, ConfigFile(4096, 14336, 32000, 32, 32, 8, 1e-
                                               num_experts_per_tok=2))
 
 PRESETS = {"tinyllama": TINYLLAMA, "mistral7b": MISTRAL_7B, "qwen25_7b": QWEN25_7B, "mixtral8x7b": MIXTRAL_8X7B}
+
+# Mean-pooled BERT sentence encoders (MiniLMModel): all-MiniLM-L6-v2 (head_dim 32), and the BERT-base / -large shapes of e5 and gte
+# (head_dim 64)
+MINILM_L6 = BertConfig(384, 12, 6, 1536, 512, 1e-12, 30522)
+BERT_BASE = BertConfig(768, 12, 12, 3072, 512, 1e-12, 30522)
+BERT_LARGE = BertConfig(1024, 16, 24, 4096, 512, 1e-12, 30522)
+BERT_PRESETS = {"minilm_l6": MINILM_L6, "bert_base": BERT_BASE, "bert_large": BERT_LARGE}

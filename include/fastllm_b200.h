@@ -182,7 +182,10 @@ FL_EXPORT int fl_forward_sample_device(fl_model* m, fl_cache* c, const uint32_t*
                                        uint32_t* next_id);
 
 /* ---- embeddings (BERT family) ------------------------------------------------------------------ */
-/* ids/mask: host u32 [b, t]; mask may be NULL (all ones).  out: host f32 [b, hidden], mean-pooled and L2-normalised. */
+/* Supported encoder shapes: head_dim (hidden / heads) 32 or 64, hidden and intermediate multiples of 64 with hidden <= 1024
+ * (all-MiniLM-L6-v2, BERT-base and BERT-large sized models such as e5 / gte), up to 512 positions; any other shape fails at
+ * fl_model_create with FL_ERR_UNSUPPORTED.
+ * ids/mask: host u32 [b, t]; mask may be NULL (all ones).  out: host f32 [b, hidden], mean-pooled and L2-normalised. */
 FL_EXPORT int fl_embed(fl_model* m, const uint32_t* ids, const uint32_t* mask, int b, int t, float* out);
 /* Sentences of different lengths in ONE encoder pass, no padding: sentence i is ids[o_i, o_i + lengths[i]) with
  * o_i = lengths[0] + ... + lengths[i-1]; every token of a sentence is pooled (the all-ones mask a lone sentence has).
