@@ -3,12 +3,11 @@
 #include <cuda.h>
 
 #include <mutex>
-#include <set>
-#include <string>
 #include <vector>
 
 #include "../../include/fastllm_b200.h"
 #include "runtime.cuh"
+#include "tensor_table.hpp"
 
 namespace fl {
 
@@ -22,12 +21,10 @@ struct BertLayerW {
 struct BertModel {
     fl_config cfg{};
     int H = 0, I = 0, V = 0, L = 0, nh = 0, d = 0, maxpos = 0;
-    DevBuf<uint8_t> slab;
+    TensorTable table;
     uint16_t *wemb = nullptr, *pemb = nullptr;
     float *lnw = nullptr, *lnb = nullptr;
     std::vector<BertLayerW> layers;
-    std::set<std::string> have;
-    bool finalized = false;
     cudaStream_t stream = nullptr;
     std::mutex mu;
     // workspace (grown on demand)
@@ -43,13 +40,12 @@ struct BertModel {
         bool mask = false;
         size_t o_pos = 0, o_starts = 0, o_short = 0, o_long = 0;
     } batch;
-    ~BertModel();
+    ~BertModel() {
+        if (stream) cudaStreamDestroy(stream);
+    }
 };
 
-void bert_build(BertModel& m);
-void bert_put_tensor(BertModel& m, const char* name, int dtype, const int64_t* shape, int rank, const void* host);
-void bert_random_init(BertModel& m, uint64_t seed, float stdv);
-void bert_finalize(BertModel& m);
+void finalize(BertModel& m);
 void bert_embed(BertModel& m, const uint32_t* ids, const uint32_t* mask, int b, int t, float* out);
 void bert_embed_packed(BertModel& m, const uint32_t* ids, const int32_t* lengths, int n, float* out);
 void bert_repeat(BertModel& m, int b, int t, int iters, float* elapsed_ms);

@@ -7,7 +7,6 @@
 #include "bert.cuh"
 #include "bert_model.cuh"
 #include "gemm_tc.cuh"
-#include "synth.cuh"
 
 namespace fl {
 
@@ -94,152 +93,15 @@ static void launch_gemm(LaunchCtx& lc, const char* tag, const CUtensorMap& tmA, 
            g);
 }
 
-// ---- weights -------------------------------------------------------------------------------------------------------------
-void bert_build(BertModel& m) {
-    const fl_config& c = m.cfg;
-    m.H = c.hidden_size; m.I = c.intermediate_size; m.V = c.vocab_size; m.L = c.num_hidden_layers; m.nh = c.num_attention_heads;
-    m.d = m.H / m.nh; m.maxpos = c.max_position_embeddings;
-    FL_CHECK(m.d * m.nh == m.H, FL_ERR_INVALID, "hidden_size must be divisible by num_attention_heads");
-    // head_dim: the attention kernels are built for 32 (all-MiniLM-L6-v2) and 64 (BERT-base / -large, e5, gte); the GEMMs take
-    // K and N in 64-column blocks; the LayerNorm kernels hold a row in one warp and pool_l2_kernel a row in one CTA: hidden <= 1024
-    FL_CHECK(m.d == 32 || m.d == 64, FL_ERR_UNSUPPORTED,
-             "BERT path is built for head_dim 32 and 64 (hidden_size / num_attention_heads = " + std::to_string(m.d) + ")");
-    FL_CHECK(m.H % 64 == 0 && m.I % 64 == 0, FL_ERR_UNSUPPORTED, "BERT path needs hidden_size and intermediate_size to be multiples of 64");
-    FL_CHECK(m.H <= 1024, FL_ERR_UNSUPPORTED, "BERT path is built for hidden_size <= 1024");
-    const size_t H = m.H, I = m.I;
-    size_t off = 0;
-    auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
-    const size_t o_w = take((size_t)m.V * H * 2), o_p = take((size_t)m.maxpos * H * 2), o_lw = take(H * 4), o_lb = take(H * 4);
-    struct LO { size_t wqkv, wo, wi, wo2, bqkv, bo, bi, bo2, l1w, l1b, l2w, l2b; };
-    std::vector<LO> lo(m.L);
-    for (auto& l : lo) {
-        l.wqkv = take(3 * H * H * 2); l.wo = take(H * H * 2); l.wi = take(I * H * 2); l.wo2 = take(H * I * 2);
-        l.bqkv = take(3 * H * 4); l.bo = take(H * 4); l.bi = take(I * 4); l.bo2 = take(H * 4);
-        l.l1w = take(H * 4); l.l1b = take(H * 4); l.l2w = take(H * 4); l.l2b = take(H * 4);
-    }
-    m.slab.alloc(off, true);
-    uint8_t* b = m.slab.p;
-    m.wemb = (uint16_t*)(b + o_w); m.pemb = (uint16_t*)(b + o_p); m.lnw = (float*)(b + o_lw); m.lnb = (float*)(b + o_lb);
-    m.layers.resize(m.L);
-    for (int i = 0; i < m.L; ++i) {
-        BertLayerW& w = m.layers[i];
-        const LO& l = lo[i];
-        w.wqkv = (uint16_t*)(b + l.wqkv); w.wo = (uint16_t*)(b + l.wo); w.wi = (uint16_t*)(b + l.wi); w.wo2 = (uint16_t*)(b + l.wo2);
-        w.bqkv = (float*)(b + l.bqkv); w.bo = (float*)(b + l.bo); w.bi = (float*)(b + l.bi); w.bo2 = (float*)(b + l.bo2);
-        w.ln1w = (float*)(b + l.l1w); w.ln1b = (float*)(b + l.l1b); w.ln2w = (float*)(b + l.l2w); w.ln2b = (float*)(b + l.l2b);
-    }
-    FL_CUDA(cudaStreamCreateWithFlags(&m.stream, cudaStreamNonBlocking));
-}
-
-struct BertRoute {
-    bool mat;
-    void* base;
-    int64_t rows, cols, row0;
-};
-
-static bool bert_route(BertModel& m, const std::string& name, BertRoute& r) {
-    const int64_t H = m.H, I = m.I;
-    auto mat = [&](uint16_t* p, int64_t rows, int64_t cols, int64_t row0 = 0) { r = {true, p, rows, cols, row0}; return true; };
-    auto vec = [&](float* p, int64_t rows, int64_t row0 = 0) { r = {false, p, rows, 1, row0}; return true; };
-    if (name == "embeddings.word_embeddings.weight") return mat(m.wemb, m.V, H);
-    if (name == "embeddings.position_embeddings.weight") return mat(m.pemb, m.maxpos, H);
-    if (name == "embeddings.LayerNorm.weight") return vec(m.lnw, H);
-    if (name == "embeddings.LayerNorm.bias") return vec(m.lnb, H);
-    const std::string pre = "encoder.layer.";
-    if (name.compare(0, pre.size(), pre) != 0) return false;
-    const size_t dot = name.find('.', pre.size());
-    if (dot == std::string::npos) return false;
-    int li = -1;
-    try { li = std::stoi(name.substr(pre.size(), dot - pre.size())); } catch (...) { return false; }
-    if (li < 0 || li >= m.L) return false;
-    BertLayerW& w = m.layers[li];
-    const std::string rest = name.substr(dot + 1);
-    if (rest == "attention.self.query.weight") return mat(w.wqkv, H, H, 0);
-    if (rest == "attention.self.key.weight") return mat(w.wqkv, H, H, H);
-    if (rest == "attention.self.value.weight") return mat(w.wqkv, H, H, 2 * H);
-    if (rest == "attention.self.query.bias") return vec(w.bqkv, H, 0);
-    if (rest == "attention.self.key.bias") return vec(w.bqkv, H, H);
-    if (rest == "attention.self.value.bias") return vec(w.bqkv, H, 2 * H);
-    if (rest == "attention.output.dense.weight") return mat(w.wo, H, H);
-    if (rest == "attention.output.dense.bias") return vec(w.bo, H);
-    if (rest == "attention.output.LayerNorm.weight") return vec(w.ln1w, H);
-    if (rest == "attention.output.LayerNorm.bias") return vec(w.ln1b, H);
-    if (rest == "intermediate.dense.weight") return mat(w.wi, I, H);
-    if (rest == "intermediate.dense.bias") return vec(w.bi, I);
-    if (rest == "output.dense.weight") return mat(w.wo2, H, I);
-    if (rest == "output.dense.bias") return vec(w.bo2, H);
-    if (rest == "output.LayerNorm.weight") return vec(w.ln2w, H);
-    if (rest == "output.LayerNorm.bias") return vec(w.ln2b, H);
-    return false;
-}
-
-static std::vector<std::string> bert_expected(const BertModel& m) {
-    std::vector<std::string> v = {"embeddings.word_embeddings.weight", "embeddings.position_embeddings.weight",
-                                  "embeddings.LayerNorm.weight", "embeddings.LayerNorm.bias"};
-    for (int l = 0; l < m.L; ++l) {
-        const std::string p = "encoder.layer." + std::to_string(l) + ".";
-        for (const char* s : {"attention.self.query", "attention.self.key", "attention.self.value", "attention.output.dense",
-                              "intermediate.dense", "output.dense", "attention.output.LayerNorm", "output.LayerNorm"}) {
-            v.push_back(p + s + ".weight");
-            v.push_back(p + s + ".bias");
-        }
-    }
-    return v;
-}
-
-void bert_put_tensor(BertModel& m, const char* name, int dtype, const int64_t* shape, int rank, const void* host) {
-    FL_CHECK(!m.finalized, FL_ERR_STATE, "model already finalized");
-    const std::string n(name);
-    // tensors the reference never reads (pooler, token-type embeddings, position_ids buffer, anything else in the checkpoint):
-    // accepted and ignored, as VarBuilder ignores the extra entries of the loaded HashMap (embeddings.rs:290-298); a MISSING tensor
-    // is still an error at finalize
-    BertRoute r;
-    if (!bert_route(m, n, r)) return;
-    FL_CHECK(dtype == FL_DTYPE_F32, FL_ERR_UNSUPPORTED, "BERT tensors must be f32 (the reference loads MiniLM as F32, embeddings.rs:298)");
-    const bool ok = r.mat ? (rank == 2 && shape[0] == r.rows && shape[1] == r.cols) : (rank == 1 && shape[0] == r.rows);
-    FL_CHECK(ok, FL_ERR_INVALID, "shape mismatch for " + n);
-    const float* f = (const float*)host;
-    if (r.mat) {
-        std::vector<uint16_t> bits((size_t)r.rows * r.cols);
-        for (size_t i = 0; i < bits.size(); ++i) bits[i] = host_f32_to_bf16(f[i]);
-        FL_CUDA(cudaMemcpy((uint16_t*)r.base + r.row0 * r.cols, bits.data(), bits.size() * 2, cudaMemcpyHostToDevice));
-    } else {
-        FL_CUDA(cudaMemcpy((float*)r.base + r.row0, f, (size_t)r.rows * 4, cudaMemcpyHostToDevice));
-    }
-    m.have.insert(n);
-}
-
-void bert_random_init(BertModel& m, uint64_t seed, float stdv) {
-    FL_CHECK(!m.finalized, FL_ERR_STATE, "model already finalized");
-    for (const std::string& n : bert_expected(m)) {
-        BertRoute r;
-        FL_CHECK(bert_route(m, n, r), FL_ERR_INVALID, "internal: unroutable " + n);
-        const bool is_ln_w = n.size() >= 16 && n.compare(n.size() - 16, 16, "LayerNorm.weight") == 0;
-        const uint64_t ts = tensor_seed(seed, n.c_str());
-        const RowMap map{r.row0, 0, 0, 0};
-        if (r.mat)
-            synth_fill_bf16_kernel<<<kNumSMs * 4, 256>>>((uint16_t*)r.base, r.rows, r.cols, r.cols, ts, stdv, map);
-        else if (is_ln_w)
-            fill_f32_kernel<<<4, 256>>>((float*)r.base + r.row0, r.rows, 1.0f);
-        else
-            synth_fill_f32_kernel<<<4, 256>>>((float*)r.base, r.rows, ts, stdv, map);
-        g_launches.fetch_add(1);
-        m.have.insert(n);
-    }
-    FL_CUDA(cudaGetLastError());
-    FL_CUDA(cudaDeviceSynchronize());
-}
-
-void bert_finalize(BertModel& m) {
-    FL_CHECK(!m.finalized, FL_ERR_STATE, "model already finalized");
-    for (const std::string& n : bert_expected(m)) FL_CHECK(m.have.count(n), FL_ERR_STATE, "missing tensor: " + n);
+void finalize(BertModel& m) {
+    m.table.check_complete();
     for (BertLayerW& w : m.layers) {   // weight-side TMA descriptors ([out, in] row-major == K-major B operand)
         w.tm_wqkv = make_tmap_bf16(w.wqkv, 3 * m.H, m.H, m.H, kBertBN);
         w.tm_wo = make_tmap_bf16(w.wo, m.H, m.H, m.H, kBertBN);
         w.tm_wi = make_tmap_bf16(w.wi, m.I, m.H, m.H, kBertBN);
         w.tm_wo2 = make_tmap_bf16(w.wo2, m.H, m.I, m.I, kBertBN);
     }
-    m.finalized = true;
+    m.table.finalized = true;
 }
 
 static void bert_reserve(BertModel& m, size_t T, size_t n, size_t words) {
@@ -267,7 +129,7 @@ static void bert_enqueue(BertModel& m, bool use_mask) {
     const BertItem* shorts = (const BertItem*)(m.ids.p + bb.o_short);
     const BertItem* longs = (const BertItem*)(m.ids.p + bb.o_long);
     LaunchCtx lc{m.stream};
-    // the model's kernel instantiations (bert_build admits head_dim 32 / 64 and hidden <= 1024); rows of up to 512 columns take the
+    // the model's kernel instantiations (bert_plan admits head_dim 32 / 64 and hidden <= 1024); rows of up to 512 columns take the
     // narrow LayerNorm kernels, which hold 16 values per lane instead of 32
     const bool wide = H > 512;
     const auto embed_ln = wide ? embed_ln_kernel<32> : embed_ln_kernel<16>;
@@ -366,7 +228,7 @@ static void bert_run(BertModel& m, const uint32_t* ids, const uint32_t* mask, co
 }
 
 void bert_embed(BertModel& m, const uint32_t* ids, const uint32_t* mask, int b, int t, float* out) {
-    FL_CHECK(m.finalized, FL_ERR_STATE, "model not finalized");
+    FL_CHECK(m.table.finalized, FL_ERR_STATE, "model not finalized");
     FL_CHECK(ids && out && b >= 1 && t >= 1, FL_ERR_INVALID, "bad arguments");
     // the reference enforces no max_seq_length (embeddings.rs:285-286); what bounds a sentence is its position table: position ids
     // 0..n index a [max_position_embeddings, H] embedding (embeddings.rs:416, 370-378), and candle's index_select fails past it
@@ -378,7 +240,7 @@ void bert_embed(BertModel& m, const uint32_t* ids, const uint32_t* mask, int b, 
 }
 
 void bert_embed_packed(BertModel& m, const uint32_t* ids, const int32_t* lengths, int n, float* out) {
-    FL_CHECK(m.finalized, FL_ERR_STATE, "model not finalized");
+    FL_CHECK(m.table.finalized, FL_ERR_STATE, "model not finalized");
     FL_CHECK(ids && lengths && out && n >= 1, FL_ERR_INVALID, "bad arguments");
     int64_t total = 0;
     for (int i = 0; i < n; ++i) {
@@ -402,10 +264,6 @@ void bert_repeat(BertModel& m, int b, int t, int iters, float* elapsed_ms) {
     FL_CUDA(cudaStreamSynchronize(m.stream));
     FL_CUDA(cudaGetLastError());
     FL_CUDA(cudaEventElapsedTime(elapsed_ms, ev.e0, ev.e1));
-}
-
-BertModel::~BertModel() {
-    if (stream) cudaStreamDestroy(stream);
 }
 
 }  // namespace fl

@@ -15,6 +15,7 @@
 #include "model.cuh"
 #include "sampler.hpp"
 #include "synth.cuh"
+#include "weights_plan.cuh"
 
 namespace fl {
 
@@ -172,322 +173,102 @@ static void validate_config(const fl_config& c) {
     FL_CHECK(d * c.num_attention_heads == c.hidden_size, FL_ERR_INVALID, "hidden_size must be divisible by num_attention_heads");
     FL_CHECK(d % 2 == 0, FL_ERR_INVALID, "head_dim must be even for RoPE embeddings");
     const int nkv = c.num_key_value_heads > 0 ? c.num_key_value_heads : c.num_attention_heads;
-    if (c.arch == FL_ARCH_BERT) return;   // remaining checks are causal-LM specific; bert_build has its own
+    if (c.arch == FL_ARCH_BERT) return;   // remaining checks are causal-LM specific; bert_plan has its own
     FL_CHECK(c.num_attention_heads % nkv == 0, FL_ERR_INVALID, "num_attention_heads must be divisible by num_key_value_heads");
     FL_CHECK(c.num_attention_heads / nkv <= kAttnMaxRep, FL_ERR_UNSUPPORTED, "GQA group size > 8 not supported");
     FL_CHECK(c.hidden_size % 8 == 0 && c.intermediate_size % 8 == 0, FL_ERR_UNSUPPORTED, "hidden/intermediate size must be a multiple of 8");
     FL_CHECK(c.max_position_embeddings > 0, FL_ERR_INVALID, "max_position_embeddings must be positive");
 }
 
-static void build_weights(Weights& w) {
-    const fl_config& c = w.cfg;
-    const int nh_f = c.num_attention_heads, nkv_f = c.num_key_value_heads > 0 ? c.num_key_value_heads : c.num_attention_heads;
-    const bool moe = c.arch == FL_ARCH_MIXTRAL;
-    // Mixtral shards by EXPERT (attention, router and head replicated); the dense models shard by tensor
-    w.ep = (moe && c.tp_size > 1) ? c.tp_size : 1;
-    w.tp = (!moe && c.tp_size > 1) ? c.tp_size : 1;
-    w.rank = c.tp_size > 1 ? c.tp_rank : 0;
-    if (moe) {
-        w.E = c.num_local_experts; w.top_k = c.num_experts_per_tok > 0 ? c.num_experts_per_tok : 2;
-        FL_CHECK(w.E >= 1 && w.E <= 64 && w.top_k >= 1 && w.top_k <= 8 && w.top_k <= w.E, FL_ERR_INVALID, "bad Mixtral expert counts");
-        FL_CHECK(w.E % w.ep == 0, FL_ERR_UNSUPPORTED, "expert parallelism needs num_local_experts divisible by the world size");
-        w.E_local = w.E / w.ep;
-        w.ep_dp = w.ep > 1 && c.ep_dp_attention != 0;
-    }
-    FL_CHECK(w.rank >= 0 && w.rank < std::max(w.tp, w.ep), FL_ERR_INVALID, "tp_rank out of range");
-    if (w.tp > 1) {
-        // column-parallel q/k/v (by head) and gate/up, row-parallel o_proj and down_proj, vocab-parallel lm_head
-        FL_CHECK((nkv_f % w.tp == 0 && nh_f % w.tp == 0) || (w.tp > nkv_f && w.tp % nkv_f == 0), FL_ERR_UNSUPPORTED,
-                 "tensor parallelism needs heads and kv heads divisible by tp_size, or tp_size a multiple of the kv heads");
-        FL_CHECK(c.intermediate_size % (8 * w.tp) == 0 && c.vocab_size % (2 * w.tp) == 0, FL_ERR_UNSUPPORTED,
-                 "tensor parallelism needs intermediate_size % (8 tp) == 0 and vocab_size % (2 tp) == 0");
-    }
-    w.H = c.hidden_size; w.L = c.num_hidden_layers;
-    w.I = c.intermediate_size / w.tp; w.Vfull = c.vocab_size; w.V = c.vocab_size / w.tp;
-    const int trank = w.tp > 1 ? w.rank : 0;       // under expert parallelism (tp == 1) the attention weights are replicated
-    if (w.tp <= nkv_f) {
-        w.nh = nh_f / w.tp; w.nkv = nkv_f / w.tp;
-        w.q_head0 = trank * w.nh; w.q_real = w.nh; w.kv_head0 = trank * w.nkv;
-    } else {
-        // more ranks than kv heads (Qwen2.5-7B at TP-8: 28 q / 4 kv heads): every kv head lives on rep = tp / nkv ranks, and the
-        // group's query heads are dealt out ceil(group / rep) per rank; the last rank of a group pads with zero heads
-        // (zero q rows and zero o_proj columns contribute nothing)
-        const int rep = w.tp / nkv_f, group = nh_f / nkv_f, hpr = (group + rep - 1) / rep;
-        const int kvh = trank / rep, sub = trank % rep;
-        w.nh = hpr; w.nkv = 1;
-        w.q_head0 = kvh * group + sub * hpr;
-        w.q_real = std::max(0, std::min(hpr, group - sub * hpr));
-        w.kv_head0 = kvh;
-    }
-    w.d = w.H / nh_f;
-    w.max_pos = c.max_position_embeddings;
-    w.nqkv = (w.nh + 2 * w.nkv) * w.d;
-    with_head_dim(w.d, [](auto) {});
-    FL_CHECK(c.arch != FL_ARCH_BERT, FL_ERR_INVALID, "internal: BERT goes through bert_build");
-
-    const size_t A = 256;
-    size_t off = 0;
-    auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, A); return o; };
-    const size_t H = w.H, I = w.I, V = w.V, nq = (size_t)w.nh * w.d;
-    const size_t o_embed = take((size_t)w.Vfull * H * 2), o_head = take(V * H * 2), o_fnorm = take(H * 4);
-    struct LO { size_t wqkv, bqkv, wo, wgu, wdown, ln1, ln2, wgate; std::vector<size_t> ewgu, ewdown; };
-    std::vector<LO> lo(w.L);
-    for (int l = 0; l < w.L; ++l) {
-        lo[l].wqkv = take((size_t)w.nqkv * H * 2);
-        lo[l].bqkv = c.qkv_bias ? take((size_t)w.nqkv * 4) : (size_t)-1;
-        lo[l].wo = take(H * nq * 2);
-        if (moe) {
-            lo[l].wgate = take((size_t)w.E * H * 4);
-            // a layer's w1|w3 matrices back to back, then its w2 matrices back to back: each set is also ONE stacked matrix
-            // ([E_local * 2I, H] / [E_local * H, I]), the A operand of the grouped expert GEMMs
-            const size_t gu0 = take((size_t)w.E_local * 2 * I * H * 2), dn0 = take((size_t)w.E_local * H * I * 2);
-            for (int e = 0; e < w.E_local; ++e) {
-                lo[l].ewgu.push_back(gu0 + (size_t)e * 2 * I * H * 2);
-                lo[l].ewdown.push_back(dn0 + (size_t)e * H * I * 2);
-            }
-            lo[l].wgu = lo[l].wdown = 0;
-        } else {
-            lo[l].wgu = take(2 * I * H * 2);
-            lo[l].wdown = take(H * I * 2);
-        }
-        lo[l].ln1 = take(H * 4);
-        lo[l].ln2 = take(H * 4);
-    }
-    const size_t o_cos = take((size_t)w.max_pos * (w.d / 2) * 4), o_sin = take((size_t)w.max_pos * (w.d / 2) * 4);
-    w.slab.alloc(off, /*zero=*/true);
-    uint8_t* base = w.slab.p;
-    w.embed = (uint16_t*)(base + o_embed);
-    w.lm_head = (uint16_t*)(base + o_head);
-    w.final_norm = (float*)(base + o_fnorm);
-    w.layers.resize(w.L);
-    for (int l = 0; l < w.L; ++l) {
-        w.layers[l].wqkv = (uint16_t*)(base + lo[l].wqkv);
-        w.layers[l].bqkv = c.qkv_bias ? (float*)(base + lo[l].bqkv) : nullptr;
-        w.layers[l].wo = (uint16_t*)(base + lo[l].wo);
-        if (moe) {
-            w.layers[l].wgate = (float*)(base + lo[l].wgate);
-            for (int e = 0; e < w.E_local; ++e) {
-                w.layers[l].ewgu.push_back((uint16_t*)(base + lo[l].ewgu[e]));
-                w.layers[l].ewdown.push_back((uint16_t*)(base + lo[l].ewdown[e]));
-            }
-        } else {
-            w.layers[l].wgu = (uint16_t*)(base + lo[l].wgu);
-            w.layers[l].wdown = (uint16_t*)(base + lo[l].wdown);
-        }
-        w.layers[l].ln1 = (float*)(base + lo[l].ln1);
-        w.layers[l].ln2 = (float*)(base + lo[l].ln2);
-    }
-    w.rope_cos = (float*)(base + o_cos);
-    w.rope_sin = (float*)(base + o_sin);
-    // bytes one decode step must stream: every parameter except the embedding table (SURVEY.md section 8d)
-    const uint64_t mlp = moe ? (uint64_t)w.E_local * 3 * I * H : 3 * I * H;     // every local expert is streamed each step
-    w.streamed_bytes = 2 * ((uint64_t)w.L * ((uint64_t)w.nqkv * H + H * nq + mlp) + V * H) +
-                       4 * ((uint64_t)w.L * (2 * H + (c.qkv_bias ? w.nqkv : 0) + (moe ? (uint64_t)w.E * H : 0)) + H);
-}
-
-struct TensorRoute {
-    enum Kind { BF16_MAT, F32_VEC } kind;
-    void* base;
-    int64_t rows, cols;             // LOCAL block held by this rank ([rows, cols] or [rows])
-    int64_t ld;                     // leading dimension of the local matrix in elements (>= cols; > cols: zero-padded heads)
-    RowMap map;
-    int64_t full_rows, full_cols;   // shape the caller hands over (the full HF tensor)
-    int64_t src_row0, src_col0;     // window of the full tensor this rank keeps
-};
-
-static bool route_tensor(Weights& w, const std::string& name, TensorRoute& r) {
-    const int64_t H = w.H, I = w.I, d = w.d, nq = (int64_t)w.nh * d, nk = (int64_t)w.nkv * d, tp = w.tp,
-                  rk = w.tp > 1 ? w.rank : 0;   // under expert parallelism (tp == 1) every dense tensor is replicated
-    // row-sharded matrix: local rows [rk*rows, (rk+1)*rows) of a [tp*rows, cols] tensor; col-sharded: the same along columns
-    auto mat_rows = [&](uint16_t* base, int64_t rows, int64_t cols, RowMap m, bool sharded) {
-        r = {TensorRoute::BF16_MAT, base, rows, cols, cols, m, sharded ? rows * tp : rows, cols, sharded ? rk * rows : 0, 0};
-        return true;
-    };
-    auto mat_cols = [&](uint16_t* base, int64_t rows, int64_t cols, RowMap m) {
-        r = {TensorRoute::BF16_MAT, base, rows, cols, cols, m, rows, cols * tp, 0, rk * cols};
-        return true;
-    };
-    auto vec = [&](float* base, int64_t rows, RowMap m, bool sharded) {
-        r = {TensorRoute::F32_VEC, base, rows, 1, 1, m, sharded ? rows * tp : rows, 1, sharded ? rk * rows : 0, 0};
-        return true;
-    };
-    // attention projections: head windows of the full tensors (w.q_head0 / w.q_real / w.kv_head0, see build_weights)
-    const int64_t nh_f = w.cfg.num_attention_heads, nkv_f = w.cfg.num_key_value_heads > 0 ? w.cfg.num_key_value_heads : nh_f;
-    const int64_t qreal = (int64_t)w.q_real * d, q0 = (int64_t)w.q_head0 * d, k0 = (int64_t)w.kv_head0 * d;
-    auto head_rows = [&](uint16_t* base, int64_t rows, RowMap m, int64_t full_heads, int64_t row0) {
-        r = {TensorRoute::BF16_MAT, base, rows, H, H, m, full_heads * d, H, row0, 0};
-        return true;
-    };
-    auto head_vec = [&](float* base, int64_t rows, RowMap m, int64_t full_heads, int64_t row0) {
-        r = {TensorRoute::F32_VEC, base, rows, 1, 1, m, full_heads * d, 1, row0, 0};
-        return true;
-    };
-    const RowMap ident{0, 0, 0, 0};
-    if (name == "model.embed_tokens.weight") return mat_rows(w.embed, w.Vfull, H, ident, false);
-    if (name == "lm_head.weight") return mat_rows(w.lm_head, w.V, H, ident, true);
-    if (name == "model.norm.weight") return vec(w.final_norm, H, ident, false);
-    const std::string pre = "model.layers.";
-    if (name.compare(0, pre.size(), pre) != 0) return false;
-    size_t dot = name.find('.', pre.size());
-    if (dot == std::string::npos) return false;
-    int li = -1;
-    try { li = std::stoi(name.substr(pre.size(), dot - pre.size())); } catch (...) { return false; }
-    if (li < 0 || li >= w.L) return false;
-    LayerW& lw = w.layers[li];
-    const std::string rest = name.substr(dot + 1);
-    const RowMap ropeq{0, 1, (int32_t)d, 0}, ropek{nq, 1, (int32_t)d, 0}, vmap{nq + nk, 0, 0, 0};
-    if (rest == "input_layernorm.weight") return vec(lw.ln1, H, ident, false);
-    if (rest == "post_attention_layernorm.weight") return vec(lw.ln2, H, ident, false);
-    if (rest == "self_attn.q_proj.weight") return head_rows(lw.wqkv, qreal, ropeq, nh_f, q0);
-    if (rest == "self_attn.k_proj.weight") return head_rows(lw.wqkv, nk, ropek, nkv_f, k0);
-    if (rest == "self_attn.v_proj.weight") return head_rows(lw.wqkv, nk, vmap, nkv_f, k0);
-    if (w.cfg.qkv_bias) {
-        if (rest == "self_attn.q_proj.bias") return head_vec(lw.bqkv, qreal, ropeq, nh_f, q0);
-        if (rest == "self_attn.k_proj.bias") return head_vec(lw.bqkv, nk, ropek, nkv_f, k0);
-        if (rest == "self_attn.v_proj.bias") return head_vec(lw.bqkv, nk, vmap, nkv_f, k0);
-    }
-    if (rest == "self_attn.o_proj.weight") {
-        r = {TensorRoute::BF16_MAT, lw.wo, H, qreal, nq, ident, H, nh_f * d, 0, q0};
-        return true;
-    }
-    if (w.cfg.arch == FL_ARCH_MIXTRAL) {
-        if (rest == "block_sparse_moe.gate.weight") return vec(lw.wgate, (int64_t)w.E * H, ident, false);   // [E, H] kept in f32
-        const std::string ep = "block_sparse_moe.experts.";
-        if (rest.compare(0, ep.size(), ep) != 0) return false;
-        const size_t d2 = rest.find('.', ep.size());
-        if (d2 == std::string::npos) return false;
-        int e = -1;
-        try { e = std::stoi(rest.substr(ep.size(), d2 - ep.size())); } catch (...) { return false; }
-        if (e < 0 || e >= w.E) return false;
-        const std::string tail = rest.substr(d2 + 1);
-        const int el = e - w.rank * w.E_local;                  // local slot, or outside this rank's range
-        const bool mine = el >= 0 && el < w.E_local;
-        uint16_t* gu = mine ? lw.ewgu[el] : nullptr;
-        uint16_t* dn = mine ? lw.ewdown[el] : nullptr;
-        bool ok = false;
-        if (tail == "w1.weight") ok = mat_rows(gu, I, H, RowMap{0, 2, 0, 0}, false);
-        else if (tail == "w3.weight") ok = mat_rows(gu, I, H, RowMap{0, 2, 0, 1}, false);
-        else if (tail == "w2.weight") ok = mat_rows(dn, H, I, ident, false);
-        return ok;      // r.base == nullptr: a valid tensor that belongs to another expert-parallel rank
-    }
-    if (rest == "mlp.gate_proj.weight") return mat_rows(lw.wgu, I, H, RowMap{0, 2, 0, 0}, true);
-    if (rest == "mlp.up_proj.weight") return mat_rows(lw.wgu, I, H, RowMap{0, 2, 0, 1}, true);
-    if (rest == "mlp.down_proj.weight") return mat_cols(lw.wdown, H, I, ident);
-    return false;
-}
-
-static std::vector<std::string> expected_tensors(const Weights& w) {
-    std::vector<std::string> v = {"model.embed_tokens.weight", "model.norm.weight"};
-    for (int l = 0; l < w.L; ++l) {
-        const std::string p = "model.layers." + std::to_string(l) + ".";
-        for (const char* s : {"input_layernorm.weight", "post_attention_layernorm.weight", "self_attn.q_proj.weight",
-                              "self_attn.k_proj.weight", "self_attn.v_proj.weight", "self_attn.o_proj.weight"})
-            v.push_back(p + s);
-        if (w.cfg.arch == FL_ARCH_MIXTRAL) {
-            v.push_back(p + "block_sparse_moe.gate.weight");
-            for (int e = w.rank * w.E_local; e < (w.rank + 1) * w.E_local; ++e)
-                for (const char* s : {"w1.weight", "w2.weight", "w3.weight"})
-                    v.push_back(p + "block_sparse_moe.experts." + std::to_string(e) + "." + s);
-        } else {
-            for (const char* s : {"mlp.gate_proj.weight", "mlp.up_proj.weight", "mlp.down_proj.weight"}) v.push_back(p + s);
-        }
-        if (w.cfg.qkv_bias)
-            for (const char* s : {"self_attn.q_proj.bias", "self_attn.k_proj.bias", "self_attn.v_proj.bias"}) v.push_back(p + s);
-    }
-    return v;
-}
-
-static void put_tensor(Weights& w, const char* name, int dtype, const int64_t* shape, int rank, const void* host) {
-    FL_CHECK(!w.finalized, FL_ERR_STATE, "model already finalized");
-    TensorRoute r;
+void TensorTable::put(const char* name, int dtype, const int64_t* shape, int rank, const void* host) {
+    FL_CHECK(!finalized, FL_ERR_STATE, "model already finalized");
     // Names the model does not read are skipped, as candle's VarBuilder ignores the extra entries of the HashMap the loader hands
     // over (huggingface.rs:81-130 loads EVERY tensor of the checkpoint: `self_attn.rotary_emb.inv_freq` in older Llama exports,
-    // `visual.*` in Qwen2_5_VLForConditionalGeneration, ...).  finalize() stays the strict gate: a MISSING tensor is an error.
-    if (!route_tensor(w, name, r)) return;
-    if (r.base == nullptr) return;       // an expert that lives on another expert-parallel rank
-    int64_t numel = 1;
-    for (int i = 0; i < rank; ++i) numel *= shape[i];
-    const bool shape_ok = (r.kind == TensorRoute::BF16_MAT) ? (rank == 2 && shape[0] == r.full_rows && shape[1] == r.full_cols)
-                                                            : ((rank == 1 && shape[0] == r.full_rows) || (rank == 2 && shape[0] * shape[1] == r.full_rows));
+    // `visual.*` in Qwen2_5_VLForConditionalGeneration, BERT's pooler, the experts of another expert-parallel rank, ...).
+    // check_complete() stays the strict gate: a MISSING tensor is an error.
+    const auto it = index.find(name);
+    if (it == index.end()) return;
+    const TensorSlot& s = slots[it->second];
+    if (f32_only) FL_CHECK(dtype == FL_DTYPE_F32, FL_ERR_UNSUPPORTED, "BERT tensors must be f32 (the reference loads MiniLM as F32, embeddings.rs:298)");
+    // a causal-LM vector may also come as [rows, cols] with rows x cols elements
+    const bool shape_ok = s.mat ? (rank == 2 && shape[0] == s.full_rows && shape[1] == s.full_cols)
+                                : ((rank == 1 && shape[0] == s.full_rows) || (!f32_only && rank == 2 && shape[0] * shape[1] == s.full_rows));
     FL_CHECK(shape_ok, FL_ERR_INVALID, std::string("shape mismatch for ") + name);
     FL_CHECK(dtype == FL_DTYPE_F32 || dtype == FL_DTYPE_BF16 || dtype == FL_DTYPE_F16, FL_ERR_INVALID, "bad dtype");
     // keep this rank's window of the full tensor, converted to bf16 bit patterns (round-to-nearest-even), the dtype the
     // reference server loads into (main.rs:120)
-    numel = r.rows * r.cols;
+    const int64_t numel = s.rows * s.cols;
     std::vector<uint16_t> bits((size_t)numel);
-    for (int64_t lr = 0; lr < r.rows; ++lr) {
-        const int64_t src = (lr + r.src_row0) * r.full_cols + r.src_col0;
-        uint16_t* dstp = bits.data() + (size_t)lr * r.cols;
+    for (int64_t lr = 0; lr < s.rows; ++lr) {
+        const int64_t src = (lr + s.row0) * s.full_cols + s.col0;
+        uint16_t* dstp = bits.data() + (size_t)lr * s.cols;
         if (dtype == FL_DTYPE_BF16) {
-            std::memcpy(dstp, (const uint16_t*)host + src, (size_t)r.cols * 2);
+            std::memcpy(dstp, (const uint16_t*)host + src, (size_t)s.cols * 2);
         } else if (dtype == FL_DTYPE_F32) {
             const float* f = (const float*)host + src;
-            for (int64_t i = 0; i < r.cols; ++i) dstp[i] = host_f32_to_bf16(f[i]);
+            for (int64_t i = 0; i < s.cols; ++i) dstp[i] = host_f32_to_bf16(f[i]);
         } else {
             const uint16_t* h = (const uint16_t*)host + src;
-            for (int64_t i = 0; i < r.cols; ++i) dstp[i] = host_f32_to_bf16(host_f16_to_f32(h[i]));
+            for (int64_t i = 0; i < s.cols; ++i) dstp[i] = host_f32_to_bf16(host_f16_to_f32(h[i]));
         }
     }
-    if (r.kind == TensorRoute::BF16_MAT) {
-        uint16_t* dst = (uint16_t*)r.base;
-        const size_t rowb = (size_t)r.cols * 2;
+    uint8_t* base = slab.p + s.off;
+    if (s.mat) {
+        uint16_t* dst = (uint16_t*)base;
+        const size_t rowb = (size_t)s.cols * 2;
         if (numel == 0) {
             // a rank that holds only padding heads of this tensor
-        } else if (r.map.mode == 0) {
-            FL_CUDA(cudaMemcpy2D(dst + r.map.dst_row0 * r.ld, (size_t)r.ld * 2, bits.data(), rowb, rowb, (size_t)r.rows, cudaMemcpyHostToDevice));
-        } else if (r.map.mode == 2) {
-            FL_CUDA(cudaMemcpy2D(dst + (size_t)r.map.lane * r.cols, 2 * rowb, bits.data(), rowb, rowb, (size_t)r.rows,
+        } else if (s.map.mode == 0) {
+            FL_CUDA(cudaMemcpy2D(dst + s.map.dst_row0 * s.ld, (size_t)s.ld * 2, bits.data(), rowb, rowb, (size_t)s.rows, cudaMemcpyHostToDevice));
+        } else if (s.map.mode == 2) {
+            FL_CUDA(cudaMemcpy2D(dst + (size_t)s.map.lane * s.cols, 2 * rowb, bits.data(), rowb, rowb, (size_t)s.rows,
                                  cudaMemcpyHostToDevice));
         } else {
             std::vector<uint16_t> perm((size_t)numel);
-            for (int64_t row = 0; row < r.rows; ++row)
-                std::memcpy(perm.data() + (size_t)(r.map.map(row) - r.map.dst_row0) * r.cols, bits.data() + (size_t)row * r.cols, rowb);
-            FL_CUDA(cudaMemcpy(dst + r.map.dst_row0 * r.cols, perm.data(), (size_t)numel * 2, cudaMemcpyHostToDevice));
+            for (int64_t row = 0; row < s.rows; ++row)
+                std::memcpy(perm.data() + (size_t)(s.map.map(row) - s.map.dst_row0) * s.cols, bits.data() + (size_t)row * s.cols, rowb);
+            FL_CUDA(cudaMemcpy(dst + s.map.dst_row0 * s.cols, perm.data(), (size_t)numel * 2, cudaMemcpyHostToDevice));
         }
     } else {
-        std::vector<float> vals((size_t)r.rows);
-        for (int64_t row = 0; row < r.rows; ++row) {
-            const uint32_t b = (uint32_t)bits[row] << 16;
+        std::vector<float> vals((size_t)s.rows);
+        for (int64_t row = 0; row < s.rows; ++row) {
             float f;
-            std::memcpy(&f, &b, 4);
-            vals[(size_t)(r.map.map(row) - r.map.dst_row0)] = f;
+            if (s.round) {
+                const uint32_t b = (uint32_t)bits[row] << 16;
+                std::memcpy(&f, &b, 4);
+            } else {
+                f = ((const float*)host)[row + s.row0];   // as uploaded (only f32-only tables keep vectors unrounded)
+            }
+            vals[(size_t)(s.map.map(row) - s.map.dst_row0)] = f;
         }
-        FL_CUDA(cudaMemcpy((float*)r.base + r.map.dst_row0, vals.data(), (size_t)r.rows * 4, cudaMemcpyHostToDevice));
+        FL_CUDA(cudaMemcpy((float*)base + s.map.dst_row0, vals.data(), (size_t)s.rows * 4, cudaMemcpyHostToDevice));
     }
-    w.have.insert(name);
-    if (std::string(name) == "lm_head.weight") w.lm_head_loaded = true;
+    have.insert(name);
 }
 
-static void random_init(Weights& w, uint64_t seed, float stdv) {
-    FL_CHECK(!w.finalized, FL_ERR_STATE, "model already finalized");
-    std::vector<std::string> names = expected_tensors(w);
-    names.push_back("lm_head.weight");
-    for (const std::string& n : names) {
-        TensorRoute r;
-        FL_CHECK(route_tensor(w, n, r), FL_ERR_INVALID, "internal: unroutable " + n);
-        const bool is_norm = n.size() >= 11 && n.compare(n.size() - 11, 11, "norm.weight") == 0;
-        const uint64_t ts = tensor_seed(seed, n.c_str());
-        if (r.kind == TensorRoute::BF16_MAT) {
-            synth_fill_bf16_kernel<<<kNumSMs * 8, 256>>>((uint16_t*)r.base, r.rows, r.cols, r.ld, ts, stdv, r.map,
-                                                         SrcWin{r.src_row0, r.src_col0, r.full_cols});
-        } else if (is_norm) {
-            fill_f32_kernel<<<8, 256>>>((float*)r.base, r.rows, 1.0f);
-        } else {
-            synth_fill_f32_kernel<<<8, 256>>>((float*)r.base, r.rows, ts, stdv, r.map, r.src_row0);
-        }
+// One launch per slot; element values depend only on the seed, the exact HF name and the full-tensor index (oracle/synth.py).
+void TensorTable::random_init(uint64_t seed, float stdv) {
+    FL_CHECK(!finalized, FL_ERR_STATE, "model already finalized");
+    for (const TensorSlot& s : slots) {
+        uint8_t* base = slab.p + s.off;
+        const uint64_t ts = tensor_seed(seed, s.name.c_str());
+        if (s.mat)
+            synth_fill_bf16_kernel<<<kNumSMs * 8, 256>>>((uint16_t*)base, s.rows, s.cols, s.ld, ts, stdv, s.map,
+                                                         SrcWin{s.row0, s.col0, s.full_cols});
+        else if (s.ones)
+            fill_f32_kernel<<<8, 256>>>((float*)base + s.map.dst_row0, s.rows, 1.0f);
+        else
+            synth_fill_f32_kernel<<<8, 256>>>((float*)base, s.rows, ts, stdv, s.map, s.row0);
         g_launches.fetch_add(1);
-        w.have.insert(n);
+        have.insert(s.name);
     }
-    w.lm_head_loaded = true;
     FL_CUDA(cudaGetLastError());
     FL_CUDA(cudaDeviceSynchronize());
 }
 
 static void finalize(Weights& w) {
-    FL_CHECK(!w.finalized, FL_ERR_STATE, "model already finalized");
-    for (const std::string& n : expected_tensors(w))
-        FL_CHECK(w.have.count(n), FL_ERR_STATE, "missing tensor: " + n);
-    if (!w.lm_head_loaded) w.lm_head = w.embed;   // candle qwen2: tied embeddings when lm_head.weight is absent
+    w.table.check_complete();
+    if (!w.table.have.count("lm_head.weight")) w.lm_head = w.embed;   // candle qwen2: tied embeddings when lm_head.weight is absent
     // RoPE tables (see oracle/candle_ops.py rope_tables for the candle rule being followed)
     const int half = w.d / 2;
     std::vector<float> cs((size_t)w.max_pos * half), sn((size_t)w.max_pos * half);
@@ -549,7 +330,7 @@ static void finalize(Weights& w) {
         w.pk_tmaps.alloc(tm.size());
         FL_CUDA(cudaMemcpy(w.pk_tmaps.p, tm.data(), tm.size() * sizeof(CUtensorMap), cudaMemcpyHostToDevice));
     }
-    w.finalized = true;
+    w.table.finalized = true;
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -728,7 +509,7 @@ static void launch_persistent(fl_cache& c, int nsteps, bool feedback) {
 
 static void cache_create(fl_cache& c, int max_batch, int max_seq) {
     const Weights& w = *c.w;
-    FL_CHECK(w.finalized, FL_ERR_STATE, "model not finalized");
+    FL_CHECK(w.table.finalized, FL_ERR_STATE, "model not finalized");
     FL_CHECK(max_batch >= 1 && max_batch <= kMaxBatch && max_seq >= 1, FL_ERR_INVALID, "bad cache dimensions");
     c.max_batch = max_batch;
     c.max_seq = max_seq;
@@ -1428,6 +1209,19 @@ static void forward_guard(fl_model* m, fl_cache* c, bool args_ok, F&& body) {
     }
 }
 
+// Body of a weight-loading entry point: f on the model's Weights (causal LM) or BertModel, under the model's mutex.
+template <typename F>
+static void with_model(fl_model* m, F&& f) {
+    auto locked = [&](auto& x) {
+        std::lock_guard<std::mutex> g(x.mu);
+        f(x);
+    };
+    if (m->bert)
+        locked(*m->bert);
+    else
+        locked(*m->w);
+}
+
 extern "C" {
 
 FL_EXPORT const char* fl_last_error(void) { return g_last_error.c_str(); }
@@ -1467,7 +1261,9 @@ FL_EXPORT int fl_model_create(const fl_config* cfg, fl_model** out) {
     if (cfg->arch == FL_ARCH_BERT) {
         auto bm = std::make_shared<BertModel>();
         bm->cfg = *cfg;
-        bert_build(*bm);
+        bert_plan(*bm);
+        bm->table.alloc();
+        FL_CUDA(cudaStreamCreateWithFlags(&bm->stream, cudaStreamNonBlocking));
         *out = new fl_model{nullptr, bm};
         return FL_OK;
     }
@@ -1477,7 +1273,9 @@ FL_EXPORT int fl_model_create(const fl_config* cfg, fl_model** out) {
     auto w = std::make_shared<Weights>();
     w->cfg = *cfg;
     w->device = g_device.load();
-    build_weights(*w);
+    plan_weights(*w);
+    with_head_dim(w->d, [](auto) {});   // a head size the kernels are built for
+    w->table.alloc();
     *out = new fl_model{w, nullptr};
     FL_API_END
 }
@@ -1486,13 +1284,7 @@ FL_EXPORT int fl_model_put_tensor(fl_model* m, const char* name, int dtype, cons
     FL_API_BEGIN
     FL_CHECK(m && name && shape && host_ptr, FL_ERR_INVALID, "NULL argument");
     use_device();
-    if (m->bert) {
-        std::lock_guard<std::mutex> g(m->bert->mu);
-        bert_put_tensor(*m->bert, name, dtype, shape, rank, host_ptr);
-        return FL_OK;
-    }
-    std::lock_guard<std::mutex> g(m->w->mu);
-    put_tensor(*m->w, name, dtype, shape, rank, host_ptr);
+    with_model(m, [&](auto& x) { x.table.put(name, dtype, shape, rank, host_ptr); });
     FL_API_END
 }
 
@@ -1500,13 +1292,7 @@ FL_EXPORT int fl_model_random_init(fl_model* m, uint64_t seed, float stdv) {
     FL_API_BEGIN
     FL_CHECK(m, FL_ERR_INVALID, "NULL argument");
     use_device();
-    if (m->bert) {
-        std::lock_guard<std::mutex> g(m->bert->mu);
-        bert_random_init(*m->bert, seed, stdv);
-        return FL_OK;
-    }
-    std::lock_guard<std::mutex> g(m->w->mu);
-    random_init(*m->w, seed, stdv);
+    with_model(m, [&](auto& x) { x.table.random_init(seed, stdv); });
     FL_API_END
 }
 
@@ -1514,13 +1300,7 @@ FL_EXPORT int fl_model_finalize(fl_model* m) {
     FL_API_BEGIN
     FL_CHECK(m, FL_ERR_INVALID, "NULL argument");
     use_device();
-    if (m->bert) {
-        std::lock_guard<std::mutex> g(m->bert->mu);
-        bert_finalize(*m->bert);
-        return FL_OK;
-    }
-    std::lock_guard<std::mutex> g(m->w->mu);
-    finalize(*m->w);
+    with_model(m, [](auto& x) { finalize(x); });
     FL_API_END
 }
 

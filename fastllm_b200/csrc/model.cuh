@@ -2,7 +2,6 @@
 #pragma once
 #include <map>
 #include <memory>
-#include <set>
 #include <string>
 #include <vector>
 
@@ -11,6 +10,7 @@
 #include "decode_persistent.cuh"
 #include "gemv.cuh"
 #include "runtime.cuh"
+#include "tensor_table.hpp"
 
 namespace fl {
 
@@ -47,7 +47,7 @@ struct Weights {
     bool ep_dp = false;         // expert parallelism with data-parallel attention (fl_config.ep_dp_attention)
     int Vfull = 0;              // full vocabulary (embedding table rows, logits length); V = Vfull / tp rows of lm_head live here
     int device = 0;
-    DevBuf<uint8_t> slab;       // every weight lives in this one allocation
+    TensorTable table;
     uint16_t* embed = nullptr;  // [V, H]
     uint16_t* lm_head = nullptr;
     float* final_norm = nullptr;
@@ -56,9 +56,6 @@ struct Weights {
     DevBuf<CUtensorMap> pk_tmaps; // [4 L + 1] 3-D TMA descriptors of the weight stream (phase g = 4 layer + {qkv, o, gate|up, down}; lm_head last)
     float* rope_cos = nullptr;  // [max_pos, d/2]
     float* rope_sin = nullptr;
-    std::set<std::string> have; // tensor names that arrived
-    bool lm_head_loaded = false;
-    bool finalized = false;
     uint64_t streamed_bytes = 0;
     CUtensorMap tm_head;
     bool dense_ok = false;      // shapes admit the dense (tcgen05) path for 3+ rows

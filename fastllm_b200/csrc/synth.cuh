@@ -1,6 +1,7 @@
 // Device side of the deterministic synthetic-weight rule (see oracle/synth.py for the specification).
 #pragma once
 #include "common.cuh"
+#include "row_map.cuh"
 
 namespace fl {
 
@@ -28,30 +29,12 @@ __device__ __forceinline__ uint16_t synth_bf16(uint64_t tseed, uint64_t i, float
     return f32_to_bf16_rne(v);
 }
 
-// Fills a [rows, cols] logical tensor into `dst`, where logical row r lands at physical row
-// dst_row0 + perm(r) * dst_row_stride_rows (see RowMap in model.cu); element index = r * cols + c.
-struct RowMap {
-    int64_t dst_row0;   // first physical row
-    int32_t mode;       // 0 identity, 1 rope-pair permutation within heads of `head_dim` rows, 2 interleave (phys = 2*r + lane)
-    int32_t head_dim;
-    int32_t lane;       // for mode 2: 0 = gate rows (even), 1 = up rows (odd)
-    __host__ __device__ int64_t map(int64_t r) const {
-        if (mode == 1) {
-            int64_t h = r / head_dim, i = r % head_dim;
-            int64_t half = head_dim / 2;
-            int64_t j = (i < half) ? 2 * i : 2 * (i - half) + 1;
-            return dst_row0 + h * head_dim + j;
-        }
-        if (mode == 2) return dst_row0 + 2 * r + lane;
-        return dst_row0 + r;
-    }
-};
-
 // The local [rows, cols] block is the window (src_row0.., src_col0..) of a full tensor with src_cols_full columns (tensor-
 // parallel shards); element values depend only on the FULL-tensor index, so every shard layout sees the same weights.
 struct SrcWin {
     int64_t row0, col0, cols_full;   // cols_full == 0: the block is the whole tensor
 };
+// Fills a [rows, cols] logical tensor into `dst`: logical row r lands at physical row map.map(r); element index = r * cols + c.
 // `ld` = leading dimension of the destination matrix (== cols unless the local matrix carries zero-padded columns).
 static __global__ void synth_fill_bf16_kernel(uint16_t* dst, int64_t rows, int64_t cols, int64_t ld, uint64_t tseed, float stdv, RowMap map,
                                               SrcWin win = SrcWin{0, 0, 0}) {

@@ -62,6 +62,18 @@ class DeviceModel:
     def finalize(self):
         _lib.check(self.lib.fl_model_finalize(self.h))
 
+    def load(self, tensors, random_seed=None, std: float = 0.02, dtype=None):
+        """Synthetic weights (tensors=None: fl_model_random_init with random_seed, default 0) or an upload of `tensors`, then
+        finalize.  `tensors` is a dict or any iterable of (name, array) -- e.g. safetensors_io.iter_tensors(dir), which hands over
+        views of the memory-mapped checkpoint one tensor at a time (huggingface.rs:81-130 without the whole-file reads); `dtype`
+        casts every array first."""
+        if tensors is None:
+            self.random_init(0 if random_seed is None else random_seed, std)
+        else:
+            for name, arr in (tensors.items() if hasattr(tensors, "items") else tensors):
+                self.put_tensor(name, np.asarray(arr, dtype=dtype))
+        self.finalize()
+
     def clone(self) -> "DeviceModel":
         h = C.c_void_p()
         _lib.check(self.lib.fl_model_clone(self.h, C.byref(h)))
@@ -313,14 +325,7 @@ class _CausalBase:
         VarBuilder::from_tensors(.., BF16, ..) would (main.rs:120).  tensors=None + random_seed = synthetic weights."""
         cfg = cls._to_fl_config(config)
         dev = DeviceModel(cfg, device)
-        if tensors is None:
-            dev.random_init(0 if random_seed is None else random_seed, std)
-        else:
-            # a dict, or any iterable of (name, array) -- e.g. safetensors_io.iter_tensors(dir), which hands over views of the
-            # memory-mapped checkpoint one tensor at a time (huggingface.rs:81-130 without the whole-file reads)
-            for name, arr in (tensors.items() if hasattr(tensors, "items") else tensors):
-                dev.put_tensor(name, np.asarray(arr))
-        dev.finalize()
+        dev.load(tensors, random_seed, std)
         self = cls(dev, cfg)
         return self, cls.initialize_cache(device, dtype)
 
@@ -665,12 +670,7 @@ class MiniLMModel:
         c.rope_theta, c.tp_rank, c.tp_size = 0.0, 0, 1
         self.config, self._model_id = config, model_id
         self.dev = DeviceModel(c, device)
-        if tensors is None:
-            self.dev.random_init(0 if random_seed is None else random_seed, std)
-        else:
-            for name, arr in tensors.items():
-                self.dev.put_tensor(name, np.asarray(arr, dtype=np.float32))
-        self.dev.finalize()
+        self.dev.load(tensors, random_seed, std, np.float32)
 
     @classmethod
     def get_family(cls) -> str:

@@ -1,6 +1,6 @@
 """Tensor-parallel plumbing on the host side: one process per GPU, torch.distributed for the rendezvous, the library
 owns the NCCL communicator (fl_comm_*).  Also the Python statement of the sharding scheme the library applies when a model
-is created with tp_size > 1 (csrc/fl_lib.cu route_tensor): column-parallel q/k/v (by head) and gate/up, row-parallel
+is created with tp_size > 1 (csrc/weights_plan.cuh plan_weights): column-parallel q/k/v (by head) and gate/up, row-parallel
 o_proj / down_proj (+ all-reduce), vocab-parallel lm_head (+ all-gather); embeddings and norms replicated.
 """
 from __future__ import annotations
@@ -38,7 +38,7 @@ def init_tensor_parallel(rank: int, world: int, device: int):
 
 
 def head_layout(nh: int, nkv: int, rank: int, tp: int):
-    """(q_head0, q_real, nh_local, kv_head0, nkv_local) of `rank`: the statement of build_weights() in csrc/fl_lib.cu.
+    """(q_head0, q_real, nh_local, kv_head0, nkv_local) of `rank`: the statement of plan_weights() in csrc/weights_plan.cuh.
     tp <= kv heads: an equal split by head.  tp > kv heads (Qwen2.5-7B at TP-8: 28 q / 4 kv heads): every kv head lives on
     rep = tp / nkv ranks and its query group is dealt out ceil(group / rep) heads per rank, the last rank of a group padding
     with zero heads (zero q rows, zero o_proj columns)."""

@@ -87,7 +87,7 @@ def test_tpN_matches_tp1_at_true_widths(n, tmp_path):
 
 
 def test_head_layout_more_ranks_than_kv_heads():
-    """tp.head_layout (the Python statement of build_weights in csrc/fl_lib.cu): Qwen2.5-7B (28 q / 4 kv heads) at TP-8 replicates each
+    """tp.head_layout (the Python statement of plan_weights in csrc/weights_plan.cuh): Qwen2.5-7B (28 q / 4 kv heads) at TP-8 replicates each
     kv head on two ranks and deals its 7 query heads 4 + 3 (+1 zero head); every q head is owned exactly once; Mistral-7B at TP-8
     is the plain split."""
     from fastllm_b200 import tp
