@@ -52,6 +52,7 @@ SYMBOLS = {
     "fl_forward": (_I, [_VP, _VP, _VP, _I, _I, _SZ, _VP]),
     "fl_forward_greedy": (_I, [_VP, _VP, _VP, _I, _I, _SZ, _VP]),
     "fl_decode_greedy_loop": (_I, [_VP, _VP, _VP, _I, _SZ, _I, _VP, C.POINTER(C.c_float)]),
+    "fl_forward_logprobs": (_I, [_VP, _VP, _VP, _VP, _I, _I, _SZ, _VP, _VP]),
     "fl_sampler_create": (_I, [_U64, C.c_double, C.POINTER(_VP)]),
     "fl_sampler_sample": (_I, [_VP, _VP, _SZ, C.POINTER(C.c_uint32)]),
     "fl_argmax_rows": (_I, [_VP, _I, _SZ, _VP]),

@@ -5,6 +5,7 @@
 // These kernels implement the same fused steps as the GEMV epilogues in gemv.cuh (SURVEY.md section 2.4 K1-K18).
 #pragma once
 #include "common.cuh"
+#include "gemm_tc.cuh"
 #include "gemv.cuh"
 
 namespace fl {
@@ -540,6 +541,36 @@ static __global__ void __launch_bounds__(1024) dense_argmax_kernel(const float* 
         for (int w = 1; w < (int)(blockDim.x >> 5); ++w)
             if (sv[w] > v || (sv[w] == v && si[w] > idx)) { v = sv[w]; idx = si[w]; }
         next_ids[blockIdx.x] = (uint32_t)idx;
+    }
+}
+
+// Scoring: one warp per row merges the row's nparts soft-max partials (the lm_head's GEPI_LOGPROB epilogue) -- lane l takes
+// partials l, l + 32, ... in order, then a fixed butterfly -- so the result does not depend on the grid.
+// logprob[row] = z[target] - (m + log s); argmax[row] = the last index among equal maxima (a NaN never wins).
+constexpr int kLogprobRowsPerCta = 8;
+static __global__ void __launch_bounds__(32 * kLogprobRowsPerCta) logprob_combine_kernel(const LogprobPart* __restrict__ part, int nparts,
+                                                                                       const float* __restrict__ target_logit, int R,
+                                                                                       float* __restrict__ logprob, uint32_t* __restrict__ argmax) {
+    pdl_launch_dependents();
+    pdl_wait();
+    const int row = blockIdx.x * kLogprobRowsPerCta + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (row >= R) return;
+    const LogprobPart* p = part + (size_t)row * nparts;
+    float m = -INFINITY, s = 0.f;
+    int idx = -1;
+    for (int i = lane; i < nparts; i += 32) {
+        const LogprobPart q = p[i];
+        logprob_merge(m, s, idx, q.m, q.s, q.idx);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const float m2 = __shfl_xor_sync(0xFFFFFFFFu, m, o), s2 = __shfl_xor_sync(0xFFFFFFFFu, s, o);
+        const int i2 = __shfl_xor_sync(0xFFFFFFFFu, idx, o);
+        logprob_merge(m, s, idx, m2, s2, i2);
+    }
+    if (lane == 0) {
+        logprob[row] = target_logit[row] - (m + logf(s));
+        argmax[row] = (uint32_t)idx;
     }
 }
 

@@ -575,7 +575,7 @@ static void cache_destroy_graphs(fl_cache& c) {
 // Enqueue the whole forward for the flattened [b, t] call on lc.stream.  Rows are processed in passes of kPassRows,
 // pass-major / layer-minor: a token's layer-l attention only needs the layer-l K/V of EARLIER tokens, which earlier
 // passes already appended, so the order is causal-correct.
-static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool loop_mode);
+static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool loop_mode, bool score = false);
 
 // A uniform call of `rows` activation rows runs on the dense (tcgen05) path: 3+ rows, or any Mixtral call.
 static bool uses_dense(const fl_cache& c, int rows) {
@@ -849,7 +849,40 @@ static int dense_gemm_grouped(fl_cache& c, LaunchCtx& lc, const char* tag, int g
     return ks;
 }
 
-static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool loop_mode) {
+// Workspace of scoring calls over `rows` rows (fl_forward_logprobs), sized on first use like the dense workspace.
+static void ensure_logprob_ws(fl_cache& c, int rows) {
+    DenseWs& d = c.dw;
+    if ((size_t)rows <= d.lp_rows) return;
+    FL_CUDA(cudaStreamSynchronize(c.stream));
+    const size_t R = rows;
+    d.lp_part.alloc(R * ((c.w->V + 255) / 256) * (kGemmEpiWarps / 4));
+    d.lp_target_logit.alloc(R);
+    d.lp_targets.alloc(R);
+    d.lp_out.alloc(2 * R);
+    d.h_lp.alloc(2 * R);
+    d.lp_rows = R;
+}
+
+// Scoring lm_head over the R final-normed rows in xhi / xlo: the prefill orientation at every R (tokens as M, 128 x 256 tiles, no
+// split-K: partial sums cannot go through a soft-max), its epilogue reducing every (row, tile) to soft-max partials, then one warp
+// per row merges them into the log-prob of the row's target and its arg-max (lp_out).  Nothing of size [R, V] is stored; pad rows
+// of the last M tile arrive zero-filled from TMA and are not stored.
+static void enqueue_lm_head_logprobs(fl_cache& c, LaunchCtx& lc, int R) {
+    const Weights& w = *c.w;
+    DenseWs& d = c.dw;
+    const int ntn = (w.V + 255) / 256, tiles = ((R + kGemmBM - 1) / kGemmBM) * ntn;
+    const CUtensorMap hi = make_tmap_bf16(d.xhi.p, R, w.H, w.H, kGemmBM), lo = make_tmap_bf16(d.xlo.p, R, w.H, w.H, kGemmBM);
+    GemmArgs g{R, w.V, w.H, nullptr, nullptr, 0, d.lp_part.p, 0, 1, 0};
+    g.lp_targets = d.lp_targets.p;
+    g.lp_target_logit = d.lp_target_logit.p;
+    launch(lc, "gemm_tc_lm_head_logprob", (uint64_t)w.V * w.H * 2, gemm_tc_kernel<256, GEPI_LOGPROB, DUAL_A>, dim3(std::min(tiles, kNumSMs)),
+           dim3(kGemmThreads), gemm_smem_bytes(256, DUAL_A), hi, lo, w.tm_head, g);
+    launch(lc, "logprob_combine", (uint64_t)R * ntn * (kGemmEpiWarps / 4) * sizeof(LogprobPart), logprob_combine_kernel,
+           dim3((R + kLogprobRowsPerCta - 1) / kLogprobRowsPerCta), dim3(32 * kLogprobRowsPerCta), 0, (const LogprobPart*)d.lp_part.p,
+           ntn * (kGemmEpiWarps / 4), (const float*)d.lp_target_logit.p, R, reinterpret_cast<float*>(d.lp_out.p), d.lp_out.p + R);
+}
+
+static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool loop_mode, bool score) {
     const Weights& w = *c.w;
     DenseWs& d = c.dw;
     const int R = b * t;
@@ -1015,10 +1048,16 @@ static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool
         if (l + 1 < w.L) {   // K16 + next layer's K2
             pa.norm_w = w.layers[l + 1].ln1;
             prep("dense_resid_rmsnorm", pa, R);
-        } else {             // K16 + K17: only the last token of every sequence goes on to the lm_head
-            pa.norm_w = w.final_norm; pa.last_only = 1;
-            prep("dense_final_rmsnorm", pa, b);
+        } else {             // K16 + K17: only the last token of every sequence goes on to the lm_head (scoring: every token)
+            pa.norm_w = w.final_norm; pa.last_only = score ? 0 : 1;
+            prep("dense_final_rmsnorm", pa, score ? R : b);
         }
+    }
+    if (score) {
+        enqueue_lm_head_logprobs(c, lc, R);
+        launch(lc, "advance_state", 0, advance_state_kernel, dim3(1), dim3(kMaxBatch), 0, c.state.p, b, t, 0, c.ids.p, (const uint32_t*)c.next_ids.p, 0,
+               (uint32_t*)nullptr, (int*)nullptr);
+        return;
     }
     const int ksh = dense_gemm(c, lc, "gemm_tc_lm_head", b, w.V, w.H, w.tm_head, d.y.p);
     if (w.tp > 1) {   // vocab-parallel head
@@ -1038,9 +1077,10 @@ static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool
 }
 
 // mode 0: one decode step of a uniform batch; 1: the same inside the device-resident greedy loop; 2: one decode step of a ragged
-// batch (fl_forward_slots: always the dense path, whatever the row count)
+// batch (fl_forward_slots: always the dense path, whatever the row count); 3: a scoring call (fl_forward_logprobs: always the
+// dense path, log-probs and arg-max of every row)
 static void enqueue_step(fl_cache& c, LaunchCtx& lc, int b, int t, int mode) {
-    if (mode == 2) enqueue_forward_dense(c, lc, b, t, false);
+    if (mode >= 2) enqueue_forward_dense(c, lc, b, t, false, mode == 3);
     else enqueue_forward(c, lc, b, t, mode == 1);
 }
 
@@ -1070,11 +1110,11 @@ static GraphEntry& get_graph(fl_cache& c, int b, int mode) {
 // Enqueues `steps` forward steps of b x t rows on the cache's stream (mode as in enqueue_step; several steps only in the greedy
 // loop) and advances kv_len by t per step (not in mode 2: ragged calls keep per-slot lengths).  Batch-1 decode runs in the
 // persistent kernel, all steps in one launch.  Other single-token steps replay the step's CUDA graph, except inside a profile
-// window, whose per-kernel events a graph cannot record.  Everything else is enqueued kernel by kernel.  `ev`, if given, brackets
-// the enqueued work; a graph is captured before it.
+// window, whose per-kernel events a graph cannot record, and scoring calls, which are prefill-shaped.  Everything else is enqueued
+// kernel by kernel.  `ev`, if given, brackets the enqueued work; a graph is captured before it.
 static void run_steps(fl_cache& c, int b, int t, int mode, int steps, const EventPair* ev = nullptr) {
-    const bool persistent = mode != 2 && b == 1 && t == 1 && c.pk.ok;
-    const bool use_graph = !persistent && t == 1 && !g_prof.on && !env_flag("FL_NO_GRAPH");
+    const bool persistent = mode <= 1 && b == 1 && t == 1 && c.pk.ok;
+    const bool use_graph = !persistent && mode != 3 && t == 1 && !g_prof.on && !env_flag("FL_NO_GRAPH");
     const GraphEntry* g = use_graph ? &get_graph(c, b, mode) : nullptr;
     if (ev) FL_CUDA(cudaEventRecord(ev->e0, c.stream));
     if (persistent) {
@@ -1109,16 +1149,27 @@ static void check_call(fl_cache& c, const uint32_t* ids, int b, int t, size_t ro
     for (int i = 0; i < b * t; ++i) FL_CHECK(ids[i] < (uint32_t)w.Vfull, FL_ERR_INVALID, "token id out of range");
 }
 
-static void run_forward(fl_cache& c, const uint32_t* ids, int b, int t, size_t rope_offset) {
+// One uniform forward of ids [b, t]; with `targets` ([b, t], the token each position is scored against) a scoring call (mode 3).
+// Everything is validated before the first device operation.
+static void run_forward(fl_cache& c, const uint32_t* ids, int b, int t, size_t rope_offset, const uint32_t* targets = nullptr) {
     check_call(c, ids, b, t, rope_offset, 0);
-    if (uses_dense(c, b * t)) ensure_dense_ws(c, b * t);
-    std::memcpy(c.h_ids.p, ids, (size_t)b * t * 4);
-    FL_CUDA(cudaMemcpyAsync(c.ids.p, c.h_ids.p, (size_t)b * t * 4, cudaMemcpyHostToDevice, c.stream));
+    const int R = b * t;
+    if (targets) {
+        for (int i = 0; i < R; ++i) FL_CHECK(targets[i] < (uint32_t)c.w->V, FL_ERR_INVALID, "target id out of range");
+        ensure_logprob_ws(c, R);
+    }
+    if (targets || uses_dense(c, R)) ensure_dense_ws(c, R);
+    std::memcpy(c.h_ids.p, ids, (size_t)R * 4);
+    FL_CUDA(cudaMemcpyAsync(c.ids.p, c.h_ids.p, (size_t)R * 4, cudaMemcpyHostToDevice, c.stream));
+    if (targets) {
+        std::memcpy(c.dw.h_lp.p, targets, (size_t)R * 4);
+        FL_CUDA(cudaMemcpyAsync(c.dw.lp_targets.p, c.dw.h_lp.p, (size_t)R * 4, cudaMemcpyHostToDevice, c.stream));
+    }
     set_state_kernel<<<1, 1, 0, c.stream>>>(c.state.p, (int)rope_offset);
     g_launches.fetch_add(1);
-    c.dw.route_rows = b * t;
+    c.dw.route_rows = R;
     c.fresh_call = c.kv_len == 0 && !c.slots_used;
-    run_steps(c, b, t, 0, 1);
+    run_steps(c, b, t, targets ? 3 : 0, 1);
 }
 
 // Ragged forward (continuous batching): batch row i is the sequence in cache slot slots[i], which holds slot_len[slots[i]]
@@ -1440,6 +1491,23 @@ FL_EXPORT int fl_forward_greedy(fl_model* m, fl_cache* c, const uint32_t* ids, i
         FL_CUDA(cudaStreamSynchronize(c.stream));
         check_peer_error();
         std::memcpy(next_ids, c.h_ids.p, (size_t)b * 4);
+    });
+    FL_API_END
+}
+
+FL_EXPORT int fl_forward_logprobs(fl_model* m, fl_cache* c, const uint32_t* ids, const uint32_t* targets, int b, int t, size_t rope_offset,
+                                  float* logprobs, uint32_t* argmax_ids) {
+    FL_API_BEGIN
+    forward_guard(m, c, targets && logprobs, [&](fl_cache& c) {
+        const Weights& w = *c.w;
+        FL_CHECK(w.cfg.tp_size <= 1, FL_ERR_UNSUPPORTED, "scoring needs an unsharded model (the vocab-parallel lm_head would need every rank's soft-max partials)");
+        FL_CHECK(w.dense_ok, FL_ERR_UNSUPPORTED, "scoring runs on the dense path: shapes must be multiples of 8");
+        run_forward(c, ids, b, t, rope_offset, targets);
+        const size_t R = (size_t)b * t;
+        FL_CUDA(cudaMemcpyAsync(c.dw.h_lp.p, c.dw.lp_out.p, (argmax_ids ? 2 : 1) * R * 4, cudaMemcpyDeviceToHost, c.stream));
+        FL_CUDA(cudaStreamSynchronize(c.stream));
+        std::memcpy(logprobs, c.dw.h_lp.p, R * 4);
+        if (argmax_ids) std::memcpy(argmax_ids, c.dw.h_lp.p + R, R * 4);
     });
     FL_API_END
 }

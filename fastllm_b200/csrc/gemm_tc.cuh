@@ -18,7 +18,7 @@
 
 namespace fl {
 
-enum : int { GEPI_BIAS_BF16 = 0, GEPI_BIAS_GELU_BF16 = 1, GEPI_BIAS_RESID_F32 = 2, GEPI_F32 = 3, GEPI_F32_T = 5, GEPI_SILU_HL = 6 };
+enum : int { GEPI_BIAS_BF16 = 0, GEPI_BIAS_GELU_BF16 = 1, GEPI_BIAS_RESID_F32 = 2, GEPI_F32 = 3, GEPI_F32_T = 5, GEPI_SILU_HL = 6, GEPI_LOGPROB = 7 };
 enum : int { DUAL_NONE = 0, DUAL_A = 1, DUAL_B = 2 };
 
 constexpr int kGemmBM = 128;
@@ -44,7 +44,24 @@ struct GemmArgs {
     int grp_m = 0;
     int grp_cap = 0;
     const int* grp_cnt = nullptr;
+    // GEPI_LOGPROB (the lm_head of a scoring call, prefill orientation): `out` receives one LogprobPart per (row, N tile, column
+    // slice), [M][ceil(N / BN)][4]; lp_target_logit[row] = D[row, lp_targets[row]]
+    const uint32_t* lp_targets = nullptr;
+    float* lp_target_logit = nullptr;
 };
+
+// Soft-max statistics of one row over a set of columns: m = the max, idx = the last column reaching it (a NaN never wins; -1 when
+// no column counted), s = sum of exp(z - m).  Partials merge in any fixed order (logprob_merge).
+struct LogprobPart {
+    float m, s;
+    int idx;
+};
+__device__ __forceinline__ void logprob_merge(float& m, float& s, int& idx, float m2, float s2, int i2) {
+    if (m2 > m || (m2 == m && i2 > idx)) idx = i2;       // the larger index among equal maxima
+    const float mn = fmaxf(m, m2);
+    s = mn == -INFINITY ? s + s2 : s * expf(m - mn) + s2 * expf(m2 - mn);
+    m = mn;
+}
 
 // ---- PTX wrappers ------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* tmap, int c0, int c1, uint64_t* bar) {
@@ -322,6 +339,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             const int row = mrow0 + q * 32 + lane;
             const int row_lim = grouped ? g.grp_m : g.M, col_lim = grouped ? gcnt : g.N;
             if (grouped) n0 = 0;
+            // GEPI_LOGPROB: this thread's soft-max statistics over its columns of the tile; -1: a pad row, or the target is elsewhere
+            float lp_m = -INFINITY, lp_s = 0.f;
+            int lp_i = -1;
+            const int lp_tgt = (EPI == GEPI_LOGPROB && row < g.M) ? (int)g.lp_targets[row] : -1;
             mbar_wait(&acc_full[as], (ti_now >> 1) & 1);
             tc_fence_after();
 #pragma unroll 1
@@ -341,6 +362,27 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 #pragma unroll
                         for (int j = 0; j < 16; ++j) r[j] = __float_as_uint(__uint_as_float(r[j]) + __uint_as_float(r[j + 16]));
                     }
+                }
+                if (EPI == GEPI_LOGPROB) {
+                    // thread == token: the reduction over the vocabulary is thread-local.  Columns >= N are the zero-filled weight
+                    // rows past the vocabulary and count nowhere.
+                    const int col = n0 + c0;
+                    float cm = -INFINITY, tz = 0.f;
+                    int ci = -1;
+#pragma unroll
+                    for (int j = 0; j < 32; ++j) {
+                        const float x = __uint_as_float(r[j]);
+                        if (col + j < g.N && x >= cm) { cm = x; ci = col + j; }      // columns ascend: >= keeps the last
+                        if (col + j == lp_tgt) tz = x;
+                    }
+                    const float cref = cm == -INFINITY ? 0.f : cm;
+                    float cs = 0.f;
+#pragma unroll
+                    for (int j = 0; j < 32; ++j)
+                        if (col + j < g.N) cs += __expf(__uint_as_float(r[j]) - cref);
+                    logprob_merge(lp_m, lp_s, lp_i, cm, cs, ci);
+                    if (lp_tgt >= col && lp_tgt < col + 32) g.lp_target_logit[row] = tz;
+                    continue;
                 }
                 if (EPI == GEPI_BIAS_RESID_F32) {
                     // f32 out = acc + bias + bf16 residual, 16 columns (64 bytes of f32) per pass: the residual rows (32 bytes each) come
@@ -467,6 +509,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                     }
                 }
             }
+            if (EPI == GEPI_LOGPROB && row < g.M)
+                reinterpret_cast<LogprobPart*>(g.out)[((size_t)row * nt + n0 / BN) * (kGemmEpiWarps / 4) + cslice] = LogprobPart{lp_m, lp_s, lp_i};
             // all TMEM reads of this warp are complete (tcgen05.wait::ld inside tmem_ld32): hand the stage back
             tc_fence_before();
             __syncwarp();

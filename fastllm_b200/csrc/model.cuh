@@ -94,6 +94,13 @@ struct DenseWs {
     DevBuf<float> comb;              // [ep sources][rows, H] expert outputs returned to this rank
     // (batched-decode attention partials: sk_acc / sk_ml above)
     DevBuf<int> counters;
+    // scoring calls (fl_forward_logprobs), sized on first use for lp_rows rows
+    size_t lp_rows = 0;
+    DevBuf<LogprobPart> lp_part;     // [rows][lm_head N tiles][4] soft-max partials of the lm_head epilogue
+    DevBuf<float> lp_target_logit;   // [rows]
+    DevBuf<uint32_t> lp_targets;     // [rows]
+    DevBuf<uint32_t> lp_out;         // [2][rows]: log-probs (f32 bits), then arg-max ids
+    PinnedBuf<uint32_t> h_lp;        // [2][rows] staging: the targets up, lp_out down
 };
 
 struct GraphKey {

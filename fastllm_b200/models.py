@@ -133,6 +133,22 @@ class DeviceCache:
                                               out.ctypes.data_as(C.c_void_p)))
         return out
 
+    def forward_logprobs(self, ids: np.ndarray, targets: np.ndarray, rope_offset: int):
+        """fl_forward_logprobs: ONE forward over ids [b, t] that feeds the cache like forward() and scores every position against
+        targets [b, t].  -> (log_softmax(logits)[target] f32 [b, t], arg-max u32 [b, t] with forward_greedy's tie rule)."""
+        ids = np.ascontiguousarray(ids, dtype=np.uint32)
+        if ids.ndim != 2:
+            raise FastllmError(-1, f"input must be [batch, seq], got shape {ids.shape}")
+        targets = np.ascontiguousarray(targets, dtype=np.uint32)
+        if targets.shape != ids.shape:
+            raise FastllmError(-1, f"targets must have the shape of ids {ids.shape}, got {targets.shape}")
+        b, t = ids.shape
+        lp = np.empty((b, t), dtype=np.float32)
+        am = np.empty((b, t), dtype=np.uint32)
+        _lib.check(self.lib.fl_forward_logprobs(self.model.h, self.h, ids.ctypes.data_as(C.c_void_p), targets.ctypes.data_as(C.c_void_p),
+                                                b, t, rope_offset, lp.ctypes.data_as(C.c_void_p), am.ctypes.data_as(C.c_void_p)))
+        return lp, am
+
     def forward_sample(self, ids: np.ndarray, rope_offset: int, logits_processor: "LogitsProcessor") -> int:
         """fl_forward + LogitsProcessor::sample of row 0 in one call (one V*4-byte read-back, no logits array on this side)."""
         ids = np.ascontiguousarray(ids, dtype=np.uint32)
@@ -312,6 +328,7 @@ class _CausalBase:
 
     def __init__(self, dev: DeviceModel, cfg: FlConfig):
         self.dev, self.cfg = dev, cfg
+        self._score: DeviceCache | None = None
 
     @classmethod
     def _to_fl_config(cls, config: ConfigFile) -> FlConfig:
@@ -339,6 +356,20 @@ class _CausalBase:
 
     def _capacity(self) -> int:
         return min(self.KV_CAPACITY, self.cfg.max_position_embeddings)
+
+    def logprobs(self, ids: np.ndarray, targets: np.ndarray):
+        """Scores ids [b, t] against targets [b, t] in one forward from an empty sequence at RoPE offset 0, for every family alike.
+        -> (log-probs f32 [b, t], arg-max u32 [b, t]).  Runs on a cache of its own, reset before and after each call, so the
+        generate caches (LlamaCache.inner, the Mistral/Qwen2 model-internal KV) are never touched."""
+        ids = np.asarray(ids)
+        b = ids.shape[0] if ids.ndim == 2 else 1
+        if self._score is None or self._score.max_batch < b:
+            self._score = DeviceCache(self.dev, max(self.MAX_BATCH, b), self._capacity())
+        self._score.reset()
+        try:
+            return self._score.forward_logprobs(ids, targets, 0)
+        finally:
+            self._score.reset()
 
 
 class LlamaWithConfig(_CausalBase):
@@ -513,6 +544,23 @@ class Model:
             logits = self.model.forward(np.array([[tok]], dtype=np.uint32), pos, self.cache)
             pos += 1
         return (out, trace) if return_logits else out
+
+    def loglikelihood(self, context_ids, continuation_ids):
+        """The `loglikelihood(context, continuation)` request of evaluation harnesses: ONE scoring call over context + continuation
+        (targets = the ids shifted left by one).  -> (sum of the continuation's log-probs, whether every continuation token is the
+        arg-max at its position).  Summed in f64 in position order, as host/fastllm_host.hpp does."""
+        ctx = np.asarray(context_ids, dtype=np.uint32).reshape(-1)
+        cont = np.asarray(continuation_ids, dtype=np.uint32).reshape(-1)
+        if ctx.size == 0 or cont.size == 0:
+            raise ValueError("loglikelihood needs a non-empty context and continuation")
+        ids = np.concatenate([ctx, cont])
+        targets = np.concatenate([ids[1:], np.zeros(1, dtype=np.uint32)])   # the last position predicts nothing asked for
+        lp, am = self.model.logprobs(ids[None], targets[None])
+        pos = range(ctx.size - 1, ids.size - 1)                               # position j predicts ids[j + 1]
+        total = 0.0
+        for j in pos:
+            total += float(lp[0, j])
+        return total, all(int(am[0, j]) == int(ids[j + 1]) for j in pos)
 
     def generate_batch(self, prompts, max_tokens: int, temperature: float = 0.0, max_batch: int = 64):
         """Request batching at the API boundary (SURVEY.md section 8f-3; the reference serialises requests at batch 1 under a

@@ -210,6 +210,33 @@ struct Model {
         }
         return out;
     }
+
+    // loglikelihood(context, continuation) -> (sum of the continuation's log-probs, whether every continuation token is the arg-max
+    // at its position): ONE fl_forward_logprobs call over context + continuation (targets = the ids shifted left by one) on a cache
+    // of its own, reset before and after at RoPE offset 0, so the generate cache is never touched.  Transliteration of
+    // fastllm_b200/models.py Model.loglikelihood (same summation order: f64, ascending positions).
+    std::unique_ptr<DeviceCache> score_cache;
+    std::pair<double, bool> loglikelihood(const std::vector<uint32_t>& context, const std::vector<uint32_t>& continuation) {
+        if (context.empty() || continuation.empty()) throw Error(FL_ERR_INVALID, "loglikelihood needs a non-empty context and continuation");
+        std::vector<uint32_t> ids(context);
+        ids.insert(ids.end(), continuation.begin(), continuation.end());
+        std::vector<uint32_t> targets(ids.begin() + 1, ids.end());
+        targets.push_back(0);                       // the last position predicts nothing asked for: any valid id
+        const int t = (int)ids.size();
+        if (!score_cache) score_cache = std::make_unique<DeviceCache>(model.dev->h, 1, std::min(kKvCapacity, model.dev->cfg.max_position_embeddings));
+        std::vector<float> lp(t);
+        std::vector<uint32_t> am(t);
+        check(fl_cache_reset(score_cache->h));
+        check(fl_forward_logprobs(model.dev->h, score_cache->h, ids.data(), targets.data(), 1, t, 0, lp.data(), am.data()));
+        check(fl_cache_reset(score_cache->h));
+        double sum = 0.0;
+        bool greedy = true;
+        for (size_t j = context.size() - 1; j + 1 < ids.size(); ++j) {     // position j predicts ids[j + 1]
+            sum += lp[j];
+            greedy = greedy && am[j] == ids[j + 1];
+        }
+        return {sum, greedy};
+    }
 };
 
 // ---- continuous batching above fl_forward_slots (SURVEY.md section 8f-3; the reference serialises requests at batch 1 under one

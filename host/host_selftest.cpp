@@ -2,6 +2,7 @@
 // Model::generate, prints the greedy ids as JSON.  tests/test_host_cpp_gpu.py compares them with the oracle.
 // `host_selftest --sampler seed temperature vocab logits.bin` needs no GPU: it runs the mirror's LogitsProcessor over the f32 rows
 // of logits.bin and prints the sampled ids (tests/test_sampling_cpu.py compares them with the oracle).
+// `host_selftest manifest weights 0 --loglikelihood context... / continuation...` prints Model::loglikelihood as [sum, is_greedy].
 // Build: g++ -std=c++17 -O2 host/host_selftest.cpp -o host/_build/host_selftest -Lfastllm_b200 -lfastllm_b200 -Wl,-rpath,...
 #include <cstdio>
 #include <cstdlib>
@@ -54,6 +55,20 @@ int main(int argc, char** argv) {
             tensors[name] = fastllm::HostTensor{FL_DTYPE_F32, shape, storage.back().data()};
         }
         const int max_tokens = std::atoi(argv[3]);
+        if (argc > 4 && std::strcmp(argv[4], "--loglikelihood") == 0) {
+            // host_selftest manifest weights 0 --loglikelihood context ids / continuation ids: Model::loglikelihood
+            std::vector<uint32_t> parts[2];
+            int k = 0;
+            for (int i = 5; i < argc; ++i) {
+                if (std::strcmp(argv[i], "/") == 0) k = 1;
+                else parts[k].push_back((uint32_t)std::strtoul(argv[i], nullptr, 10));
+            }
+            auto pr = fastllm::LlamaWithConfig::initialize_model(cfg, tensors, 0);
+            fastllm::Model<fastllm::LlamaWithConfig> model{std::move(pr.first), std::move(pr.second), std::nullopt};
+            const auto ll = model.loglikelihood(parts[0], parts[1]);
+            std::printf("[%.17g, %s]\n", ll.first, ll.second ? "true" : "false");
+            return 0;
+        }
         if (argc > 5 && std::strcmp(argv[4], "--batch") == 0) {
             // host_selftest manifest weights max_tokens --batch max_batch id id / id id id / ...: the C++ ContinuousBatcher over sequence slots
             const int max_batch = std::atoi(argv[5]);

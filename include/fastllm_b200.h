@@ -28,6 +28,8 @@
  *                                models/mod.rs:157-158,373-374 and logits_processor.sample(&last_logits)
  *                                models/mod.rs:308-310,425-428 (arg-max below 1e-7, else soft-max + WeightedIndex
  *                                over rand 0.8's StdRng seeded with seed_from_u64)
+ *   fl_forward_logprobs       <- no reference counterpart: per-position log-probs of given targets and the arg-max, in one forward
+ *                                (perplexity, loglikelihood(context, continuation), checking draft tokens)
  *   fl_forward_slots          <- the same forward for a batch of requests of different lengths (no reference counterpart: requests
  *                                are serialised at batch 1, api/chat.rs:206-208; streams run side by side, models/mod.rs:151-175)
  *   fl_embed                  <- EmbeddingModel::embed models/embeddings.rs:397-447 after tokenisation:
@@ -138,6 +140,21 @@ FL_EXPORT int fl_forward_greedy(fl_model* m, fl_cache* c, const uint32_t* ids, i
  * [steps, b] or NULL.  elapsed_ms: CUDA-event time of the whole loop on the cache's stream, or NULL. */
 FL_EXPORT int fl_decode_greedy_loop(fl_model* m, fl_cache* c, const uint32_t* first_ids, int b, size_t rope_offset, int steps,
                           uint32_t* out_ids, float* elapsed_ms);
+/* Scores ids [b, t] against targets [b, t] (host u32, row-major) in ONE forward that feeds ids to the cache exactly like
+ * fl_forward (kv_len += t; same rope_offset rule; same Llama rule for multi-token calls on a non-empty cache).
+ * logprobs:   host f32 [b, t]; logprobs[i, j] = log_softmax(z_ij)[targets[i, j]], where z_ij is the full-vocabulary logit row
+ *             at position j of sequence i (what fl_forward returns when the call ends at j), computed as
+ *             z[target] - (m + log s) in f32 with m the row maximum and s = sum exp(z - m).  No logits leave the device.
+ * argmax_ids: host u32 [b, t] or NULL; the arg-max of z_ij with the rule of fl_forward_greedy (the last index among equal maxima;
+ *             a NaN logit never wins).
+ * To score a text, pass targets = ids shifted left by one; the last target is the token that follows, or any valid id whose
+ * log-prob the caller ignores.
+ * FL_ERR_INVALID:     NULL ids / targets / logprobs, or a target >= vocab; checked before any device work (the cache is unchanged).
+ * FL_ERR_UNSUPPORTED: the model is sharded (tp_size > 1, Mixtral expert parallelism included), or its shapes do not admit the
+ *                     dense path (dimensions that are not multiples of 8).
+ * FL_ERR_STATE:       as for fl_forward (cache full, cache driven by slots). */
+FL_EXPORT int fl_forward_logprobs(fl_model* m, fl_cache* c, const uint32_t* ids, const uint32_t* targets, int b, int t,
+                                  size_t rope_offset, float* logprobs, uint32_t* argmax_ids);
 
 /* ---- continuous batching: sequence slots with their own lengths (SURVEY.md section 8f-3) -------------------------------------
  * The reference serialises requests at batch 1 under a mutex (api/chat.rs:206-208) and runs streams concurrently at batch 1 each
