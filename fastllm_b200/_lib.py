@@ -60,6 +60,7 @@ SYMBOLS = {
     "fl_sampler_destroy": (_I, [_VP]),
     "fl_forward_sample": (_I, [_VP, _VP, _VP, _I, _I, _SZ, _VP, C.POINTER(C.c_uint32)]),
     "fl_forward_slots": (_I, [_VP, _VP, _VP, _VP, _I, _I, _VP, _VP]),
+    "fl_forward_packed": (_I, [_VP, _VP, _VP, _VP, _I, _VP, _VP, _VP]),
     "fl_cache_slot_reset": (_I, [_VP, _I]),
     "fl_cache_slot_len": (_I, [_VP, _I, C.POINTER(_I)]),
     "fl_cache_moe_routing": (_I, [_VP, _I, _VP, _VP]),

@@ -37,6 +37,9 @@ struct AttnArgs {
     int nh, nkv, t, row_base;
     int sliding_window;    // <= 0: none
     float qscale;          // q is multiplied by this (1/sqrt(d))
+    // prefill kernels of attn_mma.cuh, packed calls: blockIdx.x is work item items[blockIdx.x] = (sequence, its first row, its
+    // length, query tile) instead of a query tile of the uniform [b, t] grid (null)
+    const int4* items;
 };
 
 template <int D>

@@ -430,7 +430,7 @@ __global__ void __launch_bounds__(kSkThreads) attn_sk_decode_kernel(const __grid
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
-// prefill: grid (ceil(t / 64), nh, b), 128 threads; warp w owns query rows [16w, 16w+16) of the tile
+// prefill: grid (ceil(t / 64), nh, b) or (work items, nh), 128 threads; warp w owns query rows [16w, 16w+16) of the tile
 // ---------------------------------------------------------------------------------------------------------------------
 template <int D>
 __global__ void __launch_bounds__(kMmaAttnThreads) attn_prefill_kernel(const AttnArgs a) {
@@ -441,11 +441,18 @@ __global__ void __launch_bounds__(kMmaAttnThreads) attn_prefill_kernel(const Att
     uint16_t* kv = qlo + kPrefillBM * D;                // [2 stages][K tile | V tile]
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, tq = lane & 3;
-    // heaviest (latest) query tiles first: the causal range grows with the tile index
-    const int qt = gridDim.x - 1 - blockIdx.x, head = blockIdx.y, seq = blockIdx.z;
+    const int head = blockIdx.y;
     const int n_rep = a.nh / a.nkv, kvh = head / n_rep;
     pdl_launch_dependents();
     pdl_wait();
+    // heaviest (latest) query tiles first: the causal range grows with the tile index (work items come sorted that way)
+    int qt, seq, t, row0;
+    if (a.items) {
+        const int4 it = a.items[blockIdx.x];
+        seq = it.x; row0 = it.y; t = it.z; qt = it.w;
+    } else {
+        qt = gridDim.x - 1 - blockIdx.x; seq = blockIdx.z; t = a.t; row0 = seq * a.t;
+    }
     const int i0 = qt * kPrefillBM;
     const int cslot = st_slot(a.state, seq);
     const int kv_base = a.state->kv_base[cslot];
@@ -453,7 +460,7 @@ __global__ void __launch_bounds__(kMmaAttnThreads) attn_prefill_kernel(const Att
     const int* pt = a.page_table + (size_t)cslot * a.pt_stride;
 
     // key range of the whole tile
-    const int ilast = min(i0 + kPrefillBM, a.t) - 1;
+    const int ilast = min(i0 + kPrefillBM, t) - 1;
     const int len_tile = kv_base + ilast + 1;
     // the window thins out the NEW tokens only: candle concatenates zeros for the cached columns of its [t, t] mask, so every
     // cached key (< kv_base) stays visible and a call on a non-empty cache walks all pages
@@ -468,18 +475,18 @@ __global__ void __launch_bounds__(kMmaAttnThreads) attn_prefill_kernel(const Att
     for (int i = tid; i < kPrefillBM * (D / 4); i += kMmaAttnThreads) {
         const int r = i / (D / 4), c = (i % (D / 4)) * 4;
         float4 q = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (i0 + r < a.t) q = *reinterpret_cast<const float4*>(a.q + (((size_t)seq * a.t + i0 + r) * a.nh + head) * D + c);
+        if (i0 + r < t) q = *reinterpret_cast<const float4*>(a.q + (((size_t)row0 + i0 + r) * a.nh + head) * D + c);
         const int off = swz<D>(r, c);
         store_hi_lo(qhi, qlo, off, q.x); store_hi_lo(qhi, qlo, off + 1, q.y);
         store_hi_lo(qhi, qlo, off + 2, q.z); store_hi_lo(qhi, qlo, off + 3, q.w);
     }
 
     // per-thread rows: g and g + 8 of the warp's 16 (rows past t are clamped: computed, never stored)
-    const int ir0 = min(i0 + warp * 16 + g, a.t - 1), ir1 = min(i0 + warp * 16 + g + 8, a.t - 1);
+    const int ir0 = min(i0 + warp * 16 + g, t - 1), ir1 = min(i0 + warp * 16 + g + 8, t - 1);
     const int len0 = kv_base + ir0 + 1, len1 = kv_base + ir1 + 1;
     const int st0 = (sw > 0 && ir0 - sw > 0) ? kv_base + ir0 - sw : 0;
     const int st1 = (sw > 0 && ir1 - sw > 0) ? kv_base + ir1 - sw : 0;
-    const int warp_len = kv_base + min(i0 + warp * 16 + 15, a.t - 1) + 1;    // keys >= this are masked for the whole warp
+    const int warp_len = kv_base + min(i0 + warp * 16 + 15, t - 1) + 1;    // keys >= this are masked for the whole warp
 
     float o[D / 8][4];
 #pragma unroll
@@ -582,13 +589,14 @@ __global__ void __launch_bounds__(kMmaAttnThreads) attn_prefill_kernel(const Att
 #pragma unroll
     for (int nt = 0; nt < D / 8; ++nt) {
         const int c = nt * 8 + tq * 2;
-        if (r0 < a.t) store_out2(a, (((size_t)seq * a.t + r0) * a.nh + head) * D + c, o[nt][0] * inv0, o[nt][1] * inv0);
-        if (r1 < a.t) store_out2(a, (((size_t)seq * a.t + r1) * a.nh + head) * D + c, o[nt][2] * inv1, o[nt][3] * inv1);
+        if (r0 < t) store_out2(a, (((size_t)row0 + r0) * a.nh + head) * D + c, o[nt][0] * inv0, o[nt][1] * inv0);
+        if (r1 < t) store_out2(a, (((size_t)row0 + r1) * a.nh + head) * D + c, o[nt][2] * inv1, o[nt][3] * inv1);
     }
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
-// prefill on the 5th-gen tensor cores: grid (ceil(t / 128), nh, b), 192 threads, head_dim 64 / 128, calls that start on empty caches
+// prefill on the 5th-gen tensor cores: grid (ceil(t / 128), nh, b) or (work items, nh), 352 threads, head_dim 64 / 128, sequences
+// that start on empty caches
 // ---------------------------------------------------------------------------------------------------------------------
 // One CTA owns 128 query rows of one head (M = 128 of tcgen05.mma) and walks the causal range of 64-key pages:
 //   warp 0      producer: K page (the pool's own rows, 2-D TMA, 128-byte swizzle) + the page of V^T that dense_qkv_epi_kernel wrote
@@ -606,6 +614,7 @@ struct TcPrefillArgs {
     AttnArgs a;
     int layer_row0;      // row of this layer's page 0 / kv head 0 in the pool-wide K tensor map
     int vt_pages;        // pages per (sequence, kv head) in the V^T scratch
+    const int* vt_tile0; // packed calls: first V^T tile of each sequence ([kv head][its pages]; QkvEpiArgs::vt_tile0), else null
     float tau;           // a row's reference max moves only when the tile's max exceeds it by more than this (exp2 domain)
 };
 
@@ -648,10 +657,17 @@ __global__ void __launch_bounds__(kTcThreads, 1) attn_prefill_tc_kernel(const __
     __shared__ float xsum[2][kTcQ];         // their row sums (epilogue)
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int qt = gridDim.x - 1 - blockIdx.x, head = blockIdx.y, seq = blockIdx.z;      // heaviest (latest) query tiles first
+    const int head = blockIdx.y;
     const int n_rep = a.nh / a.nkv, kvh = head / n_rep;
+    int qt, seq, t, row0;       // heaviest (latest) query tiles first (work items come sorted that way)
+    if (a.items) {
+        const int4 it = a.items[blockIdx.x];
+        seq = it.x; row0 = it.y; t = it.z; qt = it.w;
+    } else {
+        qt = gridDim.x - 1 - blockIdx.x; seq = blockIdx.z; t = a.t; row0 = seq * a.t;
+    }
     const int q0 = qt * kTcQ, sw = a.sliding_window;
-    const int kend = min(a.t, q0 + kTcQ);                            // keys [0, kend) can be visible to this tile
+    const int kend = min(t, q0 + kTcQ);                              // keys [0, kend) can be visible to this tile
     const int kt0 = (sw > 0 && q0 - sw > 0) ? (q0 - sw) / kKvPage : 0;
     const int nkt = (kend + kKvPage - 1) / kKvPage - kt0;
 
@@ -689,11 +705,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) attn_prefill_tc_kernel(const __
         }
     } else if (warp == 10) {
         if (lane == 0) {      // V^T pages of this call (written by dense_qkv_epi_kernel)
+            const int vt0 = k.vt_tile0 ? k.vt_tile0[seq] + kvh * ((t + kKvPage - 1) / kKvPage) : (seq * a.nkv + kvh) * k.vt_pages;
             for (int j = 0; j < nkt; ++j) {
                 const int st = j % NV;
                 mbar_wait(&v_empty[st], ((j / NV) & 1) ^ 1);
                 mbar_expect_tx(&v_full[st], kTile);
-                tma_load_2d(sm + kVOff + st * kTile, &tmvt, 0, ((seq * a.nkv + kvh) * k.vt_pages + kt0 + j) * D, &v_full[st]);
+                tma_load_2d(sm + kVOff + st * kTile, &tmvt, 0, (vt0 + kt0 + j) * D, &v_full[st]);
             }
         }
     } else if (warp == 1) {
@@ -746,12 +763,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) attn_prefill_tc_kernel(const __
         // warps were the critical path at ~3400 clocks per page); two per scheduler overlap one's MUFU / TMEM waits with the other's
         // arithmetic.  The halves of a row exchange their page maxima through shared memory (one 256-thread named barrier per page).
         const int grp = (warp - 2) >> 2, quarter = warp & 3, r = quarter * 32 + lane;
-        const int irow = min(q0 + r, a.t - 1);               // rows past t are clamped: computed, never stored
+        const int irow = min(q0 + r, t - 1);                 // rows past t are clamped: computed, never stored
         const uint32_t lane_addr = (uint32_t)(quarter * 32) << 16;
         auto gsync = [] { asm volatile("bar.sync 2, 256;" ::: "memory"); };
         // ---- q row -> hi / lo bf16, swizzled operand layout: 16-byte chunk c of row r at chunk (c & 7) ^ (r & 7) of k-block c >> 3 ----
         {
-            const float* qsrc = a.q + (((size_t)seq * a.t + irow) * a.nh + head) * D;
+            const float* qsrc = a.q + (((size_t)row0 + irow) * a.nh + head) * D;
 #pragma unroll
             for (int cc = 0; cc < D / 16; ++cc) {
                 const int c = grp * (D / 16) + cc;
@@ -855,12 +872,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) attn_prefill_tc_kernel(const __
         const float inv = 1.f / (l + xsum[grp ^ 1][r]);
         mbar_wait(&o_done, (nkt - 1) & 1);
         tc_fence_after();
-        const size_t obase = (((size_t)seq * a.t + irow) * a.nh + head) * D + grp * (D / 2);
+        const size_t obase = (((size_t)row0 + irow) * a.nh + head) * D + grp * (D / 2);
 #pragma unroll 1
         for (int c4 = 0; c4 < D / 64; ++c4) {
             uint32_t o[32];
             tmem_ld32(tO + lane_addr + grp * (D / 2) + c4 * 32, o);
-            if (q0 + r < a.t) {
+            if (q0 + r < t) {
 #pragma unroll
                 for (int c = 0; c < 4; ++c) {
                     float v[8];

@@ -68,6 +68,7 @@ struct PrepArgs {
     int last_only;
     uint16_t* xhi;              // [R_out, K]
     uint16_t* xlo;
+    const int* last_rows;       // optional (packed calls, dense_prep_kernel): output row j takes input row last_rows[j]
 };
 
 // one CTA per output row, float4-vectorised (K % 4 == 0); up to 1024 threads so a 4096-wide row is one load per thread
@@ -76,7 +77,7 @@ static __global__ void __launch_bounds__(1024) dense_prep_kernel(const PrepArgs 
     pdl_wait();
     __shared__ float red[32];
     const int orow = blockIdx.x;
-    const int row = a.last_only ? (orow + 1) * a.t - 1 : orow;
+    const int row = a.last_rows ? a.last_rows[orow] : (a.last_only ? (orow + 1) * a.t - 1 : orow);
     const int K = a.K, K4 = K >> 2;
     uint2* xh = reinterpret_cast<uint2*>(a.xhi + (size_t)orow * K);
     uint2* xl = reinterpret_cast<uint2*>(a.xlo + (size_t)orow * K);
@@ -215,25 +216,32 @@ struct QkvEpiArgs {
     int nh, nkv, d, max_pos, t, nqkv;
     uint16_t* vt;              // optional (prefill on the tcgen05 attention kernel): V of this call TRANSPOSED per 64-token page,
     int vt_pages;              // [sequence][kv head][vt_pages][d][64 tokens] -- the K-major B operand of O += P . V
+    // packed calls (sequences of different lengths; dense_qkv_epi_kernel<true> only):
+    int rows;                  // R: the kernel walks rows blockIdx.y, + gridDim.y, ...
+    const int2* row_tab;       // [R] (sequence, position in the sequence) of every row
+    const int* seq_len;        // [sequences] tokens each sequence is fed
+    const int* vt_tile0;       // [sequences] first [d][64] tile of the sequence's V^T pages ([kv head][its pages]), or -1: none
 };
 
-// bias + RoPE (rotate-half) + q store + paged KV append; thread per column pair, grid.y = row
-static __global__ void dense_qkv_epi_kernel(const QkvEpiArgs a) {
-    // the dependent (attention) kernel is released only AFTER this kernel's own wait: when it starts, the q|k|v GEMM -- and by
-    // induction every earlier kernel of the stream -- has completed, so its preamble may read the step state, the page table and
-    // every K/V page except the rows appended here before its own griddepcontrol.wait (attn_sk_decode_kernel streams them early)
-    pdl_wait();
-    pdl_launch_dependents();
-    const int row = blockIdx.y;
-    const int pair = blockIdx.x * blockDim.x + threadIdx.x;
-    if (pair * 2 >= a.nqkv) return;
+// bias + RoPE (rotate-half) + q store + paged KV append of one row and column pair.  PACKED (packed calls): the row's sequence and
+// position come from row_tab, its V^T tile from vt_tile0.
+template <bool PACKED>
+__device__ __forceinline__ void qkv_epi_row(const QkvEpiArgs& a, int row, int pair) {
     const int ra = pair * 2;
     const int d = a.d, half = d >> 1;
     const int hh = ra / d, j = (ra % d) >> 1;
     const float2 vab = sum_slices2(a.y + (size_t)row * a.nqkv + ra, a.sl_stride, a.nsl);
     float va = vab.x, vb = vab.y;
     if (a.bias) { va += a.bias[ra]; vb += a.bias[ra + 1]; }
-    const int seq = row / a.t, irel = row % a.t;
+    int seq, irel;
+    if constexpr (PACKED) {
+        const int2 rt = a.row_tab[row];
+        seq = rt.x;
+        irel = rt.y;
+    } else {
+        seq = row / a.t;
+        irel = row % a.t;
+    }
     const int cslot = st_slot(a.state, seq);                    // cache slot of this sequence (its own index unless the call is ragged)
     const int slot = a.state->kv_base[cslot] + irel;
     const int page = a.page_table[cslot * a.pt_stride + slot / kKvPage];
@@ -255,10 +263,35 @@ static __global__ void dense_qkv_epi_kernel(const QkvEpiArgs a) {
         uint16_t* vp = a.vpool + (((size_t)page * a.nkv + (hh - a.nh - a.nkv)) * kKvPage + slot % kKvPage) * d;
         *reinterpret_cast<uint32_t*>(vp + 2 * j) = (uint32_t)f32_to_bf16_rne(va) | ((uint32_t)f32_to_bf16_rne(vb) << 16);
         if (a.vt != nullptr) {
-            uint16_t* tp = a.vt + ((((size_t)seq * a.nkv + (hh - a.nh - a.nkv)) * a.vt_pages + irel / kKvPage) * d + 2 * j) * kKvPage + irel % kKvPage;
+            size_t tile;                // the [d][64] V^T tile of (sequence, kv head, page)
+            if constexpr (PACKED) {
+                const int t0 = a.vt_tile0[seq];
+                if (t0 < 0) return;     // this sequence's attention does not read the scratch
+                tile = (size_t)t0 + (size_t)(hh - a.nh - a.nkv) * ((a.seq_len[seq] + kKvPage - 1) / kKvPage) + irel / kKvPage;
+            } else {
+                tile = ((size_t)seq * a.nkv + (hh - a.nh - a.nkv)) * a.vt_pages + irel / kKvPage;
+            }
+            uint16_t* tp = a.vt + (tile * d + 2 * j) * kKvPage + irel % kKvPage;
             tp[0] = f32_to_bf16_rne(va);
             tp[kKvPage] = f32_to_bf16_rne(vb);
         }
+    }
+}
+
+// thread per column pair, grid.y = row (PACKED: grid.y strides over the rows, which may be more than a grid dimension holds)
+template <bool PACKED>
+static __global__ void dense_qkv_epi_kernel(const QkvEpiArgs a) {
+    // the dependent (attention) kernel is released only AFTER this kernel's own wait: when it starts, the q|k|v GEMM -- and by
+    // induction every earlier kernel of the stream -- has completed, so its preamble may read the step state, the page table and
+    // every K/V page except the rows appended here before its own griddepcontrol.wait (attn_sk_decode_kernel streams them early)
+    pdl_wait();
+    pdl_launch_dependents();
+    const int pair = blockIdx.x * blockDim.x + threadIdx.x;
+    if (pair * 2 >= a.nqkv) return;
+    if constexpr (PACKED) {
+        for (int row = blockIdx.y; row < a.rows; row += gridDim.y) qkv_epi_row<true>(a, row, pair);
+    } else {
+        qkv_epi_row<false>(a, blockIdx.y, pair);
     }
 }
 

@@ -58,14 +58,15 @@ static __global__ void argmax_finalize_kernel(const float* __restrict__ val, con
     }
 }
 
-// End of a forward call: kv_base[seq] += t.  In the device-resident greedy loop also rope_pos += 1 and ids <- next_ids.
+// End of a forward call: kv_base[seq] += t (packed calls: lens[seq]).  In the device-resident greedy loop also rope_pos += 1 and
+// ids <- next_ids.
 static __global__ void advance_state_kernel(StepState* st, int b, int t, int rope_inc, uint32_t* ids, const uint32_t* next_ids, int feedback,
-                                     uint32_t* trace, int* trace_pos) {
+                                     uint32_t* trace, int* trace_pos, const int* lens) {
     pdl_launch_dependents();
     pdl_wait();
     const int i = threadIdx.x;
     if (i < b) {
-        st->kv_base[st_slot(st, i)] += t;       // distinct slots per row (checked on the host)
+        st->kv_base[st_slot(st, i)] += lens ? lens[i] : t;       // distinct slots per row (checked on the host)
         if (feedback) ids[i] = next_ids[i];
         if (trace != nullptr) trace[(size_t)(*trace_pos) * b + i] = next_ids[i];
     }

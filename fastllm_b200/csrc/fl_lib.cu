@@ -572,10 +572,26 @@ static void cache_destroy_graphs(fl_cache& c) {
     c.graphs.clear();
 }
 
+// A packed call (fl_forward_packed) on the device: sequences of different lengths, rows in the internal order (run_forward_packed).
+// Every pointer points into fl_cache::pack_tab.
+struct PackedCall {
+    int n = 0, T = 0;                 // sequences, rows (the sum of their lengths)
+    int nd = 0;                       // length-1 sequences: sequences and rows [0, nd)
+    uint64_t kv_tokens = 0;           // keys the attention reads over all sequences (profile bytes)
+    const uint32_t* ids = nullptr;    // [T]
+    const int2* row_tab = nullptr;    // [T] (sequence, position in the sequence)
+    const int* seq_len = nullptr;     // [n]
+    const int* vt_tile0 = nullptr;    // [n] first V^T tile of a sequence on attn_prefill_tc_kernel, else -1
+    const int* last_row = nullptr;    // [n] in the CALLER's order: the row of the sequence's last token
+    const int4* tc_items = nullptr;   // attn_prefill_tc_kernel work items (sequence, first row, length, 128-row query tile)
+    const int4* mma_items = nullptr;  // attn_prefill_kernel work items (sequence, first row, length, 64-row query tile)
+    int ntc = 0, nmma = 0;
+};
+
 // Enqueue the whole forward for the flattened [b, t] call on lc.stream.  Rows are processed in passes of kPassRows,
 // pass-major / layer-minor: a token's layer-l attention only needs the layer-l K/V of EARLIER tokens, which earlier
 // passes already appended, so the order is causal-correct.
-static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool loop_mode, bool score = false);
+static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool loop_mode, bool score = false, const PackedCall* pk = nullptr);
 
 // A uniform call of `rows` activation rows runs on the dense (tcgen05) path: 3+ rows, or any Mixtral call.
 static bool uses_dense(const fl_cache& c, int rows) {
@@ -699,7 +715,7 @@ static void enqueue_forward(fl_cache& c, LaunchCtx& lc, int b, int t, bool loop_
     }
     launch(lc, "advance_state", 0, advance_state_kernel, dim3(1), dim3(kMaxBatch), 0, c.state.p, b, t, loop_mode ? 1 : 0, c.ids.p,
            (const uint32_t*)c.next_ids.p, loop_mode ? 1 : 0, loop_mode ? c.trace.p : (uint32_t*)nullptr,
-           loop_mode ? c.trace_pos.p : (int*)nullptr);
+           loop_mode ? c.trace_pos.p : (int*)nullptr, (const int*)nullptr);
 }
 
 
@@ -882,19 +898,22 @@ static void enqueue_lm_head_logprobs(fl_cache& c, LaunchCtx& lc, int R) {
            ntn * (kGemmEpiWarps / 4), (const float*)d.lp_target_logit.p, R, reinterpret_cast<float*>(d.lp_out.p), d.lp_out.p + R);
 }
 
-static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool loop_mode, bool score) {
+// Uniform calls: b sequences of t rows each.  Packed calls (pk): b = pk->n sequences of their own lengths, t unused; the window rule
+// is the lone call's per sequence (a multi-token sequence is windowed, a length-1 one is not).
+static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool loop_mode, bool score, const PackedCall* pk) {
     const Weights& w = *c.w;
     DenseWs& d = c.dw;
-    const int R = b * t;
+    const int R = pk ? pk->T : b * t;
     const int nq = w.nh * w.d;
     const float qscale = (float)(1.0 / std::sqrt((double)w.d));
-    const bool windowed = (w.cfg.arch != FL_ARCH_LLAMA) && w.cfg.sliding_window > 0 && t > 1;
+    const bool windowed = (w.cfg.arch != FL_ARCH_LLAMA) && w.cfg.sliding_window > 0 && (pk != nullptr || t > 1);
     // multi-token calls on empty sequences with head_dim 64 / 128 and more than one page of keys: attention on tcgen05
     // (attn_prefill_tc_kernel; FL_ATTN_PREFILL_MMA=1 keeps the mma.sync kernel, the A/B knob)
     const int vt_pages = (t + kKvPage - 1) / kKvPage;
     const bool prefill_mma = env_flag("FL_ATTN_PREFILL_MMA");
-    const bool tc_prefill = t > kKvPage && (w.d == 64 || w.d == 128) && c.kv_tmaps && c.fresh_call && !prefill_mma &&
+    const bool tc_prefill = !pk && t > kKvPage && (w.d == 64 || w.d == 128) && c.kv_tmaps && c.fresh_call && !prefill_mma &&
                             (size_t)b * vt_pages <= d.vt_pages_cap;
+    const float tc_tau = std::getenv("FL_ATTN_TC_TAU") ? (float)std::atof(std::getenv("FL_ATTN_TC_TAU")) : 8.f;    // 0: O is rescaled on every new row max (tests)
 
     auto prep = [&](const char* tag, PrepArgs pa, int rows_out) {
         pa.xhi = d.xhi.p; pa.xlo = d.xlo.p; pa.eps = w.cfg.norm_eps; pa.t = t;
@@ -911,7 +930,7 @@ static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool
     };
     {   // K1 + K2 of layer 0
         PrepArgs pa{};
-        pa.embed = w.embed; pa.ids = c.ids.p; pa.vocab = w.Vfull; pa.resid = d.resid.p; pa.norm_w = w.layers[0].ln1; pa.K = w.H;
+        pa.embed = w.embed; pa.ids = pk ? pk->ids : c.ids.p; pa.vocab = w.Vfull; pa.resid = d.resid.p; pa.norm_w = w.layers[0].ln1; pa.K = w.H;
         prep("dense_embed_rmsnorm", pa, R);
     }
     for (int l = 0; l < w.L; ++l) {
@@ -920,21 +939,52 @@ static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool
         uint16_t* vpool = c.vpool.p + (size_t)l * c.layer_pool_elems;
         int ks = dense_gemm(c, lc, "gemm_tc_qkv", R, w.nqkv, w.H, lw.tm_wqkv, d.y.p);
         QkvEpiArgs qa{ks, (long long)R * w.nqkv, d.y.p, lw.bqkv, d.q.p, kpool, vpool, c.page_table.p, c.pages_per_seq, c.state.p, w.rope_cos,
-                      w.rope_sin, w.nh, w.nkv, w.d, w.max_pos, t, w.nqkv, tc_prefill ? d.vt.p : nullptr, vt_pages};
-        if (t >= 64 && t % kQkvRowsPerThread == 0)      // prefill: eight rows per thread (dense_qkv_epi_rows_kernel)
+                      w.rope_sin, w.nh, w.nkv, w.d, w.max_pos, t, w.nqkv, tc_prefill ? d.vt.p : nullptr, vt_pages, R};
+        if (pk) {       // the one-row kernel: eight consecutive rows need not belong to one sequence
+            qa.row_tab = pk->row_tab; qa.seq_len = pk->seq_len; qa.vt_tile0 = pk->vt_tile0;
+            qa.vt = pk->ntc > 0 ? d.vt.p : nullptr;
+        }
+        if (pk)
+            launch(lc, "dense_qkv_rope_append", 0, dense_qkv_epi_kernel<true>, dim3((w.nqkv / 2 + 255) / 256, std::min(R, 65535)), dim3(256), 0, qa);
+        else if (t >= 64 && t % kQkvRowsPerThread == 0)      // prefill: eight rows per thread (dense_qkv_epi_rows_kernel)
             launch(lc, "dense_qkv_rope_append", 0, dense_qkv_epi_rows_kernel, dim3((w.nqkv / 2 + 255) / 256, R / kQkvRowsPerThread), dim3(256), 0, qa);
         else
-            launch(lc, "dense_qkv_rope_append", 0, dense_qkv_epi_kernel, dim3((w.nqkv / 2 + 255) / 256, R), dim3(256), 0, qa);
+            launch(lc, "dense_qkv_rope_append", 0, dense_qkv_epi_kernel<false>, dim3((w.nqkv / 2 + 255) / 256, R), dim3(256), 0, qa);
         {   // K7-K11 on tensor cores; the output lands as the hi/lo bf16 operands of the o_proj GEMM
             AttnArgs at{};
             at.q = d.q.p; at.kpool = kpool; at.vpool = vpool; at.page_table = c.page_table.p; at.pt_stride = c.pages_per_seq;
             at.state = c.state.p; at.counters = d.counters.p;
             at.out_hi = d.xhi.p; at.out_lo = d.xlo.p; at.nh = w.nh; at.nkv = w.nkv; at.t = t; at.row_base = 0;
             at.sliding_window = windowed ? w.cfg.sliding_window : 0; at.qscale = qscale;
-            const uint64_t kv_bytes = (uint64_t)b * (c.kv_len + t) * w.nkv * w.d * 4;
+            const uint64_t kv_bytes = (pk ? pk->kv_tokens : (uint64_t)b * (c.kv_len + t)) * w.nkv * w.d * 4;
             const int layer_row0 = (int)((size_t)l * (c.layer_pool_elems / w.d));
             with_head_dim(w.d, [&](auto D) {
-                if (t == 1) {
+                if (pk) {
+                    // up to three launches, each over its own rows: the length-1 sequences (rows [0, nd)) as a decode step, fresh
+                    // sequences of more than a page on tcgen05, every other multi-token sequence on mma.sync -- the kernels a lone
+                    // call of each sequence would take
+                    if (pk->nd > 0) {
+                        const SkPlan pl = attn_sk_plan<D>(w.nh / w.nkv);
+                        SkArgs sk{};
+                        sk.a = at; sk.sk_acc = d.sk_acc.p; sk.sk_ml = d.sk_ml.p; sk.b = pk->nd; sk.layer_row0 = layer_row0;
+                        launch(lc, "attn_sk_decode", kv_bytes, attn_sk_decode_kernel<D>, dim3(pl.ctas * kNumSMs), dim3(kSkThreads), pl.smem,
+                               c.tm_kpool, c.tm_vpool, sk);
+                    }
+                    if constexpr (D == 64 || D == 128) {
+                        if (pk->ntc > 0) {
+                            TcPrefillArgs tp{};
+                            tp.a = at; tp.a.items = pk->tc_items; tp.layer_row0 = layer_row0; tp.vt_tile0 = pk->vt_tile0; tp.tau = tc_tau;
+                            launch(lc, "attn_prefill_tc", kv_bytes, attn_prefill_tc_kernel<D>, dim3(pk->ntc, w.nh), dim3(kTcThreads),
+                                   attn_prefill_tc_smem_bytes(D), c.tm_kpool, d.tm_vt, tp);
+                        }
+                    }
+                    if (pk->nmma > 0) {
+                        AttnArgs am = at;
+                        am.items = pk->mma_items;
+                        launch(lc, "attn_prefill", kv_bytes, attn_prefill_kernel<D>, dim3(pk->nmma, w.nh), dim3(kMmaAttnThreads),
+                               attn_prefill_smem_bytes(D), am);
+                    }
+                } else if (t == 1) {
                     // stream-K: a fixed grid of resident CTAs, each an equal share of the step's page stream.  The grid does NOT
                     // depend on the KV length: this launch is captured into the step's CUDA graph, which is keyed by (batch, mode)
                     // only and replayed as the context grows.
@@ -948,7 +998,7 @@ static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool
                     if constexpr (D == 64 || D == 128) {
                         TcPrefillArgs tp{};
                         tp.a = at; tp.layer_row0 = layer_row0; tp.vt_pages = vt_pages;
-                        tp.tau = std::getenv("FL_ATTN_TC_TAU") ? (float)std::atof(std::getenv("FL_ATTN_TC_TAU")) : 8.f;      // 0: O is rescaled on every new row max (tests)
+                        tp.tau = tc_tau;
                         launch(lc, "attn_prefill_tc", kv_bytes, attn_prefill_tc_kernel<D>, dim3((t + kTcQ - 1) / kTcQ, w.nh, b), dim3(kTcThreads),
                                attn_prefill_tc_smem_bytes(D), c.tm_kpool, d.tm_vt, tp);
                     }
@@ -1049,14 +1099,14 @@ static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool
             pa.norm_w = w.layers[l + 1].ln1;
             prep("dense_resid_rmsnorm", pa, R);
         } else {             // K16 + K17: only the last token of every sequence goes on to the lm_head (scoring: every token)
-            pa.norm_w = w.final_norm; pa.last_only = score ? 0 : 1;
+            pa.norm_w = w.final_norm; pa.last_only = score ? 0 : 1; pa.last_rows = pk ? pk->last_row : nullptr;
             prep("dense_final_rmsnorm", pa, score ? R : b);
         }
     }
     if (score) {
         enqueue_lm_head_logprobs(c, lc, R);
         launch(lc, "advance_state", 0, advance_state_kernel, dim3(1), dim3(kMaxBatch), 0, c.state.p, b, t, 0, c.ids.p, (const uint32_t*)c.next_ids.p, 0,
-               (uint32_t*)nullptr, (int*)nullptr);
+               (uint32_t*)nullptr, (int*)nullptr, (const int*)nullptr);
         return;
     }
     const int ksh = dense_gemm(c, lc, "gemm_tc_lm_head", b, w.V, w.H, w.tm_head, d.y.p);
@@ -1073,7 +1123,7 @@ static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool
     }
     launch(lc, "advance_state", 0, advance_state_kernel, dim3(1), dim3(kMaxBatch), 0, c.state.p, b, t, loop_mode ? 1 : 0, c.ids.p,
            (const uint32_t*)c.next_ids.p, loop_mode ? 1 : 0, loop_mode ? c.trace.p : (uint32_t*)nullptr,
-           loop_mode ? c.trace_pos.p : (int*)nullptr);
+           loop_mode ? c.trace_pos.p : (int*)nullptr, pk ? pk->seq_len : (const int*)nullptr);
 }
 
 // mode 0: one decode step of a uniform batch; 1: the same inside the device-resident greedy loop; 2: one decode step of a ragged
@@ -1168,6 +1218,7 @@ static void run_forward(fl_cache& c, const uint32_t* ids, int b, int t, size_t r
     set_state_kernel<<<1, 1, 0, c.stream>>>(c.state.p, (int)rope_offset);
     g_launches.fetch_add(1);
     c.dw.route_rows = R;
+    c.pack_perm.clear();
     c.fresh_call = c.kv_len == 0 && !c.slots_used;
     run_steps(c, b, t, targets ? 3 : 0, 1);
 }
@@ -1196,6 +1247,7 @@ static void run_forward_slots(fl_cache& c, const int* slots, const uint32_t* ids
     for (int i = 0; i < n * t; ++i) FL_CHECK(ids[i] < (uint32_t)w.Vfull, FL_ERR_INVALID, "token id out of range");
     ensure_dense_ws(c, n * t);
     c.dw.route_rows = n * t;
+    c.pack_perm.clear();
     c.fresh_call = true;
     for (int i = 0; i < n; ++i) c.fresh_call = c.fresh_call && c.slot_len[slots[i]] == 0;
     c.slots_used = true;
@@ -1210,6 +1262,144 @@ static void run_forward_slots(fl_cache& c, const int* slots, const uint32_t* ids
     g_launches.fetch_add(1);
     run_steps(c, n, t, 2, 1);
     for (int i = 0; i < n; ++i) c.slot_len[slots[i]] += t;
+}
+
+// Packed forward: sequence i is cache slot slots[i], fed ids[o_i, o_i + lengths[i]) at RoPE positions rope_offsets[i] + j, all in ONE
+// forward.  Equal lengths are fl_forward_slots.  Otherwise the rows are reordered: the length-1 sequences first (by slot), then the
+// others by length descending and slot ascending, so the internal order -- and every result -- does not depend on the caller's
+// order; logits row i is the caller's sequence i.  Everything is validated before the first device operation.  Runs eagerly.
+static void run_forward_packed(fl_cache& c, const int* slots, const int32_t* lengths, int n, const uint32_t* ids, const size_t* rope_offsets) {
+    const Weights& w = *c.w;
+    FL_CHECK(!c.poisoned, FL_ERR_CUDA, "cache poisoned by an earlier CUDA error");
+    FL_CHECK(slots && lengths && ids && rope_offsets, FL_ERR_INVALID, "NULL argument");
+    FL_CHECK(w.cfg.tp_size <= 1, FL_ERR_UNSUPPORTED, "packed calls need an unsharded model");
+    FL_CHECK(w.dense_ok, FL_ERR_UNSUPPORTED, "packed calls run on the dense path: shapes must be multiples of 8");
+    FL_CHECK(n >= 1 && n <= c.max_batch, FL_ERR_INVALID, "bad number of sequences (1 <= n <= max_batch)");
+    FL_CHECK(c.slots_used || c.kv_len == 0, FL_ERR_STATE, "the cache holds tokens of uniform calls: fl_cache_reset before driving it by slots");
+    std::vector<char> seen(c.max_batch, 0);
+    int64_t T = 0;
+    bool equal = true;
+    for (int i = 0; i < n; ++i) {
+        const int sl = slots[i], len = lengths[i];
+        FL_CHECK(len >= 1, FL_ERR_INVALID, "a sequence length is < 1");
+        FL_CHECK(sl >= 0 && sl < c.max_batch, FL_ERR_INVALID, "slot index out of range");
+        FL_CHECK(!seen[sl], FL_ERR_INVALID, "a slot appears twice in one call");
+        seen[sl] = 1;
+        FL_CHECK((int64_t)c.slot_len[sl] + len <= c.max_seq, FL_ERR_STATE, "KV cache full (slot length + length > max_seq)");
+        FL_CHECK((int64_t)rope_offsets[i] + len <= w.max_pos, FL_ERR_INVALID, "RoPE position beyond max_position_embeddings");
+        FL_CHECK(!(w.cfg.arch == FL_ARCH_LLAMA && len > 1 && c.slot_len[sl] != 0), FL_ERR_INVALID,
+                 "Llama: multi-token forward needs an empty cache (candle builds a t x t mask)");
+        T += len;
+        equal = equal && len == lengths[0];
+    }
+    for (int64_t i = 0; i < T; ++i) FL_CHECK(ids[i] < (uint32_t)w.Vfull, FL_ERR_INVALID, "token id out of range");
+    if (equal) {
+        run_forward_slots(c, slots, ids, n, lengths[0], rope_offsets);
+        return;
+    }
+    int nd = 0;
+    for (int i = 0; i < n; ++i) nd += lengths[i] == 1;
+    FL_CHECK(nd == 0 || (c.kv_tmaps && w.nh / w.nkv <= 16), FL_ERR_UNSUPPORTED,
+             "batched decode attention: GQA group > 16 heads or KV pool beyond 2^31 rows");
+    ensure_dense_ws(c, (int)T);
+
+    // internal order and rows
+    std::vector<int> order(n), off(n), row0(n), tile0(n, -1);
+    for (int i = 0; i < n; ++i) order[i] = i;
+    std::sort(order.begin(), order.end(), [&](int a, int b) {
+        if ((lengths[a] == 1) != (lengths[b] == 1)) return lengths[a] == 1;
+        if (lengths[a] != lengths[b]) return lengths[a] > lengths[b];
+        return slots[a] < slots[b];
+    });
+    for (int i = 0, o = 0; i < n; o += lengths[i], ++i) off[i] = o;
+    PackedCall pc;
+    pc.n = n; pc.T = (int)T; pc.nd = nd;
+    const int sw = (w.cfg.arch != FL_ARCH_LLAMA && w.cfg.sliding_window > 0) ? w.cfg.sliding_window : 0;
+    // attention work items (sequence, first row, length, query tile), heaviest first: the most key pages, then in sequence order
+    struct Item { int cost, s, r0, len, qt; };
+    std::vector<Item> tc, mma;
+    size_t vt_pages = 0;
+    const bool tc_ok = (w.d == 64 || w.d == 128) && c.kv_tmaps && !env_flag("FL_ATTN_PREFILL_MMA");
+    for (int s = 0, r = 0; s < n; r += lengths[order[s]], ++s) {
+        const int len = lengths[order[s]], base = c.slot_len[slots[order[s]]];
+        row0[s] = r;
+        pc.kv_tokens += (uint64_t)base + len;
+        if (len == 1) continue;
+        const size_t np = (len + kKvPage - 1) / kKvPage;
+        if (tc_ok && base == 0 && len > kKvPage && vt_pages + np <= c.dw.vt_pages_cap) {
+            // the rule of a lone call: fresh sequences of more than one page on tcgen05 (their V^T pages go to the scratch)
+            tile0[s] = (int)(vt_pages * w.nkv);
+            vt_pages += np;
+            for (int qt = 0; qt * kTcQ < len; ++qt) {
+                const int q0 = qt * kTcQ, kend = std::min(len, q0 + kTcQ);
+                const int kt0 = (sw > 0 && q0 - sw > 0) ? (q0 - sw) / kKvPage : 0;
+                tc.push_back({(kend + kKvPage - 1) / kKvPage - kt0, s, r, len, qt});
+            }
+        } else {
+            for (int qt = 0; qt * kPrefillBM < len; ++qt) {      // the key range of attn_prefill_kernel's tile
+                const int i0 = qt * kPrefillBM, len_tile = base + std::min(i0 + kPrefillBM, len);
+                const int start = (sw > 0 && i0 - sw > 0 && base == 0) ? i0 - sw : 0;
+                mma.push_back({(len_tile + kKvPage - 1) / kKvPage - start / kKvPage, s, r, len, qt});
+            }
+        }
+    }
+    auto heavy_first = [](const Item& a, const Item& b) { return a.cost > b.cost; };
+    std::stable_sort(tc.begin(), tc.end(), heavy_first);
+    std::stable_sort(mma.begin(), mma.end(), heavy_first);
+    pc.ntc = (int)tc.size();
+    pc.nmma = (int)mma.size();
+
+    // one table: [row (seq, j)][ids][slot | RoPE of each sequence][lengths][V^T tiles][last rows, caller order][tc items][mma items]
+    size_t at = 0;
+    auto sect = [&](size_t ints) { const size_t o = at; at += align_up(ints, 4); return o; };
+    const size_t o_row = sect(2 * (size_t)T), o_ids = sect(T), o_slot = sect(2 * (size_t)n), o_len = sect(n), o_tile = sect(n),
+                 o_last = sect(n), o_tc = sect(4 * tc.size()), o_mma = sect(4 * mma.size());
+    if (c.h_pack_tab.n < at) {
+        c.h_pack_tab.alloc(at);
+        c.pack_tab.alloc(at);
+    }
+    int* h = c.h_pack_tab.p;
+    std::vector<int> perm((size_t)T);       // internal row -> row in the caller's ids order
+    for (int s = 0; s < n; ++s) {
+        const int i = order[s], len = lengths[i];
+        for (int j = 0; j < len; ++j) {
+            const int r = row0[s] + j;
+            h[o_row + 2 * (size_t)r] = s;
+            h[o_row + 2 * (size_t)r + 1] = j;
+            h[o_ids + r] = (int)ids[off[i] + j];
+            perm[r] = off[i] + j;
+        }
+        h[o_slot + s] = slots[i];
+        h[o_slot + n + s] = (int)rope_offsets[i];
+        h[o_len + s] = len;
+        h[o_tile + s] = tile0[s];
+        h[o_last + i] = row0[s] + len - 1;
+    }
+    auto put_items = [&](size_t o, const std::vector<Item>& v) {
+        for (size_t k = 0; k < v.size(); ++k) {
+            h[o + 4 * k] = v[k].s; h[o + 4 * k + 1] = v[k].r0; h[o + 4 * k + 2] = v[k].len; h[o + 4 * k + 3] = v[k].qt;
+        }
+    };
+    put_items(o_tc, tc);
+    put_items(o_mma, mma);
+    int* dt = c.pack_tab.p;
+    pc.row_tab = reinterpret_cast<const int2*>(dt + o_row);
+    pc.ids = reinterpret_cast<const uint32_t*>(dt + o_ids);
+    pc.seq_len = dt + o_len;
+    pc.vt_tile0 = dt + o_tile;
+    pc.last_row = dt + o_last;
+    pc.tc_items = reinterpret_cast<const int4*>(dt + o_tc);
+    pc.mma_items = reinterpret_cast<const int4*>(dt + o_mma);
+
+    c.dw.route_rows = (int)T;
+    c.pack_perm = std::move(perm);
+    c.slots_used = true;
+    FL_CUDA(cudaMemcpyAsync(dt, h, at * 4, cudaMemcpyHostToDevice, c.stream));
+    set_slots_kernel<<<1, 256, 0, c.stream>>>(c.state.p, dt + o_slot, n);
+    g_launches.fetch_add(1);
+    LaunchCtx lc{c.stream};
+    enqueue_forward_dense(c, lc, n, 0, false, false, &pc);
+    for (int i = 0; i < n; ++i) c.slot_len[slots[i]] += lengths[i];
 }
 
 }  // namespace fl
@@ -1433,6 +1623,16 @@ FL_EXPORT int fl_cache_moe_routing(fl_cache* c, int rows, int32_t* experts, floa
     FL_CUDA(cudaStreamSynchronize(c->stream));
     FL_CUDA(cudaMemcpy(experts, c->dw.route_sel.p, (size_t)w.L * rows * w.top_k * 4, cudaMemcpyDeviceToHost));
     FL_CUDA(cudaMemcpy(margins, c->dw.route_margin.p, (size_t)w.L * rows * 4, cudaMemcpyDeviceToHost));
+    if (!c->pack_perm.empty()) {     // a packed call ran its rows in its internal order: hand them back in the caller's ids order
+        const std::vector<int32_t> ex(experts, experts + (size_t)w.L * rows * w.top_k);
+        const std::vector<float> mg(margins, margins + (size_t)w.L * rows);
+        for (int l = 0; l < w.L; ++l)
+            for (int r = 0; r < rows; ++r) {
+                const size_t src = (size_t)l * rows + r, dst = (size_t)l * rows + c->pack_perm[r];
+                margins[dst] = mg[src];
+                for (int k = 0; k < w.top_k; ++k) experts[dst * w.top_k + k] = ex[src * w.top_k + k];
+            }
+    }
     FL_API_END
 }
 
@@ -1627,6 +1827,19 @@ FL_EXPORT int fl_forward_slots(fl_model* m, fl_cache* c, const int* slots, const
         FL_CUDA(cudaMemcpyAsync(c.h_logits.p, c.logits.p, cnt * 4, cudaMemcpyDeviceToHost, c.stream));
         FL_CUDA(cudaStreamSynchronize(c.stream));
         check_peer_error();
+        std::memcpy(logits_host, c.h_logits.p, cnt * 4);
+    });
+    FL_API_END
+}
+
+FL_EXPORT int fl_forward_packed(fl_model* m, fl_cache* c, const int* slots, const int32_t* lengths, int n, const uint32_t* ids,
+                                const size_t* rope_offsets, float* logits_host) {
+    FL_API_BEGIN
+    forward_guard(m, c, logits_host, [&](fl_cache& c) {
+        run_forward_packed(c, slots, lengths, n, ids, rope_offsets);
+        const size_t cnt = (size_t)n * c.w->Vfull;
+        FL_CUDA(cudaMemcpyAsync(c.h_logits.p, c.logits.p, cnt * 4, cudaMemcpyDeviceToHost, c.stream));
+        FL_CUDA(cudaStreamSynchronize(c.stream));
         std::memcpy(logits_host, c.h_logits.p, cnt * 4);
     });
     FL_API_END

@@ -131,6 +131,10 @@ struct fl_cache {
     std::vector<int> slot_len;            // host mirror of StepState.kv_base per slot
     fl::DevBuf<int> slot_tab;             // [2 * max_batch] staging of (slot, RoPE position) per batch row
     fl::PinnedBuf<int> h_slot_tab;
+    // packed calls (fl_forward_packed): ids, row table, per-sequence tables and attention work lists of one call, uploaded at once
+    fl::DevBuf<int> pack_tab;
+    fl::PinnedBuf<int> h_pack_tab;
+    std::vector<int> pack_perm;           // row of the last forward's internal row r in the caller's ids order (packed calls), else empty
     fl::DevBuf<uint32_t> sample_out;      // device-side sampling: the picked token
     fl::DevBuf<fl::StepState> state;
     fl::DevBuf<int> page_table;           // [max_batch, pages_per_seq]

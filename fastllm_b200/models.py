@@ -189,6 +189,23 @@ class DeviceCache:
                                              ro.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p)))
         return out
 
+    def forward_packed(self, slots, seqs, rope_offsets) -> np.ndarray:
+        """Packed forward (fl_forward_packed): sequence i (a 1-D id array of any length >= 1) is fed to cache slot slots[i] at RoPE
+        positions rope_offsets[i] + j, all in ONE forward -- new prompts and decode steps of running requests side by side.
+        -> f32 [n, vocab], row i = the last position of sequence i."""
+        parts = [np.asarray(s, dtype=np.uint32).reshape(-1) for s in seqs]
+        n = len(parts)
+        sl = np.ascontiguousarray(slots, dtype=np.int32).reshape(-1)
+        ro = np.ascontiguousarray(rope_offsets, dtype=np.uint64).reshape(-1)
+        if sl.size != n or ro.size != n:
+            raise FastllmError(-1, "slots / rope_offsets must have one entry per sequence")
+        ids = np.ascontiguousarray(np.concatenate(parts) if n else np.zeros(0, np.uint32), dtype=np.uint32)
+        lengths = np.array([p.size for p in parts], dtype=np.int32)
+        out = np.empty((n, self.vocab), dtype=np.float32)
+        _lib.check(self.lib.fl_forward_packed(self.model.h, self.h, sl.ctypes.data_as(C.c_void_p), lengths.ctypes.data_as(C.c_void_p), n,
+                                              ids.ctypes.data_as(C.c_void_p), ro.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p)))
+        return out
+
     def slot_reset(self, slot: int):
         _lib.check(self.lib.fl_cache_slot_reset(self.h, slot))
 
@@ -668,6 +685,63 @@ class ContinuousBatcher:
                 st = running[s]
                 st[1] += 1
                 take(logits[i].reshape(-1), st[0], s, st)
+        return out
+
+
+class PackedBatcher:
+    """Continuous batching above fl_forward_packed: every step is ONE forward that carries the next token of every running request
+    AND the prompts of newly admitted ones, so admitting a prompt neither costs a forward of its own nor stalls the running
+    requests.  A waiting request is admitted into a free slot while the step's tokens (one per running request plus the prompts
+    admitted so far) stay within `token_budget`; when a slot is free at least one prompt is admitted, even one longer than the
+    budget.  Per request the arithmetic is that of Model.generate, as in ContinuousBatcher: its own LogitsProcessor seeded 0, EOS
+    break before emitting, and the adapter's position rule (Llama: the caller's position; Mistral / Qwen2: +1 per call).
+    `cache` needs forward_packed(slots, seqs, rope_offsets) -> [n, V] and slot_reset(slot): a DeviceCache, or a stand-in in tests."""
+
+    def __init__(self, model, max_batch: int = 8, eos_token_id: int | None = 2, cache=None, token_budget: int = 4096):
+        self.model, self.max_batch, self.eos_token_id, self.token_budget = model, max_batch, eos_token_id, token_budget
+        self.position_per_call = getattr(model, "arch", "llama") != "llama"      # the Mistral/Qwen2 adapters' offset rule
+        self.cache = cache if cache is not None else DeviceCache(model.dev, max_batch, model._capacity())
+        self.forwards = 0       # packed forwards issued (tests / stats)
+
+    def generate(self, prompts, max_tokens: int, temperature: float = 0.0):
+        """-> one id list per prompt, in request order."""
+        out = [[] for _ in prompts]
+        if max_tokens <= 0:
+            return out
+        waiting = list(range(len(prompts)))[::-1]
+        free = list(range(self.max_batch))[::-1]
+        running = {}            # slot -> [request, next RoPE position, LogitsProcessor, token to feed]
+        while waiting or running:
+            slots = sorted(running)
+            seqs = [[running[s][3]] for s in slots]
+            ropes = [running[s][1] for s in slots]
+            budget = self.token_budget - len(slots)
+            admitted = 0
+            while waiting and free and (admitted == 0 or len(prompts[waiting[-1]]) <= budget):
+                req, slot = waiting.pop(), free.pop()
+                prompt = [int(x) for x in np.asarray(prompts[req]).reshape(-1)]
+                slots.append(slot)
+                seqs.append(prompt)
+                ropes.append(0)
+                budget -= len(prompt)
+                admitted += 1
+                running[slot] = [req, 0, LogitsProcessor(0, float(np.float32(temperature))), 0]
+            logits = np.asarray(self.cache.forward_packed(slots, seqs, ropes))
+            self.forwards += 1
+            for i, s in enumerate(slots):
+                st = running[s]
+                st[1] += 1 if self.position_per_call else len(seqs[i])      # a prompt starts at 0; a decode row feeds one token
+                tok = st[2].sample(logits[i].reshape(-1))
+                if self.eos_token_id is not None and tok == self.eos_token_id:
+                    done = True
+                else:
+                    out[st[0]].append(tok)
+                    st[3] = tok
+                    done = len(out[st[0]]) >= max_tokens
+                if done:
+                    running.pop(s)
+                    self.cache.slot_reset(s)
+                    free.append(s)
         return out
 
 

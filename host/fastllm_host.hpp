@@ -311,6 +311,88 @@ struct ContinuousBatcher {
     }
 };
 
+// fl_forward_packed: sequence i (any length >= 1) fed to cache slot slots[i] at RoPE positions ropes[i] + j, all in ONE forward
+// -> f32 [n, vocab], row i = the last position of sequence i
+inline std::vector<float> forward_packed(const DeviceModel& dev, const DeviceCache& cache, const std::vector<int>& slots,
+                                         const std::vector<std::vector<uint32_t>>& seqs, const std::vector<size_t>& ropes) {
+    std::vector<uint32_t> ids;
+    std::vector<int32_t> lengths;
+    for (const auto& q : seqs) {
+        ids.insert(ids.end(), q.begin(), q.end());
+        lengths.push_back((int32_t)q.size());
+    }
+    std::vector<float> logits(seqs.size() * (size_t)dev.cfg.vocab_size);
+    check(fl_forward_packed(dev.h, cache.h, slots.data(), lengths.data(), (int)seqs.size(), ids.data(), ropes.data(), logits.data()));
+    return logits;
+}
+
+// ---- continuous batching above fl_forward_packed.  Transliteration of fastllm_b200/models.py PackedBatcher: every step is ONE packed
+// forward carrying the next token of every running request and the prompts admitted into free slots while the step's tokens stay
+// within token_budget (at least one prompt when a slot is free).  Per request: as ContinuousBatcher.
+template <typename M>
+struct PackedBatcher {
+    const M& model;
+    int max_batch;
+    std::optional<uint32_t> eos_token_id = 2;
+    int token_budget = 4096;
+    DeviceCache cache;
+    int forwards = 0;   // packed forwards issued
+    PackedBatcher(const M& m, int max_batch_, std::optional<uint32_t> eos = 2, int budget = 4096)
+        : model(m), max_batch(max_batch_), eos_token_id(eos), token_budget(budget),
+          cache(m.dev->h, max_batch_, std::min(kKvCapacity, m.dev->cfg.max_position_embeddings)) {}
+
+    std::vector<std::vector<uint32_t>> generate(const std::vector<std::vector<uint32_t>>& prompts, int max_tokens, float temperature = 0.0f) {
+        struct Running { size_t req; size_t rope; std::unique_ptr<LogitsProcessor> lp; uint32_t tok; };
+        std::vector<std::vector<uint32_t>> out(prompts.size());
+        if (max_tokens <= 0) return out;
+        std::vector<size_t> waiting;
+        for (size_t i = prompts.size(); i-- > 0;) waiting.push_back(i);
+        std::vector<int> free_slots;
+        for (int s = max_batch; s-- > 0;) free_slots.push_back(s);
+        std::map<int, Running> running;
+        const size_t V = (size_t)model.dev->cfg.vocab_size;
+        while (!waiting.empty() || !running.empty()) {
+            std::vector<int> slots;
+            std::vector<std::vector<uint32_t>> seqs;
+            std::vector<size_t> ropes;
+            for (auto& kv : running) { slots.push_back(kv.first); seqs.push_back({kv.second.tok}); ropes.push_back(kv.second.rope); }   // ascending slots
+            long long budget = (long long)token_budget - (long long)slots.size();
+            int admitted = 0;
+            while (!waiting.empty() && !free_slots.empty() && (admitted == 0 || (long long)prompts[waiting.back()].size() <= budget)) {
+                const size_t req = waiting.back(); waiting.pop_back();
+                const int slot = free_slots.back(); free_slots.pop_back();
+                slots.push_back(slot);
+                seqs.push_back(prompts[req]);
+                ropes.push_back(0);
+                budget -= (long long)prompts[req].size();
+                admitted += 1;
+                running[slot] = Running{req, 0, std::make_unique<LogitsProcessor>(0, (double)temperature), 0};
+            }
+            const std::vector<float> logits = forward_packed(*model.dev, cache, slots, seqs, ropes);
+            forwards += 1;
+            for (size_t i = 0; i < slots.size(); ++i) {
+                Running& st = running[slots[i]];
+                st.rope += M::kPositionPerCall ? 1 : seqs[i].size();      // a prompt starts at 0; a decode row feeds one token
+                const uint32_t tok = st.lp->sample(logits.data() + i * V, V);
+                bool done;
+                if (eos_token_id && tok == *eos_token_id) {
+                    done = true;
+                } else {
+                    out[st.req].push_back(tok);
+                    st.tok = tok;
+                    done = (int)out[st.req].size() >= max_tokens;
+                }
+                if (done) {
+                    running.erase(slots[i]);
+                    check(fl_cache_slot_reset(cache.h, slots[i]));
+                    free_slots.push_back(slots[i]);
+                }
+            }
+        }
+        return out;
+    }
+};
+
 // ---- EmbeddingModel (models/embeddings.rs:17-38) / MiniLMModel (:245-447) after tokenisation -------------------------------------
 struct BertConfig {   // models/embeddings.rs:46-54 (+ the vocabulary size the reference takes from the tokenizer, :301-306)
     int hidden_size = 384, num_attention_heads = 12, num_hidden_layers = 6, intermediate_size = 1536, max_position_embeddings = 512;

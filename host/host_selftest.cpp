@@ -3,6 +3,7 @@
 // `host_selftest --sampler seed temperature vocab logits.bin` needs no GPU: it runs the mirror's LogitsProcessor over the f32 rows
 // of logits.bin and prints the sampled ids (tests/test_sampling_cpu.py compares them with the oracle).
 // `host_selftest manifest weights 0 --loglikelihood context... / continuation...` prints Model::loglikelihood as [sum, is_greedy].
+// `host_selftest manifest weights max_tokens --batch|--packed max_batch ids / ids / ...` prints the ContinuousBatcher's / PackedBatcher's ids.
 // Build: g++ -std=c++17 -O2 host/host_selftest.cpp -o host/_build/host_selftest -Lfastllm_b200 -lfastllm_b200 -Wl,-rpath,...
 #include <cstdio>
 #include <cstdlib>
@@ -69,8 +70,10 @@ int main(int argc, char** argv) {
             std::printf("[%.17g, %s]\n", ll.first, ll.second ? "true" : "false");
             return 0;
         }
-        if (argc > 5 && std::strcmp(argv[4], "--batch") == 0) {
+        if (argc > 5 && (std::strcmp(argv[4], "--batch") == 0 || std::strcmp(argv[4], "--packed") == 0)) {
             // host_selftest manifest weights max_tokens --batch max_batch id id / id id id / ...: the C++ ContinuousBatcher over sequence slots
+            // (--packed: the C++ PackedBatcher, prompts admitted into the decode steps' packed forwards)
+            const bool packed = std::strcmp(argv[4], "--packed") == 0;
             const int max_batch = std::atoi(argv[5]);
             std::vector<std::vector<uint32_t>> prompts(1);
             for (int i = 6; i < argc; ++i) {
@@ -78,8 +81,16 @@ int main(int argc, char** argv) {
                 else prompts.back().push_back((uint32_t)std::strtoul(argv[i], nullptr, 10));
             }
             auto pr = fastllm::LlamaWithConfig::initialize_model(cfg, tensors, 0);
-            fastllm::ContinuousBatcher<fastllm::LlamaWithConfig> cb(pr.first, max_batch, std::nullopt);
-            const auto outs = cb.generate(prompts, max_tokens);
+            std::vector<std::vector<uint32_t>> outs;
+            if (packed) {
+                fastllm::PackedBatcher<fastllm::LlamaWithConfig> pb(pr.first, max_batch, std::nullopt);
+                outs = pb.generate(prompts, max_tokens);
+                std::fprintf(stderr, "packed forwards: %d\n", pb.forwards);
+            } else {
+                fastllm::ContinuousBatcher<fastllm::LlamaWithConfig> cb(pr.first, max_batch, std::nullopt);
+                outs = cb.generate(prompts, max_tokens);
+                std::fprintf(stderr, "ragged steps: %d\n", cb.steps);
+            }
             std::printf("[");
             for (size_t r = 0; r < outs.size(); ++r) {
                 std::printf("%s[", r ? "," : "");
@@ -87,7 +98,6 @@ int main(int argc, char** argv) {
                 std::printf("]");
             }
             std::printf("]\n");
-            std::fprintf(stderr, "ragged steps: %d\n", cb.steps);
             return 0;
         }
         std::vector<uint32_t> prompt;

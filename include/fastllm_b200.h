@@ -167,6 +167,22 @@ FL_EXPORT int fl_forward_slots(fl_model* m, fl_cache* c, const int* slots, const
                                float* logits_host);
 FL_EXPORT int fl_cache_slot_reset(fl_cache* c, int slot);        /* the slot's sequence is finished: length := 0 */
 FL_EXPORT int fl_cache_slot_len(fl_cache* c, int slot, int* out);
+/* n sequences in ONE forward, each fed its own number of new tokens: sequence i is cache slot slots[i], fed
+ * ids[o_i, o_i + lengths[i]) (o_i = lengths[0] + ... + lengths[i-1]) at RoPE positions rope_offsets[i] + j.
+ * A new prompt (empty slot, lengths[i] = prompt length) and a decode step of a running request (lengths[i] = 1) can share a call.
+ * logits_host: f32 [n, vocab]; row i = the last position of sequence i (what fl_forward_slots returns for that sequence).
+ * Per sequence the call computes what fl_forward_slots(slots + i, ids + o_i, 1, lengths[i], rope_offsets + i) would: slot_len grows
+ * by lengths[i], the Llama rule and the Mistral/Qwen2 sliding window (multi-token sequences only) apply per sequence.  Results do not
+ * depend on the order of the sequences; when every length is the same t the call is fl_forward_slots(slots, ids, n, t, ...).
+ * Like fl_forward_slots it drives the cache by slots (uniform calls are refused until fl_cache_reset).  After a packed call,
+ * fl_cache_moe_routing reports rows = the sum of the lengths, in ids order.
+ * FL_ERR_INVALID:     a NULL pointer, n < 1 or n > max_batch, a length < 1, a slot out of range or repeated, an id >= vocab, a RoPE
+ *                     position >= max_position_embeddings, or a multi-token sequence on a non-empty slot of a Llama model.
+ * FL_ERR_STATE:       slot_len + length > max_seq, or the cache holds tokens of uniform calls.
+ * FL_ERR_UNSUPPORTED: the model is sharded (tp_size > 1, Mixtral expert parallelism included), or its shapes do not admit the dense path.
+ * All are checked before any device work: a failed call leaves the cache unchanged. */
+FL_EXPORT int fl_forward_packed(fl_model* m, fl_cache* c, const int* slots, const int32_t* lengths, int n, const uint32_t* ids,
+                                const size_t* rope_offsets, float* logits_host);
 
 /* Diagnostics (no reference counterpart): the router's decisions in the LAST forward on this cache (Mixtral only) -- experts
  * [layers][rows][num_experts_per_tok] in pick order (MixtralSparseMoeBlock's sort, models/mixtral.rs via candle-transformers) and
