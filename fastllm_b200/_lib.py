@@ -45,6 +45,9 @@ SYMBOLS = {
     "fl_model_destroy": (_I, [_VP]),
     "fl_model_weight_bytes": (_I, [_VP, C.POINTER(_U64)]),
     "fl_cache_create": (_I, [_VP, _I, _I, C.POINTER(_VP)]),
+    "fl_cache_create_pool": (_I, [_VP, _I, _I, _I, C.POINTER(_VP)]),
+    "fl_cache_pool_pages": (_I, [_VP, C.POINTER(_I), C.POINTER(_I)]),
+    "fl_cache_slot_fork": (_I, [_VP, _I, _I]),
     "fl_cache_reset": (_I, [_VP]),
     "fl_cache_kv_len": (_I, [_VP, C.POINTER(_I)]),
     "fl_cache_fill_synthetic": (_I, [_VP, _I, _I, _U64]),

@@ -176,5 +176,19 @@ static __global__ void set_slots_kernel(StepState* st, const int* __restrict__ t
     if (threadIdx.x == 0) st->ragged = 1;
 }
 static __global__ void reset_slot_kernel(StepState* st, int slot) { st->kv_base[slot] = 0; }
+// fl_cache_slot_fork: the forked slot's length
+static __global__ void set_slot_len_kernel(StepState* st, int slot, int len) { st->kv_base[slot] = len; }
+// Page-table entries a call changed: table[upd[i].x] = upd[i].y
+static __global__ void page_table_scatter_kernel(int* __restrict__ table, const int2* __restrict__ upd, int n) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) table[upd[i].x] = upd[i].y;
+}
+// fl_cache_slot_fork: copy one K or V page (blockIdx.z) of every layer (blockIdx.y) from page src to page dst; elems = nkv * 64 * d
+static __global__ void kv_page_copy_kernel(uint16_t* kpool, uint16_t* vpool, size_t layer_elems, int src, int dst, int elems) {
+    uint16_t* pool = (blockIdx.z ? vpool : kpool) + (size_t)blockIdx.y * layer_elems;
+    const uint4* s = reinterpret_cast<const uint4*>(pool + (size_t)src * elems);
+    uint4* d = reinterpret_cast<uint4*>(pool + (size_t)dst * elems);
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < elems / 8; i += gridDim.x * blockDim.x) d[i] = s[i];
+}
 
 }  // namespace fl

@@ -507,20 +507,23 @@ static void launch_persistent(fl_cache& c, int nsteps, bool feedback) {
     }
 }
 
-static void cache_create(fl_cache& c, int max_batch, int max_seq) {
+// pool_tokens <= 0: the pool of max_batch * ceil(max_seq / 64) pages, in which every slot's home pages exist
+static void cache_create(fl_cache& c, int max_batch, int max_seq, int64_t pool_tokens) {
     const Weights& w = *c.w;
     FL_CHECK(w.table.finalized, FL_ERR_STATE, "model not finalized");
     FL_CHECK(max_batch >= 1 && max_batch <= kMaxBatch && max_seq >= 1, FL_ERR_INVALID, "bad cache dimensions");
     c.max_batch = max_batch;
     c.max_seq = max_seq;
     c.pages_per_seq = (max_seq + kKvPage - 1) / kKvPage;
+    const int64_t pool_pages = pool_tokens > 0 ? (pool_tokens + kKvPage - 1) / kKvPage : (int64_t)max_batch * c.pages_per_seq;
+    FL_CHECK(pool_pages < (1ll << 31) && (int64_t)max_batch * c.pages_per_seq < (1ll << 31), FL_ERR_INVALID, "bad cache dimensions");
     FL_CUDA(cudaStreamCreateWithFlags(&c.stream, cudaStreamNonBlocking));
     c.state.alloc(1, true);
-    std::vector<int> pt((size_t)max_batch * c.pages_per_seq);
-    for (size_t i = 0; i < pt.size(); ++i) pt[i] = (int)i;   // static page assignment; the layout stays paged
+    c.pool.init(max_batch, c.pages_per_seq, (int)pool_pages);
+    const std::vector<int>& pt = c.pool.table();     // no page taken yet: every entry names its home page (or page 0)
     c.page_table.alloc(pt.size());
     FL_CUDA(cudaMemcpy(c.page_table.p, pt.data(), pt.size() * 4, cudaMemcpyHostToDevice));
-    c.layer_pool_elems = (size_t)max_batch * c.pages_per_seq * w.nkv * kKvPage * w.d;
+    c.layer_pool_elems = (size_t)pool_pages * w.nkv * kKvPage * w.d;
     c.kpool.alloc(c.layer_pool_elems * w.L, true);
     c.vpool.alloc(c.layer_pool_elems * w.L, true);
     {
@@ -570,6 +573,32 @@ static void cache_destroy_graphs(fl_cache& c) {
     for (auto& kv : c.graphs)
         if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
     c.graphs.clear();
+}
+
+// Takes the pages a call will write -- (slot, tokens it holds after the call) per sequence -- after the call's validation and before
+// its first device operation, then writes the table entries that changed since the last call.  When every page is in place (always
+// on a default pool without forks) nothing is launched.  The scatter is a plain launch on the cache's stream, complete before the
+// forward's first kernel starts, as set_slots_kernel's tables are: the stream-K decode attention reads the table before
+// griddepcontrol.wait.  The staging buffer is free again at the next call: every forward entry point synchronises the stream.
+static void reserve_pages(fl_cache& c, std::vector<std::pair<int, int64_t>> req) {
+    FL_CHECK(c.pool.reserve(std::move(req)), FL_ERR_STATE, "KV page pool exhausted");
+    const std::vector<std::pair<int, int>> upd = c.pool.flush();
+    if (upd.empty()) return;
+    const size_t n = upd.size();
+    if (c.h_pt_upd.n < n) {
+        c.h_pt_upd.alloc(n);
+        c.pt_upd.alloc(n);
+    }
+    for (size_t i = 0; i < n; ++i) c.h_pt_upd.p[i] = make_int2(upd[i].first, upd[i].second);
+    FL_CUDA(cudaMemcpyAsync(c.pt_upd.p, c.h_pt_upd.p, n * sizeof(int2), cudaMemcpyHostToDevice, c.stream));
+    page_table_scatter_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c.stream>>>(c.page_table.p, c.pt_upd.p, (int)n);
+    g_launches.fetch_add(1);
+}
+// The uniform calls: slots 0..b-1, each holding `tokens` tokens after the call.
+static void reserve_uniform(fl_cache& c, int b, int64_t tokens) {
+    std::vector<std::pair<int, int64_t>> req;
+    for (int s = 0; s < b; ++s) req.push_back({s, tokens});
+    reserve_pages(c, std::move(req));
 }
 
 // A packed call (fl_forward_packed) on the device: sequences of different lengths, rows in the internal order (run_forward_packed).
@@ -1204,10 +1233,10 @@ static void check_call(fl_cache& c, const uint32_t* ids, int b, int t, size_t ro
 static void run_forward(fl_cache& c, const uint32_t* ids, int b, int t, size_t rope_offset, const uint32_t* targets = nullptr) {
     check_call(c, ids, b, t, rope_offset, 0);
     const int R = b * t;
-    if (targets) {
+    if (targets)
         for (int i = 0; i < R; ++i) FL_CHECK(targets[i] < (uint32_t)c.w->V, FL_ERR_INVALID, "target id out of range");
-        ensure_logprob_ws(c, R);
-    }
+    reserve_uniform(c, b, (int64_t)c.kv_len + t);
+    if (targets) ensure_logprob_ws(c, R);
     if (targets || uses_dense(c, R)) ensure_dense_ws(c, R);
     std::memcpy(c.h_ids.p, ids, (size_t)R * 4);
     FL_CUDA(cudaMemcpyAsync(c.ids.p, c.h_ids.p, (size_t)R * 4, cudaMemcpyHostToDevice, c.stream));
@@ -1245,6 +1274,9 @@ static void run_forward_slots(fl_cache& c, const int* slots, const uint32_t* ids
                  "Llama: multi-token forward needs an empty cache (candle builds a t x t mask)");
     }
     for (int i = 0; i < n * t; ++i) FL_CHECK(ids[i] < (uint32_t)w.Vfull, FL_ERR_INVALID, "token id out of range");
+    std::vector<std::pair<int, int64_t>> req;
+    for (int i = 0; i < n; ++i) req.push_back({slots[i], (int64_t)c.slot_len[slots[i]] + t});
+    reserve_pages(c, std::move(req));
     ensure_dense_ws(c, n * t);
     c.dw.route_rows = n * t;
     c.pack_perm.clear();
@@ -1301,6 +1333,11 @@ static void run_forward_packed(fl_cache& c, const int* slots, const int32_t* len
     for (int i = 0; i < n; ++i) nd += lengths[i] == 1;
     FL_CHECK(nd == 0 || (c.kv_tmaps && w.nh / w.nkv <= 16), FL_ERR_UNSUPPORTED,
              "batched decode attention: GQA group > 16 heads or KV pool beyond 2^31 rows");
+    {
+        std::vector<std::pair<int, int64_t>> req;
+        for (int i = 0; i < n; ++i) req.push_back({slots[i], (int64_t)c.slot_len[slots[i]] + lengths[i]});
+        reserve_pages(c, std::move(req));
+    }
     ensure_dense_ws(c, (int)T);
 
     // internal order and rows
@@ -1576,8 +1613,56 @@ FL_EXPORT int fl_cache_create(fl_model* m, int max_batch, int max_seq, fl_cache*
     use_device();
     std::unique_ptr<fl_cache> c(new fl_cache);
     c->w = m->w;
-    cache_create(*c, max_batch, max_seq);
+    cache_create(*c, max_batch, max_seq, 0);
     *out = c.release();
+    FL_API_END
+}
+
+FL_EXPORT int fl_cache_create_pool(fl_model* m, int max_batch, int max_seq, int pool_tokens, fl_cache** out) {
+    FL_API_BEGIN
+    FL_CHECK(m && out, FL_ERR_INVALID, "NULL argument");
+    FL_CHECK(m->w != nullptr, FL_ERR_INVALID, "BERT models have no KV cache");
+    FL_CHECK(pool_tokens >= 1, FL_ERR_INVALID, "pool_tokens must be >= 1");
+    use_device();
+    std::unique_ptr<fl_cache> c(new fl_cache);
+    c->w = m->w;
+    cache_create(*c, max_batch, max_seq, pool_tokens);
+    *out = c.release();
+    FL_API_END
+}
+
+FL_EXPORT int fl_cache_pool_pages(fl_cache* c, int* free_pages, int* total_pages) {
+    FL_API_BEGIN
+    FL_CHECK(c && free_pages && total_pages, FL_ERR_INVALID, "NULL argument");
+    *free_pages = c->pool.free_pages();
+    *total_pages = c->pool.total_pages();
+    FL_API_END
+}
+
+FL_EXPORT int fl_cache_slot_fork(fl_cache* c, int src, int dst) {
+    FL_API_BEGIN
+    FL_CHECK(c, FL_ERR_INVALID, "NULL argument");
+    FL_CHECK(src >= 0 && src < c->max_batch && dst >= 0 && dst < c->max_batch, FL_ERR_INVALID, "slot index out of range");
+    FL_CHECK(src != dst, FL_ERR_INVALID, "a slot cannot be forked into itself");
+    FL_CHECK(!c->poisoned, FL_ERR_CUDA, "cache poisoned by an earlier CUDA error");
+    FL_CHECK(c->slots_used || c->kv_len == 0, FL_ERR_STATE, "the cache holds tokens of uniform calls: fl_cache_reset before driving it by slots");
+    const int len = c->slot_len[src];
+    FL_CHECK(len > 0, FL_ERR_INVALID, "the source slot is empty");
+    FL_CHECK(c->slot_len[dst] == 0, FL_ERR_STATE, "the destination slot is not empty: fl_cache_slot_reset it first");
+    use_device();
+    std::pair<int, int> copy;
+    FL_CHECK(c->pool.fork(src, dst, len, &copy), FL_ERR_STATE, "KV page pool exhausted (no free page for the partial last page)");
+    const Weights& w = *c->w;
+    if (copy.first >= 0) {      // the partial last page: K and V of every layer
+        const int elems = w.nkv * kKvPage * w.d;
+        LaunchCtx lc{c->stream, /*pdl=*/false};     // a plain launch (named in fl_prof profiles)
+        launch(lc, "kv_page_copy", (uint64_t)2 * 2 * w.L * elems * 2, kv_page_copy_kernel, dim3(std::max(1, std::min(16, elems / 8 / 256)), w.L, 2),
+               dim3(256), 0, c->kpool.p, c->vpool.p, c->layer_pool_elems, copy.first, copy.second, elems);
+    }
+    set_slot_len_kernel<<<1, 1, 0, c->stream>>>(c->state.p, dst, len);
+    g_launches.fetch_add(1);
+    c->slot_len[dst] = len;
+    c->slots_used = true;
     FL_API_END
 }
 
@@ -1591,6 +1676,7 @@ FL_EXPORT int fl_cache_reset(fl_cache* c) {
     c->kv_len = 0;
     c->slots_used = false;
     std::fill(c->slot_len.begin(), c->slot_len.end(), 0);
+    c->pool.release_all();
     FL_API_END
 }
 
@@ -1602,6 +1688,8 @@ FL_EXPORT int fl_cache_slot_reset(fl_cache* c, int slot) {
     reset_slot_kernel<<<1, 1, 0, c->stream>>>(c->state.p, slot);
     g_launches.fetch_add(1);
     c->slot_len[slot] = 0;
+    // a cache driven by uniform calls keeps the row's pages: its common length kv_len still covers them (fl_cache_reset frees them)
+    if (c->slots_used || c->kv_len == 0) c->pool.release(slot);
     FL_API_END
 }
 
@@ -1647,7 +1735,14 @@ FL_EXPORT int fl_cache_fill_synthetic(fl_cache* c, int batch, int kv_len, uint64
     FL_API_BEGIN
     FL_CHECK(c, FL_ERR_INVALID, "NULL argument");
     FL_CHECK(batch >= 1 && batch <= c->max_batch && kv_len >= 0 && kv_len <= c->max_seq, FL_ERR_INVALID, "bad synthetic fill size");
+    FL_CHECK((int64_t)batch * KvPool::pages_for(kv_len) <= c->pool.total_pages(), FL_ERR_STATE, "KV page pool exhausted");
     use_device();
+    // the fill overwrites the whole pool: earlier sequences are gone, and the cache holds a uniform prefill of kv_len tokens in slots
+    // 0..batch-1 (a slot-driven cache becomes a uniform one, as after fl_cache_reset)
+    c->pool.release_all();
+    c->slots_used = false;
+    std::fill(c->slot_len.begin(), c->slot_len.end(), 0);
+    reserve_uniform(*c, batch, kv_len);
     const RowMap ident{0, 0, 0, 0};
     synth_fill_bf16_kernel<<<kNumSMs * 8, 256, 0, c->stream>>>(c->kpool.p, 1, (int64_t)c->kpool.n, (int64_t)c->kpool.n, tensor_seed(seed, "kv.k"), 0.5f, ident);
     synth_fill_bf16_kernel<<<kNumSMs * 8, 256, 0, c->stream>>>(c->vpool.p, 1, (int64_t)c->vpool.n, (int64_t)c->vpool.n, tensor_seed(seed, "kv.v"), 0.5f, ident);
@@ -1718,6 +1813,7 @@ FL_EXPORT int fl_decode_greedy_loop(fl_model* m, fl_cache* c, const uint32_t* fi
     forward_guard(m, c, true, [&](fl_cache& c) {
         FL_CHECK(steps >= 1, FL_ERR_INVALID, "steps must be >= 1");
         check_call(c, first_ids, b, 1, rope_offset, steps - 1);
+        reserve_uniform(c, b, (int64_t)c.kv_len + steps);      // the loop never returns to the host: every step's pages up front
         if (uses_dense(c, b)) ensure_dense_ws(c, b);
         if (c.trace_cap < (size_t)steps * b) {
             c.trace.alloc((size_t)steps * b);

@@ -9,6 +9,7 @@
 #include "bert_model.cuh"
 #include "decode_persistent.cuh"
 #include "gemv.cuh"
+#include "kv_pool.hpp"
 #include "runtime.cuh"
 #include "tensor_table.hpp"
 
@@ -138,7 +139,10 @@ struct fl_cache {
     fl::DevBuf<uint32_t> sample_out;      // device-side sampling: the picked token
     fl::DevBuf<fl::StepState> state;
     fl::DevBuf<int> page_table;           // [max_batch, pages_per_seq]
-    fl::DevBuf<uint16_t> kpool, vpool;    // [L][pages][nkv][kKvPage][d]
+    fl::KvPool pool;                      // owner of every page: refcounts, per-slot page lists, the host side of page_table
+    fl::DevBuf<int2> pt_upd;              // (table index, page) of the entries a call changed, scattered into page_table
+    fl::PinnedBuf<int2> h_pt_upd;
+    fl::DevBuf<uint16_t> kpool, vpool;    // [L][pool pages][nkv][kKvPage][d]
     size_t layer_pool_elems = 0;
     CUtensorMap tm_kpool{}, tm_vpool{};   // the pools as [rows, d] matrices (stream-K decode attention); valid when kv_tmaps
     bool kv_tmaps = false;

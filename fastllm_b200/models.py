@@ -94,14 +94,19 @@ class DeviceModel:
 
 
 class DeviceCache:
-    """fl_cache*: paged KV cache + per-cache stream/workspaces."""
+    """fl_cache*: paged KV cache + per-cache stream/workspaces.  pool_tokens=None: every slot can reach max_seq (a pool of
+    max_batch * ceil(max_seq / 64) pages); otherwise the slots share a pool of pool_tokens tokens (rounded up to 64-token pages),
+    taken as sequences grow."""
 
-    def __init__(self, model: DeviceModel, max_batch: int, max_seq: int):
+    def __init__(self, model: DeviceModel, max_batch: int, max_seq: int, pool_tokens: int | None = None):
         self.model, self.lib = model, model.lib
         self.max_batch, self.max_seq = max_batch, max_seq
         self.vocab = model.cfg.vocab_size
         h = C.c_void_p()
-        _lib.check(self.lib.fl_cache_create(model.h, max_batch, max_seq, C.byref(h)))
+        if pool_tokens is None:
+            _lib.check(self.lib.fl_cache_create(model.h, max_batch, max_seq, C.byref(h)))
+        else:
+            _lib.check(self.lib.fl_cache_create_pool(model.h, max_batch, max_seq, pool_tokens, C.byref(h)))
         self.h = h
 
     def reset(self):
@@ -213,6 +218,16 @@ class DeviceCache:
         n = C.c_int()
         _lib.check(self.lib.fl_cache_slot_len(self.h, slot, C.byref(n)))
         return n.value
+
+    def slot_fork(self, src: int, dst: int):
+        """fl_cache_slot_fork: the empty slot dst continues from src's cached tokens (full pages shared, the partial one copied)."""
+        _lib.check(self.lib.fl_cache_slot_fork(self.h, src, dst))
+
+    def pool_pages(self):
+        """-> (free pages, total pages) of the KV pool."""
+        f, t = C.c_int(), C.c_int()
+        _lib.check(self.lib.fl_cache_pool_pages(self.h, C.byref(f), C.byref(t)))
+        return f.value, t.value
 
     def moe_routing(self, rows: int):
         """Router decisions of the last forward (Mixtral): experts [layers, rows, top_k] int32 in pick order, margins [layers, rows] f32."""
@@ -688,6 +703,13 @@ class ContinuousBatcher:
         return out
 
 
+KV_PAGE = 64        # tokens per KV page
+
+
+def _pages(tokens: int) -> int:
+    return -(-tokens // KV_PAGE)
+
+
 class PackedBatcher:
     """Continuous batching above fl_forward_packed: every step is ONE forward that carries the next token of every running request
     AND the prompts of newly admitted ones, so admitting a prompt neither costs a forward of its own nor stalls the running
@@ -695,53 +717,115 @@ class PackedBatcher:
     admitted so far) stay within `token_budget`; when a slot is free at least one prompt is admitted, even one longer than the
     budget.  Per request the arithmetic is that of Model.generate, as in ContinuousBatcher: its own LogitsProcessor seeded 0, EOS
     break before emitting, and the adapter's position rule (Llama: the caller's position; Mistral / Qwen2: +1 per call).
-    `cache` needs forward_packed(slots, seqs, rope_offsets) -> [n, V] and slot_reset(slot): a DeviceCache, or a stand-in in tests."""
+    `cache` needs forward_packed(slots, seqs, rope_offsets) -> [n, V] and slot_reset(slot) (and slot_fork(src, dst) for a shared
+    prefix): a DeviceCache, or a stand-in in tests.
 
-    def __init__(self, model, max_batch: int = 8, eos_token_id: int | None = 2, cache=None, token_budget: int = 4096):
+    pool_tokens: the slots share a KV pool of that many tokens instead of max_seq each.  A waiting request is then also admitted only
+    if the pages it can ever need -- its prompt plus max_tokens, less the prefix pages it shares -- fit the pool minus the pages
+    reserved for running requests (and the shared prefix), so no call can run out of pages and nothing is preempted.  Requests are
+    admitted in order: one that does not fit waits for pages to free up."""
+
+    def __init__(self, model, max_batch: int = 8, eos_token_id: int | None = 2, cache=None, token_budget: int = 4096,
+                 pool_tokens: int | None = None):
         self.model, self.max_batch, self.eos_token_id, self.token_budget = model, max_batch, eos_token_id, token_budget
         self.position_per_call = getattr(model, "arch", "llama") != "llama"      # the Mistral/Qwen2 adapters' offset rule
-        self.cache = cache if cache is not None else DeviceCache(model.dev, max_batch, model._capacity())
+        self.sliding_window = getattr(getattr(model, "cfg", None), "sliding_window", 0) if self.position_per_call else 0
+        self.cache = cache if cache is not None else DeviceCache(model.dev, max_batch, model._capacity(), pool_tokens)
+        self.pool_pages = None if pool_tokens is None else _pages(pool_tokens)
+        self.slot_pages = _pages(self.cache.max_seq) if hasattr(self.cache, "max_seq") else None   # a slot never holds more
         self.forwards = 0       # packed forwards issued (tests / stats)
+        self.prefill_tokens = 0  # prompt tokens fed (tests / stats): a shared prefix counts once
+        self.peak_pages = 0      # most pages reserved at once (with pool_tokens)
 
-    def generate(self, prompts, max_tokens: int, temperature: float = 0.0):
-        """-> one id list per prompt, in request order."""
+    def _uses_prefix(self, prompt, prefix) -> bool:
+        """A request continues from the shared prefix's slot when its prompt extends the prefix and splitting the prompt there
+        computes what the one-call prompt does: not on Llama (a multi-token call on a non-empty sequence is refused there), and not
+        for a prompt longer than the sliding window (the window of a multi-token call applies to an empty sequence only)."""
+        return (prefix is not None and self.position_per_call and len(prompt) > len(prefix) and list(prompt[:len(prefix)]) == prefix
+                and not (self.sliding_window and len(prompt) > self.sliding_window))
+
+    def generate(self, prompts, max_tokens: int, temperature: float = 0.0, shared_prefix=None):
+        """-> one id list per prompt, in request order.  shared_prefix: token ids that many prompts start with; it is fed once into a
+        slot held for the call, and each request that extends it starts as a fork of that slot, fed only the rest of its prompt at
+        RoPE offset len(shared_prefix) (the positions of the one-call prompt).  Other requests take the normal path."""
         out = [[] for _ in prompts]
         if max_tokens <= 0:
             return out
+        prompts = [[int(x) for x in np.asarray(p).reshape(-1)] for p in prompts]
+        prefix = None if shared_prefix is None else [int(x) for x in np.asarray(shared_prefix).reshape(-1)]
+        if not prefix or self.max_batch < 2:
+            prefix = None       # nothing to share, or no slot left for requests beside the prefix's
+        forked = [self._uses_prefix(p, prefix) for p in prompts]
         waiting = list(range(len(prompts)))[::-1]
         free = list(range(self.max_batch))[::-1]
-        running = {}            # slot -> [request, next RoPE position, LogitsProcessor, token to feed]
-        while waiting or running:
-            slots = sorted(running)
-            seqs = [[running[s][3]] for s in slots]
-            ropes = [running[s][1] for s in slots]
-            budget = self.token_budget - len(slots)
-            admitted = 0
-            while waiting and free and (admitted == 0 or len(prompts[waiting[-1]]) <= budget):
-                req, slot = waiting.pop(), free.pop()
-                prompt = [int(x) for x in np.asarray(prompts[req]).reshape(-1)]
-                slots.append(slot)
-                seqs.append(prompt)
-                ropes.append(0)
-                budget -= len(prompt)
-                admitted += 1
-                running[slot] = [req, 0, LogitsProcessor(0, float(np.float32(temperature))), 0]
-            logits = np.asarray(self.cache.forward_packed(slots, seqs, ropes))
+        running = {}            # slot -> [request, next RoPE position, LogitsProcessor, token to feed, pages reserved]
+        reserved = 0            # pages the admission rule holds for running requests and the prefix
+
+        def need(req):
+            n = _pages(len(prompts[req]) + max_tokens)
+            if self.slot_pages is not None:
+                n = min(n, self.slot_pages)
+            return n - (len(prefix) // KV_PAGE if forked[req] else 0)
+
+        pslot = None
+        if any(forked):
+            pslot = free.pop()
+            reserved = _pages(len(prefix))
+            self.cache.forward_packed([pslot], [prefix], [0])
             self.forwards += 1
-            for i, s in enumerate(slots):
-                st = running[s]
-                st[1] += 1 if self.position_per_call else len(seqs[i])      # a prompt starts at 0; a decode row feeds one token
-                tok = st[2].sample(logits[i].reshape(-1))
-                if self.eos_token_id is not None and tok == self.eos_token_id:
-                    done = True
-                else:
-                    out[st[0]].append(tok)
-                    st[3] = tok
-                    done = len(out[st[0]]) >= max_tokens
-                if done:
-                    running.pop(s)
-                    self.cache.slot_reset(s)
-                    free.append(s)
+            self.prefill_tokens += len(prefix)
+        try:
+            while waiting or running:
+                slots = sorted(running)
+                seqs = [[running[s][3]] for s in slots]
+                ropes = [running[s][1] for s in slots]
+                budget = self.token_budget - len(slots)
+                admitted = 0
+                while waiting and free:
+                    req = waiting[-1]
+                    seq = prompts[req][len(prefix):] if forked[req] else prompts[req]
+                    if admitted and len(seq) > budget:
+                        break
+                    if self.pool_pages is not None and reserved + need(req) > self.pool_pages:
+                        if not running and not admitted:
+                            raise ValueError(f"request {req} needs {need(req)} KV pages; the pool holds {self.pool_pages - reserved}")
+                        break
+                    waiting.pop()
+                    slot = free.pop()
+                    if forked[req]:
+                        self.cache.slot_fork(pslot, slot)
+                    slots.append(slot)
+                    seqs.append(seq)
+                    ropes.append(len(prefix) if forked[req] else 0)
+                    budget -= len(seq)
+                    admitted += 1
+                    self.prefill_tokens += len(seq)
+                    pages = need(req) if self.pool_pages is not None else 0
+                    reserved += pages
+                    running[slot] = [req, 0, LogitsProcessor(0, float(np.float32(temperature))), 0, pages]
+                self.peak_pages = max(self.peak_pages, reserved)
+                logits = np.asarray(self.cache.forward_packed(slots, seqs, ropes))
+                self.forwards += 1
+                for i, s in enumerate(slots):
+                    st = running[s]
+                    # a prompt starts at 0; a decode row feeds one token.  A forked request's suffix is the rest of its prompt: the
+                    # Mistral/Qwen2 rule then continues from 1, as after the one-call prompt.
+                    st[1] += 1 if self.position_per_call else len(seqs[i])
+                    tok = st[2].sample(logits[i].reshape(-1))
+                    if self.eos_token_id is not None and tok == self.eos_token_id:
+                        done = True
+                    else:
+                        out[st[0]].append(tok)
+                        st[3] = tok
+                        done = len(out[st[0]]) >= max_tokens
+                    if done:
+                        running.pop(s)
+                        reserved -= st[4]
+                        self.cache.slot_reset(s)
+                        free.append(s)
+        finally:
+            if pslot is not None:
+                self.cache.slot_reset(pslot)
         return out
 
 

@@ -77,6 +77,14 @@ struct DeviceModel {   // shared device weights (fl_model*)
 struct DeviceCache {   // paged KV cache + stream (fl_cache*)
     fl_cache* h = nullptr;
     DeviceCache(fl_model* m, int max_batch, int max_seq) { check(fl_cache_create(m, max_batch, max_seq, &h)); }
+    // the slots share a pool of pool_tokens tokens of KV (fl_cache_create_pool)
+    DeviceCache(fl_model* m, int max_batch, int max_seq, int pool_tokens) { check(fl_cache_create_pool(m, max_batch, max_seq, pool_tokens, &h)); }
+    void slot_fork(int src, int dst) const { check(fl_cache_slot_fork(h, src, dst)); }
+    std::pair<int, int> pool_pages() const {   // (free, total)
+        int f = 0, t = 0;
+        check(fl_cache_pool_pages(h, &f, &t));
+        return {f, t};
+    }
     ~DeviceCache() { if (h) fl_cache_destroy(h); }
     DeviceCache(const DeviceCache&) = delete;
     DeviceCache& operator=(const DeviceCache&) = delete;
@@ -328,29 +336,70 @@ inline std::vector<float> forward_packed(const DeviceModel& dev, const DeviceCac
 
 // ---- continuous batching above fl_forward_packed.  Transliteration of fastllm_b200/models.py PackedBatcher: every step is ONE packed
 // forward carrying the next token of every running request and the prompts admitted into free slots while the step's tokens stay
-// within token_budget (at least one prompt when a slot is free).  Per request: as ContinuousBatcher.
+// within token_budget (at least one prompt when a slot is free).  Per request: as ContinuousBatcher.  With pool_tokens the slots share
+// a KV pool, and a request is admitted only if the pages it can ever need fit the pool minus those reserved for running requests and
+// the shared prefix.  A shared prefix is fed once into a slot held for the call; requests that extend it start as forks of that slot.
+constexpr int kKvPage = 64;
+inline int kv_pages(long long tokens) { return (int)((tokens + kKvPage - 1) / kKvPage); }
+
 template <typename M>
 struct PackedBatcher {
     const M& model;
     int max_batch;
     std::optional<uint32_t> eos_token_id = 2;
     int token_budget = 4096;
+    std::optional<int> pool_pages;
+    int max_seq;
     DeviceCache cache;
     int forwards = 0;   // packed forwards issued
-    PackedBatcher(const M& m, int max_batch_, std::optional<uint32_t> eos = 2, int budget = 4096)
+    PackedBatcher(const M& m, int max_batch_, std::optional<uint32_t> eos = 2, int budget = 4096, std::optional<int> pool_tokens = std::nullopt)
         : model(m), max_batch(max_batch_), eos_token_id(eos), token_budget(budget),
-          cache(m.dev->h, max_batch_, std::min(kKvCapacity, m.dev->cfg.max_position_embeddings)) {}
+          pool_pages(pool_tokens ? std::optional<int>(kv_pages(*pool_tokens)) : std::nullopt),
+          max_seq(std::min(kKvCapacity, m.dev->cfg.max_position_embeddings)),
+          cache(pool_tokens ? DeviceCache(m.dev->h, max_batch_, max_seq, *pool_tokens) : DeviceCache(m.dev->h, max_batch_, max_seq)) {}
 
-    std::vector<std::vector<uint32_t>> generate(const std::vector<std::vector<uint32_t>>& prompts, int max_tokens, float temperature = 0.0f) {
-        struct Running { size_t req; size_t rope; std::unique_ptr<LogitsProcessor> lp; uint32_t tok; };
+    // as models.PackedBatcher._uses_prefix: not on Llama, not for a prompt longer than the sliding window
+    bool uses_prefix(const std::vector<uint32_t>& prompt, const std::vector<uint32_t>* prefix) const {
+        if (!prefix || !M::kPositionPerCall || prompt.size() <= prefix->size()) return false;
+        if (!std::equal(prefix->begin(), prefix->end(), prompt.begin())) return false;
+        const int window = model.dev->cfg.sliding_window;
+        return !(window > 0 && (long long)prompt.size() > window);
+    }
+
+    std::vector<std::vector<uint32_t>> generate(const std::vector<std::vector<uint32_t>>& prompts, int max_tokens, float temperature = 0.0f,
+                                                const std::vector<uint32_t>* shared_prefix = nullptr) {
+        struct Running { size_t req; size_t rope; std::unique_ptr<LogitsProcessor> lp; uint32_t tok; int pages; };
         std::vector<std::vector<uint32_t>> out(prompts.size());
         if (max_tokens <= 0) return out;
+        std::vector<char> forked(prompts.size());
+        bool any = false;
+        if (shared_prefix && (shared_prefix->empty() || max_batch < 2))
+            shared_prefix = nullptr;      // nothing to share, or no slot left for requests beside the prefix's
+        for (size_t i = 0; i < prompts.size(); ++i) any |= (forked[i] = uses_prefix(prompts[i], shared_prefix));
+        const size_t plen = shared_prefix ? shared_prefix->size() : 0;
+        auto need = [&](size_t req) {
+            const int n = std::min(kv_pages((long long)prompts[req].size() + max_tokens), kv_pages(max_seq));
+            return n - (forked[req] ? (int)(plen / kKvPage) : 0);
+        };
         std::vector<size_t> waiting;
         for (size_t i = prompts.size(); i-- > 0;) waiting.push_back(i);
         std::vector<int> free_slots;
         for (int s = max_batch; s-- > 0;) free_slots.push_back(s);
         std::map<int, Running> running;
+        long long reserved = 0;
         const size_t V = (size_t)model.dev->cfg.vocab_size;
+        int pslot = -1;
+        struct PrefixSlot {       // the prefix slot is handed back however generate ends, as models.py's try / finally does
+            const DeviceCache& c;
+            const int& slot;
+            ~PrefixSlot() { if (slot >= 0) fl_cache_slot_reset(c.h, slot); }
+        } prefix_guard{cache, pslot};
+        if (any) {
+            pslot = free_slots.back(); free_slots.pop_back();
+            reserved = kv_pages((long long)plen);
+            forward_packed(*model.dev, cache, {pslot}, {*shared_prefix}, {0});
+            forwards += 1;
+        }
         while (!waiting.empty() || !running.empty()) {
             std::vector<int> slots;
             std::vector<std::vector<uint32_t>> seqs;
@@ -358,15 +407,25 @@ struct PackedBatcher {
             for (auto& kv : running) { slots.push_back(kv.first); seqs.push_back({kv.second.tok}); ropes.push_back(kv.second.rope); }   // ascending slots
             long long budget = (long long)token_budget - (long long)slots.size();
             int admitted = 0;
-            while (!waiting.empty() && !free_slots.empty() && (admitted == 0 || (long long)prompts[waiting.back()].size() <= budget)) {
-                const size_t req = waiting.back(); waiting.pop_back();
+            while (!waiting.empty() && !free_slots.empty()) {
+                const size_t req = waiting.back();
+                std::vector<uint32_t> seq = forked[req] ? std::vector<uint32_t>(prompts[req].begin() + plen, prompts[req].end()) : prompts[req];
+                if (admitted && (long long)seq.size() > budget) break;
+                if (pool_pages && reserved + need(req) > *pool_pages) {
+                    if (running.empty() && !admitted) throw Error(FL_ERR_STATE, "a request needs more KV pages than the pool holds");
+                    break;
+                }
+                waiting.pop_back();
                 const int slot = free_slots.back(); free_slots.pop_back();
+                if (forked[req]) cache.slot_fork(pslot, slot);
+                budget -= (long long)seq.size();
                 slots.push_back(slot);
-                seqs.push_back(prompts[req]);
-                ropes.push_back(0);
-                budget -= (long long)prompts[req].size();
+                seqs.push_back(std::move(seq));
+                ropes.push_back(forked[req] ? plen : 0);
                 admitted += 1;
-                running[slot] = Running{req, 0, std::make_unique<LogitsProcessor>(0, (double)temperature), 0};
+                const int pages = pool_pages ? need(req) : 0;
+                reserved += pages;
+                running[slot] = Running{req, 0, std::make_unique<LogitsProcessor>(0, (double)temperature), 0, pages};
             }
             const std::vector<float> logits = forward_packed(*model.dev, cache, slots, seqs, ropes);
             forwards += 1;
@@ -383,6 +442,7 @@ struct PackedBatcher {
                     done = (int)out[st.req].size() >= max_tokens;
                 }
                 if (done) {
+                    reserved -= st.pages;
                     running.erase(slots[i]);
                     check(fl_cache_slot_reset(cache.h, slots[i]));
                     free_slots.push_back(slots[i]);

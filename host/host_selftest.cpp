@@ -4,6 +4,8 @@
 // of logits.bin and prints the sampled ids (tests/test_sampling_cpu.py compares them with the oracle).
 // `host_selftest manifest weights 0 --loglikelihood context... / continuation...` prints Model::loglikelihood as [sum, is_greedy].
 // `host_selftest manifest weights max_tokens --batch|--packed max_batch ids / ids / ...` prints the ContinuousBatcher's / PackedBatcher's ids.
+// `host_selftest manifest weights max_tokens --packed-pool max_batch pool_tokens prefix_len ids / ...`: the Mistral PackedBatcher on a KV
+// pool with a shared prefix.
 // Build: g++ -std=c++17 -O2 host/host_selftest.cpp -o host/_build/host_selftest -Lfastllm_b200 -lfastllm_b200 -Wl,-rpath,...
 #include <cstdio>
 #include <cstdlib>
@@ -68,6 +70,29 @@ int main(int argc, char** argv) {
             fastllm::Model<fastllm::LlamaWithConfig> model{std::move(pr.first), std::move(pr.second), std::nullopt};
             const auto ll = model.loglikelihood(parts[0], parts[1]);
             std::printf("[%.17g, %s]\n", ll.first, ll.second ? "true" : "false");
+            return 0;
+        }
+        if (argc > 7 && std::strcmp(argv[4], "--packed-pool") == 0) {
+            // host_selftest manifest weights max_tokens --packed-pool max_batch pool_tokens prefix_len id id / id ... : the C++ PackedBatcher
+            // of the Mistral adapter on a KV pool of pool_tokens, with the first prefix_len ids of the first prompt as the shared prefix
+            const int max_batch = std::atoi(argv[5]), pool_tokens = std::atoi(argv[6]), prefix_len = std::atoi(argv[7]);
+            std::vector<std::vector<uint32_t>> prompts(1);
+            for (int i = 8; i < argc; ++i) {
+                if (std::strcmp(argv[i], "/") == 0) prompts.emplace_back();
+                else prompts.back().push_back((uint32_t)std::strtoul(argv[i], nullptr, 10));
+            }
+            const std::vector<uint32_t> prefix(prompts[0].begin(), prompts[0].begin() + prefix_len);
+            auto pr = fastllm::MistralWithConfig::initialize_model(cfg, tensors, 0);
+            fastllm::PackedBatcher<fastllm::MistralWithConfig> pb(pr.first, max_batch, std::nullopt, 4096, pool_tokens);
+            const auto outs = pb.generate(prompts, max_tokens, 0.0f, &prefix);
+            std::fprintf(stderr, "packed forwards: %d\n", pb.forwards);
+            std::printf("[");
+            for (size_t r = 0; r < outs.size(); ++r) {
+                std::printf("%s[", r ? "," : "");
+                for (size_t i = 0; i < outs[r].size(); ++i) std::printf("%s%u", i ? "," : "", outs[r][i]);
+                std::printf("]");
+            }
+            std::printf("]\n");
             return 0;
         }
         if (argc > 5 && (std::strcmp(argv[4], "--batch") == 0 || std::strcmp(argv[4], "--packed") == 0)) {

@@ -123,10 +123,25 @@ FL_EXPORT int fl_model_destroy(fl_model* m);
 FL_EXPORT int fl_model_weight_bytes(fl_model* m, uint64_t* streamed_bytes); /* bytes one decode step must stream (no embedding table) */
 
 /* ---- KV cache ---------------------------------------------------------------------------------- */
+/* KV lives in 64-token pages drawn from the cache's pool.  Every entry point that grows a sequence takes the pages it will write
+ * after its other checks and before any device work: the uniform calls (fl_forward*, including logprobs, greedy, sample and
+ * sample_device) for slots 0..b-1 over [0, kv_len + t); fl_decode_greedy_loop over [0, kv_len + steps), up front; fl_forward_slots
+ * and fl_forward_packed per slot over [0, slot_len + length); fl_cache_fill_synthetic for slots 0..batch-1 up to kv_len.  When the
+ * free pages do not cover the call it returns FL_ERR_STATE ("KV page pool exhausted") and the cache is unchanged.
+ * Page p of slot s takes the slot's home page s * ceil(max_seq/64) + p when it exists in the pool and is free, else the lowest
+ * free page; pages return to the pool when no slot holds them any more (fl_cache_slot_reset, fl_cache_reset).
+ * fl_cache_create(m, B, S, out) is the pool of B * ceil(S/64) pages: every slot can reach max_seq, and results are those of a
+ * static per-slot layout. */
 FL_EXPORT int fl_cache_create(fl_model* m, int max_batch, int max_seq, fl_cache** out);
-FL_EXPORT int fl_cache_reset(fl_cache* c);                       /* kv length := 0 for every sequence */
+/* A cache of max_batch slots, each up to max_seq tokens, sharing a pool of pool_tokens (rounded up to 64-token pages) of KV.
+ * fl_cache_create(m, B, S, out) is the pool of B * ceil(S/64) pages.  FL_ERR_INVALID: pool_tokens < 1 or bad dimensions. */
+FL_EXPORT int fl_cache_create_pool(fl_model* m, int max_batch, int max_seq, int pool_tokens, fl_cache** out);
+FL_EXPORT int fl_cache_pool_pages(fl_cache* c, int* free_pages, int* total_pages);   /* pages no slot holds / pages of the pool */
+FL_EXPORT int fl_cache_reset(fl_cache* c);                       /* kv length := 0 for every sequence; every page returns to the pool */
 FL_EXPORT int fl_cache_kv_len(fl_cache* c, int* out);            /* tokens currently held (same for every sequence) */
-FL_EXPORT int fl_cache_fill_synthetic(fl_cache* c, int batch, int kv_len, uint64_t seed); /* benchmark: pretend a kv_len-token prefill */
+/* benchmark: pretend a kv_len-token uniform prefill of slots 0..batch-1 (the whole pool is overwritten; earlier sequences, slot
+ * lengths included, are dropped, and the cache takes uniform calls again) */
+FL_EXPORT int fl_cache_fill_synthetic(fl_cache* c, int batch, int kv_len, uint64_t seed);
 FL_EXPORT int fl_cache_destroy(fl_cache* c);
 
 /* ---- forward (causal LMs) ---------------------------------------------------------------------- */
@@ -165,8 +180,18 @@ FL_EXPORT int fl_forward_logprobs(fl_model* m, fl_cache* c, const uint32_t* ids,
  * A cache is driven either by the uniform calls above or by slots; fl_cache_reset switches back. */
 FL_EXPORT int fl_forward_slots(fl_model* m, fl_cache* c, const int* slots, const uint32_t* ids, int n, int t, const size_t* rope_offsets,
                                float* logits_host);
-FL_EXPORT int fl_cache_slot_reset(fl_cache* c, int slot);        /* the slot's sequence is finished: length := 0 */
+/* the slot's sequence is finished: length := 0, pages released (on a cache of uniform calls the row keeps its pages until
+ * fl_cache_reset: the common length still covers them) */
+FL_EXPORT int fl_cache_slot_reset(fl_cache* c, int slot);
 FL_EXPORT int fl_cache_slot_len(fl_cache* c, int slot, int* out);
+/* The empty slot dst becomes a copy of slot src: the same length, and every later call on dst computes what the same call on src
+ * would.  The full 64-token pages of src are shared, not copied (they are never written again: appends only touch positions at or
+ * beyond a slot's length); a partial last page is copied at once into a fresh page for dst.  A shared system prompt is thus
+ * prefilled once, and one sequence can continue as several (parallel samples, beams).  Drives the cache by slots.
+ * FL_ERR_INVALID: NULL, a slot out of range, src == dst, or an empty src.
+ * FL_ERR_STATE:   dst not empty, the cache holds tokens of uniform calls, or no free page for the partial copy.
+ * All are checked before any device work: a failed call leaves the cache unchanged. */
+FL_EXPORT int fl_cache_slot_fork(fl_cache* c, int src, int dst);
 /* n sequences in ONE forward, each fed its own number of new tokens: sequence i is cache slot slots[i], fed
  * ids[o_i, o_i + lengths[i]) (o_i = lengths[0] + ... + lengths[i-1]) at RoPE positions rope_offsets[i] + j.
  * A new prompt (empty slot, lengths[i] = prompt length) and a decode step of a running request (lengths[i] = 1) can share a call.
@@ -178,7 +203,7 @@ FL_EXPORT int fl_cache_slot_len(fl_cache* c, int slot, int* out);
  * fl_cache_moe_routing reports rows = the sum of the lengths, in ids order.
  * FL_ERR_INVALID:     a NULL pointer, n < 1 or n > max_batch, a length < 1, a slot out of range or repeated, an id >= vocab, a RoPE
  *                     position >= max_position_embeddings, or a multi-token sequence on a non-empty slot of a Llama model.
- * FL_ERR_STATE:       slot_len + length > max_seq, or the cache holds tokens of uniform calls.
+ * FL_ERR_STATE:       slot_len + length > max_seq, the cache holds tokens of uniform calls, or the KV page pool is exhausted.
  * FL_ERR_UNSUPPORTED: the model is sharded (tp_size > 1, Mixtral expert parallelism included), or its shapes do not admit the dense path.
  * All are checked before any device work: a failed call leaves the cache unchanged. */
 FL_EXPORT int fl_forward_packed(fl_model* m, fl_cache* c, const int* slots, const int32_t* lengths, int n, const uint32_t* ids,
