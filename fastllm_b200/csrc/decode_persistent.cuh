@@ -19,8 +19,10 @@
 //     (RMSNorm prologue; bias+RoPE+KV append; residual add; SiLU*up; logits+arg-max).
 //   * phases of a layer are separated by a grid barrier (monotonic atomic counter, release/acquire fences); data that
 //     crosses CTAs is read with ld.global.cg (L2) because L1 is not coherent across SMs.
-//   * attention: split-K over the sequence, (kv_head, split) items spread over the CTAs, K/V read straight from the paged
-//     cache with 128-bit ld.global.cg, online softmax, last-arriver merge (same algorithm as attn_decode.cuh).
+//   * attention: split-K over the sequence, (kv_head, split) items spread over the CTAs, online softmax, last-arriver merge
+//     (same algorithm as attn_decode.cuh).  The K/V pages an item needs are stages of the same ring: the producer bulk-copies
+//     them right after the q|k|v phase's chunks, so they land while the consumers run the q|k|v epilogue and its grid
+//     barrier; only the row appended in the current step is read from L2 after the barrier.
 //   * `nsteps` decode steps can run inside one launch (greedy feedback on device), so the device-resident loop has no
 //     launch gaps at all.
 #pragma once
@@ -231,6 +233,19 @@ __global__ void __launch_bounds__(kPkThreads, 1) decode_persistent_kernel(const 
     const int cta = blockIdx.x, ncta = gridDim.x;
     const int NS = a.nstages;
     const int nq = a.nh * a.d;
+    const int n_rep = a.nh / a.nkv;
+    // attention geometry shared by the producer (which streams the K/V stages) and the consumers (which read them)
+    constexpr int LPT = D / 8, TPW = 32 / LPT;      // lanes per token (8 bf16 each), tokens per warp
+    constexpr int HG = 4;                           // query heads per pass (register budget)
+    constexpr int NG = kPkConsumerWarps * TPW;      // lane groups per CTA
+    constexpr int BATCH = 4;                        // tokens per lane group per pass
+    constexpr int SPT = NG * BATCH;                 // tokens per K/V stage: 64 (D = 128) or 128 (D = 64)
+    constexpr int SKV = SPT * D * 2;                // bytes of K (then of V) in a stage: 16 KB, so a stage is 32 KB
+    static_assert(2 * SKV == kPkStageBytes && SPT % kKvPage == 0, "a K/V stage is one ring stage of whole pages");
+    // the KV length of step 0, read before the role split: CTA 0's consumers advance it by exactly 1 at the end of every step,
+    // which is after a grid barrier that every CTA reaches only past the __syncthreads below
+    int kv_base0 = 0;
+    if (warp == kPkConsumerWarps) kv_base0 = __ldcg(&a.state->kv_base[0]);
 
     if (tid == 0) {
         for (int s = 0; s < NS; ++s) {
@@ -251,6 +266,57 @@ __global__ void __launch_bounds__(kPkThreads, 1) decode_persistent_kernel(const 
         const uint64_t pol_first = l2_policy_evict_first();
         const bool dynamic = a.tp == 1 && a.pool != nullptr;
         for (int step = 0; step < a.nsteps; ++step) {
+            const int len = kv_base0 + step + 1, slot = len - 1;
+            const int npages = (len + kKvPage - 1) / kKvPage;
+            const int per = (npages + a.nsplit - 1) / a.nsplit;
+            // page-table entries of this CTA's items (constant during the launch): towards L1 once per step, off the ring's path
+            for (int item = cta; item < a.nkv * a.nsplit; item += ncta) {
+                const int p1 = min((item % a.nsplit + 1) * per, npages);
+                for (int p = item % a.nsplit * per; p < p1; p += 32) asm volatile("prefetch.global.L1 [%0];" ::"l"(a.page_table + p));
+            }
+            // K/V stages of layer l's attention items, emitted right after the q|k|v phase so that they land while the consumers
+            // run the q|k|v epilogue and its grid barrier.  Stage = one pass of the consumers' token loop (SPT tokens of one kv
+            // head), K rows at +0 and V rows at +SKV, one 1-D bulk copy per page and K / V.  Only rows < slot are copied: row
+            // `slot` is appended in this very step by some CTA's q|k|v epilogue, the consumer that owns it loads it from L2.
+            // Ordering of the row appended at step s (read by these copies from step s+1 on): writer's store -> its grid-barrier
+            // release -> acquire by this CTA's consumers -> their `empty` arrive on a stage consumed after that barrier -> this
+            // thread's wait on it -> fence.proxy.async -> bulk copy.  The stage waited on is NS uses back; between the q|k|v
+            // phase of (s, l) and the K/V stages of (s+1, l) the stream holds at least 4 L + 1 end-of-phase stages, all consumed
+            // after that barrier, and plan_persistent keeps NS <= 4 L + 1, so this holds however far the producer runs ahead
+            // (e.g. under tensor parallelism, where many CTAs own no q|k|v block).
+            auto fetch_kv = [&](int l) {
+                const uint16_t* kl = a.kpool + (size_t)l * a.layer_pool_elems;
+                const uint16_t* vl = a.vpool + (size_t)l * a.layer_pool_elems;
+                bool fenced = false;
+                for (int item = cta; item < a.nkv * a.nsplit; item += ncta) {
+                    const int kvh = item / a.nsplit, split = item % a.nsplit;
+                    const int tok0 = split * per * kKvPage, tok1 = min(min((split + 1) * per, npages) * kKvPage, len);
+                    for (int h0 = 0; h0 < n_rep; h0 += HG) {
+                        for (int tb0 = tok0; tb0 < tok1; tb0 += SPT) {
+                            const int st = c % NS;
+                            mbar_wait(&empty[st], ((c / NS) & 1) ^ 1);
+                            ++c;
+                            const int cend = min(min(tb0 + SPT, tok1), slot);      // rows [tb0, cend) come by bulk copy
+                            if (cend <= tb0) {      // nothing below the slot: a zero-byte stage keeps both sides in step
+                                mbar_arrive(&full[st]);
+                                continue;
+                            }
+                            if (!fenced) {
+                                asm volatile("fence.proxy.async;" ::: "memory");
+                                fenced = true;
+                            }
+                            uint8_t* dst = ring + (size_t)st * kPkStageBytes;
+                            mbar_expect_tx(&full[st], (uint32_t)(cend - tb0) * D * 4u);
+                            for (int p = tb0; p < cend; p += kKvPage) {
+                                const uint32_t bytes = (uint32_t)min(kKvPage, cend - p) * D * 2u;
+                                const size_t src = ((size_t)__ldg(a.page_table + p / kKvPage) * a.nkv + kvh) * kKvPage * D;
+                                bulk_g2s(dst + (p - tb0) * D * 2, kl + src, bytes, &full[st]);
+                                bulk_g2s(dst + SKV + (p - tb0) * D * 2, vl + src, bytes, &full[st]);
+                            }
+                        }
+                    }
+                }
+            };
             for (int g = 0; g <= 4 * a.L; ++g) {
                 const uint16_t* W;
                 int N, K;
@@ -293,6 +359,7 @@ __global__ void __launch_bounds__(kPkThreads, 1) decode_persistent_kernel(const 
                 meta[st] = make_int2(0, kPkMetaEnd);
                 mbar_arrive(&full[st]);
                 ++c;
+                if (g < 4 * a.L && (g & 3) == 0) fetch_kv(g >> 2);
             }
         }
         return;
@@ -526,8 +593,6 @@ __global__ void __launch_bounds__(kPkThreads, 1) decode_persistent_kernel(const 
         }
         ++dbg_i;
     };
-    const int n_rep = a.nh / a.nkv;
-    constexpr int LPT = D / 8, TPW = 32 / LPT;
     const int grp = lane / LPT, gl = lane % LPT;
     // this CTA's first attention item, opaque to the optimiser: starting the item loop at `cta` itself lets the compiler keep values
     // derived from it live across every weight phase, and the q|k|v phase then spills its MMA accumulators (ptxas at 168 registers;
@@ -539,9 +604,8 @@ __global__ void __launch_bounds__(kPkThreads, 1) decode_persistent_kernel(const 
         const uint32_t tok_id = __ldcg(a.ids);
         const int rope_pos = min(__ldcg(&a.state->rope_pos), a.max_pos - 1);
         const int kv_base = __ldcg(&a.state->kv_base[0]);
-        const int slot = kv_base;                       // cache slot of the token being decoded
-        const int len = kv_base + 1;
-        const int page_of_slot = __ldg(a.page_table + slot / kKvPage);
+        const int slot_s = kv_base;                       // cache slot of the token being decoded
+        const int page_of_slot_s = __ldg(a.page_table + slot_s / kKvPage);
 
         for (int l = 0; l < a.L; ++l) {
             const PkLayer& lw = a.layers[l];
@@ -553,11 +617,6 @@ __global__ void __launch_bounds__(kPkThreads, 1) decode_persistent_kernel(const 
             dbg_i = 0;
             dbg_layer = l;
             stamp(l);
-            if (l == 0) {      // page-table entries of this CTA's attention items (constant during the launch): towards L1, off the
-                               // load -> load dependency chain of every layer's attention phase
-                const int npages = (len + kKvPage - 1) / kKvPage;
-                for (int i = tid * 32; i < npages; i += kPkConsumers * 32) asm volatile("prefetch.global.L1 [%0];" ::"l"(a.page_table + i));
-            }
             if (l == 0)
                 load_x_rmsnorm(nullptr, true, a.embed + (size_t)tok_id * a.H, lw.ln1, a.H, cta == 0 ? a.resid : nullptr);
             else
@@ -579,12 +638,12 @@ __global__ void __launch_bounds__(kPkThreads, 1) decode_persistent_kernel(const 
                             a.q[(size_t)hh * d + j] = o1;
                             a.q[(size_t)hh * d + j + half] = o2;
                         } else {
-                            uint16_t* kp = kpool + (((size_t)page_of_slot * a.nkv + (hh - a.nh)) * kKvPage + slot % kKvPage) * d;
+                            uint16_t* kp = kpool + (((size_t)page_of_slot_s * a.nkv + (hh - a.nh)) * kKvPage + slot_s % kKvPage) * d;
                             kp[j] = f32_to_bf16_rne(o1);
                             kp[j + half] = f32_to_bf16_rne(o2);
                         }
                     } else {
-                        uint16_t* vp = vpool + (((size_t)page_of_slot * a.nkv + (hh - a.nh - a.nkv)) * kKvPage + slot % kKvPage) * d;
+                        uint16_t* vp = vpool + (((size_t)page_of_slot_s * a.nkv + (hh - a.nh - a.nkv)) * kKvPage + slot_s % kKvPage) * d;
                         *reinterpret_cast<uint32_t*>(vp + 2 * j) = (uint32_t)f32_to_bf16_rne(va) | ((uint32_t)f32_to_bf16_rne(vb) << 16);
                     }
                 }
@@ -595,13 +654,17 @@ __global__ void __launch_bounds__(kPkThreads, 1) decode_persistent_kernel(const 
             stamp(l);
 
             // ---------------- P2: split-K attention over (kv head, split) items + last-arriver merge ----------------
-            // Latency-optimised: every 16-lane group (two per warp, 16 per CTA) runs its OWN online softmax over a strided
-            // subset of the item's tokens with all of its K/V loads in flight at once and q held in registers (loaded from L2
-            // concurrently with K/V); the 16 partial states meet in shared memory after ONE block sync.
+            // Latency-optimised: every lane group (D / 8 lanes; 16 or 32 per CTA) runs its OWN online softmax over a strided
+            // subset of the item's tokens with q held in registers; the K/V rows of every token but the one appended in this step
+            // are already in the ring (streamed by the producer during the q|k|v phase, one stage per SPT tokens, see fetch_kv),
+            // and the lane group that owns token `slot` loads that row from L2 together with q.  The partial states meet in
+            // shared memory after ONE block sync.
             {
-                constexpr int HG = 4;                       // query heads per pass (register budget)
-                constexpr int NG = kPkConsumerWarps * TPW;  // lane groups per CTA
-                constexpr int BATCH = 4;                    // tokens in flight per lane group
+                // the step's slot, opaque to the optimiser: otherwise values derived from it are hoisted out of the layer loop and
+                // kept live across the weight phases, whose MMA accumulators then spill (ptxas -v, D = 128: 328 -> 192 bytes of spill loads)
+                int slot = slot_s, page_of_slot = page_of_slot_s;
+                asm volatile("" : "+r"(slot), "+r"(page_of_slot));
+                const int len = slot + 1;
                 const int npages = (len + kKvPage - 1) / kKvPage;
                 const int per = (npages + a.nsplit - 1) / a.nsplit;
                 float* gacc = xs;                            // [NG][HG][D]
@@ -628,22 +691,36 @@ __global__ void __launch_bounds__(kPkThreads, 1) decode_persistent_kernel(const 
                                 for (int i = 0; i < 8; ++i) qv[h][i] = 0.f;
                             }
                         }
-                        // trip count is uniform across the CTA (the shuffles below use the full mask); validity is per lane group
-                        for (int tb0 = tok0; tb0 < tok1; tb0 += NG * BATCH) {
+                        // the row appended in this step: in the item's last stage, owned by one lane group
+                        uint4 ks = make_uint4(0u, 0u, 0u, 0u), vs = ks;
+                        if (slot >= tok0 && slot < tok1 && (slot - tok0) % NG == gidx) {
+                            const size_t base = (((size_t)page_of_slot * a.nkv + kvh) * kKvPage + slot % kKvPage) * D + gl * 8;
+                            ks = ldcg_u4(kpool + base);
+                            vs = ldcg_u4(vpool + base);
+                        }
+                        // one ring stage per pass; the trip count is uniform across the CTA (the shuffles below use the full
+                        // mask, and every consumer warp releases every stage); validity is per lane group
+                        const int tend = min(tok1, slot);      // tokens [tok0, tend) are in the ring
+                        for (int tb0 = tok0; tb0 < tok1; tb0 += SPT) {
                             const int tb = tb0 + gidx;
+                            const int st = c % NS;
+                            mbar_wait(&full[st], (c / NS) & 1);
+                            ++c;
+                            const uint8_t* kst = ring + (size_t)st * kPkStageBytes + (size_t)gidx * D * 2 + gl * 16;
                             uint4 kw[BATCH], vw[BATCH];
 #pragma unroll
                             for (int it = 0; it < BATCH; ++it) {
                                 const int tk = tb + it * NG;
-                                if (tk < tok1) {
-                                    const size_t base = (((size_t)__ldg(a.page_table + tk / kKvPage) * a.nkv + kvh) * kKvPage + tk % kKvPage) * D + gl * 8;
-                                    kw[it] = ldcg_u4(kpool + base);
-                                    vw[it] = ldcg_u4(vpool + base);
+                                if (tk < tend) {
+                                    kw[it] = *reinterpret_cast<const uint4*>(kst + it * NG * D * 2);
+                                    vw[it] = *reinterpret_cast<const uint4*>(kst + SKV + it * NG * D * 2);
                                 } else {
-                                    kw[it] = make_uint4(0u, 0u, 0u, 0u);
-                                    vw[it] = kw[it];
+                                    kw[it] = tk == slot ? ks : make_uint4(0u, 0u, 0u, 0u);
+                                    vw[it] = tk == slot ? vs : make_uint4(0u, 0u, 0u, 0u);
                                 }
                             }
+                            __syncwarp();
+                            if (lane == 0) mbar_arrive(&empty[st]);
 #pragma unroll
                             for (int it = 0; it < BATCH; ++it) {
                                 const bool valid = tb + it * NG < tok1;
@@ -704,15 +781,19 @@ __global__ void __launch_bounds__(kPkThreads, 1) decode_persistent_kernel(const 
                                 }
                             }
                         }
-                        pk_named_sync();      // gacc / gml are reused by the next head group
+                        pk_named_sync();      // gacc / gml are reused by the next head group; part_* of this item are written
                     }
-                    __threadfence();
-                    pk_named_sync();
-                    if (tid == 0) *s_flag = (atomicAdd(&a.counters[kvh], 1) == a.nsplit - 1);
+                    // arrive on the kv head's counter with ONE acq_rel atomic, as pk_grid_barrier does: the CTA barrier above
+                    // orders every thread's part_* stores before it (cumulativity), and for the last arriver its acquire side
+                    // plus the CTA barrier below order the other splits' part_* before the merge's loads
+                    if (tid == 0) {
+                        int old;
+                        asm volatile("atom.add.acq_rel.gpu.global.s32 %0, [%1], 1;" : "=r"(old) : "l"(a.counters + kvh) : "memory");
+                        *s_flag = old == a.nsplit - 1;
+                    }
                     pk_named_sync();
                     if (*s_flag) {
-                        __threadfence();
-                        float* cm = xs;                      // [n_rep][nsplit] weights
+                        float* cm = xs;                     // [n_rep][nsplit] weights
                         float* cden = cm + kAttnMaxRep * a.nsplit;
                         if (warp < n_rep) {
                             const int h = warp;

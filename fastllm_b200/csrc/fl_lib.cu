@@ -408,7 +408,9 @@ static void plan_persistent(fl_cache& c) {
     const size_t fixed = (size_t)p.xs_floats * 4 + (size_t)p.partial_rows * kPkConsumerWarps * 4 + (size_t)kAttnMaxRep * kKvPage * 4 + 64 * 4;
     const size_t avail = 232448 - 2048;   // 227 KB opt-in limit minus static shared memory and slack
     if (fixed + 2 * (size_t)kPkStageBytes > avail) return;
-    p.nstages = (int)std::min<size_t>(kPkMaxStages, (avail - fixed) / kPkStageBytes);
+    // at most 4 L + 1 stages: a ring use then always waits on a stage consumed after the previous step's K/V append of its
+    // layer (the ordering argument of fetch_kv in decode_persistent.cuh)
+    p.nstages = (int)std::min<size_t>(std::min(kPkMaxStages, 4 * w.L + 1), (avail - fixed) / kPkStageBytes);
     p.smem = (size_t)p.nstages * kPkStageBytes + fixed;
     p.nsplit = std::max(1, std::min(c.pages_per_seq, kNumSMs / w.nkv));
     if (p.nsplit > c.nsplit) p.nsplit = c.nsplit;            // partial buffers are sized for c.nsplit
