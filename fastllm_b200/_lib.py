@@ -46,6 +46,7 @@ SYMBOLS = {
     "fl_model_weight_bytes": (_I, [_VP, C.POINTER(_U64)]),
     "fl_cache_create": (_I, [_VP, _I, _I, C.POINTER(_VP)]),
     "fl_cache_create_pool": (_I, [_VP, _I, _I, _I, C.POINTER(_VP)]),
+    "fl_cache_create_pool_kv": (_I, [_VP, _I, _I, _I, _I, C.POINTER(_VP)]),
     "fl_cache_pool_pages": (_I, [_VP, C.POINTER(_I), C.POINTER(_I)]),
     "fl_cache_slot_fork": (_I, [_VP, _I, _I]),
     "fl_cache_reset": (_I, [_VP]),

@@ -8,6 +8,8 @@
 //       style loop over the causal range of 64-key pages, S = Q K^T and O += P V on mma.sync, online softmax in registers.
 //       Replaces the row-per-CTA decode kernel in prefill (84 % of the Qwen2.5-7B 4k prefill before).
 //
+// FP8 caches (FL_KV_FP8_E4M3): every kernel is also instantiated for e4m3 pages and widens them to bf16 (exactly) before the same
+// bf16 MMAs; the tcgen05 prefill reads the call's K from a bf16 scratch the q|k|v epilogue writes (DESIGN.md section 3.7).
 // Precision: q and the softmax probabilities are f32 in the oracle.  Both are split hi + lo into two bf16 operands and
 // multiplied against the same K / V fragments (as the dense GEMMs do with their activations), K/V are bf16 in the cache
 // already, accumulation is f32: results stay inside the kernel tolerance of the f32 oracle.
@@ -42,6 +44,38 @@ __device__ __forceinline__ void stage_kv_tile(uint16_t* kd, uint16_t* vd, const 
         cp_async16(vd + swz<D>(r, c * 8), vsrc + r * D + c * 8);
     }
     cp_async_commit();
+}
+
+// FP8 pages: the K and V page of one kv head land unchanged ([64][D] e4m3 each, back to back) ...
+template <int D>
+__device__ __forceinline__ void stage_kv_raw8(uint8_t* dst, const uint8_t* ksrc, const uint8_t* vsrc, int tid) {
+    constexpr int CH = D / 16;
+#pragma unroll
+    for (int i = tid; i < kKvPage * CH; i += kMmaAttnThreads) {
+        cp_async16(dst + i * 16, ksrc + i * 16);
+        cp_async16(dst + kKvPage * D + i * 16, vsrc + i * 16);
+    }
+    cp_async_commit();
+}
+// ... and are widened (exactly) into the swizzled bf16 K and V tiles the bf16 path stages
+template <int D>
+__device__ __forceinline__ void widen_kv_tile8(uint16_t* kd, const uint8_t* raw, int tid) {
+    constexpr int CH = D / 16;
+#pragma unroll
+    for (int i = tid; i < 2 * kKvPage * CH; i += kMmaAttnThreads) {
+        const int kvsel = i / (kKvPage * CH), r = (i / CH) % kKvPage, c = i % CH;
+        const uint4 x = *reinterpret_cast<const uint4*>(raw + i * 16);
+        const uint32_t w[4] = {x.x, x.y, x.z, x.w};
+        uint32_t b[8];
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+            b[2 * e] = e4m3x2_to_bf16x2((uint16_t)(w[e] & 0xFFFFu));
+            b[2 * e + 1] = e4m3x2_to_bf16x2((uint16_t)(w[e] >> 16));
+        }
+        uint16_t* t = kd + kvsel * kKvPage * D;
+        *reinterpret_cast<uint4*>(t + swz<D>(r, c * 16)) = make_uint4(b[0], b[1], b[2], b[3]);
+        *reinterpret_cast<uint4*>(t + swz<D>(r, c * 16 + 8)) = make_uint4(b[4], b[5], b[6], b[7]);
+    }
 }
 
 // f32 q rows -> hi/lo bf16 tiles [NR][D] (rows >= valid rows are zero)
@@ -87,6 +121,9 @@ constexpr int kSkThreads = kSkConsumers + 32;
 // batch 64 is the same with 3 stages x 2 CTAs (6.83 vs 6.84 ms/step), batch 8 is better with more, smaller ranges (4.07 vs
 // 4.17 ms/step); 4 stages x 1 CTA loses 14 %.
 constexpr int kSkStages = 2;
+// K|V stages of an FP8 cache: a stage is half the bytes, so twice as many keep the same bytes in flight per CTA
+template <typename KV>
+constexpr int sk_stages = kv_is_fp8<KV> ? 2 * kSkStages : kSkStages;
 
 // element offset of (row, col) inside a staged 64 x D K or V page.  D >= 64: [D / 64 halves][64 rows][128 bytes] with the TMA
 // engine's 128-byte swizzle (16-byte chunk index XOR row & 7); D < 64 (test-size heads): the plain [64][D] box, no swizzle.
@@ -94,6 +131,23 @@ template <int D>
 __device__ __forceinline__ int kv_off(int row, int col) {
     if constexpr (D >= 64) return (col >> 6) * (kKvPage * 64) + row * 64 + (((((col >> 3) & 7) ^ (row & 7))) << 3) + (col & 7);
     else return row * D + col;
+}
+
+// byte offset of 16-byte chunk `ch` of row `row` inside a staged 64 x D e4m3 K or V page: one [64 rows][D bytes] box with the TMA
+// engine's 128-byte swizzle (D = 128: chunk XOR row & 7), 64-byte swizzle (D = 64: chunk XOR (row >> 1) & 3), none below.  Eight
+// rows of one chunk column are then conflict-free for ldmatrix.
+template <int D>
+__device__ __forceinline__ int kv_off8(int row, int ch) {
+    if constexpr (D == 128) return row * 128 + ((ch ^ (row & 7)) << 4);
+    else if constexpr (D == 64) return row * 64 + ((ch ^ ((row >> 1) & 3)) << 4);
+    else return row * D + ch * 16;
+}
+// FP8 S = Q.K^T: the B fragment of dims [16c, 16c + 16) comes from ONE ldmatrix row of 16 e4m3 bytes, thread quad tq holding physical
+// dims 16c + 4tq .. 4tq + 3, which the MMA sees as k = 2tq, 2tq + 1 (b0) and 8 + 2tq, 9 + 2tq (b1).  q is staged with the same
+// permutation of each 16-dim block: physical dim p sits at logical column sk_kperm(p).
+__device__ __forceinline__ int sk_kperm(int p) {
+    const int q = p & 15, tq = q >> 2;
+    return (p & ~15) | ((q & 2) ? 8 + 2 * tq + (q & 1) : 2 * tq + (q & 1));
 }
 
 struct SkArgs {
@@ -104,11 +158,16 @@ struct SkArgs {
     int layer_row0;       // row of this layer's page 0 / kv head 0 in the pool-wide tensor maps
 };
 
-template <int D>
+// KV: element type of the pages (uint16_t = bf16, uint8_t = e4m3).  The e4m3 instantiation stages 1-byte pages and widens them to
+// bf16 (exactly) in the consumers' registers before the same mma.sync m16n8k16; see kv_off8 / sk_kperm for its fragment layout.
+template <int D, typename KV = uint16_t>
 __global__ void __launch_bounds__(kSkThreads) attn_sk_decode_kernel(const __grid_constant__ CUtensorMap tmk, const __grid_constant__ CUtensorMap tmv,
                                                                     const SkArgs k) {
     const AttnArgs& a = k.a;
+    constexpr bool FP8 = kv_is_fp8<KV>;
     constexpr int TILE = kKvPage * D;
+    constexpr int NST = sk_stages<KV>;
+    constexpr uint32_t STAGE = 2u * TILE * sizeof(KV);      // bytes of a K|V stage
     constexpr int NW = kSkConsumerWarps;
     extern __shared__ __align__(1024) uint8_t sksm[];
     const int n_rep = a.nh / a.nkv;
@@ -118,9 +177,9 @@ __global__ void __launch_bounds__(kSkThreads) attn_sk_decode_kernel(const __grid
     uint16_t* qhi = reinterpret_cast<uint16_t*>(sksm);
     uint16_t* qlo = qhi + 16 * D;
     float* red_o = reinterpret_cast<float*>(sksm);
-    uint16_t* ring = reinterpret_cast<uint16_t*>(sksm + ((front + 1023) & ~1023));
-    __shared__ __align__(8) uint64_t full[kSkStages];
-    __shared__ __align__(8) uint64_t empty[kSkStages];
+    uint8_t* ring = sksm + ((front + 1023) & ~1023);
+    __shared__ __align__(8) uint64_t full[NST];
+    __shared__ __align__(8) uint64_t empty[NST];
     __shared__ float red_m[NW][16], red_l[NW][16], mrg_w[NW][16], mrg_den[16], mrg_star[16];
     __shared__ int prefix[kMaxBatch + 1];        // pages of the sequences before s
     __shared__ int s_len[kMaxBatch], s_slot[kMaxBatch];
@@ -128,7 +187,7 @@ __global__ void __launch_bounds__(kSkThreads) attn_sk_decode_kernel(const __grid
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, tq = lane & 3;
     if (tid == 0) {
-        for (int s = 0; s < kSkStages; ++s) {
+        for (int s = 0; s < NST; ++s) {
             mbar_init(&full[s], 1);
             mbar_init(&empty[s], NW);
         }
@@ -206,11 +265,14 @@ __global__ void __launch_bounds__(kSkThreads) attn_sk_decode_kernel(const __grid
                 }
                 r &= 0x7FFFFFFF;
                 if (lane == 0) {
-                    const int st = c % kSkStages;
-                    mbar_wait(&empty[st], ((c / kSkStages) & 1) ^ 1);
-                    mbar_expect_tx(&full[st], 2u * TILE * 2u);
-                    uint16_t* kd = ring + (size_t)st * 2 * TILE;
-                    if constexpr (D >= 64) {
+                    const int st = c % NST;
+                    mbar_wait(&empty[st], ((c / NST) & 1) ^ 1);
+                    mbar_expect_tx(&full[st], STAGE);
+                    uint16_t* kd = reinterpret_cast<uint16_t*>(ring + (size_t)st * STAGE);
+                    if constexpr (FP8) {          // one [64 rows][D bytes] box per page
+                        tma_load_2d(ring + (size_t)st * STAGE, &tmk, 0, r, &full[st]);
+                        tma_load_2d(ring + (size_t)st * STAGE + STAGE / 2, &tmv, 0, r, &full[st]);
+                    } else if constexpr (D >= 64) {
 #pragma unroll
                         for (int hf = 0; hf < D / 64; ++hf) {
                             tma_load_2d(kd + hf * (kKvPage * 64), &tmk, hf * 64, r, &full[st]);
@@ -244,7 +306,7 @@ __global__ void __launch_bounds__(kSkThreads) attn_sk_decode_kernel(const __grid
             for (int i = tid; i < 16 * D; i += kSkConsumers) {
                 const int hh = i / D, dd = i % D;
                 const float q = hh < n_rep ? a.q[((size_t)s * a.nh + h * n_rep + hh) * D + dd] : 0.f;
-                store_hi_lo(qhi, qlo, swz<D>(hh, dd), q);
+                store_hi_lo(qhi, qlo, swz<D>(hh, FP8 ? sk_kperm(dd) : dd), q);
             }
             csync();
 #pragma unroll
@@ -254,13 +316,43 @@ __global__ void __launch_bounds__(kSkThreads) attn_sk_decode_kernel(const __grid
             open = true;
             from_start = (p == 0);
         }
-        const int st = c % kSkStages;
-        mbar_wait(&full[st], (c / kSkStages) & 1);
-        const uint16_t* kt = ring + (size_t)st * 2 * TILE;
+        const int st = c % NST;
+        mbar_wait(&full[st], (c / NST) & 1);
+        const uint16_t* kt = reinterpret_cast<const uint16_t*>(ring + (size_t)st * STAGE);
         const uint16_t* vt = kt + TILE;
+        const uint8_t* kt8 = ring + (size_t)st * STAGE;
+        const uint8_t* vt8 = kt8 + STAGE / 2;
+        // FP8: lane l addresses row (l >> 3 & 1) * 8 + (l & 7) of the warp's 16 keys, 16-byte chunk c0 + (l >> 4): ldmatrix x4 then
+        // yields the matrices (keys 0-7, c0), (keys 8-15, c0), (keys 0-7, c0 + 1), (keys 8-15, c0 + 1) (D = 16: c0 twice)
+        auto ld8 = [&](uint32_t (&r)[4], const uint8_t* base, int c0, bool trans) {
+            const uint8_t* ptr = base + kv_off8<D>(warp * 16 + ((lane >> 3) & 1) * 8 + (lane & 7), min(c0 + (lane >> 4), D / 16 - 1));
+            if (trans) ldmatrix_x4_trans(r, ptr); else ldmatrix_x4(r, ptr);
+        };
         const int key0 = p * kKvPage + warp * 16;
         if (key0 < len) {
             float sc[2][4] = {{0.f, 0.f, 0.f, 0.f}, {0.f, 0.f, 0.f, 0.f}};
+            if constexpr (FP8) {
+#pragma unroll
+                for (int c0 = 0; c0 < D / 16; c0 += 2) {
+                    uint32_t kb[4];
+                    ld8(kb, kt8, c0, false);
+#pragma unroll
+                    for (int hc = 0; hc < 2; ++hc) {
+                        const int ks = c0 + hc;
+                        if (ks >= D / 16) break;
+                        uint32_t ah[4], al[4];
+                        ldmatrix_x4(ah, qhi + swz<D>(lane & 15, ks * 16 + (lane >> 4) * 8));
+                        ldmatrix_x4(al, qlo + swz<D>(lane & 15, ks * 16 + (lane >> 4) * 8));
+#pragma unroll
+                        for (int nt = 0; nt < 2; ++nt) {
+                            const uint32_t u = kb[2 * hc + nt];
+                            const uint32_t b0 = e4m3x2_to_bf16x2((uint16_t)(u & 0xFFFFu)), b1 = e4m3x2_to_bf16x2((uint16_t)(u >> 16));
+                            mma_bf16_16816(sc[nt], ah, b0, b1);
+                            mma_bf16_16816(sc[nt], al, b0, b1);
+                        }
+                    }
+                }
+            } else {
 #pragma unroll
             for (int ks = 0; ks < D / 16; ++ks) {
                 uint32_t ah[4], al[4], kb[4];
@@ -271,6 +363,7 @@ __global__ void __launch_bounds__(kSkThreads) attn_sk_decode_kernel(const __grid
                 mma_bf16_16816(sc[0], al, kb[0], kb[1]);
                 mma_bf16_16816(sc[1], ah, kb[2], kb[3]);
                 mma_bf16_16816(sc[1], al, kb[2], kb[3]);
+            }
             }
             float mx0 = -INFINITY, mx1 = -INFINITY;
 #pragma unroll
@@ -303,6 +396,31 @@ __global__ void __launch_bounds__(kSkThreads) attn_sk_decode_kernel(const __grid
             pl[1] = pack_bf16x2(sc[0][2] - bf16lo(ph[1]), sc[0][3] - bf16hi(ph[1]));
             pl[2] = pack_bf16x2(sc[1][0] - bf16lo(ph[2]), sc[1][1] - bf16hi(ph[2]));
             pl[3] = pack_bf16x2(sc[1][2] - bf16lo(ph[3]), sc[1][3] - bf16hi(ph[3]));
+            if constexpr (FP8) {
+                // O += P.V: ldmatrix.trans of 16-bit pairs gives thread (g, tq) keys 2tq, 2tq + 1 (the keys of its P fragment) x dims
+                // 2g, 2g + 1 of a chunk; byte permutes pair the two keys of one dim.  Output tile 2c (2c + 1) column n is then dim
+                // 16c + 2n (16c + 2n + 1): the emit below stores o in that order.
+#pragma unroll
+                for (int c0 = 0; c0 < D / 16; c0 += 2) {
+                    uint32_t vb[4];
+                    ld8(vb, vt8, c0, true);
+#pragma unroll
+                    for (int hc = 0; hc < 2; ++hc) {
+                        const int cc = c0 + hc;
+                        if (cc >= D / 16) break;
+#pragma unroll
+                        for (int par = 0; par < 2; ++par) {
+                            const uint32_t sel = par ? 0x0031u : 0x0020u;
+                            const uint32_t b0 = e4m3x2_to_bf16x2((uint16_t)__byte_perm(vb[2 * hc], 0u, sel));
+                            const uint32_t b1 = e4m3x2_to_bf16x2((uint16_t)__byte_perm(vb[2 * hc + 1], 0u, sel));
+                            float(&oc)[4] = o[2 * cc + par];
+                            oc[0] *= al0; oc[1] *= al0; oc[2] *= al1; oc[3] *= al1;
+                            mma_bf16_16816(oc, ph, b0, b1);
+                            mma_bf16_16816(oc, pl, b0, b1);
+                        }
+                    }
+                }
+            } else {
 #pragma unroll
             for (int dt = 0; dt < D / 16; ++dt) {
                 uint32_t vb[4];
@@ -315,6 +433,7 @@ __global__ void __launch_bounds__(kSkThreads) attn_sk_decode_kernel(const __grid
                 mma_bf16_16816(oa, pl, vb[0], vb[1]);
                 mma_bf16_16816(ob, ph, vb[2], vb[3]);
                 mma_bf16_16816(ob, pl, vb[2], vb[3]);
+            }
             }
         }
         __syncwarp();
@@ -331,10 +450,20 @@ __global__ void __launch_bounds__(kSkThreads) attn_sk_decode_kernel(const __grid
                 red_m[warp][g] = m0; red_m[warp][g + 8] = m1;
                 red_l[warp][g] = l0; red_l[warp][g + 8] = l1;
             }
+            if constexpr (FP8) {      // tiles 2c, 2c + 1 hold dims 16c + 4tq + {0, 2} and {1, 3}
+#pragma unroll
+                for (int cc = 0; cc < D / 16; ++cc) {
+                    const float(&e)[4] = o[2 * cc];
+                    const float(&f)[4] = o[2 * cc + 1];
+                    if (g < n_rep) *reinterpret_cast<float4*>(red_o + ((size_t)warp * n_rep + g) * D + cc * 16 + tq * 4) = make_float4(e[0], f[0], e[1], f[1]);
+                    if (g + 8 < n_rep) *reinterpret_cast<float4*>(red_o + ((size_t)warp * n_rep + g + 8) * D + cc * 16 + tq * 4) = make_float4(e[2], f[2], e[3], f[3]);
+                }
+            } else {
 #pragma unroll
             for (int nt = 0; nt < D / 8; ++nt) {
                 if (g < n_rep) *reinterpret_cast<float2*>(red_o + ((size_t)warp * n_rep + g) * D + nt * 8 + tq * 2) = make_float2(o[nt][0], o[nt][1]);
                 if (g + 8 < n_rep) *reinterpret_cast<float2*>(red_o + ((size_t)warp * n_rep + g + 8) * D + nt * 8 + tq * 2) = make_float2(o[nt][2], o[nt][3]);
+            }
             }
             csync();
             const int part = cta * 2 + (from_start ? 1 : 0);      // this CTA's partial slot for the pair
@@ -432,13 +561,18 @@ __global__ void __launch_bounds__(kSkThreads) attn_sk_decode_kernel(const __grid
 // ---------------------------------------------------------------------------------------------------------------------
 // prefill: grid (ceil(t / 64), nh, b) or (work items, nh), 128 threads; warp w owns query rows [16w, 16w+16) of the tile
 // ---------------------------------------------------------------------------------------------------------------------
-template <int D>
+// KV = uint8_t (FP8 cache): the two stages hold the raw e4m3 pages ([2 stages][K | V] bytes, the same bytes as one bf16 stage) and
+// each page is widened into ONE bf16 K | V tile after it landed; the loads stay asynchronous, a page costs one more barrier.
+template <int D, typename KV = uint16_t>
 __global__ void __launch_bounds__(kMmaAttnThreads) attn_prefill_kernel(const AttnArgs a) {
+    constexpr bool FP8 = kv_is_fp8<KV>;
     constexpr int TILE = kKvPage * D;
     extern __shared__ __align__(128) uint8_t dsm[];
     uint16_t* qhi = reinterpret_cast<uint16_t*>(dsm);   // [64][D]
     uint16_t* qlo = qhi + kPrefillBM * D;
-    uint16_t* kv = qlo + kPrefillBM * D;                // [2 stages][K tile | V tile]
+    uint16_t* kv = qlo + kPrefillBM * D;                // [2 stages][K tile | V tile]; FP8: [2 stages][K | V] e4m3, then the bf16 K | V tile
+    uint8_t* raw8 = reinterpret_cast<uint8_t*>(kv);
+    uint16_t* wide = kv + 2 * TILE;
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, tq = lane & 3;
     const int head = blockIdx.y;
@@ -469,7 +603,10 @@ __global__ void __launch_bounds__(kMmaAttnThreads) attn_prefill_kernel(const Att
 
     auto load = [&](int p, int st) {
         const size_t off = ((size_t)pt[p] * a.nkv + kvh) * (size_t)TILE;
-        stage_kv_tile<D>(kv + st * 2 * TILE, kv + st * 2 * TILE + TILE, a.kpool + off, a.vpool + off, tid);
+        if constexpr (FP8)
+            stage_kv_raw8<D>(raw8 + st * 2 * TILE, reinterpret_cast<const uint8_t*>(a.kpool) + off, reinterpret_cast<const uint8_t*>(a.vpool) + off, tid);
+        else
+            stage_kv_tile<D>(kv + st * 2 * TILE, kv + st * 2 * TILE + TILE, a.kpool + off, a.vpool + off, tid);
     };
     if (p0 < p1) load(p0, 0);
     for (int i = tid; i < kPrefillBM * (D / 4); i += kMmaAttnThreads) {
@@ -503,6 +640,11 @@ __global__ void __launch_bounds__(kMmaAttnThreads) attn_prefill_kernel(const Att
         }
         __syncthreads();
         const uint16_t* kt = kv + st * 2 * TILE;
+        if constexpr (FP8) {      // the previous page's readers of the tile passed the barrier at the end of its iteration
+            widen_kv_tile8<D>(wide, raw8 + st * 2 * TILE, tid);
+            __syncthreads();
+            kt = wide;
+        }
         const uint16_t* vt = kt + TILE;
         const int key0 = p * kKvPage;
         if (key0 < warp_len) {
@@ -612,7 +754,7 @@ constexpr int kTcThreads = 352;
 
 struct TcPrefillArgs {
     AttnArgs a;
-    int layer_row0;      // row of this layer's page 0 / kv head 0 in the pool-wide K tensor map
+    int layer_row0;      // row of this layer's page 0 / kv head 0 in the pool-wide K tensor map (bf16 caches)
     int vt_pages;        // pages per (sequence, kv head) in the V^T scratch
     const int* vt_tile0; // packed calls: first V^T tile of each sequence ([kv head][its pages]; QkvEpiArgs::vt_tile0), else null
     float tau;           // a row's reference max moves only when the tile's max exceeds it by more than this (exp2 domain)
@@ -638,9 +780,11 @@ __device__ __forceinline__ void sts128(uint32_t addr, const uint4& v) {
     asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
 }
 
-template <int D>
-__global__ void __launch_bounds__(kTcThreads, 1) attn_prefill_tc_kernel(const __grid_constant__ CUtensorMap tmk, const __grid_constant__ CUtensorMap tmvt,
-                                                                        const TcPrefillArgs k) {
+// KV = uint8_t (FP8 cache, attn_prefill_tc_fp8_kernel): kind::f16 needs bf16 K in shared memory, so tmk is the call's K scratch
+// (QkvEpiArgs::kt: the e4m3-rounded K as bf16, [tile][64 tokens][d], tiles numbered as the V^T tiles) and K pages are addressed by
+// tile instead of through the page table.
+template <int D, typename KV>
+__device__ __forceinline__ void attn_prefill_tc_body(const CUtensorMap& tmk, const CUtensorMap& tmvt, const TcPrefillArgs& k) {
     static_assert(D == 64 || D == 128, "head_dim 64 or 128");
     const AttnArgs& a = k.a;
     constexpr int HALF = D / 64;
@@ -668,6 +812,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) attn_prefill_tc_kernel(const __
     }
     const int q0 = qt * kTcQ, sw = a.sliding_window;
     const int kend = min(t, q0 + kTcQ);                              // keys [0, kend) can be visible to this tile
+    // first V^T (and, FP8, K scratch) tile of (sequence, kv head)
+    auto tile0 = [&] { return k.vt_tile0 ? k.vt_tile0[seq] + kvh * ((t + kKvPage - 1) / kKvPage) : (seq * a.nkv + kvh) * k.vt_pages; };
     const int kt0 = (sw > 0 && q0 - sw > 0) ? (q0 - sw) / kKvPage : 0;
     const int nkt = (kend + kKvPage - 1) / kKvPage - kt0;
 
@@ -691,12 +837,13 @@ __global__ void __launch_bounds__(kTcThreads, 1) attn_prefill_tc_kernel(const __
     const uint32_t tO = tmem + kTcSBufs * 64;
 
     if (warp == 0) {
-        if (lane == 0) {      // K pages: the pool's own rows
+        if (lane == 0) {      // K pages: the pool's own rows (FP8: the K scratch's)
             const int cslot = st_slot(a.state, seq);
             const int* pt = a.page_table + (size_t)cslot * a.pt_stride;
+            const int kt_tile0 = kv_is_fp8<KV> ? tile0() : 0;
             for (int j = 0; j < nkt; ++j) {
                 const int st = j % NK;
-                const int row = k.layer_row0 + (pt[kt0 + j] * a.nkv + kvh) * kKvPage;
+                const int row = kv_is_fp8<KV> ? (kt_tile0 + kt0 + j) * kKvPage : k.layer_row0 + (pt[kt0 + j] * a.nkv + kvh) * kKvPage;
                 mbar_wait(&k_empty[st], ((j / NK) & 1) ^ 1);
                 mbar_expect_tx(&k_full[st], kTile);
 #pragma unroll
@@ -705,7 +852,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) attn_prefill_tc_kernel(const __
         }
     } else if (warp == 10) {
         if (lane == 0) {      // V^T pages of this call (written by dense_qkv_epi_kernel)
-            const int vt0 = k.vt_tile0 ? k.vt_tile0[seq] + kvh * ((t + kKvPage - 1) / kKvPage) : (seq * a.nkv + kvh) * k.vt_pages;
+            const int vt0 = tile0();
             for (int j = 0; j < nkt; ++j) {
                 const int st = j % NV;
                 mbar_wait(&v_empty[st], ((j / NV) & 1) ^ 1);
@@ -899,6 +1046,17 @@ __global__ void __launch_bounds__(kTcThreads, 1) attn_prefill_tc_kernel(const __
         tc_fence_after();
         tmem_dealloc(tmem, 512);
     }
+}
+
+template <int D>
+__global__ void __launch_bounds__(kTcThreads, 1) attn_prefill_tc_kernel(const __grid_constant__ CUtensorMap tmk, const __grid_constant__ CUtensorMap tmvt,
+                                                                        const TcPrefillArgs k) {
+    attn_prefill_tc_body<D, uint16_t>(tmk, tmvt, k);
+}
+template <int D>
+__global__ void __launch_bounds__(kTcThreads, 1) attn_prefill_tc_fp8_kernel(const __grid_constant__ CUtensorMap tmk, const __grid_constant__ CUtensorMap tmvt,
+                                                                            const TcPrefillArgs k) {
+    attn_prefill_tc_body<D, uint8_t>(tmk, tmvt, k);
 }
 
 }  // namespace fl

@@ -51,6 +51,6 @@ void bert_embed_packed(BertModel& m, const uint32_t* ids, const int32_t* lengths
 void bert_repeat(BertModel& m, int b, int t, int iters, float* elapsed_ms);
 CUtensorMap make_tmap_bf16(const void* ptr, uint64_t rows, uint64_t cols, uint64_t ld, uint32_t box_rows);
 CUtensorMap make_tmap_pk(const void* ptr, uint64_t N, uint64_t K);
-CUtensorMap make_tmap_kv(const void* ptr, uint64_t rows, uint32_t head_dim);
+CUtensorMap make_tmap_kv(const void* ptr, uint64_t rows, uint32_t head_dim, uint32_t elem_bytes = 2);
 
 }  // namespace fl

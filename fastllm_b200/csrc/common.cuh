@@ -60,6 +60,39 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
     return r;
 }
 
+// ---- FP8 e4m3 KV elements (FL_KV_FP8_E4M3).  Kernels that read or write K/V pages are templated on the element type KV:
+// uint16_t = bf16, uint8_t = e4m3.
+template <typename KV>
+constexpr bool kv_is_fp8 = sizeof(KV) == 1;
+
+// two f32 -> packed e4m3x2 (lo in bits 0-7): round-to-nearest-even, saturating (|x| > 448 -> +-448, never NaN)
+__device__ __forceinline__ uint16_t f32x2_to_e4m3x2(float lo, float hi) {
+    uint16_t r;
+    asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(r) : "f"(hi), "f"(lo));
+    return r;
+}
+// packed e4m3x2 -> packed bf16x2, exact (every e4m3 value is a bf16 value): e4m3 -> f16 -> f32 -> bf16
+__device__ __forceinline__ uint32_t e4m3x2_to_bf16x2(uint16_t v) {
+    uint32_t h;
+    asm("cvt.rn.f16x2.e4m3x2 %0, %1;" : "=r"(h) : "h"(v));
+    float lo, hi;
+    asm("cvt.f32.f16 %0, %1;" : "=f"(lo) : "h"((uint16_t)(h & 0xFFFFu)));
+    asm("cvt.f32.f16 %0, %1;" : "=f"(hi) : "h"((uint16_t)(h >> 16)));
+    return pack_bf16x2(lo, hi);
+}
+// the value a K/V element of type KV holds for x, as the bf16 bits the attention operands carry
+template <typename KV>
+__device__ __forceinline__ uint16_t kv_round_bf16(float x) {
+    if constexpr (kv_is_fp8<KV>) return (uint16_t)e4m3x2_to_bf16x2(f32x2_to_e4m3x2(x, 0.f));
+    else return f32_to_bf16_rne(x);
+}
+// two K/V elements of type KV for (lo, hi), packed as KV's storage of a pair
+template <typename KV>
+__device__ __forceinline__ uint32_t kv_pack2(float lo, float hi) {
+    if constexpr (kv_is_fp8<KV>) return f32x2_to_e4m3x2(lo, hi);
+    else return (uint32_t)f32_to_bf16_rne(lo) | ((uint32_t)f32_to_bf16_rne(hi) << 16);
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xFFFFFFFFu, v, o);

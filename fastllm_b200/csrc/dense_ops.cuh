@@ -206,8 +206,8 @@ struct QkvEpiArgs {
     const float* y;            // [nsl][R, nqkv] GEMM output in the permuted row order of wqkv
     const float* bias;         // [nqkv] or null
     float* q_out;              // [R, nh*d]
-    uint16_t* kpool;
-    uint16_t* vpool;
+    void* kpool;               // this layer's K / V pages, elements of the kernel's KV type (bf16 or e4m3)
+    void* vpool;
     const int* page_table;
     int pt_stride;
     const StepState* state;
@@ -221,11 +221,26 @@ struct QkvEpiArgs {
     const int2* row_tab;       // [R] (sequence, position in the sequence) of every row
     const int* seq_len;        // [sequences] tokens each sequence is fed
     const int* vt_tile0;       // [sequences] first [d][64] tile of the sequence's V^T pages ([kv head][its pages]), or -1: none
+    uint16_t* kt;              // FP8 caches with vt: K of this call as bf16 (the e4m3-rounded values) in pages [tile][64 tokens][d], the
+                               // tiles numbered as the V^T tiles (the K operand of the tcgen05 prefill, which needs bf16 K)
 };
 
-// bias + RoPE (rotate-half) + q store + paged KV append of one row and column pair.  PACKED (packed calls): the row's sequence and
-// position come from row_tab, its V^T tile from vt_tile0.
+// The V^T / K scratch tile of (sequence, kv head hkv, position irel), or -1 when the sequence's attention does not read the scratch.
 template <bool PACKED>
+__device__ __forceinline__ long long qkv_scratch_tile(const QkvEpiArgs& a, int seq, int irel, int hkv) {
+    if constexpr (PACKED) {
+        const int t0 = a.vt_tile0[seq];
+        if (t0 < 0) return -1;
+        return (long long)t0 + (long long)hkv * ((a.seq_len[seq] + kKvPage - 1) / kKvPage) + irel / kKvPage;
+    } else {
+        return ((long long)seq * a.nkv + hkv) * a.vt_pages + irel / kKvPage;
+    }
+}
+
+// bias + RoPE (rotate-half) + q store + paged KV append of one row and column pair.  PACKED (packed calls): the row's sequence and
+// position come from row_tab, its V^T tile from vt_tile0.  KV: element type of the pages (uint16_t = bf16, uint8_t = e4m3, each
+// value rounded once from f32); the scratch copies for the tcgen05 prefill carry the stored value as bf16.
+template <bool PACKED, typename KV>
 __device__ __forceinline__ void qkv_epi_row(const QkvEpiArgs& a, int row, int pair) {
     const int ra = pair * 2;
     const int d = a.d, half = d >> 1;
@@ -255,31 +270,42 @@ __device__ __forceinline__ void qkv_epi_row(const QkvEpiArgs& a, int row, int pa
             q[j] = o1;
             q[j + half] = o2;
         } else {
-            uint16_t* kp = a.kpool + (((size_t)page * a.nkv + (hh - a.nh)) * kKvPage + slot % kKvPage) * d;
-            kp[j] = f32_to_bf16_rne(o1);
-            kp[j + half] = f32_to_bf16_rne(o2);
+            KV* kp = static_cast<KV*>(a.kpool) + (((size_t)page * a.nkv + (hh - a.nh)) * kKvPage + slot % kKvPage) * d;
+            if constexpr (kv_is_fp8<KV>) {
+                const uint16_t e = f32x2_to_e4m3x2(o1, o2);
+                kp[j] = (uint8_t)(e & 0xFFu);
+                kp[j + half] = (uint8_t)(e >> 8);
+                if (a.kt != nullptr) {
+                    const long long tile = qkv_scratch_tile<PACKED>(a, seq, irel, hh - a.nh);
+                    if (tile < 0) return;
+                    uint16_t* tk = a.kt + ((size_t)tile * kKvPage + irel % kKvPage) * d;
+                    const uint32_t b = e4m3x2_to_bf16x2(e);
+                    tk[j] = (uint16_t)(b & 0xFFFFu);
+                    tk[j + half] = (uint16_t)(b >> 16);
+                }
+            } else {
+                kp[j] = f32_to_bf16_rne(o1);
+                kp[j + half] = f32_to_bf16_rne(o2);
+            }
         }
     } else {
-        uint16_t* vp = a.vpool + (((size_t)page * a.nkv + (hh - a.nh - a.nkv)) * kKvPage + slot % kKvPage) * d;
-        *reinterpret_cast<uint32_t*>(vp + 2 * j) = (uint32_t)f32_to_bf16_rne(va) | ((uint32_t)f32_to_bf16_rne(vb) << 16);
+        KV* vp = static_cast<KV*>(a.vpool) + (((size_t)page * a.nkv + (hh - a.nh - a.nkv)) * kKvPage + slot % kKvPage) * d;
+        if constexpr (kv_is_fp8<KV>)
+            *reinterpret_cast<uint16_t*>(vp + 2 * j) = f32x2_to_e4m3x2(va, vb);
+        else
+            *reinterpret_cast<uint32_t*>(vp + 2 * j) = (uint32_t)f32_to_bf16_rne(va) | ((uint32_t)f32_to_bf16_rne(vb) << 16);
         if (a.vt != nullptr) {
-            size_t tile;                // the [d][64] V^T tile of (sequence, kv head, page)
-            if constexpr (PACKED) {
-                const int t0 = a.vt_tile0[seq];
-                if (t0 < 0) return;     // this sequence's attention does not read the scratch
-                tile = (size_t)t0 + (size_t)(hh - a.nh - a.nkv) * ((a.seq_len[seq] + kKvPage - 1) / kKvPage) + irel / kKvPage;
-            } else {
-                tile = ((size_t)seq * a.nkv + (hh - a.nh - a.nkv)) * a.vt_pages + irel / kKvPage;
-            }
-            uint16_t* tp = a.vt + (tile * d + 2 * j) * kKvPage + irel % kKvPage;
-            tp[0] = f32_to_bf16_rne(va);
-            tp[kKvPage] = f32_to_bf16_rne(vb);
+            const long long tile = qkv_scratch_tile<PACKED>(a, seq, irel, hh - a.nh - a.nkv);      // the [d][64] V^T tile
+            if (tile < 0) return;       // this sequence's attention does not read the scratch
+            uint16_t* tp = a.vt + ((size_t)tile * d + 2 * j) * kKvPage + irel % kKvPage;
+            tp[0] = kv_round_bf16<KV>(va);
+            tp[kKvPage] = kv_round_bf16<KV>(vb);
         }
     }
 }
 
 // thread per column pair, grid.y = row (PACKED: grid.y strides over the rows, which may be more than a grid dimension holds)
-template <bool PACKED>
+template <bool PACKED, typename KV>
 static __global__ void dense_qkv_epi_kernel(const QkvEpiArgs a) {
     // the dependent (attention) kernel is released only AFTER this kernel's own wait: when it starts, the q|k|v GEMM -- and by
     // induction every earlier kernel of the stream -- has completed, so its preamble may read the step state, the page table and
@@ -289,9 +315,9 @@ static __global__ void dense_qkv_epi_kernel(const QkvEpiArgs a) {
     const int pair = blockIdx.x * blockDim.x + threadIdx.x;
     if (pair * 2 >= a.nqkv) return;
     if constexpr (PACKED) {
-        for (int row = blockIdx.y; row < a.rows; row += gridDim.y) qkv_epi_row<true>(a, row, pair);
+        for (int row = blockIdx.y; row < a.rows; row += gridDim.y) qkv_epi_row<true, KV>(a, row, pair);
     } else {
-        qkv_epi_row<false>(a, blockIdx.y, pair);
+        qkv_epi_row<false, KV>(a, blockIdx.y, pair);
     }
 }
 
@@ -301,6 +327,7 @@ static __global__ void dense_qkv_epi_kernel(const QkvEpiArgs a) {
 // 25 us memory floor on Qwen2.5-7B); here the chain is paid once per eight rows, their loads travel together, and the eight tokens of
 // a V^T row are one 16-byte store.  Same arithmetic per element.
 constexpr int kQkvRowsPerThread = 8;
+template <typename KV>
 static __global__ void __launch_bounds__(256) dense_qkv_epi_rows_kernel(const QkvEpiArgs a) {
     pdl_wait();
     pdl_launch_dependents();
@@ -352,9 +379,21 @@ static __global__ void __launch_bounds__(256) dense_qkv_epi_rows_kernel(const Qk
             } else {
                 const int slot = slot0 + r;
                 const int page = a.page_table[cslot * a.pt_stride + slot / kKvPage];
-                uint16_t* kp = a.kpool + (((size_t)page * a.nkv + (hh - a.nh)) * kKvPage + slot % kKvPage) * d;
-                kp[j] = f32_to_bf16_rne(o1);
-                kp[j + half] = f32_to_bf16_rne(o2);
+                KV* kp = static_cast<KV*>(a.kpool) + (((size_t)page * a.nkv + (hh - a.nh)) * kKvPage + slot % kKvPage) * d;
+                if constexpr (kv_is_fp8<KV>) {
+                    const uint16_t e = f32x2_to_e4m3x2(o1, o2);
+                    kp[j] = (uint8_t)(e & 0xFFu);
+                    kp[j + half] = (uint8_t)(e >> 8);
+                    if (a.kt != nullptr) {      // the eight rows lie in one page: irel0 % 8 == 0
+                        uint16_t* tk = a.kt + ((size_t)qkv_scratch_tile<false>(a, seq, irel0, hh - a.nh) * kKvPage + (irel0 + r) % kKvPage) * d;
+                        const uint32_t b = e4m3x2_to_bf16x2(e);
+                        tk[j] = (uint16_t)(b & 0xFFFFu);
+                        tk[j + half] = (uint16_t)(b >> 16);
+                    }
+                } else {
+                    kp[j] = f32_to_bf16_rne(o1);
+                    kp[j + half] = f32_to_bf16_rne(o2);
+                }
             }
         }
     } else {
@@ -364,9 +403,19 @@ static __global__ void __launch_bounds__(256) dense_qkv_epi_rows_kernel(const Qk
         for (int r = 0; r < RPT; ++r) {
             const int slot = slot0 + r;
             const int page = a.page_table[cslot * a.pt_stride + slot / kKvPage];
-            uint16_t* vp = a.vpool + (((size_t)page * a.nkv + hv) * kKvPage + slot % kKvPage) * d;
-            const uint32_t ba = f32_to_bf16_rne(y[r].x), bb = f32_to_bf16_rne(y[r].y);
-            *reinterpret_cast<uint32_t*>(vp + 2 * j) = ba | (bb << 16);
+            KV* vp = static_cast<KV*>(a.vpool) + (((size_t)page * a.nkv + hv) * kKvPage + slot % kKvPage) * d;
+            uint32_t ba, bb;
+            if constexpr (kv_is_fp8<KV>) {
+                const uint16_t e = f32x2_to_e4m3x2(y[r].x, y[r].y);
+                *reinterpret_cast<uint16_t*>(vp + 2 * j) = e;
+                const uint32_t b = e4m3x2_to_bf16x2(e);
+                ba = b & 0xFFFFu;
+                bb = b >> 16;
+            } else {
+                ba = f32_to_bf16_rne(y[r].x);
+                bb = f32_to_bf16_rne(y[r].y);
+                *reinterpret_cast<uint32_t*>(vp + 2 * j) = ba | (bb << 16);
+            }
             if (r & 1) { va[r >> 1] |= ba << 16; vb[r >> 1] |= bb << 16; } else { va[r >> 1] = ba; vb[r >> 1] = bb; }
         }
         if (a.vt != nullptr) {      // irel0 % 8 == 0: the eight tokens are 16 aligned bytes of one V^T row

@@ -183,12 +183,13 @@ static __global__ void page_table_scatter_kernel(int* __restrict__ table, const 
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) table[upd[i].x] = upd[i].y;
 }
-// fl_cache_slot_fork: copy one K or V page (blockIdx.z) of every layer (blockIdx.y) from page src to page dst; elems = nkv * 64 * d
-static __global__ void kv_page_copy_kernel(uint16_t* kpool, uint16_t* vpool, size_t layer_elems, int src, int dst, int elems) {
-    uint16_t* pool = (blockIdx.z ? vpool : kpool) + (size_t)blockIdx.y * layer_elems;
-    const uint4* s = reinterpret_cast<const uint4*>(pool + (size_t)src * elems);
-    uint4* d = reinterpret_cast<uint4*>(pool + (size_t)dst * elems);
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < elems / 8; i += gridDim.x * blockDim.x) d[i] = s[i];
+// fl_cache_slot_fork: copy one K or V page (blockIdx.z) of every layer (blockIdx.y) from page src to page dst, in bytes (any element
+// type); page_bytes = nkv * 64 * d * element size, a multiple of 16
+static __global__ void kv_page_copy_kernel(uint8_t* kpool, uint8_t* vpool, size_t layer_bytes, int src, int dst, int page_bytes) {
+    uint8_t* pool = (blockIdx.z ? vpool : kpool) + (size_t)blockIdx.y * layer_bytes;
+    const uint4* s = reinterpret_cast<const uint4*>(pool + (size_t)src * page_bytes);
+    uint4* d = reinterpret_cast<uint4*>(pool + (size_t)dst * page_bytes);
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < page_bytes / 16; i += gridDim.x * blockDim.x) d[i] = s[i];
 }
 
 }  // namespace fl

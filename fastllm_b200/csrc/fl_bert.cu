@@ -65,18 +65,22 @@ CUtensorMap make_tmap_pk(const void* ptr, uint64_t N, uint64_t K) {
     return m;
 }
 
-// K or V pool of a cache seen as one [rows, head_dim] bf16 matrix (rows = layers x pages x kv heads x 64 tokens): the stream-K decode
-// attention fetches a page of one kv head as 64-row boxes of 64 columns (128 bytes, 128-byte swizzle); test-size heads (< 64) as one
-// unswizzled [64, head_dim] box.
-CUtensorMap make_tmap_kv(const void* ptr, uint64_t rows, uint32_t head_dim) {
+// K or V pool of a cache seen as one [rows, head_dim] matrix (rows = layers x pages x kv heads x 64 tokens) of bf16 (elem_bytes 2) or
+// e4m3 (elem_bytes 1) elements: the stream-K decode attention fetches a page of one kv head as 64-row boxes of 128 bytes with the
+// 128-byte swizzle (bf16: 64 columns per box; e4m3: the 128-byte row of head_dim 128), or as one [64, head_dim] box of 64-byte rows
+// with the 64-byte swizzle (e4m3, head_dim 64); test-size heads (< 64) as one unswizzled [64, head_dim] box.
+CUtensorMap make_tmap_kv(const void* ptr, uint64_t rows, uint32_t head_dim, uint32_t elem_bytes) {
     CUtensorMap m;
     const cuuint64_t dims[2] = {head_dim, rows};
-    const cuuint64_t strides[1] = {(cuuint64_t)head_dim * 2};
-    const cuuint32_t box[2] = {head_dim >= 64 ? 64u : head_dim, 64u};
+    const cuuint64_t strides[1] = {(cuuint64_t)head_dim * elem_bytes};
+    const uint32_t row_bytes = head_dim * elem_bytes;
+    const cuuint32_t box[2] = {row_bytes >= 128 ? 128u / elem_bytes : head_dim, 64u};
     const cuuint32_t estr[2] = {1, 1};
-    const CUresult r = encode_tiled_fn()(&m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides, box, estr,
-                                         CU_TENSOR_MAP_INTERLEAVE_NONE, head_dim >= 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE,
-                                         CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    const CUtensorMapSwizzle swz = row_bytes >= 128 ? CU_TENSOR_MAP_SWIZZLE_128B : (row_bytes == 64 && elem_bytes == 1 ? CU_TENSOR_MAP_SWIZZLE_64B
+                                                                                                                      : CU_TENSOR_MAP_SWIZZLE_NONE);
+    const CUresult r = encode_tiled_fn()(&m, elem_bytes == 1 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr),
+                                         dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     FL_CHECK(r == CUDA_SUCCESS, -2, "cuTensorMapEncodeTiled (KV pool) failed (" + std::to_string((int)r) + ")");
     return m;
 }

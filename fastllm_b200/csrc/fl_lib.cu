@@ -136,14 +136,23 @@ static size_t attn_prefill_smem_bytes(int d) {
     return (size_t)(2 * kPrefillBM + 4 * kKvPage) * d * 2;
 }
 
-// stream-K batched decode (attn_sk_decode_kernel): q tiles / merge scratch in front, then the K|V ring
+// tcgen05 prefill attention of a cache of KV elements
+template <int D, typename KV>
+static auto tc_prefill_kernel() {
+    if constexpr (kv_is_fp8<KV>) return attn_prefill_tc_fp8_kernel<D>;
+    else return attn_prefill_tc_kernel<D>;
+}
+
+// stream-K batched decode (attn_sk_decode_kernel): q tiles / merge scratch in front, then the K|V ring of KV elements
+template <typename KV>
 static size_t attn_sk_smem_bytes(int d, int n_rep) {
     const size_t front = std::max<size_t>((size_t)2 * 16 * d * 2, (size_t)kSkConsumerWarps * n_rep * d * 4);
-    return ((front + 1023) & ~(size_t)1023) + (size_t)kSkStages * 2 * kKvPage * d * 2;
+    return ((front + 1023) & ~(size_t)1023) + (size_t)sk_stages<KV> * 2 * kKvPage * d * sizeof(KV);
 }
 struct SkPlan { int ctas = 0; size_t smem = 0; };
-// resident CTAs per SM: 3, capped by the runtime's occupancy answer (the ring depth and why: kSkStages in attn_mma.cuh)
-template <int D>
+// resident CTAs per SM: 3, capped by the runtime's occupancy answer (the ring depth and why: kSkStages in attn_mma.cuh).  An FP8
+// ring has twice the stages of half the size (sk_stages): the same shared memory, so the same 3 CTAs per SM.
+template <int D, typename KV = uint16_t>
 static SkPlan attn_sk_plan(int n_rep) {
     static std::map<int, SkPlan> memo;
     static std::mutex mu;
@@ -151,10 +160,10 @@ static SkPlan attn_sk_plan(int n_rep) {
     auto it = memo.find(n_rep);
     if (it != memo.end()) return it->second;
     SkPlan p;
-    p.smem = attn_sk_smem_bytes(D, n_rep);
-    ensure_smem_optin((const void*)attn_sk_decode_kernel<D>, p.smem);    // the occupancy answer is 0 above the opt-in limit
+    p.smem = attn_sk_smem_bytes<KV>(D, n_rep);
+    ensure_smem_optin((const void*)attn_sk_decode_kernel<D, KV>, p.smem);    // the occupancy answer is 0 above the opt-in limit
     int fit = 0;
-    FL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fit, attn_sk_decode_kernel<D>, kSkThreads, p.smem));
+    FL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fit, attn_sk_decode_kernel<D, KV>, kSkThreads, p.smem));
     p.ctas = std::min(3, fit);
     FL_CHECK(p.ctas >= 1, FL_ERR_UNSUPPORTED, "stream-K attention does not fit an SM");
     memo[n_rep] = p;
@@ -509,11 +518,18 @@ static void launch_persistent(fl_cache& c, int nsteps, bool feedback) {
     }
 }
 
-// pool_tokens <= 0: the pool of max_batch * ceil(max_seq / 64) pages, in which every slot's home pages exist
-static void cache_create(fl_cache& c, int max_batch, int max_seq, int64_t pool_tokens) {
+// pool_tokens <= 0: the pool of max_batch * ceil(max_seq / 64) pages, in which every slot's home pages exist.  kv_dtype: fl_kv_dtype.
+static void cache_create(fl_cache& c, int max_batch, int max_seq, int64_t pool_tokens, int kv_dtype = FL_KV_BF16) {
     const Weights& w = *c.w;
     FL_CHECK(w.table.finalized, FL_ERR_STATE, "model not finalized");
     FL_CHECK(max_batch >= 1 && max_batch <= kMaxBatch && max_seq >= 1, FL_ERR_INVALID, "bad cache dimensions");
+    FL_CHECK(kv_dtype == FL_KV_BF16 || kv_dtype == FL_KV_FP8_E4M3, FL_ERR_INVALID, "unknown kv_dtype");
+    c.kv_fp8 = kv_dtype == FL_KV_FP8_E4M3;
+    c.kv_bytes = c.kv_fp8 ? 1 : 2;
+    if (c.kv_fp8) {      // FP8 caches are driven by slot and packed calls, which run on the dense path of an unsharded model
+        FL_CHECK(w.cfg.tp_size <= 1, FL_ERR_UNSUPPORTED, "an FP8 KV cache needs an unsharded model");
+        FL_CHECK(w.dense_ok, FL_ERR_UNSUPPORTED, "an FP8 KV cache runs on the dense path: shapes must be multiples of 8");
+    }
     c.max_batch = max_batch;
     c.max_seq = max_seq;
     c.pages_per_seq = (max_seq + kKvPage - 1) / kKvPage;
@@ -526,14 +542,14 @@ static void cache_create(fl_cache& c, int max_batch, int max_seq, int64_t pool_t
     c.page_table.alloc(pt.size());
     FL_CUDA(cudaMemcpy(c.page_table.p, pt.data(), pt.size() * 4, cudaMemcpyHostToDevice));
     c.layer_pool_elems = (size_t)pool_pages * w.nkv * kKvPage * w.d;
-    c.kpool.alloc(c.layer_pool_elems * w.L, true);
-    c.vpool.alloc(c.layer_pool_elems * w.L, true);
+    c.kpool.alloc(c.layer_pool_elems * w.L * c.kv_bytes / 2, true);      // the buffers hold 2-byte units
+    c.vpool.alloc(c.layer_pool_elems * w.L * c.kv_bytes / 2, true);
     {
         const uint64_t rows = (uint64_t)c.layer_pool_elems / w.d * w.L;
         c.kv_tmaps = rows < (1ull << 31) && (w.d == 16 || w.d == 32 || w.d == 64 || w.d == 128);
         if (c.kv_tmaps) {
-            c.tm_kpool = make_tmap_kv(c.kpool.p, rows, (uint32_t)w.d);
-            c.tm_vpool = make_tmap_kv(c.vpool.p, rows, (uint32_t)w.d);
+            c.tm_kpool = make_tmap_kv(c.kpool.p, rows, (uint32_t)w.d, (uint32_t)c.kv_bytes);
+            c.tm_vpool = make_tmap_kv(c.vpool.p, rows, (uint32_t)w.d, (uint32_t)c.kv_bytes);
         }
     }
     int ns = (2 * kNumSMs + w.nkv * kPassRows - 1) / (w.nkv * kPassRows);
@@ -567,7 +583,7 @@ static void cache_create(fl_cache& c, int max_batch, int max_seq, int64_t pool_t
     c.slot_tab.alloc(2 * (size_t)max_batch);
     c.h_slot_tab.alloc(2 * (size_t)max_batch);
     c.sample_out.alloc(1, true);
-    plan_persistent(c);
+    if (!c.kv_fp8) plan_persistent(c);      // batch-1 uniform decode only: an FP8 cache never takes it
     FL_CUDA(cudaDeviceSynchronize());
 }
 
@@ -818,6 +834,10 @@ static void ensure_dense_ws(fl_cache& c, int rows) {
         d.vt_pages_cap = R / kKvPage + std::min<size_t>(R, kMaxBatch);
         d.vt.alloc(d.vt_pages_cap * w.nkv * w.d * kKvPage, true);        // zero: the last page's tail multiplies P = 0 and must stay finite
         d.tm_vt = make_tmap_bf16(d.vt.p, d.vt_pages_cap * w.nkv * w.d, kKvPage, kKvPage, (uint32_t)w.d);
+        if (c.kv_fp8) {      // the tcgen05 prefill's bf16 K operand: same tiles as vt, [64 tokens][d] each (the pool's row layout)
+            d.kt.alloc(d.vt_pages_cap * w.nkv * kKvPage * w.d, true);
+            d.tm_kt = make_tmap_kv(d.kt.p, d.vt_pages_cap * w.nkv * kKvPage, (uint32_t)w.d);
+        }
     }
     d.rows = R;
 }
@@ -966,8 +986,8 @@ static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool
     }
     for (int l = 0; l < w.L; ++l) {
         const LayerW& lw = w.layers[l];
-        uint16_t* kpool = c.kpool.p + (size_t)l * c.layer_pool_elems;
-        uint16_t* vpool = c.vpool.p + (size_t)l * c.layer_pool_elems;
+        uint16_t* kpool = reinterpret_cast<uint16_t*>(reinterpret_cast<uint8_t*>(c.kpool.p) + (size_t)l * c.layer_pool_elems * c.kv_bytes);
+        uint16_t* vpool = reinterpret_cast<uint16_t*>(reinterpret_cast<uint8_t*>(c.vpool.p) + (size_t)l * c.layer_pool_elems * c.kv_bytes);
         int ks = dense_gemm(c, lc, "gemm_tc_qkv", R, w.nqkv, w.H, lw.tm_wqkv, d.y.p);
         QkvEpiArgs qa{ks, (long long)R * w.nqkv, d.y.p, lw.bqkv, d.q.p, kpool, vpool, c.page_table.p, c.pages_per_seq, c.state.p, w.rope_cos,
                       w.rope_sin, w.nh, w.nkv, w.d, w.max_pos, t, w.nqkv, tc_prefill ? d.vt.p : nullptr, vt_pages, R};
@@ -975,44 +995,55 @@ static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool
             qa.row_tab = pk->row_tab; qa.seq_len = pk->seq_len; qa.vt_tile0 = pk->vt_tile0;
             qa.vt = pk->ntc > 0 ? d.vt.p : nullptr;
         }
-        if (pk)
-            launch(lc, "dense_qkv_rope_append", 0, dense_qkv_epi_kernel<true>, dim3((w.nqkv / 2 + 255) / 256, std::min(R, 65535)), dim3(256), 0, qa);
-        else if (t >= 64 && t % kQkvRowsPerThread == 0)      // prefill: eight rows per thread (dense_qkv_epi_rows_kernel)
-            launch(lc, "dense_qkv_rope_append", 0, dense_qkv_epi_rows_kernel, dim3((w.nqkv / 2 + 255) / 256, R / kQkvRowsPerThread), dim3(256), 0, qa);
-        else
-            launch(lc, "dense_qkv_rope_append", 0, dense_qkv_epi_kernel<false>, dim3((w.nqkv / 2 + 255) / 256, R), dim3(256), 0, qa);
+        qa.kt = c.kv_fp8 && qa.vt ? d.kt.p : nullptr;      // FP8: the tcgen05 prefill reads K as bf16 from this scratch
+        // the kernels below are instantiated per K/V element type: uint16_t (bf16) or uint8_t (e4m3, FP8 caches)
+        auto with_kv = [&](auto f) {
+            if (c.kv_fp8) f(uint8_t{}); else f(uint16_t{});
+        };
+        with_kv([&](auto kv) {
+            using KV = decltype(kv);
+            if (pk)
+                launch(lc, "dense_qkv_rope_append", 0, dense_qkv_epi_kernel<true, KV>, dim3((w.nqkv / 2 + 255) / 256, std::min(R, 65535)), dim3(256), 0, qa);
+            else if (t >= 64 && t % kQkvRowsPerThread == 0)      // prefill: eight rows per thread (dense_qkv_epi_rows_kernel)
+                launch(lc, "dense_qkv_rope_append", 0, dense_qkv_epi_rows_kernel<KV>, dim3((w.nqkv / 2 + 255) / 256, R / kQkvRowsPerThread), dim3(256), 0, qa);
+            else
+                launch(lc, "dense_qkv_rope_append", 0, dense_qkv_epi_kernel<false, KV>, dim3((w.nqkv / 2 + 255) / 256, R), dim3(256), 0, qa);
+        });
         {   // K7-K11 on tensor cores; the output lands as the hi/lo bf16 operands of the o_proj GEMM
             AttnArgs at{};
             at.q = d.q.p; at.kpool = kpool; at.vpool = vpool; at.page_table = c.page_table.p; at.pt_stride = c.pages_per_seq;
             at.state = c.state.p; at.counters = d.counters.p;
             at.out_hi = d.xhi.p; at.out_lo = d.xlo.p; at.nh = w.nh; at.nkv = w.nkv; at.t = t; at.row_base = 0;
             at.sliding_window = windowed ? w.cfg.sliding_window : 0; at.qscale = qscale;
-            const uint64_t kv_bytes = (pk ? pk->kv_tokens : (uint64_t)b * (c.kv_len + t)) * w.nkv * w.d * 4;
+            const uint64_t kv_bytes = (pk ? pk->kv_tokens : (uint64_t)b * (c.kv_len + t)) * w.nkv * w.d * 2 * c.kv_bytes;
             const int layer_row0 = (int)((size_t)l * (c.layer_pool_elems / w.d));
+            const CUtensorMap& tm_tc_k = c.kv_fp8 ? d.tm_kt : c.tm_kpool;      // K of the tcgen05 prefill
+            with_kv([&](auto kv) {
+            using KV = decltype(kv);
             with_head_dim(w.d, [&](auto D) {
                 if (pk) {
                     // up to three launches, each over its own rows: the length-1 sequences (rows [0, nd)) as a decode step, fresh
                     // sequences of more than a page on tcgen05, every other multi-token sequence on mma.sync -- the kernels a lone
                     // call of each sequence would take
                     if (pk->nd > 0) {
-                        const SkPlan pl = attn_sk_plan<D>(w.nh / w.nkv);
+                        const SkPlan pl = attn_sk_plan<D, KV>(w.nh / w.nkv);
                         SkArgs sk{};
                         sk.a = at; sk.sk_acc = d.sk_acc.p; sk.sk_ml = d.sk_ml.p; sk.b = pk->nd; sk.layer_row0 = layer_row0;
-                        launch(lc, "attn_sk_decode", kv_bytes, attn_sk_decode_kernel<D>, dim3(pl.ctas * kNumSMs), dim3(kSkThreads), pl.smem,
+                        launch(lc, "attn_sk_decode", kv_bytes, attn_sk_decode_kernel<D, KV>, dim3(pl.ctas * kNumSMs), dim3(kSkThreads), pl.smem,
                                c.tm_kpool, c.tm_vpool, sk);
                     }
                     if constexpr (D == 64 || D == 128) {
                         if (pk->ntc > 0) {
                             TcPrefillArgs tp{};
                             tp.a = at; tp.a.items = pk->tc_items; tp.layer_row0 = layer_row0; tp.vt_tile0 = pk->vt_tile0; tp.tau = tc_tau;
-                            launch(lc, "attn_prefill_tc", kv_bytes, attn_prefill_tc_kernel<D>, dim3(pk->ntc, w.nh), dim3(kTcThreads),
-                                   attn_prefill_tc_smem_bytes(D), c.tm_kpool, d.tm_vt, tp);
+                            launch(lc, "attn_prefill_tc", kv_bytes, tc_prefill_kernel<D, KV>(), dim3(pk->ntc, w.nh), dim3(kTcThreads),
+                                   attn_prefill_tc_smem_bytes(D), tm_tc_k, d.tm_vt, tp);
                         }
                     }
                     if (pk->nmma > 0) {
                         AttnArgs am = at;
                         am.items = pk->mma_items;
-                        launch(lc, "attn_prefill", kv_bytes, attn_prefill_kernel<D>, dim3(pk->nmma, w.nh), dim3(kMmaAttnThreads),
+                        launch(lc, "attn_prefill", kv_bytes, attn_prefill_kernel<D, KV>, dim3(pk->nmma, w.nh), dim3(kMmaAttnThreads),
                                attn_prefill_smem_bytes(D), am);
                     }
                 } else if (t == 1) {
@@ -1020,23 +1051,24 @@ static void enqueue_forward_dense(fl_cache& c, LaunchCtx& lc, int b, int t, bool
                     // depend on the KV length: this launch is captured into the step's CUDA graph, which is keyed by (batch, mode)
                     // only and replayed as the context grows.
                     FL_CHECK(c.kv_tmaps && w.nh / w.nkv <= 16, FL_ERR_UNSUPPORTED, "batched decode attention: GQA group > 16 heads or KV pool beyond 2^31 rows");
-                    const SkPlan pl = attn_sk_plan<D>(w.nh / w.nkv);
+                    const SkPlan pl = attn_sk_plan<D, KV>(w.nh / w.nkv);
                     SkArgs sk{};
                     sk.a = at; sk.sk_acc = d.sk_acc.p; sk.sk_ml = d.sk_ml.p; sk.b = b; sk.layer_row0 = layer_row0;
-                    launch(lc, "attn_sk_decode", kv_bytes, attn_sk_decode_kernel<D>, dim3(pl.ctas * kNumSMs), dim3(kSkThreads), pl.smem, c.tm_kpool,
+                    launch(lc, "attn_sk_decode", kv_bytes, attn_sk_decode_kernel<D, KV>, dim3(pl.ctas * kNumSMs), dim3(kSkThreads), pl.smem, c.tm_kpool,
                            c.tm_vpool, sk);
                 } else if (tc_prefill) {
                     if constexpr (D == 64 || D == 128) {
                         TcPrefillArgs tp{};
                         tp.a = at; tp.layer_row0 = layer_row0; tp.vt_pages = vt_pages;
                         tp.tau = tc_tau;
-                        launch(lc, "attn_prefill_tc", kv_bytes, attn_prefill_tc_kernel<D>, dim3((t + kTcQ - 1) / kTcQ, w.nh, b), dim3(kTcThreads),
-                               attn_prefill_tc_smem_bytes(D), c.tm_kpool, d.tm_vt, tp);
+                        launch(lc, "attn_prefill_tc", kv_bytes, tc_prefill_kernel<D, KV>(), dim3((t + kTcQ - 1) / kTcQ, w.nh, b), dim3(kTcThreads),
+                               attn_prefill_tc_smem_bytes(D), tm_tc_k, d.tm_vt, tp);
                     }
                 } else {
-                    launch(lc, "attn_prefill", kv_bytes, attn_prefill_kernel<D>, dim3((t + kPrefillBM - 1) / kPrefillBM, w.nh, b), dim3(kMmaAttnThreads),
+                    launch(lc, "attn_prefill", kv_bytes, attn_prefill_kernel<D, KV>, dim3((t + kPrefillBM - 1) / kPrefillBM, w.nh, b), dim3(kMmaAttnThreads),
                            attn_prefill_smem_bytes(D), at);
                 }
+            });
             });
         }
         ks = dense_gemm(c, lc, "gemm_tc_o", R, w.H, nq, lw.tm_wo, d.y.p);
@@ -1219,6 +1251,7 @@ static void run_steps(fl_cache& c, int b, int t, int mode, int steps, const Even
 static void check_call(fl_cache& c, const uint32_t* ids, int b, int t, size_t rope_offset, int extra_steps) {
     const Weights& w = *c.w;
     FL_CHECK(!c.poisoned, FL_ERR_CUDA, "cache poisoned by an earlier CUDA error");
+    FL_CHECK(!c.kv_fp8, FL_ERR_UNSUPPORTED, "an FP8 KV cache takes slot and packed calls only (fl_forward_slots, fl_forward_packed)");
     FL_CHECK(!c.slots_used, FL_ERR_STATE, "this cache is driven by sequence slots (fl_forward_slots): call fl_cache_reset before a uniform call");
     FL_CHECK(ids != nullptr, FL_ERR_INVALID, "ids is NULL");
     FL_CHECK(b >= 1 && b <= c.max_batch && t >= 1, FL_ERR_INVALID, "bad batch / sequence length");
@@ -1633,6 +1666,20 @@ FL_EXPORT int fl_cache_create_pool(fl_model* m, int max_batch, int max_seq, int 
     FL_API_END
 }
 
+FL_EXPORT int fl_cache_create_pool_kv(fl_model* m, int max_batch, int max_seq, int pool_tokens, int kv_dtype, fl_cache** out) {
+    FL_API_BEGIN
+    FL_CHECK(m && out, FL_ERR_INVALID, "NULL argument");
+    FL_CHECK(m->w != nullptr, FL_ERR_INVALID, "BERT models have no KV cache");
+    FL_CHECK(pool_tokens >= 1, FL_ERR_INVALID, "pool_tokens must be >= 1");
+    FL_CHECK(kv_dtype == FL_KV_BF16 || kv_dtype == FL_KV_FP8_E4M3, FL_ERR_INVALID, "unknown kv_dtype");
+    use_device();
+    std::unique_ptr<fl_cache> c(new fl_cache);
+    c->w = m->w;
+    cache_create(*c, max_batch, max_seq, pool_tokens, kv_dtype);
+    *out = c.release();
+    FL_API_END
+}
+
 FL_EXPORT int fl_cache_pool_pages(fl_cache* c, int* free_pages, int* total_pages) {
     FL_API_BEGIN
     FL_CHECK(c && free_pages && total_pages, FL_ERR_INVALID, "NULL argument");
@@ -1656,10 +1703,11 @@ FL_EXPORT int fl_cache_slot_fork(fl_cache* c, int src, int dst) {
     FL_CHECK(c->pool.fork(src, dst, len, &copy), FL_ERR_STATE, "KV page pool exhausted (no free page for the partial last page)");
     const Weights& w = *c->w;
     if (copy.first >= 0) {      // the partial last page: K and V of every layer
-        const int elems = w.nkv * kKvPage * w.d;
+        const int elems = w.nkv * kKvPage * w.d, bytes = elems * c->kv_bytes;
         LaunchCtx lc{c->stream, /*pdl=*/false};     // a plain launch (named in fl_prof profiles)
-        launch(lc, "kv_page_copy", (uint64_t)2 * 2 * w.L * elems * 2, kv_page_copy_kernel, dim3(std::max(1, std::min(16, elems / 8 / 256)), w.L, 2),
-               dim3(256), 0, c->kpool.p, c->vpool.p, c->layer_pool_elems, copy.first, copy.second, elems);
+        launch(lc, "kv_page_copy", (uint64_t)2 * 2 * w.L * bytes, kv_page_copy_kernel, dim3(std::max(1, std::min(16, elems / 8 / 256)), w.L, 2),
+               dim3(256), 0, reinterpret_cast<uint8_t*>(c->kpool.p), reinterpret_cast<uint8_t*>(c->vpool.p), c->layer_pool_elems * c->kv_bytes,
+               copy.first, copy.second, bytes);
     }
     set_slot_len_kernel<<<1, 1, 0, c->stream>>>(c->state.p, dst, len);
     g_launches.fetch_add(1);
@@ -1736,6 +1784,7 @@ FL_EXPORT int fl_cache_kv_len(fl_cache* c, int* out) {
 FL_EXPORT int fl_cache_fill_synthetic(fl_cache* c, int batch, int kv_len, uint64_t seed) {
     FL_API_BEGIN
     FL_CHECK(c, FL_ERR_INVALID, "NULL argument");
+    FL_CHECK(!c->kv_fp8, FL_ERR_UNSUPPORTED, "the synthetic fill is a uniform prefill: an FP8 KV cache takes slot and packed calls only");
     FL_CHECK(batch >= 1 && batch <= c->max_batch && kv_len >= 0 && kv_len <= c->max_seq, FL_ERR_INVALID, "bad synthetic fill size");
     FL_CHECK((int64_t)batch * KvPool::pages_for(kv_len) <= c->pool.total_pages(), FL_ERR_STATE, "KV page pool exhausted");
     use_device();

@@ -81,6 +81,8 @@ struct DenseWs {
     DevBuf<uint16_t> vt;            // V of the current multi-token call transposed per page: [seq][kv head][page][d][64] (tcgen05 prefill attention)
     size_t vt_pages_cap = 0;        // pages the scratch holds (over all sequences of a call)
     CUtensorMap tm_vt{};
+    DevBuf<uint16_t> kt;            // FP8 caches: K of the call as bf16 in pages [tile][64][d], tiles numbered as vt's (tcgen05 prefill attention)
+    CUtensorMap tm_kt{};
     DevBuf<float> sk_acc, sk_ml;    // stream-K decode attention: [CTAs][2][n_rep][d] / [CTAs][2][n_rep][2] partials of shared pairs
     DevBuf<float> moe_out, route_w;
     DevBuf<int> route_sel;          // [L][rows of the call][top_k] picked experts of the last forward (fl_cache_moe_routing)
@@ -142,8 +144,10 @@ struct fl_cache {
     fl::KvPool pool;                      // owner of every page: refcounts, per-slot page lists, the host side of page_table
     fl::DevBuf<int2> pt_upd;              // (table index, page) of the entries a call changed, scattered into page_table
     fl::PinnedBuf<int2> h_pt_upd;
-    fl::DevBuf<uint16_t> kpool, vpool;    // [L][pool pages][nkv][kKvPage][d]
+    fl::DevBuf<uint16_t> kpool, vpool;    // [L][pool pages][nkv][kKvPage][d] elements of kv_bytes bytes (bf16, or e4m3 when kv_fp8)
     size_t layer_pool_elems = 0;
+    bool kv_fp8 = false;                  // FL_KV_FP8_E4M3: K/V pages hold e4m3; driven by slot and packed calls only
+    int kv_bytes = 2;                     // bytes per K/V element
     CUtensorMap tm_kpool{}, tm_vpool{};   // the pools as [rows, d] matrices (stream-K decode attention); valid when kv_tmaps
     bool kv_tmaps = false;
     bool fresh_call = false;              // the forward being enqueued starts on empty sequences (every row's KV length is 0)

@@ -96,14 +96,22 @@ class DeviceModel:
 class DeviceCache:
     """fl_cache*: paged KV cache + per-cache stream/workspaces.  pool_tokens=None: every slot can reach max_seq (a pool of
     max_batch * ceil(max_seq / 64) pages); otherwise the slots share a pool of pool_tokens tokens (rounded up to 64-token pages),
-    taken as sequences grow."""
+    taken as sequences grow.  kv_dtype="fp8_e4m3" stores K and V as FP8 e4m3 (fl_cache_create_pool_kv): half the bytes per token,
+    slot and packed calls only."""
 
-    def __init__(self, model: DeviceModel, max_batch: int, max_seq: int, pool_tokens: int | None = None):
+    KV_DTYPES = {"bf16": 0, "fp8_e4m3": 1}      # fl_kv_dtype
+
+    def __init__(self, model: DeviceModel, max_batch: int, max_seq: int, pool_tokens: int | None = None, kv_dtype: str = "bf16"):
+        if kv_dtype not in self.KV_DTYPES:
+            raise ValueError(f"kv_dtype must be one of {sorted(self.KV_DTYPES)}, not {kv_dtype!r}")
         self.model, self.lib = model, model.lib
-        self.max_batch, self.max_seq = max_batch, max_seq
+        self.max_batch, self.max_seq, self.kv_dtype = max_batch, max_seq, kv_dtype
         self.vocab = model.cfg.vocab_size
         h = C.c_void_p()
-        if pool_tokens is None:
+        if kv_dtype != "bf16":
+            tokens = pool_tokens if pool_tokens is not None else max_batch * _pages(max_seq) * KV_PAGE
+            _lib.check(self.lib.fl_cache_create_pool_kv(model.h, max_batch, max_seq, tokens, self.KV_DTYPES[kv_dtype], C.byref(h)))
+        elif pool_tokens is None:
             _lib.check(self.lib.fl_cache_create(model.h, max_batch, max_seq, C.byref(h)))
         else:
             _lib.check(self.lib.fl_cache_create_pool(model.h, max_batch, max_seq, pool_tokens, C.byref(h)))
@@ -723,14 +731,16 @@ class PackedBatcher:
     pool_tokens: the slots share a KV pool of that many tokens instead of max_seq each.  A waiting request is then also admitted only
     if the pages it can ever need -- its prompt plus max_tokens, less the prefix pages it shares -- fit the pool minus the pages
     reserved for running requests (and the shared prefix), so no call can run out of pages and nothing is preempted.  Requests are
-    admitted in order: one that does not fit waits for pages to free up."""
+    admitted in order: one that does not fit waits for pages to free up.
+
+    kv_dtype: element type of the cache the batcher builds ("bf16" or "fp8_e4m3"; DeviceCache)."""
 
     def __init__(self, model, max_batch: int = 8, eos_token_id: int | None = 2, cache=None, token_budget: int = 4096,
-                 pool_tokens: int | None = None):
+                 pool_tokens: int | None = None, kv_dtype: str = "bf16"):
         self.model, self.max_batch, self.eos_token_id, self.token_budget = model, max_batch, eos_token_id, token_budget
         self.position_per_call = getattr(model, "arch", "llama") != "llama"      # the Mistral/Qwen2 adapters' offset rule
         self.sliding_window = getattr(getattr(model, "cfg", None), "sliding_window", 0) if self.position_per_call else 0
-        self.cache = cache if cache is not None else DeviceCache(model.dev, max_batch, model._capacity(), pool_tokens)
+        self.cache = cache if cache is not None else DeviceCache(model.dev, max_batch, model._capacity(), pool_tokens, kv_dtype)
         self.pool_pages = None if pool_tokens is None else _pages(pool_tokens)
         self.slot_pages = _pages(self.cache.max_seq) if hasattr(self.cache, "max_seq") else None   # a slot never holds more
         self.forwards = 0       # packed forwards issued (tests / stats)

@@ -79,6 +79,10 @@ struct DeviceCache {   // paged KV cache + stream (fl_cache*)
     DeviceCache(fl_model* m, int max_batch, int max_seq) { check(fl_cache_create(m, max_batch, max_seq, &h)); }
     // the slots share a pool of pool_tokens tokens of KV (fl_cache_create_pool)
     DeviceCache(fl_model* m, int max_batch, int max_seq, int pool_tokens) { check(fl_cache_create_pool(m, max_batch, max_seq, pool_tokens, &h)); }
+    // the same pool with K/V pages of element type kv_dtype (fl_cache_create_pool_kv; FL_KV_FP8_E4M3: slot and packed calls only)
+    DeviceCache(fl_model* m, int max_batch, int max_seq, int pool_tokens, fl_kv_dtype kv_dtype) {
+        check(fl_cache_create_pool_kv(m, max_batch, max_seq, pool_tokens, kv_dtype, &h));
+    }
     void slot_fork(int src, int dst) const { check(fl_cache_slot_fork(h, src, dst)); }
     std::pair<int, int> pool_pages() const {   // (free, total)
         int f = 0, t = 0;
@@ -352,11 +356,15 @@ struct PackedBatcher {
     int max_seq;
     DeviceCache cache;
     int forwards = 0;   // packed forwards issued
-    PackedBatcher(const M& m, int max_batch_, std::optional<uint32_t> eos = 2, int budget = 4096, std::optional<int> pool_tokens = std::nullopt)
+    // kv_dtype: element type of the cache's K/V pages (FL_KV_FP8_E4M3: half the bytes per token)
+    PackedBatcher(const M& m, int max_batch_, std::optional<uint32_t> eos = 2, int budget = 4096, std::optional<int> pool_tokens = std::nullopt,
+                  fl_kv_dtype kv_dtype = FL_KV_BF16)
         : model(m), max_batch(max_batch_), eos_token_id(eos), token_budget(budget),
           pool_pages(pool_tokens ? std::optional<int>(kv_pages(*pool_tokens)) : std::nullopt),
           max_seq(std::min(kKvCapacity, m.dev->cfg.max_position_embeddings)),
-          cache(pool_tokens ? DeviceCache(m.dev->h, max_batch_, max_seq, *pool_tokens) : DeviceCache(m.dev->h, max_batch_, max_seq)) {}
+          cache(kv_dtype != FL_KV_BF16 ? DeviceCache(m.dev->h, max_batch_, max_seq, pool_tokens ? *pool_tokens : max_batch_ * kv_pages(max_seq) * kKvPage, kv_dtype)
+                : pool_tokens       ? DeviceCache(m.dev->h, max_batch_, max_seq, *pool_tokens)
+                                    : DeviceCache(m.dev->h, max_batch_, max_seq)) {}
 
     // as models.PackedBatcher._uses_prefix: not on Llama, not for a prompt longer than the sliding window
     bool uses_prefix(const std::vector<uint32_t>& prompt, const std::vector<uint32_t>* prefix) const {

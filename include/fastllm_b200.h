@@ -136,6 +136,21 @@ FL_EXPORT int fl_cache_create(fl_model* m, int max_batch, int max_seq, fl_cache*
 /* A cache of max_batch slots, each up to max_seq tokens, sharing a pool of pool_tokens (rounded up to 64-token pages) of KV.
  * fl_cache_create(m, B, S, out) is the pool of B * ceil(S/64) pages.  FL_ERR_INVALID: pool_tokens < 1 or bad dimensions. */
 FL_EXPORT int fl_cache_create_pool(fl_model* m, int max_batch, int max_seq, int pool_tokens, fl_cache** out);
+/* Element type of a cache's K and V pages. */
+typedef enum fl_kv_dtype { FL_KV_BF16 = 0, FL_KV_FP8_E4M3 = 1 } fl_kv_dtype;
+/* fl_cache_create_pool with the K/V element type kv_dtype (an fl_kv_dtype); FL_KV_BF16 is exactly fl_cache_create_pool.
+ * FL_KV_FP8_E4M3 stores K (after RoPE) and V as FP8 e4m3, each value rounded once from the f32 value of the q|k|v projection:
+ * round-to-nearest-even, saturating (a magnitude above 448 becomes +-448, never NaN), scale 1, not rounded through bf16 first.
+ * Every attention reads the rounded values, a call's attention over its own new tokens included.  pool_tokens keeps its meaning
+ * (tokens): an FP8 pool of N tokens takes half the bytes of a bf16 pool of N tokens.
+ * An FP8 cache is driven by slots only.  It takes fl_forward_slots, fl_forward_packed, fl_cache_slot_fork, fl_cache_slot_reset,
+ * fl_cache_slot_len, fl_cache_pool_pages, fl_cache_reset and fl_cache_moe_routing.  The uniform calls (fl_forward,
+ * fl_forward_greedy, fl_decode_greedy_loop, fl_forward_logprobs, fl_forward_sample, fl_forward_sample_device) and
+ * fl_cache_fill_synthetic return FL_ERR_UNSUPPORTED before any device work and leave the cache unchanged.
+ * FL_ERR_INVALID:     as fl_cache_create_pool, or an unknown kv_dtype.
+ * FL_ERR_UNSUPPORTED: FL_KV_FP8_E4M3 on a sharded model (tp_size > 1, Mixtral expert parallelism included) or on one whose shapes
+ *                     do not admit the dense path (dimensions that are not multiples of 8). */
+FL_EXPORT int fl_cache_create_pool_kv(fl_model* m, int max_batch, int max_seq, int pool_tokens, int kv_dtype, fl_cache** out);
 FL_EXPORT int fl_cache_pool_pages(fl_cache* c, int* free_pages, int* total_pages);   /* pages no slot holds / pages of the pool */
 FL_EXPORT int fl_cache_reset(fl_cache* c);                       /* kv length := 0 for every sequence; every page returns to the pool */
 FL_EXPORT int fl_cache_kv_len(fl_cache* c, int* out);            /* tokens currently held (same for every sequence) */
